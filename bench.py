@@ -2,7 +2,7 @@
 """bench.py — the headline benchmark: BASELINE.json's metric (Mpaths/s, with Mrays/s beside it) on config C2,
 `semesterbild.json` at its native 800x600 / 256 spp / 30 bounces, on N B200s of one node.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config C1|C2|C3|C3s|C4|C5]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config C1|C2|C3|C3s|C4|C5] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A "step" is one full render of the frame (render_scene, src/renderer.rs:67-123 of the reference, timed like the
@@ -38,6 +38,7 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 DEFAULT_POOL = 0  # the library's default: the whole job in flight at once if it fits a quarter of the free memory, else 48 Mi slots
+DUMP_PIXELS = 1 << 20  # --dump-outputs: frames up to 1 Mi pixels (C1-C4) whole, 32 MiB at most; larger ones (C5) as a sample of this many
 
 
 def metric_name(cfg, w, h, spp, depth):
@@ -190,6 +191,29 @@ def cpu_baseline(scene):
                       "(oracle/), row-parallel, ChaCha12 per-row RNG as the reference"}
 
 
+def dump_outputs(out_dir, film, packed, w, h, counts):
+    """What the timed path hands its caller in its last step, as DIR/<name>.npy:
+      film   [H, W, 3] float32  the radiance sum ptc_render_accumulate leaves in the device film (reduced over ranks)
+      image  [H, W, 3] float32  the 0x00RRGGBB pixels of ptc_resolve_device as channel levels 0-255
+      stats  [2]       float64  paths and rays of the step, summed over ranks
+    A frame of more than DUMP_PIXELS pixels keeps a fixed, seeded sample of them: film and image are [DUMP_PIXELS, 3]
+    and pixel_index (float64) holds their row-major indices into the frame."""
+    import numpy as np
+    u = packed.reshape(-1).view(np.uint32)
+    arrays = {"film": film.reshape(h * w, 3).astype(np.float32),
+              "image": np.stack([(u >> 16) & 255, (u >> 8) & 255, u & 255], -1).astype(np.float32)}
+    if h * w > DUMP_PIXELS:
+        idx = np.sort(np.random.default_rng(0).choice(h * w, DUMP_PIXELS, replace=False))
+        arrays = {k: v[idx] for k, v in arrays.items()}
+        arrays["pixel_index"] = idx.astype(np.float64)
+    else:
+        arrays = {k: v.reshape(h, w, 3) for k, v in arrays.items()}
+    arrays["stats"] = np.asarray(counts, np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -201,7 +225,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-weak", action="store_true", help="N > 1: skip the extra weak-scaling measurement")
     ap.add_argument("--no-inprocess", action="store_true", help="N > 1: skip the in-process ptc_multi_* measurement on rank 0")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the film, image and path / ray counts of the last timed step "
+                                                          "as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        # the reference arm sizes its sample by a CPU timing, so its output is not the same from run to run
+        ap.error("--dump-outputs applies to --impl b200")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -313,6 +344,10 @@ def main():
     # brackets every stage launch with CUDA events on the launching stream (a few per cent slower): these give the
     # per-kernel share and the roofline's launch durations.  Clocks are sampled across both.
     ms_total, vstats = timed(lambda: step_device("strong", 0), args.steps)
+    if args.dump_outputs:
+        last = summed(vstats[-1:], "paths", "rays")  # a collective: every rank takes part
+        if rank == 0:
+            dump_outputs(args.dump_outputs, accum.cpu().numpy(), out_u32.cpu().numpy(), w, h, last)
     _, stats = timed(lambda: step_device("strong", pt.FLAG_TIMING), args.steps)
     clocks = sampler.stop() if rank == 0 else None
 

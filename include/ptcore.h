@@ -164,8 +164,13 @@ int ptc_scene_commit(ptc_scene *, int device);
 /* Same with options.  PTC_COMMIT_FAST_BUILD: flatten the meshes entirely on the device — the reference's own median-split
  * tree (src/acceleration/bvh.rs:15-76), which has to be restated anyway for the dead-triangle mask, doubles as the
  * traversal tree: 2 M triangles commit in ~0.2 s instead of ~1 s, the render is ~20 % slower than through the default
- * SAH tree (host-built from the device-restated mask).  Results (hit records, images) are identical either way. */
-enum { PTC_COMMIT_FAST_BUILD = 1 };
+ * SAH tree (host-built from the device-restated mask).  Results (hit records, images) are identical either way.
+ * PTC_COMMIT_DEVICE_SAH: flatten the meshes entirely on the device AND build the default's traversal tree there — the
+ * binned SAH tree and 8-wide collapse of the host builder, decision for decision, for meshes of every size (same wide
+ * nodes and leaves, same node and triangle tests per ray).  Meshes of 2^27
+ * triangles or more, and a non-default PTC_REF_TIE, still take the host builder; PTC_COLLAPSE=greedy applies to the host
+ * builder only.  Combined with PTC_COMMIT_FAST_BUILD: PTC_E_INVALID. */
+enum { PTC_COMMIT_FAST_BUILD = 1, PTC_COMMIT_DEVICE_SAH = 2 };
 int ptc_scene_commit_ex(ptc_scene *, int device, int flags);
 /* Path-pool slots the last render on this handle used (what pool_paths = 0 resolved to). */
 int64_t ptc_scene_last_pool_slots(const ptc_scene *);

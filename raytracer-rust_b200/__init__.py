@@ -23,6 +23,7 @@ MAT_LAMBERT, MAT_LAMBERT_CHECKER, MAT_METAL, MAT_DIELECTRIC, MAT_EMISSIVE, MAT_P
 DIST_GGX, DIST_BECKMANN = 0, 1
 FLAG_COUNTERS, FLAG_TIMING, FLAG_NEE = 1, 2, 4
 COMMIT_FAST_BUILD = 1
+COMMIT_DEVICE_SAH = 2
 LOAD_INFINITE_SPHERE_SKY, LOAD_WO3_STRIDE16, LOAD_SKIP_UNKNOWN = 1, 2, 4
 OBJ_SPHERE, OBJ_PLANE, OBJ_QUAD, OBJ_CUBE, OBJ_MESH = range(5)
 
@@ -503,9 +504,11 @@ class CoreScene:
         _ck(core().ptc_scene_build(self._h))
         return self
 
-    def commit(self, device=0, fast_build=False):
-        """fast_build: PTC_COMMIT_FAST_BUILD — flatten the meshes entirely on the device (quick commit, slower traversal)."""
-        _ck(core().ptc_scene_commit_ex(self._h, device, COMMIT_FAST_BUILD if fast_build else 0))
+    def commit(self, device=0, fast_build=False, device_sah=False):
+        """fast_build: PTC_COMMIT_FAST_BUILD — flatten the meshes entirely on the device (quick commit, slower traversal).
+        device_sah: PTC_COMMIT_DEVICE_SAH — flatten them on the device into the default's SAH tree (quick commit, same tree)."""
+        flags = (COMMIT_FAST_BUILD if fast_build else 0) | (COMMIT_DEVICE_SAH if device_sah else 0)
+        _ck(core().ptc_scene_commit_ex(self._h, device, flags))
         self.device = device
         return self
 

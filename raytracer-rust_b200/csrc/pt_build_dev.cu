@@ -6,10 +6,13 @@
 
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
+#include <cub/device/device_select.cuh>
 
 #include <algorithm>
 #include <chrono>
+#include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <stdexcept>
 #include <string>
 #include <unordered_map>
@@ -418,6 +421,538 @@ __global__ void k_emit_level(const WNode *wn, const uint32_t *sid, uint32_t leve
   out[4] = make_float4(pack4(qhi[1]), pack4(qhi[1] + 4), pack4(qhi[2]), pack4(qhi[2] + 4));
 }
 
+// ---- step 2, DevBuildMode::Sah: pt_build.cpp's binned SAH tree and collapse plan, decision for decision ------------
+// A split decision depends on the SET of triangles in a node only (bins hold min / max / counts; the sweep runs over the
+// non-empty bins in double, axes x -> y -> z, strict <), so kernels that see the same sets make the same decisions.
+// Triangles are addressed by ORIGINAL index; `prim` is the permutation of the live ones, initially ascending (the host's
+// live_ids), and every node owns a contiguous range of it.  Node ids depend on ranges alone, not on scheduling: a range
+// [f, f + c) owns ids [2f, 2f + 2c - 1); a leaf takes 2f, an inner node split at `mid` takes 2 mid - 1, its children the
+// ranges below and above.
+constexpr int kBins = 16, kLeafMax = 3;
+constexpr uint32_t kWarpMax = 32;  // nodes of at most this many triangles: one warp builds the whole subtree (k_small)
+constexpr int kBinWords = 13;      // per bin: box lo / hi keys, centroid lo / hi keys (fkey), count
+constexpr int kNodeBinWords = 3 * kBins * kBinWords;
+
+struct OpenNode {  // a node of > kWarpMax triangles waiting for its level
+  uint32_t first, count;
+  int32_t parent, side;  // side 1: right child
+  float cb[6];           // centroid bounds lo xyz, hi xyz
+};
+struct SmallNode {
+  uint32_t first, count;
+  int32_t parent, side;
+};
+struct SplitDev {  // decision for one open node: axis < 0 = all centroids coincide, split at mid
+  int32_t axis, split;
+  uint32_t mid;
+  float lo, k;
+};
+struct B2Dev {  // binary tree by node id; count == 0: no node has this id
+  Box *box;
+  uint32_t *first, *count;
+  int32_t *left, *right, *parent;
+};
+
+__device__ __forceinline__ bool bin_word_is_min(int w) { return w < 3 || (w >= 6 && w < 9); }
+
+__device__ __forceinline__ double box_area(const Box &b) {  // pt_build.cpp: Box3::area
+  const double x = (double)b.hi[0] - b.lo[0], y = (double)b.hi[1] - b.lo[1], z = (double)b.hi[2] - b.lo[2];
+  if (x < 0) return 0.0;
+  return 2.0 * (x * y + y * z + z * x);
+}
+
+__device__ __forceinline__ void link_node(const B2Dev &b2, int32_t id, int32_t parent, int32_t side, int32_t *root_id) {
+  b2.parent[id] = parent;
+  if (parent < 0) *root_id = id;
+  else (side ? b2.right : b2.left)[parent] = id;
+}
+
+// live triangles in ascending original index, centroids 0.5 (lo + hi) of every triangle's box (pt_build.cpp:872-884)
+__global__ void k_live_flags(const uint8_t *dead, uint32_t n, uint32_t *flag) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) flag[i] = dead[i] ? 0u : 1u;
+}
+__global__ void k_live_scatter(const uint32_t *flag, const uint32_t *rank, const float *tbox, uint32_t n, uint32_t *prim, float *pcen) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  if (flag[i]) prim[rank[i]] = i;
+  for (int a = 0; a < 3; a++) pcen[(size_t)i * 3 + a] = 0.5f * (tbox[(size_t)i * 6 + a] + tbox[(size_t)i * 6 + 3 + a]);
+}
+
+// centroid bounds of the root (only when it is an open node)
+__global__ void k_root_cb(const uint32_t *prim, const float *pcen, uint32_t nl, uint32_t *keys) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  uint32_t k[6] = {0xffffffffu, 0xffffffffu, 0xffffffffu, 0u, 0u, 0u};
+  if (i < nl) {
+    const float *c = pcen + (size_t)prim[i] * 3;
+    for (int a = 0; a < 3; a++) k[a] = k[3 + a] = fkey(c[a], false);
+  }
+  for (int a = 0; a < 3; a++) k[a] = __reduce_min_sync(0xffffffffu, k[a]), k[3 + a] = __reduce_max_sync(0xffffffffu, k[3 + a]);
+  if ((threadIdx.x & 31u) == 0u)
+    for (int a = 0; a < 3; a++) atomicMin(keys + a, k[a]), atomicMax(keys + 3 + a, k[3 + a]);
+}
+__global__ void k_root_open(const uint32_t *keys, uint32_t nl, OpenNode *open, uint32_t *off) {
+  OpenNode o;
+  o.first = 0u, o.count = nl, o.parent = -1, o.side = 0;
+  for (int a = 0; a < 6; a++) o.cb[a] = fkey_inv(keys[a]);
+  open[0] = o;
+  off[0] = 0u;
+}
+
+// the open node that holds active element t: the last j with off[j] <= t
+__device__ __forceinline__ uint32_t find_open(const uint32_t *off, uint32_t n_open, uint32_t t) {
+  uint32_t lo = 0u, hi = n_open;
+  while (hi - lo > 1u) {
+    const uint32_t m = (lo + hi) >> 1;
+    if (off[m] <= t) lo = m;
+    else hi = m;
+  }
+  return lo;
+}
+
+__device__ __forceinline__ void axis_scale(const float *cb, bool ok[3], float kk[3]) {  // pt_build.cpp:276-280
+  for (int a = 0; a < 3; a++) {
+    const float cext = cb[3 + a] - cb[a];
+    ok[a] = cext > 0.0f;
+    kk[a] = ok[a] ? (float)kBins / cext : 0.0f;
+  }
+}
+__device__ __forceinline__ int bin_of(float c, float lo, float k) {
+  const int bi = (int)((c - lo) * k);
+  return min(max(bi, 0), kBins - 1);
+}
+
+__global__ void k_bins_init(uint32_t *bins, size_t words) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < words) bins[i] = bin_word_is_min((int)(i % kBinWords)) ? 0xffffffffu : 0u;
+}
+
+// One thread per triangle of an open node: its box, centroid and count into the node's 3 x 16 bins.  A block whose
+// triangles all belong to one node aggregates in shared memory first.  Min, max and integer sums do not depend on the
+// order of the updates.  A node whose centroids coincide on every axis is binned into bin 0 of axis 0 (box and count only).
+__global__ void k_bin(const OpenNode *open, const uint32_t *off, uint32_t n_open, uint32_t total, const uint32_t *prim, const float *tbox,
+                      const float *pcen, uint32_t *bins) {
+  __shared__ uint32_t sb[kNodeBinWords];
+  const uint32_t t0 = blockIdx.x * blockDim.x, t = t0 + threadIdx.x;
+  const uint32_t j0 = find_open(off, n_open, t0), j1 = find_open(off, n_open, min(total, t0 + blockDim.x) - 1u);
+  const bool shared = j0 == j1;
+  if (shared) {
+    for (int w = threadIdx.x; w < kNodeBinWords; w += blockDim.x) sb[w] = bin_word_is_min(w % kBinWords) ? 0xffffffffu : 0u;
+    __syncthreads();
+  }
+  if (t < total) {
+    const uint32_t j = shared ? j0 : find_open(off, n_open, t);
+    const OpenNode &o = open[j];
+    const uint32_t p = prim[o.first + (t - off[j])];
+    uint32_t key[12];
+    for (int a = 0; a < 6; a++) key[a] = fkey(tbox[(size_t)p * 6 + a], false);
+    for (int a = 0; a < 3; a++) key[6 + a] = key[9 + a] = fkey(pcen[(size_t)p * 3 + a], false);
+    bool ok[3];
+    float kk[3];
+    axis_scale(o.cb, ok, kk);
+    const bool none = !ok[0] && !ok[1] && !ok[2];
+    uint32_t *base = shared ? sb : bins + (size_t)j * kNodeBinWords;
+    for (int a = 0; a < 3; a++) {
+      if (!ok[a] && !(none && a == 0)) continue;
+      const int bi = ok[a] ? bin_of(pcen[(size_t)p * 3 + a], o.cb[a], kk[a]) : 0;
+      uint32_t *d = base + (a * kBins + bi) * kBinWords;
+      for (int w = 0; w < 12; w++) {
+        if (bin_word_is_min(w)) atomicMin(d + w, key[w]);
+        else atomicMax(d + w, key[w]);
+      }
+      atomicAdd(d + 12, 1u);
+    }
+  }
+  if (shared) {
+    __syncthreads();
+    uint32_t *d = bins + (size_t)j0 * kNodeBinWords;
+    for (int w = threadIdx.x; w < kNodeBinWords; w += blockDim.x) {
+      const int k = w % kBinWords;
+      if (sb[w - k + 12] == 0u) continue;  // empty bin
+      if (k == 12) atomicAdd(d + w, sb[w]);
+      else if (bin_word_is_min(k)) atomicMin(d + w, sb[w]);
+      else atomicMax(d + w, sb[w]);
+    }
+  }
+}
+
+__device__ __forceinline__ Box bin_box(const uint32_t *b, int first_word) {
+  Box r;
+  for (int a = 0; a < 3; a++) r.lo[a] = fkey_inv(b[first_word + a]), r.hi[a] = fkey_inv(b[first_word + 3 + a]);
+  return r;
+}
+__device__ __forceinline__ void box_union(Box &acc, const Box &b) {
+  for (int a = 0; a < 3; a++) acc.lo[a] = fminf(acc.lo[a], b.lo[a]), acc.hi[a] = fmaxf(acc.hi[a], b.hi[a]);
+}
+__device__ __forceinline__ Box box_empty() {
+  Box r;
+  for (int a = 0; a < 3; a++) r.lo[a] = INFINITY, r.hi[a] = -INFINITY;
+  return r;
+}
+
+// One thread per open node: the sweep of pt_build.cpp:321-370 over its bins, the node's record, its children.  Children
+// of more than kWarpMax triangles become candidates of the next level (slots 2j, 2j + 1, compacted in order by the
+// caller: the next level's nodes stay sorted by range); the others go to the list k_small works on.
+__global__ void k_sweep(const OpenNode *open, uint32_t n_open, const uint32_t *bins, SplitDev *splits, B2Dev b2, int32_t *root_id,
+                        OpenNode *cand, uint8_t *cand_flag, SmallNode *small, uint32_t *counters) {
+  const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= n_open) return;
+  const OpenNode o = open[j];
+  const uint32_t *B = bins + (size_t)j * kNodeBinWords;
+  bool ok[3];
+  float kk[3];
+  axis_scale(o.cb, ok, kk);
+  const int a0 = ok[0] ? 0 : (ok[1] ? 1 : (ok[2] ? 2 : 0));  // every triangle sits in one bin of this axis
+  Box nb = box_empty();
+  for (int bi = 0; bi < kBins; bi++)
+    if (B[(a0 * kBins + bi) * kBinWords + 12]) box_union(nb, bin_box(B + (a0 * kBins + bi) * kBinWords, 0));
+  int best_axis = -1, best_split = -1;
+  double best_cost = 1.7976931348623157e308;
+  for (int a = 0; a < 3; a++) {
+    if (!ok[a]) continue;
+    const uint32_t *ba = B + a * kBins * kBinWords;
+    int idx[kBins], m = 0;
+    for (int bi = 0; bi < kBins; bi++)
+      if (ba[bi * kBinWords + 12]) idx[m++] = bi;
+    if (m < 2) continue;
+    double right_area[kBins];
+    uint32_t right_n[kBins];
+    Box acc = box_empty();
+    uint32_t cnt = 0u;
+    for (int q = m - 1; q > 0; q--) {
+      box_union(acc, bin_box(ba + idx[q] * kBinWords, 0));
+      cnt += ba[idx[q] * kBinWords + 12];
+      right_area[q] = box_area(acc);
+      right_n[q] = cnt;
+    }
+    acc = box_empty();
+    cnt = 0u;
+    for (int q = 0; q < m - 1; q++) {
+      box_union(acc, bin_box(ba + idx[q] * kBinWords, 0));
+      cnt += ba[idx[q] * kBinWords + 12];
+      const double cost = box_area(acc) * (double)(int32_t)cnt + right_area[q + 1] * (double)(int32_t)right_n[q + 1];
+      if (cost < best_cost) best_cost = cost, best_axis = a, best_split = idx[q] + 1;
+    }
+  }
+  SplitDev sp;
+  sp.axis = best_axis, sp.split = best_split, sp.lo = 0.0f, sp.k = 0.0f;
+  float cbl[6], cbr[6];
+  uint32_t nleft;
+  if (best_axis < 0) {  // all centroids coincide: both halves keep the node's (point) centroid bounds
+    nleft = o.count / 2u;
+    for (int a = 0; a < 6; a++) cbl[a] = cbr[a] = o.cb[a];
+  } else {
+    sp.lo = o.cb[best_axis], sp.k = kk[best_axis];
+    for (int a = 0; a < 3; a++) cbl[a] = cbr[a] = INFINITY, cbl[3 + a] = cbr[3 + a] = -INFINITY;
+    nleft = 0u;
+    const uint32_t *ba = B + best_axis * kBins * kBinWords;
+    for (int bi = 0; bi < kBins; bi++) {
+      const uint32_t c = ba[bi * kBinWords + 12];
+      if (!c) continue;
+      const Box cbox = bin_box(ba + bi * kBinWords, 6);
+      float *dst = bi < best_split ? cbl : cbr;
+      if (bi < best_split) nleft += c;
+      for (int a = 0; a < 3; a++) dst[a] = fminf(dst[a], cbox.lo[a]), dst[3 + a] = fmaxf(dst[3 + a], cbox.hi[a]);
+    }
+  }
+  const uint32_t mid = o.first + nleft;
+  sp.mid = mid;
+  splits[j] = sp;
+  const int32_t id = (int32_t)(2u * mid - 1u);
+  b2.box[id] = nb, b2.first[id] = o.first, b2.count[id] = o.count;
+  link_node(b2, id, o.parent, o.side, root_id);
+  atomicAdd(counters + 3, 1u);  // inner nodes
+  for (int s = 0; s < 2; s++) {
+    const uint32_t cf = s ? mid : o.first, cc = s ? o.first + o.count - mid : nleft;
+    if (cc > kWarpMax) {
+      OpenNode c;
+      c.first = cf, c.count = cc, c.parent = id, c.side = s;
+      for (int a = 0; a < 6; a++) c.cb[a] = s ? cbr[a] : cbl[a];
+      cand[2 * j + s] = c;
+      cand_flag[2 * j + s] = 1;
+      atomicAdd(counters + 1, cc);  // elements of the next level
+    } else {
+      cand_flag[2 * j + s] = 0;
+      small[atomicAdd(counters + 2, 1u)] = SmallNode{cf, cc, id, s};
+    }
+  }
+}
+
+// Partition of every open node's range as pt_build.cpp's std::partition does it — from the left the first element that
+// goes right, from the right the first that goes left, swap, repeat (the bidirectional algorithm of libstdc++ and libc++) —
+// so that every leaf ends up with the host's triangles in the host's order (the traversal's triangle order, hence its
+// node and triangle test counts, depends on it).  In closed form: the k-th element (ascending) left of `mid` that goes
+// right trades places with the k-th element (descending) right of `mid` that goes left.  Flag, one exclusive scan
+// (caller), ranks of the right-hand movers, swaps.  All centroids coincide: the host keeps the order and splits at mid.
+__global__ void k_part_flag(const OpenNode *open, const uint32_t *off, uint32_t n_open, uint32_t total, const uint32_t *prim, const float *pcen,
+                            const SplitDev *splits, uint32_t *flag) {
+  const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= total) return;
+  const uint32_t j = find_open(off, n_open, t);
+  const uint32_t pos = open[j].first + (t - off[j]);
+  const SplitDev sp = splits[j];
+  if (sp.axis < 0) flag[t] = pos < sp.mid ? 1u : 0u;
+  else flag[t] = bin_of(pcen[(size_t)prim[pos] * 3 + sp.axis], sp.lo, sp.k) < sp.split ? 1u : 0u;
+}
+__global__ void k_part_rank(const OpenNode *open, const uint32_t *off, uint32_t n_open, uint32_t total, const SplitDev *splits, const uint32_t *flag,
+                            const uint32_t *scan, uint32_t *partner) {
+  const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= total) return;
+  const uint32_t j = find_open(off, n_open, t), oj = off[j];
+  const uint32_t first = open[j].first, pos = first + (t - oj), mid = splits[j].mid;
+  if (pos >= mid && flag[t]) partner[first + (mid - first - 1u - (scan[t] - scan[oj]))] = pos;
+}
+__global__ void k_part_swap(const OpenNode *open, const uint32_t *off, uint32_t n_open, uint32_t total, const SplitDev *splits, const uint32_t *flag,
+                            const uint32_t *scan, const uint32_t *partner, uint32_t *prim) {
+  const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= total) return;
+  const uint32_t j = find_open(off, n_open, t), oj = off[j];
+  const uint32_t first = open[j].first, pos = first + (t - oj);
+  if (pos >= splits[j].mid || flag[t]) return;
+  const uint32_t q = partner[first + (pos - first) - (scan[t] - scan[oj])];
+  const uint32_t x = prim[pos];
+  prim[pos] = prim[q];
+  prim[q] = x;
+}
+__global__ void k_open_counts(const OpenNode *open, uint32_t n_open, uint32_t *cnt) {
+  const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j < n_open) cnt[j] = open[j].count;
+}
+
+// One warp per node of <= kWarpMax triangles builds its whole subtree: lane i holds the i-th triangle of the range.  The
+// bins of the host's sweep are not needed here — a split position after a non-empty bin is the same as "every triangle
+// whose bin is <= this lane's bin goes left", so each lane evaluates the candidate of its own bin, per axis, over the
+// exact left and right boxes (min / max over the lanes), and the warp takes the host's first minimum: lowest cost, then
+// lowest axis, then lowest bin.
+constexpr int kSmallWarps = 4;
+__global__ void __launch_bounds__(32 * kSmallWarps) k_small(const SmallNode *small, uint32_t n_small, uint32_t *prim, const float *tbox,
+                                                            const float *pcen, B2Dev b2, int32_t *root_id, uint32_t *counters) {
+  __shared__ uint32_t s_prim[kSmallWarps][32], s_slot[kSmallWarps][32];
+  __shared__ float s_val[kSmallWarps][32][9];
+  const int wib = threadIdx.x >> 5;
+  const uint32_t lane = threadIdx.x & 31u;
+  const uint32_t w = blockIdx.x * kSmallWarps + wib;
+  if (w >= n_small) return;  // whole warps
+  const SmallNode sn = small[w];
+  uint32_t p = 0u;
+  float v[9];  // box lo xyz, hi xyz, centroid xyz
+  for (int a = 0; a < 3; a++) v[a] = INFINITY, v[3 + a] = -INFINITY, v[6 + a] = 0.0f;
+  if (lane < sn.count) {
+    p = prim[sn.first + lane];
+    for (int a = 0; a < 6; a++) v[a] = tbox[(size_t)p * 6 + a];
+    for (int a = 0; a < 3; a++) v[6 + a] = pcen[(size_t)p * 3 + a];
+  }
+  struct Item {
+    int32_t f, c, parent, side;
+  } stack[32];
+  int sp = 0;
+  stack[sp++] = Item{0, (int32_t)sn.count, sn.parent, sn.side};
+  uint32_t inner = 0u;
+  while (sp > 0) {
+    const Item it = stack[--sp];
+    const bool in = (int)lane >= it.f && (int)lane < it.f + it.c;
+    Box nb;
+    float cb[6];
+    for (int a = 0; a < 3; a++) {
+      nb.lo[a] = in ? v[a] : INFINITY, nb.hi[a] = in ? v[3 + a] : -INFINITY;
+      cb[a] = in ? v[6 + a] : INFINITY, cb[3 + a] = in ? v[6 + a] : -INFINITY;
+    }
+    for (int o = 16; o > 0; o >>= 1)
+      for (int a = 0; a < 3; a++) {
+        nb.lo[a] = fminf(nb.lo[a], __shfl_xor_sync(0xffffffffu, nb.lo[a], o));
+        nb.hi[a] = fmaxf(nb.hi[a], __shfl_xor_sync(0xffffffffu, nb.hi[a], o));
+        cb[a] = fminf(cb[a], __shfl_xor_sync(0xffffffffu, cb[a], o));
+        cb[3 + a] = fmaxf(cb[3 + a], __shfl_xor_sync(0xffffffffu, cb[3 + a], o));
+      }
+    const uint32_t gfirst = sn.first + (uint32_t)it.f;
+    if (it.c <= kLeafMax) {
+      if (lane == 0u) {
+        const int32_t id = (int32_t)(2u * gfirst);
+        b2.box[id] = nb, b2.first[id] = gfirst, b2.count[id] = (uint32_t)it.c, b2.left[id] = -1, b2.right[id] = -1;
+        link_node(b2, id, it.parent, it.side, root_id);
+      }
+      continue;
+    }
+    bool ok[3];
+    float kk[3];
+    axis_scale(cb, ok, kk);
+    int bin[3];
+    for (int a = 0; a < 3; a++) bin[a] = (in && ok[a]) ? bin_of(v[6 + a], cb[a], kk[a]) : -1;
+    Box L[3], R[3];
+    int nl[3] = {0, 0, 0}, nr[3] = {0, 0, 0};
+    for (int a = 0; a < 3; a++) L[a] = box_empty(), R[a] = box_empty();
+    for (int q = it.f; q < it.f + it.c; q++) {
+      float u[6];
+      int bq[3];
+      for (int a = 0; a < 6; a++) u[a] = __shfl_sync(0xffffffffu, v[a], q);
+      for (int a = 0; a < 3; a++) bq[a] = __shfl_sync(0xffffffffu, bin[a], q);
+      for (int a = 0; a < 3; a++) {
+        const bool left = bq[a] <= bin[a];
+        Box &d = left ? L[a] : R[a];
+        for (int e = 0; e < 3; e++) d.lo[e] = fminf(d.lo[e], u[e]), d.hi[e] = fmaxf(d.hi[e], u[3 + e]);
+        (left ? nl[a] : nr[a])++;
+      }
+    }
+    bool valid = false;
+    double best = 0.0;
+    int ba = 3, bb = kBins;
+    for (int a = 0; a < 3; a++) {
+      if (bin[a] < 0 || nr[a] == 0) continue;
+      const double cost = box_area(L[a]) * (double)nl[a] + box_area(R[a]) * (double)nr[a];
+      if (!valid || cost < best) valid = true, best = cost, ba = a, bb = bin[a];
+    }
+    for (int o = 16; o > 0; o >>= 1) {
+      const bool ov = __shfl_xor_sync(0xffffffffu, (int)valid, o) != 0;
+      const double oc = __shfl_xor_sync(0xffffffffu, best, o);
+      const int oa = __shfl_xor_sync(0xffffffffu, ba, o), ob = __shfl_xor_sync(0xffffffffu, bb, o);
+      if (ov && (!valid || oc < best || (oc == best && (oa < ba || (oa == ba && ob < bb))))) valid = true, best = oc, ba = oa, bb = ob;
+    }
+    int32_t mid_l;
+    if (!valid) {
+      mid_l = it.f + it.c / 2;  // all centroids coincide
+    } else {
+      // the host's std::partition (see k_part_rank): the k-th right-goer left of mid <-> the k-th left-goer from the right
+      const bool go_left = in && bin[ba] <= bb;
+      const int32_t nleft = __popc(__ballot_sync(0xffffffffu, go_left));
+      const bool mis_l = in && (int)lane < it.f + nleft && !go_left, mis_r = (int)lane >= it.f + nleft && go_left;
+      const uint32_t ml = __ballot_sync(0xffffffffu, mis_l), mr = __ballot_sync(0xffffffffu, mis_r), below = (1u << lane) - 1u;
+      const int k = mis_l ? __popc(ml & below) : __popc(mr & ~below & ~(1u << lane));
+      if (mis_l) s_slot[wib][16 + k] = lane;
+      if (mis_r) s_slot[wib][k] = lane;
+      __syncwarp();
+      const uint32_t dest = mis_l ? s_slot[wib][k] : (mis_r ? s_slot[wib][16 + k] : lane);
+      __syncwarp();
+      s_prim[wib][dest] = p;
+      for (int a = 0; a < 9; a++) s_val[wib][dest][a] = v[a];
+      __syncwarp();
+      p = s_prim[wib][lane];
+      for (int a = 0; a < 9; a++) v[a] = s_val[wib][lane][a];
+      __syncwarp();
+      mid_l = it.f + nleft;
+    }
+    const int32_t id = (int32_t)(2u * (sn.first + (uint32_t)mid_l) - 1u);
+    if (lane == 0u) {
+      b2.box[id] = nb, b2.first[id] = gfirst, b2.count[id] = (uint32_t)it.c;
+      link_node(b2, id, it.parent, it.side, root_id);
+    }
+    inner++;
+    stack[sp++] = Item{mid_l, it.f + it.c - mid_l, id, 1};
+    stack[sp++] = Item{it.f, mid_l - it.f, id, 0};
+  }
+  if (lane < sn.count) prim[sn.first + lane] = p;
+  if (lane == 0u && inner) atomicAdd(counters + 3, inner);
+}
+
+// The collapse plan of pt_build.cpp:449-526, bottom-up: a thread starts at a leaf and climbs while it is the second of
+// two children to arrive at the parent.  Costs are stored as float, temporaries are double, like the host's.
+__device__ void plan_inner(const B2Dev &b2, int32_t n, double c_n, float *cost, uint8_t *split) {
+  const double area = box_area(b2.box[n]);
+  const float *L = cost + (size_t)b2.left[n] * 8, *R = cost + (size_t)b2.right[n] * 8;
+  float l[7], r[7];
+  for (int i = 0; i < 7; i++) l[i] = __ldcg(L + i), r[i] = __ldcg(R + i);
+  double D[9];
+  uint8_t K[9];
+  for (int j = 2; j <= 8; j++) {
+    D[j] = 1.7976931348623157e308, K[j] = 1;
+    for (int k = 1; k < j; k++) {
+      const double v = (double)l[k - 1] + (double)r[j - k - 1];
+      if (v < D[j]) D[j] = v, K[j] = (uint8_t)k;
+    }
+  }
+  const uint32_t count = b2.count[n];
+  const double c_leaf = count <= (uint32_t)kLeafMax ? area * (double)count * 1.0 : 1.7976931348623157e308;
+  const double c_inner = area * c_n + D[8];
+  float *C = cost + (size_t)n * 8;
+  uint8_t *S = split + (size_t)n * 8;
+  C[0] = (float)(c_inner < c_leaf ? c_inner : c_leaf);
+  S[7] = K[8];
+  for (int i = 2; i <= 7; i++) {
+    if (D[i] < (double)C[i - 2]) C[i - 1] = (float)D[i], S[i - 1] = K[i];
+    else C[i - 1] = C[i - 2], S[i - 1] = 0;
+  }
+}
+__global__ void k_plan(B2Dev b2, uint32_t n_ids, double c_n, float *cost, uint8_t *split, uint32_t *arrive) {
+  const uint32_t id = blockIdx.x * blockDim.x + threadIdx.x;
+  if (id >= n_ids || b2.count[id] == 0u || b2.left[id] >= 0) return;
+  const float leaf_cost = (float)(box_area(b2.box[id]) * (double)b2.count[id] * 1.0);
+  for (int i = 0; i < 8; i++) cost[(size_t)id * 8 + i] = leaf_cost;
+  int32_t n = (int32_t)id;
+  for (;;) {
+    const int32_t p = b2.parent[n];
+    if (p < 0) return;
+    __threadfence();
+    if (atomicAdd(arrive + p, 1u) == 0u) return;  // the sibling's subtree is still being planned
+    __threadfence();
+    plan_inner(b2, p, c_n, cost, split);
+    n = p;
+  }
+}
+
+// Wide structure, one level per launch pair: the children of every node of the level (pt_build.cpp: plan_children, left
+// before right), then — after two exclusive scans give each node its first inner child and first triangle record — the
+// WNode records in breadth-first order (gen_structure's layout: inner children consecutive in child order) and the next
+// level's node list.  A binary node is a leaf of the wide tree exactly when it has <= 3 triangles (a binary leaf; an inner
+// binary node has >= 4 and its c_leaf is infinite), so WNode's count rule holds for these trees too.
+__global__ void k_wide_children(const int32_t *lvl, uint32_t count, B2Dev b2, const uint8_t *split, int32_t *ch, uint32_t *n_inner, uint32_t *n_tris) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= count) return;
+  const int32_t n = lvl[i];
+  int32_t c[8];
+  int nch = 0;
+  if (b2.left[n] < 0) {
+    c[nch++] = n;  // a mesh of <= 3 live triangles: a root with one leaf
+  } else {
+    int32_t st_node[16], st_slots[16];
+    int sp = 0;
+    const int k = split[(size_t)n * 8 + 7];
+    st_node[sp] = b2.right[n], st_slots[sp++] = 8 - k;
+    st_node[sp] = b2.left[n], st_slots[sp++] = k;
+    while (sp > 0) {
+      const int32_t x = st_node[--sp];
+      const int s = st_slots[sp];
+      if (b2.left[x] < 0 || s == 1) {
+        c[nch++] = x;
+        continue;
+      }
+      const int kk = split[(size_t)x * 8 + s - 1];
+      if (kk == 0) {
+        st_node[sp] = x, st_slots[sp++] = s - 1;
+      } else {
+        st_node[sp] = b2.right[x], st_slots[sp++] = s - kk;
+        st_node[sp] = b2.left[x], st_slots[sp++] = kk;
+      }
+    }
+  }
+  uint32_t ni = 0u, nt = 0u;
+  for (int q = 0; q < 8; q++) {
+    ch[(size_t)i * 8 + q] = q < nch ? c[q] : -1;
+    if (q < nch) {
+      const uint32_t cnt = b2.count[c[q]];
+      if (cnt > (uint32_t)kLeafMax) ni++;
+      else nt += cnt;
+    }
+  }
+  n_inner[i] = ni, n_tris[i] = nt;
+}
+__global__ void k_wide_write(const int32_t *lvl, uint32_t count, const int32_t *ch, B2Dev b2, const uint32_t *n_inner, const uint32_t *n_tris,
+                             const uint32_t *cbase, const uint32_t *tbase, uint32_t level_first, uint32_t next_first, uint32_t tri_first, WNode *wn,
+                             int32_t *lvl_next, uint32_t *totals) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= count) return;
+  WNode w;
+  w.child_base = next_first + cbase[i];
+  w.tri_base = tri_first + tbase[i];
+  uint32_t r = 0u;
+  for (int q = 0; q < 8; q++) {
+    const int32_t x = ch[(size_t)i * 8 + q];
+    w.child_lo[q] = x < 0 ? 0u : b2.first[x];
+    w.child_cnt[q] = x < 0 ? 0u : b2.count[x];
+    if (x >= 0 && w.child_cnt[q] > (uint32_t)kLeafMax) lvl_next[cbase[i] + r++] = x;
+  }
+  wn[level_first + i] = w;
+  if (i == count - 1u) totals[0] = cbase[i] + n_inner[i], totals[1] = tbase[i] + n_tris[i];
+}
+
 // ---- host side ----------------------------------------------------------------------------------------------------
 // The wide tree's structure from the live counts alone.  Binary tree = the reference's own (split at size / 2 while
 // size > 4, bvh.rs:19-27,55-56) with every range measured in LIVE triangles (R = live rank of a DFS position); ranges
@@ -520,9 +1055,216 @@ double ms_between(std::chrono::steady_clock::time_point a, std::chrono::steady_c
   return std::chrono::duration<double, std::milli>(b - a).count();
 }
 
+uint32_t widest_level(const std::vector<uint32_t> &level_first) {
+  uint32_t widest = 0;
+  for (size_t l = 0; l + 1 < level_first.size(); l++) widest = std::max(widest, level_first[l + 1] - level_first[l]);
+  return widest;
+}
+size_t scan_temp_bytes(uint32_t items) {
+  size_t bytes = 0;
+  CKB(cub::DeviceScan::ExclusiveSum(nullptr, bytes, (uint32_t *)nullptr, (uint32_t *)nullptr, (int)items, nullptr));
+  return bytes;
+}
+// arena bytes emit_wide takes for a wide tree of this shape (level l = ids [level_first[l], level_first[l + 1]))
+size_t emit_need(const std::vector<uint32_t> &level_first) {
+  const uint32_t widest = widest_level(level_first);
+  return Arena::need(level_first.back(), sizeof(Box)) + Arena::need(6, 4) + Arena::need(1, sizeof(int)) + 4 * Arena::need(widest, 4) +
+         Arena::need(scan_temp_bytes(widest), 1);
+}
+
+// Boxes, frames, slots, quantised nodes and triangle records of the wide tree described by `wn` (breadth-first
+// structural ids, level l = [level_first[l], level_first[l + 1])) — shared by both device step-2 builders.
+void emit_wide(Arena &a, cudaStream_t stream, const WNode *wn, const uint32_t *live, const std::vector<uint32_t> &level_first, uint32_t n_tri_records,
+               const float *tris, const int32_t *order, Buf<float4> &d_nodes, Buf<float4> &d_tri48, MeshBuild &m) {
+  const uint32_t n_nodes = level_first.back(), n_levels = (uint32_t)level_first.size() - 1, widest = widest_level(level_first);
+  const size_t scan_bytes = scan_temp_bytes(widest);
+  Box *d_box = a.get<Box>(n_nodes);
+  d_nodes.alloc((size_t)n_nodes * 5), d_tri48.alloc((size_t)std::max(n_tri_records, 1u) * 3);
+  float *d_root = a.get<float>(6);
+  int *d_err = a.get<int>(1);
+  CKB(cudaMemsetAsync(d_err, 0, sizeof(int), stream));
+  for (uint32_t l = n_levels; l-- > 0;) {
+    const uint32_t first = level_first[l], count = level_first[l + 1] - first;
+    k_boxes_level<<<blocks_for(count), kThreads, 0, stream>>>(wn, first, count, live, tris, d_box);
+  }
+  CKB(cudaGetLastError());
+  uint32_t *d_sid[2] = {a.get<uint32_t>(widest), a.get<uint32_t>(widest)}, *d_cnt = a.get<uint32_t>(widest), *d_cbase = a.get<uint32_t>(widest);
+  uint8_t *d_scan = a.get<uint8_t>(scan_bytes);
+  CKB(cudaMemsetAsync(d_sid[0], 0, 4, stream));  // level 0: final position 0 holds structural node 0
+  for (uint32_t l = 0; l < n_levels; l++) {
+    const uint32_t first = level_first[l], count = level_first[l + 1] - first;
+    k_inner_count<<<blocks_for(count), kThreads, 0, stream>>>(wn, d_sid[l & 1], count, d_cnt);
+    size_t sb = scan_bytes;
+    CKB(cub::DeviceScan::ExclusiveSum(d_scan, sb, d_cnt, d_cbase, (int)count, stream));
+    k_emit_level<<<blocks_for(count), kThreads, 0, stream>>>(wn, d_sid[l & 1], first, count, d_cbase, level_first[l + 1], d_sid[(l + 1) & 1], live, tris,
+                                                        order, d_box, d_nodes.p, d_tri48.p, d_root, d_err);
+    CKB(cudaGetLastError());
+  }
+  int err = 0;
+  float root[6];
+  CKB(cudaMemcpyAsync(&err, d_err, sizeof(int), cudaMemcpyDeviceToHost, stream));
+  CKB(cudaMemcpyAsync(root, d_root, sizeof(root), cudaMemcpyDeviceToHost, stream));
+  CKB(cudaStreamSynchronize(stream));
+  if (err) throw std::runtime_error("mesh extent too large for the quantised BVH frame");
+  for (int a3 = 0; a3 < 3; a3++) m.root_lo[a3] = root[a3], m.root_hi[a3] = root[3 + a3];
+  m.wide_depth = (int32_t)n_levels - 1;
+}
+
+// DevBuildMode::Sah, step 2 up to the WNode records: binary SAH tree (large nodes level by level, then one warp per small
+// subtree), collapse plan, wide structure.
+struct SahTree {
+  std::unique_ptr<Arena> work, wide;  // binary tree + plan; wide structure + room for emit_wide
+  const WNode *wn = nullptr;
+  const uint32_t *live = nullptr;  // triangle (original index) at every position of the final permutation
+  std::vector<uint32_t> level_first;
+  int sah_levels = 0;
+  double sah_ms = 0, plan_ms = 0, structure_ms = 0;
+};
+
+SahTree build_sah(uint32_t n, uint32_t nl, const uint8_t *d_dead, const float *d_tbox, cudaStream_t stream) {
+  auto now = [] { return std::chrono::steady_clock::now(); };
+  const auto t0 = now();
+  SahTree r;
+  const uint32_t max_open = nl / (kWarpMax + 1u) + 1u;  // an open node holds > kWarpMax triangles
+  const size_t n_ids = 2 * (size_t)nl;
+  size_t sel_bytes = 0;
+  CKB(cub::DeviceSelect::Flagged(nullptr, sel_bytes, (OpenNode *)nullptr, (uint8_t *)nullptr, (OpenNode *)nullptr, (uint32_t *)nullptr,
+                                 (int)(2 * max_open), stream));
+  const size_t temp_bytes = std::max(scan_temp_bytes(n), sel_bytes);
+  r.work.reset(new Arena(2 * Arena::need(n, 4) + 2 * Arena::need(nl, 4) + Arena::need((size_t)n * 3, 4) + Arena::need(n_ids, sizeof(Box)) +
+                         5 * Arena::need(n_ids, 4) + Arena::need(n_ids * 8, 4) + Arena::need(n_ids * 8, 1) + Arena::need(n_ids, 4) +
+                         4 * Arena::need(max_open, sizeof(OpenNode)) + Arena::need(2 * max_open, 1) + 2 * Arena::need(max_open, 4) +
+                         Arena::need(max_open, sizeof(SplitDev)) + Arena::need((size_t)max_open * kNodeBinWords, 4) + Arena::need(nl, sizeof(SmallNode)) +
+                         Arena::need(10, 4) + Arena::need(1, 4) + Arena::need(temp_bytes, 1) + 8192));
+  Arena &a = *r.work;
+  uint32_t *d_flag = a.get<uint32_t>(n), *d_scan = a.get<uint32_t>(n), *d_prim = a.get<uint32_t>(nl), *d_tmp = a.get<uint32_t>(nl);
+  float *d_pcen = a.get<float>((size_t)n * 3);
+  B2Dev b2;
+  b2.box = a.get<Box>(n_ids), b2.first = a.get<uint32_t>(n_ids), b2.count = a.get<uint32_t>(n_ids);
+  b2.left = a.get<int32_t>(n_ids), b2.right = a.get<int32_t>(n_ids), b2.parent = a.get<int32_t>(n_ids);
+  float *d_cost = a.get<float>(n_ids * 8);
+  uint8_t *d_split = a.get<uint8_t>(n_ids * 8);
+  uint32_t *d_arrive = a.get<uint32_t>(n_ids);
+  OpenNode *d_open[2] = {a.get<OpenNode>(max_open), a.get<OpenNode>(max_open)}, *d_cand = a.get<OpenNode>(2 * max_open);
+  uint8_t *d_cand_flag = a.get<uint8_t>(2 * max_open);
+  uint32_t *d_off = a.get<uint32_t>(max_open), *d_cnt = a.get<uint32_t>(max_open);
+  SplitDev *d_splits = a.get<SplitDev>(max_open);
+  uint32_t *d_bins = a.get<uint32_t>((size_t)max_open * kNodeBinWords);
+  SmallNode *d_small = a.get<SmallNode>(nl);
+  uint32_t *d_counters = a.get<uint32_t>(10);  // next level's nodes, next level's triangles, small nodes, inner nodes, root centroid keys
+  int32_t *d_root = a.get<int32_t>(1);
+  uint8_t *d_temp = a.get<uint8_t>(temp_bytes);
+
+  CKB(cudaMemsetAsync(b2.count, 0, n_ids * 4, stream));
+  CKB(cudaMemsetAsync(d_arrive, 0, n_ids * 4, stream));
+  uint32_t counters[10] = {0u, 0u, nl <= kWarpMax ? 1u : 0u, 0u, 0xffffffffu, 0xffffffffu, 0xffffffffu, 0u, 0u, 0u};
+  CKB(cudaMemcpy(d_counters, counters, sizeof(counters), cudaMemcpyHostToDevice));
+  if (nl <= kWarpMax) {
+    const SmallNode root{0u, nl, -1, 0};
+    CKB(cudaMemcpy(d_small, &root, sizeof(root), cudaMemcpyHostToDevice));
+  }
+  size_t tb = temp_bytes;
+  k_live_flags<<<blocks_for(n), kThreads, 0, stream>>>(d_dead, n, d_flag);
+  CKB(cub::DeviceScan::ExclusiveSum(d_temp, tb, d_flag, d_scan, (int)n, stream));
+  k_live_scatter<<<blocks_for(n), kThreads, 0, stream>>>(d_flag, d_scan, d_tbox, n, d_prim, d_pcen);
+  CKB(cudaGetLastError());
+
+  // large nodes, one level per pass
+  uint32_t n_open = 0, total = 0, n_small = counters[2];
+  if (nl > kWarpMax) {
+    k_root_cb<<<blocks_for(nl), kThreads, 0, stream>>>(d_prim, d_pcen, nl, d_counters + 4);
+    k_root_open<<<1, 1, 0, stream>>>(d_counters + 4, nl, d_open[0], d_off);
+    CKB(cudaGetLastError());
+    n_open = 1, total = nl;
+  }
+  int cur = 0;
+  while (n_open > 0) {
+    r.sah_levels++;
+    const size_t words = (size_t)n_open * kNodeBinWords;
+    k_bins_init<<<blocks_for(words), kThreads, 0, stream>>>(d_bins, words);
+    k_bin<<<blocks_for(total), kThreads, 0, stream>>>(d_open[cur], d_off, n_open, total, d_prim, d_tbox, d_pcen, d_bins);
+    CKB(cudaMemsetAsync(d_counters, 0, 8, stream));
+    k_sweep<<<blocks_for(n_open), kThreads, 0, stream>>>(d_open[cur], n_open, d_bins, d_splits, b2, d_root, d_cand, d_cand_flag, d_small, d_counters);
+    k_part_flag<<<blocks_for(total), kThreads, 0, stream>>>(d_open[cur], d_off, n_open, total, d_prim, d_pcen, d_splits, d_flag);
+    CKB(cudaGetLastError());
+    tb = temp_bytes;
+    CKB(cub::DeviceScan::ExclusiveSum(d_temp, tb, d_flag, d_scan, (int)total, stream));
+    k_part_rank<<<blocks_for(total), kThreads, 0, stream>>>(d_open[cur], d_off, n_open, total, d_splits, d_flag, d_scan, d_tmp);
+    k_part_swap<<<blocks_for(total), kThreads, 0, stream>>>(d_open[cur], d_off, n_open, total, d_splits, d_flag, d_scan, d_tmp, d_prim);
+    CKB(cudaGetLastError());
+    tb = temp_bytes;
+    CKB(cub::DeviceSelect::Flagged(d_temp, tb, d_cand, d_cand_flag, d_open[cur ^ 1], d_counters, (int)(2 * n_open), stream));
+    CKB(cudaMemcpyAsync(counters, d_counters, 4 * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+    CKB(cudaStreamSynchronize(stream));
+    cur ^= 1;
+    n_open = counters[0], total = counters[1], n_small = counters[2];
+    if (n_open > 0) {
+      k_open_counts<<<blocks_for(n_open), kThreads, 0, stream>>>(d_open[cur], n_open, d_cnt);
+      CKB(cudaGetLastError());
+      tb = temp_bytes;
+      CKB(cub::DeviceScan::ExclusiveSum(d_temp, tb, d_cnt, d_off, (int)n_open, stream));
+    }
+  }
+  // small nodes: one warp each, whole subtrees
+  k_small<<<(n_small + kSmallWarps - 1) / kSmallWarps, 32 * kSmallWarps, 0, stream>>>(d_small, n_small, d_prim, d_tbox, d_pcen, b2, d_root, d_counters);
+  CKB(cudaGetLastError());
+  int32_t root = -1;
+  CKB(cudaMemcpyAsync(counters, d_counters, 4 * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+  CKB(cudaMemcpyAsync(&root, d_root, sizeof(root), cudaMemcpyDeviceToHost, stream));
+  CKB(cudaStreamSynchronize(stream));
+  const uint32_t n_inner = counters[3];
+  if (root < 0 || (nl <= (uint32_t)kLeafMax) != (n_inner == 0u)) throw std::runtime_error("pt_build_dev: inconsistent SAH tree");
+  const auto t1 = now();
+
+  // collapse plan (PTC_SAH_CN: node cost, as pt_build.cpp)
+  const double c_n = getenv("PTC_SAH_CN") ? atof(getenv("PTC_SAH_CN")) : 1.8;
+  k_plan<<<blocks_for(n_ids), kThreads, 0, stream>>>(b2, (uint32_t)n_ids, c_n, d_cost, d_split, d_arrive);
+  CKB(cudaGetLastError());
+  CKB(cudaStreamSynchronize(stream));
+  const auto t2 = now();
+
+  // wide structure: at most one wide node per inner binary node (one when the root is a leaf)
+  const uint32_t cap = std::max(n_inner, 1u);
+  const std::vector<uint32_t> cap_shape{0u, cap};
+  r.wide.reset(new Arena(Arena::need(cap, sizeof(WNode)) + 2 * Arena::need(cap, 4) + Arena::need((size_t)cap * 8, 4) + 4 * Arena::need(cap, 4) +
+                         Arena::need(scan_temp_bytes(cap), 1) + Arena::need(2, 4) + emit_need(cap_shape) + 8192));
+  Arena &w = *r.wide;
+  WNode *d_wn = w.get<WNode>(cap);
+  int32_t *d_lvl[2] = {w.get<int32_t>(cap), w.get<int32_t>(cap)}, *d_ch = w.get<int32_t>((size_t)cap * 8);
+  uint32_t *d_ni = w.get<uint32_t>(cap), *d_nt = w.get<uint32_t>(cap), *d_cb = w.get<uint32_t>(cap), *d_tb = w.get<uint32_t>(cap);
+  const size_t scan2 = scan_temp_bytes(cap);
+  uint8_t *d_scan2 = w.get<uint8_t>(scan2);
+  uint32_t *d_tot = w.get<uint32_t>(2);
+  CKB(cudaMemcpyAsync(d_lvl[0], d_root, 4, cudaMemcpyDeviceToDevice, stream));
+  r.level_first.assign(1, 0u);
+  uint32_t count = 1, tri_first = 0;
+  for (int c = 0; count > 0; c ^= 1) {
+    const uint32_t first = r.level_first.back(), next_first = first + count;
+    if (next_first > cap) throw std::runtime_error("pt_build_dev: wide tree larger than its bound");
+    k_wide_children<<<blocks_for(count), kThreads, 0, stream>>>(d_lvl[c], count, b2, d_split, d_ch, d_ni, d_nt);
+    CKB(cudaGetLastError());
+    size_t sb = scan2;
+    CKB(cub::DeviceScan::ExclusiveSum(d_scan2, sb, d_ni, d_cb, (int)count, stream));
+    sb = scan2;
+    CKB(cub::DeviceScan::ExclusiveSum(d_scan2, sb, d_nt, d_tb, (int)count, stream));
+    k_wide_write<<<blocks_for(count), kThreads, 0, stream>>>(d_lvl[c], count, d_ch, b2, d_ni, d_nt, d_cb, d_tb, first, next_first, tri_first, d_wn,
+                                                         d_lvl[c ^ 1], d_tot);
+    CKB(cudaGetLastError());
+    uint32_t tot[2];
+    CKB(cudaMemcpyAsync(tot, d_tot, sizeof(tot), cudaMemcpyDeviceToHost, stream));
+    CKB(cudaStreamSynchronize(stream));
+    r.level_first.push_back(next_first);
+    count = tot[0], tri_first += tot[1];
+  }
+  if (tri_first != nl) throw std::runtime_error("pt_build_dev: wide tree does not hold every live triangle once");
+  r.wn = d_wn, r.live = d_prim;
+  r.sah_ms = ms_between(t0, t1), r.plan_ms = ms_between(t1, t2), r.structure_ms = ms_between(t2, now());
+  return r;
+}
+
 }  // namespace
 
-void build_mesh_device(MeshBuild &m, DevMeshBuffers &out, DevBuildTiming *timing, bool ref_only) {
+void build_mesh_device(MeshBuild &m, DevMeshBuffers &out, DevBuildTiming *timing, DevBuildMode mode) {
   const int64_t n64 = m.n;
   if (n64 <= 0) throw std::runtime_error("mesh without triangles");
   if (n64 >= ((int64_t)1 << 27)) throw std::runtime_error("mesh too large for the device builder");
@@ -587,12 +1329,15 @@ void build_mesh_device(MeshBuild &m, DevMeshBuffers &out, DevBuildTiming *timing
   CKB(cudaGetLastError());
   m.dead.resize(n);
   m.order.resize(n);
-  std::vector<uint8_t> dead_pos(n);
-  std::vector<uint32_t> idx_host(n);
+  std::vector<uint8_t> dead_pos;
+  std::vector<uint32_t> idx_host;
   CKB(cudaMemcpyAsync(m.dead.data(), d_dead.p, n, cudaMemcpyDeviceToHost, stream));
   CKB(cudaMemcpyAsync(m.order.data(), d_order.p, (size_t)n * 4, cudaMemcpyDeviceToHost, stream));
-  CKB(cudaMemcpyAsync(dead_pos.data(), d_dead_pos.p, n, cudaMemcpyDeviceToHost, stream));
-  CKB(cudaMemcpyAsync(idx_host.data(), d_idx[cur].p, (size_t)n * 4, cudaMemcpyDeviceToHost, stream));
+  if (mode == DevBuildMode::Median) {  // the host derives the median tree's structure from them
+    dead_pos.resize(n), idx_host.resize(n);
+    CKB(cudaMemcpyAsync(dead_pos.data(), d_dead_pos.p, n, cudaMemcpyDeviceToHost, stream));
+    CKB(cudaMemcpyAsync(idx_host.data(), d_idx[cur].p, (size_t)n * 4, cudaMemcpyDeviceToHost, stream));
+  }
   CKB(cudaStreamSynchronize(stream));
   {
     int64_t nodes = 0, leaves = 0;
@@ -602,7 +1347,7 @@ void build_mesh_device(MeshBuild &m, DevMeshBuffers &out, DevBuildTiming *timing
     m.ref_nodes = nodes, m.ref_leaves = leaves, m.ref_depth = depth;
   }
   const auto t2 = now();
-  if (ref_only) {  // the caller builds the traversal tree itself (host SAH + collapse) from this dead mask and order
+  if (mode == DevBuildMode::RefOnly) {  // the caller builds the traversal tree itself (host SAH + collapse) from this dead mask and order
     m.ref_done = true;
     if (timing) {
       timing->upload_ms = ms_between(t0, t1), timing->ref_ms = ms_between(t1, t2), timing->total_ms = ms_between(t0, t2);
@@ -611,16 +1356,20 @@ void build_mesh_device(MeshBuild &m, DevMeshBuffers &out, DevBuildTiming *timing
     return;
   }
 
-  // ---- step 2: structure on the host (live ranks only), boxes + nodes + triangle records on the device
-  std::vector<uint32_t> R((size_t)n + 1);
-  std::vector<uint32_t> live_tri;
-  live_tri.reserve(n);
-  R[0] = 0;
-  for (uint32_t p = 0; p < n; p++) {
-    R[p + 1] = R[p] + (dead_pos[p] ? 0u : 1u);
-    if (!dead_pos[p]) live_tri.push_back(idx_host[p]);
+  // ---- step 2
+  std::vector<uint32_t> R, live_tri;
+  if (mode == DevBuildMode::Median) {  // structure on the host (live ranks only), boxes + nodes + triangle records on the device
+    R.resize((size_t)n + 1);
+    live_tri.reserve(n);
+    R[0] = 0;
+    for (uint32_t p = 0; p < n; p++) {
+      R[p + 1] = R[p] + (dead_pos[p] ? 0u : 1u);
+      if (!dead_pos[p]) live_tri.push_back(idx_host[p]);
+    }
+    m.live = (int64_t)R[n];
+  } else {
+    m.live = (int64_t)std::count(m.dead.begin(), m.dead.end(), (uint8_t)0);
   }
-  m.live = (int64_t)R[n];
   Buf<float4> d_normals(n);
   k_normals<<<blocks_for(n), kThreads, 0, stream>>>(d_tris.p, d_order.p, n, d_normals.p);
   CKB(cudaGetLastError());
@@ -649,68 +1398,42 @@ void build_mesh_device(MeshBuild &m, DevMeshBuffers &out, DevBuildTiming *timing
     m.built = true;
     return;
   }
-  const Structure st = gen_structure(n, R);
-  const uint32_t n_nodes = (uint32_t)st.nodes.size(), n_levels = (uint32_t)st.level_first.size() - 1;
-  const auto t3 = now();
-  uint32_t widest = 0;
-  for (uint32_t l = 0; l < n_levels; l++) widest = std::max(widest, st.level_first[l + 1] - st.level_first[l]);
-  size_t scan_bytes = 0;
-  CKB(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, (uint32_t *)nullptr, (uint32_t *)nullptr, (int)widest, stream));
-  Arena a2(Arena::need(n_nodes, sizeof(WNode)) + Arena::need(live_tri.size(), 4) + Arena::need(st.quads.size(), 4) + Arena::need(n_nodes, sizeof(Box)) +
-           4 * Arena::need(widest, 4) + Arena::need(scan_bytes, 1) + 8192);
-  struct PW {
-    WNode *p;
-  } d_wn{a2.get<WNode>(n_nodes)};
-  PU d_live{a2.get<uint32_t>(live_tri.size())};
-  CKB(cudaMemcpyAsync(d_wn.p, st.nodes.data(), (size_t)n_nodes * sizeof(WNode), cudaMemcpyHostToDevice, stream));
-  CKB(cudaMemcpyAsync(d_live.p, live_tri.data(), live_tri.size() * 4, cudaMemcpyHostToDevice, stream));
-  if (!st.quads.empty()) {
-    PU d_quads{a2.get<uint32_t>(st.quads.size())};
-    CKB(cudaMemcpyAsync(d_quads.p, st.quads.data(), st.quads.size() * 4, cudaMemcpyHostToDevice, stream));
-    k_pair_quads<<<blocks_for(st.quads.size()), kThreads, 0, stream>>>(d_quads.p, (uint32_t)st.quads.size(), d_live.p, d_tris.p);
-    CKB(cudaGetLastError());
+  uint32_t n_nodes = 0, n_tri_records = 0;
+  Buf<float4> d_nodes, d_tri48;
+  auto t3 = now();
+  if (mode == DevBuildMode::Median) {
+    const Structure st = gen_structure(n, R);
+    n_nodes = (uint32_t)st.nodes.size(), n_tri_records = st.n_tri_records;
+    t3 = now();
+    Arena a2(Arena::need(n_nodes, sizeof(WNode)) + Arena::need(live_tri.size(), 4) + Arena::need(st.quads.size(), 4) + emit_need(st.level_first) + 8192);
+    struct PW {
+      WNode *p;
+    } d_wn{a2.get<WNode>(n_nodes)};
+    PU d_live{a2.get<uint32_t>(live_tri.size())};
+    CKB(cudaMemcpyAsync(d_wn.p, st.nodes.data(), (size_t)n_nodes * sizeof(WNode), cudaMemcpyHostToDevice, stream));
+    CKB(cudaMemcpyAsync(d_live.p, live_tri.data(), live_tri.size() * 4, cudaMemcpyHostToDevice, stream));
+    if (!st.quads.empty()) {
+      PU d_quads{a2.get<uint32_t>(st.quads.size())};
+      CKB(cudaMemcpyAsync(d_quads.p, st.quads.data(), st.quads.size() * 4, cudaMemcpyHostToDevice, stream));
+      k_pair_quads<<<blocks_for(st.quads.size()), kThreads, 0, stream>>>(d_quads.p, (uint32_t)st.quads.size(), d_live.p, d_tris.p);
+      CKB(cudaGetLastError());
+    }
+    emit_wide(a2, stream, d_wn.p, d_live.p, st.level_first, n_tri_records, d_tris.p, d_order.p, d_nodes, d_tri48, m);
+  } else {
+    SahTree sah = build_sah(n, (uint32_t)m.live, d_dead.p, d_tbox.p, stream);
+    n_nodes = sah.level_first.back(), n_tri_records = (uint32_t)m.live;
+    t3 = now();
+    emit_wide(*sah.wide, stream, sah.wn, sah.live, sah.level_first, n_tri_records, d_tris.p, d_order.p, d_nodes, d_tri48, m);
+    if (timing) {
+      timing->sah_ms = sah.sah_ms, timing->plan_ms = sah.plan_ms, timing->sah_levels = sah.sah_levels;
+      timing->structure_ms = sah.structure_ms;
+    }
   }
-  struct PX {
-    Box *p;
-  } d_box{a2.get<Box>(n_nodes)};
-  Buf<float4> d_nodes((size_t)n_nodes * 5), d_tri48((size_t)std::max(st.n_tri_records, 1u) * 3);
-  struct PF {
-    float *p;
-  } d_root{a2.get<float>(6)};
-  struct PE {
-    int *p;
-  } d_err{a2.get<int>(1)};
-  CKB(cudaMemsetAsync(d_err.p, 0, sizeof(int), stream));
-  for (uint32_t l = n_levels; l-- > 0;) {
-    const uint32_t first = st.level_first[l], count = st.level_first[l + 1] - first;
-    k_boxes_level<<<blocks_for(count), kThreads, 0, stream>>>(d_wn.p, first, count, d_live.p, d_tris.p, d_box.p);
-  }
-  CKB(cudaGetLastError());
-  PU d_sid[2] = {{a2.get<uint32_t>(widest)}, {a2.get<uint32_t>(widest)}}, d_cnt{a2.get<uint32_t>(widest)}, d_cbase{a2.get<uint32_t>(widest)};
-  PB d_scan{a2.get<uint8_t>(scan_bytes)};
-  CKB(cudaMemsetAsync(d_sid[0].p, 0, 4, stream));  // level 0: final position 0 holds structural node 0
-  for (uint32_t l = 0; l < n_levels; l++) {
-    const uint32_t first = st.level_first[l], count = st.level_first[l + 1] - first;
-    k_inner_count<<<blocks_for(count), kThreads, 0, stream>>>(d_wn.p, d_sid[l & 1].p, count, d_cnt.p);
-    size_t sb = scan_bytes;
-    CKB(cub::DeviceScan::ExclusiveSum(d_scan.p, sb, d_cnt.p, d_cbase.p, (int)count, stream));
-    k_emit_level<<<blocks_for(count), kThreads, 0, stream>>>(d_wn.p, d_sid[l & 1].p, first, count, d_cbase.p, st.level_first[l + 1], d_sid[(l + 1) & 1].p,
-                                                        d_live.p, d_tris.p, d_order.p, d_box.p, d_nodes.p, d_tri48.p, d_root.p, d_err.p);
-    CKB(cudaGetLastError());
-  }
-  int err = 0;
-  float root[6];
-  CKB(cudaMemcpyAsync(&err, d_err.p, sizeof(int), cudaMemcpyDeviceToHost, stream));
-  CKB(cudaMemcpyAsync(root, d_root.p, sizeof(root), cudaMemcpyDeviceToHost, stream));
-  CKB(cudaStreamSynchronize(stream));
-  if (err) throw std::runtime_error("mesh extent too large for the quantised BVH frame");
-  for (int a = 0; a < 3; a++) m.root_lo[a] = root[a], m.root_hi[a] = root[3 + a];
-  m.wide_depth = (int32_t)n_levels - 1;
   const auto t4 = now();
 
   // ---- host copies (ptc_scene_mesh_info, replicas of ptc_multi_create)
   m.nodes.resize(n_nodes);
-  m.tri48.resize(std::max(st.n_tri_records, 1u));
+  m.tri48.resize(std::max(n_tri_records, 1u));
   m.normals.resize(n);
   CKB(cudaMemcpyAsync(m.nodes.data(), d_nodes.p, (size_t)n_nodes * 80, cudaMemcpyDeviceToHost, stream));
   CKB(cudaMemcpyAsync(m.tri48.data(), d_tri48.p, m.tri48.size() * 48, cudaMemcpyDeviceToHost, stream));
@@ -720,8 +1443,9 @@ void build_mesh_device(MeshBuild &m, DevMeshBuffers &out, DevBuildTiming *timing
   m.built = true;
   const auto t5 = now();
   if (timing) {
-    timing->upload_ms = ms_between(t0, t1), timing->ref_ms = ms_between(t1, t2), timing->structure_ms = ms_between(t2, t3);
-    timing->emit_ms = ms_between(t3, t4), timing->download_ms = ms_between(t4, t5), timing->total_ms = ms_between(t0, t5);
+    timing->upload_ms = ms_between(t0, t1), timing->ref_ms = ms_between(t1, t2), timing->emit_ms = ms_between(t3, t4);
+    if (mode == DevBuildMode::Median) timing->structure_ms = ms_between(t2, t3);
+    timing->download_ms = ms_between(t4, t5), timing->total_ms = ms_between(t0, t5);
     timing->ref_levels = sort_levels + 1;
   }
 }

@@ -815,6 +815,8 @@ int ptc_scene_commit_ex(ptc_scene *s, int device, int flags) {
   PTC_GUARD_BEGIN
   if (!s) throw std::invalid_argument("null argument");
   if (s->committed) throw std::logic_error("scene already committed");
+  if ((flags & PTC_COMMIT_FAST_BUILD) && (flags & PTC_COMMIT_DEVICE_SAH))
+    throw std::invalid_argument("PTC_COMMIT_FAST_BUILD and PTC_COMMIT_DEVICE_SAH exclude each other");
   int n = 0;
   if (cudaGetDeviceCount(&n) != cudaSuccess || n == 0) {
     cudaGetLastError();
@@ -825,26 +827,31 @@ int ptc_scene_commit_ex(ptc_scene *s, int device, int flags) {
   // large meshes: 10-30 ms instead of ~400 ms for 2 M triangles.  The traversal tree then comes from the host's SAH +
   // dynamic-programming collapse by default — the better tree: C5 renders 22 % faster through it than through the
   // device-built one — or, with PTC_COMMIT_FAST_BUILD / PTC_BUILD=device, from the device too (the reference tree itself,
-  // re-used as the wide tree: the whole commit of 2 M triangles in ~0.2 s).  PTC_BUILD=host keeps everything on the host;
+  // re-used as the wide tree: the whole commit of 2 M triangles in ~0.2 s).  PTC_COMMIT_DEVICE_SAH / PTC_BUILD=device-sah
+  // builds the host's SAH tree on the device, for meshes of every size.  PTC_BUILD=host keeps everything on the host;
   // a non-default tie order (PTC_REF_TIE, a measurement switch) exists on the host only.
   {
     const char *mode = getenv("PTC_BUILD"), *tie = getenv("PTC_REF_TIE");
     const bool tie_default = !tie || !*tie || !strcmp(tie, "stable");
     const bool force_host = mode && !strcmp(mode, "host");
-    const bool fast = (mode && !strcmp(mode, "device")) || (flags & PTC_COMMIT_FAST_BUILD) != 0;
+    const bool sah = (mode && !strcmp(mode, "device-sah")) || (flags & PTC_COMMIT_DEVICE_SAH) != 0;
+    const bool fast = !sah && ((mode && !strcmp(mode, "device")) || (flags & PTC_COMMIT_FAST_BUILD) != 0);
+    const DevBuildMode dev_mode = sah ? DevBuildMode::Sah : (fast ? DevBuildMode::Median : DevBuildMode::RefOnly);
     s->dev_built.assign(s->hs.meshes.size(), DevMeshBuffers());
     for (size_t mi = 0; mi < s->hs.meshes.size(); mi++) {
       MeshBuild &mb = *s->hs.meshes[mi];
       if (mb.built || force_host || !tie_default || mb.n >= ((int64_t)1 << 27)) continue;  // (the device builder's index width)
-      if (!fast && mb.n < kDeviceRefMinTriangles) continue;
+      if (dev_mode == DevBuildMode::RefOnly && mb.n < kDeviceRefMinTriangles) continue;
       CK(cudaSetDevice(device));
       DevBuildTiming tm;
-      build_mesh_device(mb, s->dev_built[mi], &tm, /*ref_only=*/!fast);
+      build_mesh_device(mb, s->dev_built[mi], &tm, dev_mode);
       if (getenv("PTC_BUILD_TIMING"))
-        fprintf(stderr, "[pt_build_dev] %lld triangles (%lld live)%s: upload %.1f ms, reference-BVH restatement %.1f ms (%d levels), structure %.1f ms, "
+        fprintf(stderr, "[pt_build_dev] %lld triangles (%lld live)%s: upload %.1f ms, reference-BVH restatement %.1f ms (%d levels), "
+                        "binned SAH %.1f ms (%d levels), collapse plan %.1f ms, structure %.1f ms, "
                         "boxes + nodes + triangle records %.1f ms, download %.1f ms, total %.1f ms; %zu wide nodes, depth %d\n",
-                (long long)mb.n, (long long)mb.live, fast ? "" : " [step 1 only]", tm.upload_ms, tm.ref_ms, tm.ref_levels, tm.structure_ms, tm.emit_ms,
-                tm.download_ms, tm.total_ms, mb.nodes.size(), mb.wide_depth);
+                (long long)mb.n, (long long)mb.live, dev_mode == DevBuildMode::RefOnly ? " [step 1 only]" : (sah ? " [SAH]" : ""), tm.upload_ms,
+                tm.ref_ms, tm.ref_levels, tm.sah_ms, tm.sah_levels, tm.plan_ms, tm.structure_ms, tm.emit_ms, tm.download_ms, tm.total_ms,
+                mb.nodes.size(), mb.wide_depth);
     }
   }
   const auto t_host = std::chrono::steady_clock::now();

@@ -8,6 +8,10 @@ pub const PTC_E_CUDA: c_int = -2;
 pub const PTC_E_NOMEM: c_int = -3;
 pub const PTC_E_STATE: c_int = -4;
 
+/// ptc_scene_commit_ex flags
+pub const PTC_COMMIT_FAST_BUILD: c_int = 1;
+pub const PTC_COMMIT_DEVICE_SAH: c_int = 2;
+
 pub const PTC_MAT_LAMBERT: i32 = 0;
 pub const PTC_MAT_LAMBERT_CHECKER: i32 = 1;
 pub const PTC_MAT_METAL: i32 = 2;
@@ -104,7 +108,8 @@ extern "C" {
     pub fn ptc_scene_build(s: *mut ptc_scene) -> c_int;
     pub fn ptc_scene_last_pool_slots(s: *const ptc_scene) -> i64;
     pub fn ptc_scene_commit(s: *mut ptc_scene, device: c_int) -> c_int;
-    /// flags: PTC_COMMIT_FAST_BUILD = 1 (flatten meshes entirely on the device: quick commit, slower traversal)
+    /// flags: PTC_COMMIT_FAST_BUILD (flatten meshes entirely on the device: quick commit, slower traversal) or
+    /// PTC_COMMIT_DEVICE_SAH (flatten them on the device into the default SAH tree: quick commit, same traversal)
     pub fn ptc_scene_commit_ex(s: *mut ptc_scene, device: c_int, flags: c_int) -> c_int;
     pub fn ptc_render(s: *mut ptc_scene, cam: *const ptc_camera, st: *const ptc_render_settings, out_rgb: *mut f32,
                       stats: *mut ptc_stats) -> c_int;

@@ -1,7 +1,10 @@
 #!/usr/bin/env python3
-"""Commit time and traversal quality of the two mesh builders on one B200: host (SAH + DP collapse) against device
-(reference tree as the wide tree), for C5 (2 M triangles), C3 (teapot) and C2's text mesh.  PTC_BUILD_TIMING=1 prints the
-builders' own step times on stderr.  One JSON line per (config, builder)."""
+"""Commit time and traversal quality of the mesh builders on one B200: host (SAH + DP collapse), device (reference tree
+as the wide tree), device-sah (the host's SAH tree built on the device) and hybrid (the default commit), for C5
+(2 M triangles), C3 (teapot) and C2's text mesh.  PTC_BUILD_TIMING=1 prints the builders' own step times on stderr.  One
+JSON line per (config, builder) plus one naming the GPU and its power limit.
+
+  python tools/build_probe.py [config ...] [--modes host,device,device-sah,hybrid]"""
 import json
 import os
 import sys
@@ -15,12 +18,25 @@ pt = ptload.load()
 from raytracer_rust_b200 import workloads  # noqa: E402
 
 os.environ["PTC_BUILD_TIMING"] = "1"
+args = sys.argv[1:]
+modes = ("host", "device", "device")
+if "--modes" in args:
+    i = args.index("--modes")
+    modes = tuple(args[i + 1].split(","))
+    del args[i:i + 2]
+import torch  # noqa: E402
+import subprocess  # noqa: E402
+smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True, text=True).stdout.strip()
+print(json.dumps({"gpu": torch.cuda.get_device_name(0), "nvidia_smi": smi}), flush=True)
 pt.synthetic_scene(cells=32).to_core().commit(0)  # context + module load outside the timings
-for cfg in sys.argv[1:] or ["C5", "C3", "C2"]:
+for cfg in args or ["C5", "C3", "C2"]:
     label, scene = workloads.workload(cfg)
     w, h, spp, depth = scene.settings
-    for mode in ("host", "device", "device"):
-        os.environ["PTC_BUILD"] = mode
+    for mode in modes:
+        if mode == "hybrid":
+            os.environ.pop("PTC_BUILD", None)
+        else:
+            os.environ["PTC_BUILD"] = mode
         t0 = time.perf_counter()
         cs = scene.to_core().commit(0)
         commit_s = time.perf_counter() - t0

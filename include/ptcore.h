@@ -85,12 +85,17 @@ typedef struct ptc_render_settings {
 enum {
   PTC_FLAG_COUNTERS = 1, /* run the instrumented extend kernel: fills nodes_visited / tris_tested (slower) */
   PTC_FLAG_TIMING = 2,   /* record CUDA events around every extend / shade launch: fills extend_ms / shade_ms */
-  PTC_FLAG_NEE = 4       /* next-event estimation + multiple importance sampling (SURVEY.md 8f-4; the Tungsten scenes ask for
+  PTC_FLAG_NEE = 4,      /* next-event estimation + multiple importance sampling (SURVEY.md 8f-4; the Tungsten scenes ask for
                             it with "enable_mis", which the reference's IntegratorConfig ignores, src/tungsten/parser.rs:167-171).
                             OFF by default: the default integrator is the reference's, sample for sample.  With the flag every
                             non-specular hit also samples one emissive sphere / quad through a shadow ray, and emitters found
                             by BSDF sampling are weighted with the power heuristic.  Same expected image, far less noise where
                             emitters are small (veach-mis).  stats.rays then counts the shadow rays too. */
+  PTC_FLAG_NEE_SKY = 8   /* with PTC_FLAG_NEE only (alone: PTC_E_INVALID): NEE also samples the HDR sky as an environment light,
+                            importance-sampled by its radiance over the cells of the reference's equirectangular lookup, with
+                            the power heuristic against BSDF sampling (the Tungsten scenes' "enable_light_sampling").  Same
+                            expected image, less noise under a sky with bright spots (the teapot's envmap).  On a scene
+                            without an HDR sky, or with an all-zero one, it changes nothing: the image is PTC_FLAG_NEE's. */
 };
 
 /* HitRecord (src/hittable.rs:10-16) plus the ids the parity bar is stated on. */
@@ -224,6 +229,11 @@ int ptc_primary_rays(ptc_scene *, const ptc_camera *, const ptc_render_settings 
 int ptc_scatter(ptc_scene *, int material, const float *ray_dirs, const float *positions, const float *normals,
                 const int32_t *front_face, const float *u4, int64_t n, int32_t *scattered, float *out_origin,
                 float *out_dir, float *attenuation, float *emitted);
+/* The HDR sky as a light (PTC_FLAG_NEE_SKY): n directions drawn from u4 (n x 4 uniforms in [0, 1)), their solid-angle
+ * pdf and the sky's radiance along them (out_dir / out_rgb n x 3 floats, out_pdf n floats); and the pdf of n directions.
+ * PTC_E_STATE when the committed scene has no sky distribution (no HDR sky, or an all-zero one). */
+int ptc_sky_sample(ptc_scene *, const float *u4, int64_t n, float *out_dir, float *out_pdf, float *out_rgb);
+int ptc_sky_pdf(ptc_scene *, const float *dirs, int64_t n, float *out_pdf);
 /* Philox4x32-10 known-answer hook (runs on the device). */
 int ptc_philox(ptc_scene *, const uint32_t ctr[4], const uint32_t key[2], uint32_t out[4]);
 

@@ -21,7 +21,7 @@ REPO_ROOT = os.path.dirname(_HERE)
 PTC_OK, PTC_E_INVALID, PTC_E_CUDA, PTC_E_NOMEM, PTC_E_STATE = 0, -1, -2, -3, -4
 MAT_LAMBERT, MAT_LAMBERT_CHECKER, MAT_METAL, MAT_DIELECTRIC, MAT_EMISSIVE, MAT_PLASTIC, MAT_ROUGH_CONDUCTOR, MAT_NULL = range(8)
 DIST_GGX, DIST_BECKMANN = 0, 1
-FLAG_COUNTERS, FLAG_TIMING, FLAG_NEE = 1, 2, 4
+FLAG_COUNTERS, FLAG_TIMING, FLAG_NEE, FLAG_NEE_SKY = 1, 2, 4, 8
 COMMIT_FAST_BUILD = 1
 COMMIT_DEVICE_SAH = 2
 LOAD_INFINITE_SPHERE_SKY, LOAD_WO3_STRIDE16, LOAD_SKIP_UNKNOWN = 1, 2, 4
@@ -152,6 +152,8 @@ def core():
     L.ptc_primary_rays.argtypes = [_vp, C.POINTER(Camera), C.POINTER(RenderSettings), C.c_int32, _F, _F]
     L.ptc_scatter.argtypes = [_vp, C.c_int, _F, _F, _F, _vp, _F, C.c_int64, _vp, _F, _F, _F, _F]
     L.ptc_philox.argtypes = [_vp, _vp, _vp, _vp]
+    L.ptc_sky_sample.argtypes = [_vp, _F, C.c_int64, _F, _F, _F]
+    L.ptc_sky_pdf.argtypes = [_vp, _F, C.c_int64, _F]
     L.ptc_multi_create.argtypes = [_vp, C.POINTER(C.c_int), C.c_int, C.POINTER(_vp)]
     L.ptc_multi_destroy.argtypes = [_vp]
     L.ptc_multi_destroy.restype = None
@@ -574,6 +576,22 @@ class CoreScene:
         _ck(core().ptc_scatter(self._h, material, _fptr(d), _fptr(p), _fptr(nn), ff.ctypes.data, _fptr(u), n, sc.ctypes.data,
                                _fptr(oo), _fptr(od), _fptr(att), _fptr(em)))
         return sc, oo, od, att, em
+
+    def sky_sample(self, u4):
+        """The HDR sky as a light (FLAG_NEE_SKY): u4 = n x 4 uniforms in [0, 1) -> (directions n x 3, solid-angle pdf n,
+        sky radiance along them n x 3), by the shade stage's own device functions."""
+        u = _f32(u4, (-1, 4))
+        n = len(u)
+        d, pdf, rgb = np.empty((n, 3), np.float32), np.empty(n, np.float32), np.empty((n, 3), np.float32)
+        _ck(core().ptc_sky_sample(self._h, _fptr(u), n, _fptr(d), _fptr(pdf), _fptr(rgb)))
+        return d, pdf, rgb
+
+    def sky_pdf(self, dirs):
+        """Solid-angle pdf with which FLAG_NEE_SKY samples each direction of dirs (n x 3)."""
+        d = _f32(dirs, (-1, 3))
+        pdf = np.empty(len(d), np.float32)
+        _ck(core().ptc_sky_pdf(self._h, _fptr(d), len(d), _fptr(pdf)))
+        return pdf
 
     def philox(self, ctr, key):
         c = np.asarray(ctr, np.uint32)

@@ -352,21 +352,70 @@ PT_HD uint32_t f32_as_u32_sat(float f) {  // Rust `as u32`
   if (f >= 4294967296.0f) return 0xffffffffu;
   return (uint32_t)f;
 }
+// the texel of the HDR sky a direction looks up (renderer.rs:40-54); shared by sky_color and the sky light's pdf
+PT_HD void sky_texel(const DScene &sc, V3 ray_d, uint32_t &xp, uint32_t &yp) {
+  const V3 dir = normalized(ray_d);
+  const float theta = acosf(dir.y);
+  const float phi = atan2f(dir.z, dir.x) + kPi;
+  const float u = phi / (2.0f * kPi);
+  const float v = theta / kPi;
+  xp = f32_as_u32_sat(fmaxf(u * (float)(sc.sky_w - 1), 0.0f));
+  yp = f32_as_u32_sat(fmaxf(v * (float)(sc.sky_h - 1), 0.0f));
+  if (xp > (uint32_t)(sc.sky_w - 1)) xp = (uint32_t)(sc.sky_w - 1);
+  if (yp > (uint32_t)(sc.sky_h - 1)) yp = (uint32_t)(sc.sky_h - 1);
+}
 PT_HD V3 sky_color(const DScene &sc, V3 ray_d) {
   if (sc.sky != nullptr) {
-    const V3 dir = normalized(ray_d);
-    const float theta = acosf(dir.y);
-    const float phi = atan2f(dir.z, dir.x) + kPi;
-    const float u = phi / (2.0f * kPi);
-    const float v = theta / kPi;
-    uint32_t xp = f32_as_u32_sat(fmaxf(u * (float)(sc.sky_w - 1), 0.0f));
-    uint32_t yp = f32_as_u32_sat(fmaxf(v * (float)(sc.sky_h - 1), 0.0f));
-    if (xp > (uint32_t)(sc.sky_w - 1)) xp = (uint32_t)(sc.sky_w - 1);
-    if (yp > (uint32_t)(sc.sky_h - 1)) yp = (uint32_t)(sc.sky_h - 1);
+    uint32_t xp, yp;
+    sky_texel(sc, ray_d, xp, yp);
     const float *px = sc.sky + ((size_t)yp * sc.sky_w + xp) * 3;
     return v3(px[0], px[1], px[2]);
   }
   return v3(0.5f, 0.5f, 0.5f);  // Color::GRAY
+}
+
+// The HDR sky as a light (PTC_FLAG_NEE_SKY; layout and cell mapping: pt_types.h, SkyDist).  Needs sc.sky_dist != nullptr.
+// P(cell) is a product of differences of the stored CDF entries the sampler searches, so sampler and pdf agree.
+PT_HD float sky_cell_prob(const SkyDist &d, uint32_t x, uint32_t y) {
+  const float *row = d.cond + (size_t)y * (uint32_t)(d.wc + 1);
+  return (d.marg[y + 1] - d.marg[y]) * (row[x + 1] - row[x]);
+}
+// solid-angle density of direction ray_d (0 in the last texel column / row, which the lookup reaches on a null set only)
+PT_HD float sky_pdf(const DScene &sc, V3 ray_d) {
+  const SkyDist d = sky_dist_view(sc.sky_dist, sc.sky_w, sc.sky_h);
+  uint32_t x, y;
+  sky_texel(sc, ray_d, x, y);
+  if (x >= (uint32_t)d.wc || y >= (uint32_t)d.hc) return 0.0f;
+  return sky_cell_prob(d, x, y) * d.inv_sa[y];
+}
+// first i in [0, n) with cdf[i + 1] > u, for cdf[0] = 0 <= u < cdf[n] = 1: never an interval of width 0
+PT_HD uint32_t cdf_search(const float *cdf, uint32_t n, float u) {
+  uint32_t lo = 0, hi = n - 1;
+  while (lo < hi) {
+    const uint32_t mid = (lo + hi) >> 1;
+    if (cdf[mid + 1] > u) hi = mid;
+    else lo = mid + 1;
+  }
+  return lo;
+}
+// a direction with density sky_pdf from four uniforms: row, column, then uniform in phi and cos(theta) inside the cell
+// (uniform in solid angle), mapped back through the lookup's angles: atan2(z, x) = phi - pi, y = cos(theta)
+PT_HD V3 sky_sample(const DScene &sc, const float *u4, float &pdf) {
+  const SkyDist d = sky_dist_view(sc.sky_dist, sc.sky_w, sc.sky_h);
+  const uint32_t y = cdf_search(d.marg, (uint32_t)d.hc, u4[0]);
+  const uint32_t x = cdf_search(d.cond + (size_t)y * (uint32_t)(d.wc + 1), (uint32_t)d.wc, u4[1]);
+  pdf = sky_cell_prob(d, x, y) * d.inv_sa[y];
+  const float ct = d.cos[y] + u4[3] * (d.cos[y + 1] - d.cos[y]);
+  const float st = sqrtf(fmaxf(0.0f, 1.0f - ct * ct));
+  const float a = (2.0f * kPi) * (((float)x + u4[2]) / (float)d.wc) - kPi;
+  float s, c;
+#if defined(__CUDA_ARCH__)
+  sincosf(a, &s, &c);
+#else
+  s = sinf(a);
+  c = cosf(a);
+#endif
+  return v3(st * c, ct, st * s);
 }
 
 // Camera::get_ray (src/camera.rs:33-42)

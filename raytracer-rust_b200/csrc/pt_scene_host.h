@@ -1,6 +1,7 @@
 // pt_scene_host.h — host-side scene under construction: what the add_* calls of include/ptcore.h collect before
 // ptc_scene_commit flattens it (object table in Scene.object_list order, material table, one MeshBuild per Mesh).
 #pragma once
+#include <algorithm>
 #include <cmath>
 #include <cstring>
 #include <memory>
@@ -32,6 +33,7 @@ struct HostScene {
   std::vector<float> sky;
   int32_t sky_w = 0, sky_h = 0;
   std::vector<DLight> lights;  // filled by build_all
+  std::vector<float> sky_dist;  // filled by build_all: SkyDist of the sky, or empty
 
   int add_material(const ptc_material *m) {
     if (m->type < PTC_MAT_LAMBERT || m->type > PTC_MAT_NULL) throw std::invalid_argument("unknown material type");
@@ -146,6 +148,51 @@ struct HostScene {
       }
       o.hit_bits = (m.type << 26) | (light_id << 20) | o.material;
     }
+    build_sky_dist();
+  }
+  // the sky as a light (PTC_FLAG_NEE_SKY, layout in pt_types.h: SkyDist): cell weight = max(r, g, b) x solid angle, summed
+  // in double in a fixed order; left empty without a sky or when every weight is 0
+  void build_sky_dist() {
+    sky_dist.clear();
+    if (sky.empty()) return;
+    const int32_t wc = sky_cells(sky_w), hc = sky_cells(sky_h);
+    std::vector<float> d(sky_dist_size(sky_w, sky_h));
+    const SkyDist v = sky_dist_view(d.data(), sky_w, sky_h);
+    float *marg = d.data(), *cosv = marg + (v.cos - v.marg), *inv_sa = marg + (v.inv_sa - v.marg), *cond = marg + (v.cond - v.marg);
+    const double pi = 3.14159265358979323846;
+    std::vector<double> row_w((size_t)hc), cum((size_t)wc + 1);
+    double total = 0.0;
+    for (int32_t y = 0; y < hc; y++) {
+      const double c0 = std::cos(pi * y / hc), c1 = std::cos(pi * (y + 1) / hc);
+      const double sa = 2.0 * pi / wc * (c0 - c1);
+      cosv[y] = (float)c0;
+      inv_sa[y] = (float)(1.0 / sa);
+      cum[0] = 0.0;
+      for (int32_t x = 0; x < wc; x++) {
+        const float *px = sky.data() + ((size_t)y * sky_w + x) * 3;
+        double wgt = 0.0;
+        if (!std::isnan(px[0]) && !std::isnan(px[1]) && !std::isnan(px[2])) {
+          wgt = (double)std::max(px[0], std::max(px[1], px[2])) * sa;
+          if (!std::isfinite(wgt) || wgt < 0.0) wgt = 0.0;
+        }
+        cum[(size_t)x + 1] = cum[(size_t)x] + wgt;
+      }
+      const double rw = cum[(size_t)wc];
+      float *row = cond + (size_t)y * (size_t)(wc + 1);
+      for (int32_t x = 0; x < wc; x++) row[x] = rw > 0.0 ? (float)(cum[(size_t)x] / rw) : (float)x / (float)wc;
+      row[wc] = 1.0f;
+      row_w[(size_t)y] = rw;
+      total += rw;
+    }
+    cosv[hc] = -1.0f;
+    if (!(total > 0.0) || !std::isfinite(total)) return;
+    double c = 0.0;
+    for (int32_t y = 0; y < hc; y++) {
+      marg[y] = (float)(c / total);
+      c += row_w[(size_t)y];
+    }
+    marg[hc] = 1.0f;
+    sky_dist = std::move(d);
   }
 };
 

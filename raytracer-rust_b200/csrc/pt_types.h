@@ -84,6 +84,34 @@ struct alignas(16) DLight {
 };
 constexpr int kMaxLights = 63;  // light id 1..63 in the hit record's 6 bits; further emitters are simply not sampled
 
+// The HDR sky as a light (PTC_FLAG_NEE_SKY).  The reference's lookup (pt_bsdf.h: sky_texel) makes a w x h sky piecewise
+// constant over Wc x Hc cells, Wc = max(w - 1, 1), Hc = max(h - 1, 1): cell (x, y) has the radiance of texel (x, y) and
+// covers phi in [2 pi x / Wc, 2 pi (x + 1) / Wc), theta in [pi y / Hc, pi (y + 1) / Hc).  (The last texel column and row
+// are looked up on a set of measure zero only: they have probability 0.)  DScene::sky_dist holds, as floats:
+//   marg   [Hc + 1]         marginal CDF over the rows, 0 ... 1
+//   cos    [Hc + 1]         cos(pi y / Hc): the theta bounds of the rows
+//   inv_sa [Hc]             1 / solid angle of one cell of row y
+//   cond   [Hc][Wc + 1]     conditional CDF over the columns of row y, 0 ... 1
+// Built on the host (HostScene::build_all), from weights max(r, g, b) x solid angle summed in double.
+struct SkyDist {
+  const float *marg, *cos, *inv_sa, *cond;
+  int32_t wc, hc;
+};
+PT_HD int32_t sky_cells(int32_t texels) { return texels > 1 ? texels - 1 : 1; }
+PT_HD size_t sky_dist_size(int32_t w, int32_t h) {
+  const size_t wc = (size_t)sky_cells(w), hc = (size_t)sky_cells(h);
+  return 3 * hc + 2 + hc * (wc + 1);
+}
+PT_HD SkyDist sky_dist_view(const float *p, int32_t w, int32_t h) {
+  SkyDist d;
+  d.wc = sky_cells(w), d.hc = sky_cells(h);
+  d.marg = p;
+  d.cos = p + d.hc + 1;
+  d.inv_sa = p + 2 * d.hc + 2;
+  d.cond = p + 3 * d.hc + 2;
+  return d;
+}
+
 struct DScene {
   const DObject *objects;
   const DMaterial *materials;
@@ -93,6 +121,11 @@ struct DScene {
   int32_t n_objects, n_materials, n_meshes;
   int32_t sky_w, sky_h;
   int32_t n_lights;
+  // PTC_FLAG_NEE_SKY: the sky as a light (pt_bsdf.h: sky_sample / sky_pdf); nullptr without a sky or with an all-zero one.
+  // sky_dist_size(sky_w, sky_h) floats, see SkyDist.  (Last, and padded to 16 bytes: the kernels' other parameters keep
+  // their offsets modulo 16, hence their 128-bit constant loads.)
+  const float *sky_dist;
+  int32_t pad[2];
 };
 
 // HitRecord (src/hittable.rs:10-16) + the ids the parity bar is stated on.

@@ -518,11 +518,16 @@ __device__ __forceinline__ uint32_t block_rank(bool flag, uint32_t *s_warp /* [k
 // weighted with the power heuristic against the light pdf of that point (the sampling pdf travels with the ray in `aux`).
 // The path count of a segment is capped at cap / 2 so that paths + their shadow rays always fit.  The estimator's
 // expectation is the plain integrator's (tested): same image, less variance where the lights are small.
+// Mode 2 (PTC_FLAG_NEE_SKY, the scene has a sky distribution): NEE also samples the HDR sky as an environment light.  The
+// sky is chosen with probability p_sky = 0.5 when there are analytic lights (1 otherwise; each light then has (1 - p_sky) /
+// n_lights), its direction is drawn from the sky's own distribution (pt_bsdf.h: sky_sample, Philox block 2) and the
+// shadow ray has an infinite distance: any hit occludes.  A BSDF-sampled ray that misses is weighted with the power
+// heuristic against p_sky * sky_pdf.  Mode 0 = plain, 1 = NEE.
 // Returns the new ray count of the segment.
 // `seg_done` (or nullptr): one word per segment, set when the segment is found empty with the path supply exhausted — it
 // will never hold a ray again — and counted off ctl->n_active, once.
 // (The path state is read with plain loads: launches overlap, see stage_begin, so it is not read-only while a k_shade runs.)
-template <bool NEE>
+template <int Mode>
 __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, uint32_t *seg_done, Ctl *ctl, const DScene &sc, const RenderParams &rp,
                                                 const Buffers &b, const Film &film) {
   __shared__ uint16_t s_perm[kShadeWindow];
@@ -530,6 +535,7 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
   __shared__ uint32_t s_warp[kBlock / 32 + 1];
   __shared__ unsigned long long s_first;
   __shared__ uint32_t s_avail, s_more, s_w, s_wp;
+  constexpr bool NEE = Mode != 0, SKY = Mode == 2;
   const uint32_t n = b.cnt[seg], seg_base = seg * b.cap;
   const uint32_t tid = threadIdx.x, lane = tid & 31u;
   const uint32_t lt_mask = (1u << lane) - 1u;
@@ -605,6 +611,13 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
           if (!(bits & kHitBit) || !(b.hit0[i].w < t_light * (1.0f - 2e-4f))) radiance = beta, add = true;
         } else if (!(bits & kHitBit)) {
           radiance = beta * sky_color(sc, ray_d);
+          if (SKY) {  // power heuristic against the sky's light-sampling pdf (camera rays and delta lobes: weight 1)
+            const float pb = b.aux[i];
+            if (pb >= 0.0f) {
+              const float pe = (sc.n_lights > 0 ? 0.5f : 1.0f) * sky_pdf(sc, ray_d);
+              if (pe > 0.0f) radiance = radiance * (pb * pb / (pb * pb + pe * pe));
+            }
+          }
           add = true;
         } else {
           const float4 h0 = b.hit0[i];
@@ -617,7 +630,8 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
               const float pb = b.aux[i];
               const uint32_t light = (bits >> kLightShift) & 63u;
               if (pb >= 0.0f && light != 0u) {
-                const float pl = light_pdf(sc.lights[light - 1u], h0.w, fabsf(dot(nrm, ray_d))) * (1.0f / (float)sc.n_lights);
+                // selection probability 1 / n_lights, or (1 - p_sky) / n_lights when the sky is sampled too
+                const float pl = light_pdf(sc.lights[light - 1u], h0.w, fabsf(dot(nrm, ray_d))) * ((SKY ? 0.5f : 1.0f) / (float)sc.n_lights);
                 w_mis = pb * pb / (pb * pb + pl * pl);
               }
             }
@@ -638,7 +652,38 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
               if (NEE) {
                 npdf = mat_sampled_pdf(m, ray_d, pos, nrm, u.u, sc_ray.d);
                 // light sampling: what the NEXT segment could find at an emitter (hence the same depth rule as the continuation)
-                if (sc.n_lights > 0) {
+                if (SKY) {
+                  // one emitter: the sky with probability p_sky (own uniforms, Philox block 2; infinitely far, so any hit
+                  // occludes), else a uniformly chosen analytic light with the rest of u[0]
+                  const Uniforms4 ul = philox_uniforms(rp.seed, pixel, sample, bounce, 1u);
+                  const float p_sky = sc.n_lights > 0 ? 0.5f : 1.0f;
+                  const V3 so = pos + nrm * kEps;
+                  V3 wi, fcos, le;
+                  float dist, pl, pb;
+                  bool ok;
+                  if (ul.u[0] < p_sky) {
+                    const Uniforms4 us = philox_uniforms(rp.seed, pixel, sample, bounce, 2u);
+                    wi = sky_sample(sc, us.u, pl);
+                    pl *= p_sky;
+                    dist = INFINITY;
+                    le = sky_color(sc, wi);
+                    ok = pl > 0.0f;
+                  } else {
+                    const uint32_t li = min((uint32_t)((ul.u[0] - p_sky) * 2.0f * (float)sc.n_lights), (uint32_t)sc.n_lights - 1u);
+                    const DLight L = sc.lights[li];
+                    ok = light_sample(L, so, ul.u[1], ul.u[2], wi, dist, pl);
+                    pl *= 0.5f / (float)sc.n_lights;  // (1 - p_sky) / n_lights, as where a BSDF-sampled ray hits the light
+                    le = v3(L.emission[0], L.emission[1], L.emission[2]);
+                  }
+                  if (ok && mat_eval_pdf(m, ray_d, pos, nrm, wi, fcos, pb) && (fcos.x > 0.0f || fcos.y > 0.0f || fcos.z > 0.0f)) {
+                    const float w_mis = pl * pl / (pl * pl + pb * pb);
+                    const V3 c = beta * fcos * le * (w_mis / pl);
+                    shadow = true;
+                    so4 = make_float4(so.x, so.y, so.z, u2f(pixel | kShadowBit));
+                    sd4 = make_float4(wi.x, wi.y, wi.z, dist);
+                    sb4 = make_float4(c.x, c.y, c.z, u2f(bounce + 1u));
+                  }
+                } else if (sc.n_lights > 0) {
                   const Uniforms4 ul = philox_uniforms(rp.seed, pixel, sample, bounce, 1u);
                   const uint32_t li = min((uint32_t)(ul.u[0] * (float)sc.n_lights), (uint32_t)sc.n_lights - 1u);
                   const DLight L = sc.lights[li];
@@ -905,10 +950,10 @@ __global__ void __launch_bounds__(kBlock, kSegPerSM) k_extend_post(Ctl *ctl, Seg
   else stage_post<false>(sr.seg0 + blockIdx.x, sr.n_seg, sc, out, tq, round, t_min, t_max);
   stage_end(sr, sr.seg0 + blockIdx.x);
 }
-template <bool NEE>
+template <int Mode>  // 0 = plain, 1 = PTC_FLAG_NEE, 2 = PTC_FLAG_NEE | PTC_FLAG_NEE_SKY on a scene with a sky distribution
 __global__ void __launch_bounds__(kBlock, kSegPerSM) k_shade(Ctl *ctl, SegRange sr, DScene sc, RenderParams rp, Buffers b, Film film) {
   stage_begin(sr, sr.seg0 + blockIdx.x, ctl);
-  stage_shade<NEE>(sr.seg0 + blockIdx.x, sr.n_seg, sr.flags ? sr.flags + sr.n_seg : nullptr, ctl, sc, rp, b, film);
+  stage_shade<Mode>(sr.seg0 + blockIdx.x, sr.n_seg, sr.flags ? sr.flags + sr.n_seg : nullptr, ctl, sc, rp, b, film);
   stage_end(sr, sr.seg0 + blockIdx.x);
 }
 
@@ -988,6 +1033,23 @@ __global__ void k_scatter(DMaterial m, const float *dirs, const float *pos, cons
   out_d[i * 3] = sr.d.x, out_d[i * 3 + 1] = sr.d.y, out_d[i * 3 + 2] = sr.d.z;
   att_out[i * 3] = att.x, att_out[i * 3 + 1] = att.y, att_out[i * 3 + 2] = att.z;
   emitted[i * 3] = e.x, emitted[i * 3 + 1] = e.y, emitted[i * 3 + 2] = e.z;
+}
+
+// PTC_FLAG_NEE_SKY parity hooks: sky_sample / sky_pdf as the shade stage runs them
+__global__ void k_sky_sample(DScene sc, const float *u4, size_t n, float *dirs, float *pdf, float *rgb) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const float u[4] = {u4[i * 4], u4[i * 4 + 1], u4[i * 4 + 2], u4[i * 4 + 3]};
+  float p;
+  const V3 d = sky_sample(sc, u, p);
+  const V3 c = sky_color(sc, d);
+  dirs[i * 3] = d.x, dirs[i * 3 + 1] = d.y, dirs[i * 3 + 2] = d.z;
+  pdf[i] = p;
+  rgb[i * 3] = c.x, rgb[i * 3 + 1] = c.y, rgb[i * 3 + 2] = c.z;
+}
+__global__ void k_sky_pdf(DScene sc, const float *dirs, size_t n, float *pdf) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) pdf[i] = sky_pdf(sc, v3(dirs[i * 3], dirs[i * 3 + 1], dirs[i * 3 + 2]));
 }
 
 __global__ void k_philox(U4 c, uint32_t k0, uint32_t k1, uint32_t *out) {

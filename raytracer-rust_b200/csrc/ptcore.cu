@@ -140,6 +140,7 @@ struct ptc_scene {
   DevBuf<DMesh> d_meshes;
   DevBuf<float> d_sky;
   DevBuf<DLight> d_lights;
+  DevBuf<float> d_sky_dist;
   std::vector<std::unique_ptr<DevBuf<float4>>> mesh_bufs;
   std::vector<DevMeshBuffers> dev_built;  // per mesh: device arrays left behind by the device-side builder (adopted by upload_scene)
   DScene ds;
@@ -238,6 +239,10 @@ void require_committed(const ptc_scene *s) {
   if (!s->committed) throw std::logic_error("scene not committed (call ptc_scene_commit first)");
 }
 
+void check_render_flags(const ptc_render_settings *st) {
+  if ((st->flags & PTC_FLAG_NEE_SKY) && !(st->flags & PTC_FLAG_NEE)) throw std::invalid_argument("PTC_FLAG_NEE_SKY needs PTC_FLAG_NEE");
+}
+
 void ensure_ctl(ptc_scene *s) {
   if (s->h_ctl) return;
   s->d_ctl.alloc(1);
@@ -256,6 +261,7 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
   if (!cam || !st) throw std::invalid_argument("null argument");
   if (st->width <= 0 || st->height <= 0 || st->spp <= 0) throw std::invalid_argument("bad render settings");
   if ((int64_t)st->width * st->height > (int64_t)0x3fffffff) throw std::invalid_argument("image too large");
+  check_render_flags(st);
   CK(cudaSetDevice(s->device));
   int s_begin = st->sample_begin, s_end = st->sample_end;
   if (s_begin == 0 && s_end == 0) s_end = st->spp;
@@ -264,6 +270,8 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
   const int tile_rem = st->tile_mod > 0 ? st->tile_rem : 0;
   if (tile_rem < 0 || tile_rem >= tile_mod) throw std::invalid_argument("tile_rem out of range");
   const bool nee = (st->flags & PTC_FLAG_NEE) != 0;
+  // the sky joins the sampled lights only where there is a sky distribution; elsewhere the flag changes nothing
+  const bool nee_sky = nee && (st->flags & PTC_FLAG_NEE_SKY) != 0 && s->ds.sky_dist != nullptr;
   // paths this call starts (its tiles x its samples; border tiles padded to 32 x 32 like the path index space)
   uint64_t want_paths;
   {
@@ -436,8 +444,9 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
     auto run_shade = [&]() {  // reads set `flip`, writes the other one, which the next extend then reads
       if (timing) mark(ST_SHADE);
       const SegRange ssr = seg_range(0u, 1u);
-      if (nee) launch_stage(pdl, stream, segments, k_shade<true>, s->d_ctl.p, ssr, s->ds, rp, bufs[flip], film);
-      else launch_stage(pdl, stream, segments, k_shade<false>, s->d_ctl.p, ssr, s->ds, rp, bufs[flip], film);
+      if (nee_sky) launch_stage(pdl, stream, segments, k_shade<2>, s->d_ctl.p, ssr, s->ds, rp, bufs[flip], film);
+      else if (nee) launch_stage(pdl, stream, segments, k_shade<1>, s->d_ctl.p, ssr, s->ds, rp, bufs[flip], film);
+      else launch_stage(pdl, stream, segments, k_shade<0>, s->d_ctl.p, ssr, s->ds, rp, bufs[flip], film);
       launches += 1;
       flip ^= 1;
     };
@@ -651,6 +660,8 @@ void upload_scene(ptc_scene *s, const HostScene &hs, int device) {
   s->ds.sky = hs.sky.empty() ? nullptr : s->d_sky.p;
   s->d_lights.upload(hs.lights.data(), hs.lights.size());
   s->ds.lights = s->d_lights.p;
+  if (!hs.sky_dist.empty()) s->d_sky_dist.upload(hs.sky_dist.data(), hs.sky_dist.size());
+  s->ds.sky_dist = hs.sky_dist.empty() ? nullptr : s->d_sky_dist.p;
   s->ds.n_lights = (int32_t)hs.lights.size();
   s->ds.n_objects = (int32_t)hs.objects.size();
   s->ds.n_materials = (int32_t)hs.materials.size();
@@ -1092,6 +1103,46 @@ int ptc_scatter(ptc_scene *s, int material, const float *ray_dirs, const float *
   PTC_GUARD_END
 }
 
+int ptc_sky_sample(ptc_scene *s, const float *u4, int64_t n, float *out_dir, float *out_pdf, float *out_rgb) {
+  PTC_GUARD_BEGIN
+  require_committed(s);
+  if (n < 0 || (n > 0 && (!u4 || !out_dir || !out_pdf || !out_rgb))) throw std::invalid_argument("bad argument");
+  if (!s->ds.sky_dist) throw std::logic_error("the committed scene has no sky distribution (no HDR sky, or an all-zero one)");
+  if (n == 0) return 0;
+  CK(cudaSetDevice(s->device));
+  const size_t N = (size_t)n;
+  DevBuf<float> d_u, d_dir, d_pdf, d_rgb;
+  d_u.upload(u4, N * 4);
+  d_dir.alloc(N * 3), d_pdf.alloc(N), d_rgb.alloc(N * 3);
+  k_sky_sample<<<(unsigned)((N + 127) / 128), 128, 0, s->own_stream>>>(s->ds, d_u.p, N, d_dir.p, d_pdf.p, d_rgb.p);
+  CK(cudaGetLastError());
+  CK(cudaMemcpyAsync(out_dir, d_dir.p, N * 12, cudaMemcpyDeviceToHost, s->own_stream));
+  CK(cudaMemcpyAsync(out_pdf, d_pdf.p, N * 4, cudaMemcpyDeviceToHost, s->own_stream));
+  CK(cudaMemcpyAsync(out_rgb, d_rgb.p, N * 12, cudaMemcpyDeviceToHost, s->own_stream));
+  CK(cudaStreamSynchronize(s->own_stream));
+  return 0;
+  PTC_GUARD_END
+}
+
+int ptc_sky_pdf(ptc_scene *s, const float *dirs, int64_t n, float *out_pdf) {
+  PTC_GUARD_BEGIN
+  require_committed(s);
+  if (n < 0 || (n > 0 && (!dirs || !out_pdf))) throw std::invalid_argument("bad argument");
+  if (!s->ds.sky_dist) throw std::logic_error("the committed scene has no sky distribution (no HDR sky, or an all-zero one)");
+  if (n == 0) return 0;
+  CK(cudaSetDevice(s->device));
+  const size_t N = (size_t)n;
+  DevBuf<float> d_dir, d_pdf;
+  d_dir.upload(dirs, N * 3);
+  d_pdf.alloc(N);
+  k_sky_pdf<<<(unsigned)((N + 127) / 128), 128, 0, s->own_stream>>>(s->ds, d_dir.p, N, d_pdf.p);
+  CK(cudaGetLastError());
+  CK(cudaMemcpyAsync(out_pdf, d_pdf.p, N * 4, cudaMemcpyDeviceToHost, s->own_stream));
+  CK(cudaStreamSynchronize(s->own_stream));
+  return 0;
+  PTC_GUARD_END
+}
+
 int ptc_philox(ptc_scene *s, const uint32_t ctr[4], const uint32_t key[2], uint32_t out[4]) {
   PTC_GUARD_BEGIN
   require_committed(s);
@@ -1149,6 +1200,7 @@ static int multi_render(ptc_multi *m, const ptc_camera *cam, const ptc_render_se
   if (st->width <= 0 || st->height <= 0 || st->spp <= 0) throw std::invalid_argument("bad render settings");
   if (st->tile_mod > 0) throw std::invalid_argument("ptc_multi_render shards by itself: tile_mod must be 0");
   if (shard_mode != PTC_SHARD_SAMPLES && shard_mode != PTC_SHARD_TILES) throw std::invalid_argument("bad shard mode");
+  check_render_flags(st);
   const int n = (int)m->scenes.size();
   int s_begin = st->sample_begin, s_end = st->sample_end;
   if (s_begin == 0 && s_end == 0) s_end = st->spp;

@@ -12,6 +12,13 @@ pub const PTC_E_STATE: c_int = -4;
 pub const PTC_COMMIT_FAST_BUILD: c_int = 1;
 pub const PTC_COMMIT_DEVICE_SAH: c_int = 2;
 
+/// ptc_render_settings.flags
+pub const PTC_FLAG_COUNTERS: i32 = 1;
+pub const PTC_FLAG_TIMING: i32 = 2;
+pub const PTC_FLAG_NEE: i32 = 4;
+/// with PTC_FLAG_NEE only: NEE also samples the HDR sky as an environment light
+pub const PTC_FLAG_NEE_SKY: i32 = 8;
+
 pub const PTC_MAT_LAMBERT: i32 = 0;
 pub const PTC_MAT_LAMBERT_CHECKER: i32 = 1;
 pub const PTC_MAT_METAL: i32 = 2;
@@ -118,6 +125,9 @@ extern "C" {
     pub fn ptc_render_accumulate(s: *mut ptc_scene, cam: *const ptc_camera, st: *const ptc_render_settings, d_accum: *mut f32,
                                  cuda_stream: *mut c_void, stats: *mut ptc_stats) -> c_int;
     pub fn ptc_resolve_u32(s: *mut ptc_scene, rgb: *const f32, n_pixels: i64, scale: f32, out: *mut u32) -> c_int;
+    /// the HDR sky as a light (PTC_FLAG_NEE_SKY): sample / pdf hooks; PTC_E_STATE without a sky distribution
+    pub fn ptc_sky_sample(s: *mut ptc_scene, u4: *const f32, n: i64, out_dir: *mut f32, out_pdf: *mut f32, out_rgb: *mut f32) -> c_int;
+    pub fn ptc_sky_pdf(s: *mut ptc_scene, dirs: *const f32, n: i64, out_pdf: *mut f32) -> c_int;
     pub fn ptc_resolve_device(d_rgb: *const f32, n_pixels: i64, scale: f32, d_out: *mut u32, cuda_stream: *mut c_void) -> c_int;
 
     // in-process multi-GPU: one host thread per device inside the library, one ncclReduce of the film (include/ptcore.h)

@@ -26,8 +26,9 @@ $(PKG)/libpthost.so: $(PKG)/host/pthost.cpp $(PKG)/host/json.hpp include/pthost.
 oracle/liboracle.so: oracle/oracle.cpp oracle/oracle.h
 	$(MAKE) -C oracle
 
-tests/hostsim/libhostsim.so: tests/hostsim/hostsim.cpp tests/hostsim/wfsim.cpp tests/hostsim/skysim.cpp $(CSRC)/pt_build.cpp $(HDRS)
-	$(CXX) $(CXXFLAGS) -shared -o $@ tests/hostsim/hostsim.cpp tests/hostsim/wfsim.cpp tests/hostsim/skysim.cpp $(CSRC)/pt_build.cpp
+tests/hostsim/libhostsim.so: tests/hostsim/hostsim.cpp tests/hostsim/wfsim.cpp tests/hostsim/skysim.cpp tests/hostsim/adaptsim.cpp $(CSRC)/pt_build.cpp $(HDRS)
+	$(CXX) $(CXXFLAGS) -shared -o $@ tests/hostsim/hostsim.cpp tests/hostsim/wfsim.cpp tests/hostsim/skysim.cpp tests/hostsim/adaptsim.cpp \
+		$(CSRC)/pt_build.cpp
 
 clean:
 	rm -f $(PKG)/libptcore.so $(PKG)/libpthost.so oracle/liboracle.so tests/hostsim/libhostsim.so

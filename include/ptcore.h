@@ -194,6 +194,25 @@ int ptc_render_u32(ptc_scene *, const ptc_camera *, const ptc_render_settings *,
  * Returns after the work is enqueued AND finished (the wavefront loop polls its queue counters). */
 int ptc_render_accumulate(ptc_scene *, const ptc_camera *, const ptc_render_settings *, float *d_accum,
                           void *cuda_stream, ptc_stats *stats);
+/* Adaptive sampling: every pixel is rendered until its noise estimate converges, at most settings->spp samples.
+ * Schedule: samples [0, min_spp/2) and [min_spp/2, min_spp) of every pixel, then [n, min(2n, spp)) of the pixels still
+ * active.  After each pass from m to n samples a pixel with fp32 film sum V (Vp before the pass) NEEDS MORE iff
+ * e = sum_c |V_c/n - (V_c-Vp_c)/(n-m)| / (1e-4 + sqrt(sum_c V_c/n)) >= threshold (Dammertz et al. 2009) and every channel
+ * of V is finite; it stays active iff some active pixel of its 3x3 neighbourhood (itself included) needs more.  A pixel
+ * that leaves never returns.  Philox is keyed on (pixel, sample) and the film sums are fixed-point, so every pixel ends
+ * with exactly the film, the image and the packed value of a uniform render at its own sample count.
+ * settings: sample_begin = sample_end = 0 and tile_mod = 0, else PTC_E_INVALID; flags as in ptc_render.  Single device:
+ * ptc_multi_* has no adaptive variant.  Outputs are host buffers, each may be NULL: out_rgb W*H*3 linear mean radiance
+ * (the pixel's sum / its own count), out_u32 W*H 0x00RRGGBB as ptc_render_u32, out_spp W*H samples each pixel received.
+ * stats: paths = sum of the counts; rays, iterations, launches and stage times summed over the passes; render_ms from
+ * the first pass to the end of the resolve (device events).  The ptc_adaptive arguments are checked before the scene's
+ * state: PTC_E_INVALID for bad ones even on an uncommitted scene. */
+typedef struct ptc_adaptive {
+  int32_t min_spp; /* every pixel gets at least this many samples; even, >= 2, <= settings->spp */
+  float threshold; /* a pixel keeps sampling while its error estimate is >= threshold; 0 = never stop early, +inf = stop at min_spp */
+} ptc_adaptive;
+int ptc_render_adaptive(ptc_scene *, const ptc_camera *, const ptc_render_settings *, const ptc_adaptive *, float *out_rgb,
+                        uint32_t *out_u32, int32_t *out_spp, ptc_stats *stats);
 /* Film resolve, renderer.rs:112-120 + color.rs:87-93: out = pack(sqrt(rgb * scale)).  Device and host buffers. */
 int ptc_resolve_device(const float *d_rgb, int64_t n_pixels, float scale, uint32_t *d_out, void *cuda_stream);
 int ptc_resolve_u32(ptc_scene *, const float *rgb, int64_t n_pixels, float scale, uint32_t *out);

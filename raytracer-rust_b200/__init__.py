@@ -45,6 +45,10 @@ class RenderSettings(C.Structure):  # ptc_render_settings
                 ("tile_rem", C.c_int32), ("pool_paths", C.c_int32), ("flags", C.c_int32)]
 
 
+class Adaptive(C.Structure):  # ptc_adaptive
+    _fields_ = [("min_spp", C.c_int32), ("threshold", C.c_float)]
+
+
 class Hit(C.Structure):  # ptc_hit
     _fields_ = [("object", C.c_int32), ("triangle", C.c_int32), ("t", C.c_float), ("position", C.c_float * 3),
                 ("normal", C.c_float * 3), ("front_face", C.c_int32), ("material", C.c_int32)]
@@ -145,6 +149,8 @@ def core():
     L.ptc_scene_last_pool_slots.restype = C.c_int64
     L.ptc_render.argtypes = [_vp, C.POINTER(Camera), C.POINTER(RenderSettings), _F, C.POINTER(Stats)]
     L.ptc_render_u32.argtypes = [_vp, C.POINTER(Camera), C.POINTER(RenderSettings), _vp, C.POINTER(Stats)]
+    L.ptc_render_adaptive.argtypes = [_vp, C.POINTER(Camera), C.POINTER(RenderSettings), C.POINTER(Adaptive), _F, _vp, _vp,
+                                      C.POINTER(Stats)]
     L.ptc_render_accumulate.argtypes = [_vp, C.POINTER(Camera), C.POINTER(RenderSettings), _vp, _vp, C.POINTER(Stats)]
     L.ptc_resolve_device.argtypes = [_vp, C.c_int64, C.c_float, _vp, _vp]
     L.ptc_resolve_u32.argtypes = [_vp, _F, C.c_int64, C.c_float, _vp]
@@ -538,6 +544,20 @@ class CoreScene:
         st = Stats()
         _ck(core().ptc_render_u32(self._h, C.byref(camera), C.byref(settings), out.ctypes.data, C.byref(st)))
         return out, st
+
+    def render_adaptive(self, camera, settings, min_spp, threshold):
+        """Adaptive sampling (ptc_render_adaptive): every pixel gets min_spp samples, then more, doubling, up to
+        settings.spp while the noise estimate of its 3x3 neighbourhood is >= threshold.  -> (rgb [H,W,3] float32 linear
+        mean radiance, u32 [H*W] 0x00RRGGBB, spp [H,W] int32 samples per pixel, Stats); each pixel is the uniform render
+        at its own count."""
+        rgb = np.empty((settings.height, settings.width, 3), np.float32)
+        u32 = np.empty(settings.height * settings.width, np.uint32)
+        spp = np.empty((settings.height, settings.width), np.int32)
+        st = Stats()
+        ad = Adaptive(min_spp, threshold)
+        _ck(core().ptc_render_adaptive(self._h, C.byref(camera), C.byref(settings), C.byref(ad), _fptr(rgb), u32.ctypes.data,
+                                       spp.ctypes.data, C.byref(st)))
+        return rgb, u32, spp, st
 
     def multi(self, devices):
         """In-process multi-GPU (ptc_multi_*): this committed scene replicated on `devices` (devices[0] = its own)."""

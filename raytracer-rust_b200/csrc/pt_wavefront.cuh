@@ -28,6 +28,7 @@
 #include <cuda_runtime.h>
 
 #include "../../include/ptcore.h"
+#include "pt_adaptive.h"
 #include "pt_bsdf.h"
 #include "pt_philox.h"
 #include "pt_prims.h"
@@ -77,6 +78,10 @@ struct RenderParams {
   int32_t tiles_x, n_my_tiles, tile_mod, tile_rem;
   uint32_t row_mult;  // odd, coprime with n_my_tiles: scatters consecutive 32-pixel rows over the image (see k_shade)
   uint64_t seed;
+  // ptc_render_adaptive's later passes: the pixels to start paths for (ascending; padded to a multiple of 32 by index
+  // space only, entries >= n_list start no path); read by k_shade<Mode, true> only, nullptr otherwise
+  const uint32_t *pixel_list;
+  uint32_t n_list;
 };
 
 // Path state, SoA of float4.  Segment b = slots [b * cap, b * cap + cnt[b]).
@@ -527,7 +532,9 @@ __device__ __forceinline__ uint32_t block_rank(bool flag, uint32_t *s_warp /* [k
 // `seg_done` (or nullptr): one word per segment, set when the segment is found empty with the path supply exhausted — it
 // will never hold a ray again — and counted off ctl->n_active, once.
 // (The path state is read with plain loads: launches overlap, see stage_begin, so it is not read-only while a k_shade runs.)
-template <int Mode>
+// List: regeneration starts paths from rp.pixel_list instead of the tiles (ptc_render_adaptive's later passes); a
+// template argument, so that the shade kernels of every other render compile to the instructions they had.
+template <int Mode, bool List>
 __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, uint32_t *seg_done, Ctl *ctl, const DScene &sc, const RenderParams &rp,
                                                 const Buffers &b, const Film &film) {
   __shared__ uint16_t s_perm[kShadeWindow];
@@ -747,8 +754,9 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
   // distinct film addresses), but consecutive rows are scattered over the image by a multiplicative bijection, so every
   // segment holds a uniform sample of the frame — segments are statically owned by blocks, and a segment that got all
   // the rays of the mesh's screen region would make its block the straggler of every traversal pass.  Pixels of partial
-  // border tiles that fall outside the image start no path.
-  const unsigned long long per_sample = (unsigned long long)rp.n_my_tiles * 1024ull;
+  // border tiles that fall outside the image start no path.  With a pixel list the 32-pixel rows are 32 consecutive
+  // list entries instead, and the padding of the last row starts no path.
+  const unsigned long long per_sample = List ? (unsigned long long)((rp.n_list + 31u) & ~31u) : (unsigned long long)rp.n_my_tiles * 1024ull;
   for (;;) {
     if (tid == 0) {
       const unsigned long long total = ctl->total_paths;
@@ -778,12 +786,19 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
         const uint32_t r0 = (uint32_t)(p - (unsigned long long)s * per_sample);
         const uint32_t row = (uint32_t)(((unsigned long long)(r0 >> 5) * rp.row_mult) % (unsigned long long)(per_sample >> 5));
         const uint32_t r = (row << 5) | (r0 & 31u);
-        const uint32_t local_tile = r >> 10, in_tile = r & 1023u;
-        const uint32_t tile = local_tile * (uint32_t)rp.tile_mod + (uint32_t)rp.tile_rem;
-        x = (int)((tile % (uint32_t)rp.tiles_x) * 32u + (in_tile & 31u));
-        y = (int)((tile / (uint32_t)rp.tiles_x) * 32u + (in_tile >> 5));
-        valid = x < rp.width && y < rp.height;
-        pixel = (uint32_t)(y * rp.width + x);
+        if (List) {
+          valid = r < rp.n_list;
+          pixel = valid ? rp.pixel_list[r] : 0u;
+          x = (int)(pixel % (uint32_t)rp.width);
+          y = (int)(pixel / (uint32_t)rp.width);
+        } else {
+          const uint32_t local_tile = r >> 10, in_tile = r & 1023u;
+          const uint32_t tile = local_tile * (uint32_t)rp.tile_mod + (uint32_t)rp.tile_rem;
+          x = (int)((tile % (uint32_t)rp.tiles_x) * 32u + (in_tile & 31u));
+          y = (int)((tile / (uint32_t)rp.tiles_x) * 32u + (in_tile >> 5));
+          valid = x < rp.width && y < rp.height;
+          pixel = (uint32_t)(y * rp.width + x);
+        }
         sample = (uint32_t)rp.sample_begin + s;
       }
       uint32_t total;
@@ -950,10 +965,12 @@ __global__ void __launch_bounds__(kBlock, kSegPerSM) k_extend_post(Ctl *ctl, Seg
   else stage_post<false>(sr.seg0 + blockIdx.x, sr.n_seg, sc, out, tq, round, t_min, t_max);
   stage_end(sr, sr.seg0 + blockIdx.x);
 }
-template <int Mode>  // 0 = plain, 1 = PTC_FLAG_NEE, 2 = PTC_FLAG_NEE | PTC_FLAG_NEE_SKY on a scene with a sky distribution
+// Mode: 0 = plain, 1 = PTC_FLAG_NEE, 2 = PTC_FLAG_NEE | PTC_FLAG_NEE_SKY on a scene with a sky distribution.  List: paths
+// start from rp.pixel_list (stage_shade).
+template <int Mode, bool List = false>
 __global__ void __launch_bounds__(kBlock, kSegPerSM) k_shade(Ctl *ctl, SegRange sr, DScene sc, RenderParams rp, Buffers b, Film film) {
   stage_begin(sr, sr.seg0 + blockIdx.x, ctl);
-  stage_shade<Mode>(sr.seg0 + blockIdx.x, sr.n_seg, sr.flags ? sr.flags + sr.n_seg : nullptr, ctl, sc, rp, b, film);
+  stage_shade<Mode, List>(sr.seg0 + blockIdx.x, sr.n_seg, sr.flags ? sr.flags + sr.n_seg : nullptr, ctl, sc, rp, b, film);
   stage_end(sr, sr.seg0 + blockIdx.x);
 }
 
@@ -973,6 +990,50 @@ __global__ void k_scale(const float *in, float *out, size_t n, float scale) {
 __global__ void k_resolve(const float *rgb, size_t n_pixels, float scale, uint32_t *out) {
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n_pixels) out[i] = resolve_pixel(rgb[i * 3] * scale, rgb[i * 3 + 1] * scale, rgb[i * 3 + 2] * scale);
+}
+
+// ---- ptc_render_adaptive (pt_adaptive.h): decision, dilation and the per-pixel resolve ------------------------
+// every pixel active, none needing more, every final count spp until the pixel leaves earlier
+__global__ void k_adapt_init(uint32_t n_pixels, int32_t spp, uint32_t *list, uint8_t *needs, int32_t *counts) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n_pixels) return;
+  list[i] = i, needs[i] = 0u, counts[i] = spp;
+}
+// needs[p] = the decision of every active pixel p at n samples against its snapshot vp at m; vp <- the film now
+__global__ void k_adapt_decide(Film film, const uint32_t *list, uint32_t n_list, int32_t n, int32_t m, float threshold, float *vp,
+                               uint8_t *needs) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n_list) return;
+  const uint32_t p = list[i];
+  const unsigned long long flags = film.flags[p];
+  float V[3], P[3];
+  for (int c = 0; c < 3; c++) V[c] = film_value(film.sum[(size_t)p * 3 + c], flags, c), P[c] = vp[(size_t)p * 3 + c];
+  needs[p] = adapt_needs_more(V, P, n, m, threshold) ? 1u : 0u;
+  for (int c = 0; c < 3; c++) vp[(size_t)p * 3 + c] = V[c];
+}
+// keep[i] = list entry i stays active (3x3 dilation of needs over the active set)
+__global__ void k_adapt_keep(const uint32_t *list, uint32_t n_list, const uint8_t *needs, int32_t width, int32_t height, uint8_t *keep) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n_list) keep[i] = adapt_keep(needs, width, height, list[i]) ? 1u : 0u;
+}
+// a pixel that leaves keeps its count n and stops counting as needing more (after every k_adapt_keep read of needs)
+__global__ void k_adapt_leave(const uint32_t *list, uint32_t n_list, const uint8_t *keep, int32_t n, uint8_t *needs, int32_t *counts) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n_list || keep[i]) return;
+  const uint32_t p = list[i];
+  needs[p] = 0u, counts[p] = n;
+}
+// rgb = film sum x (1 / its own count), packed = resolve_pixel of that: per pixel what k_film_to_accum into a zeroed
+// film, then k_scale / k_resolve with 1 / spp compute for a uniform render at that count.  Either output may be nullptr.
+__global__ void k_resolve_adaptive(Film film, size_t n_pixels, const int32_t *counts, float *rgb, uint32_t *packed) {
+  const size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= n_pixels) return;
+  const float scale = 1.0f / (float)counts[p];
+  const unsigned long long flags = film.flags[p];
+  float c[3];
+  for (int k = 0; k < 3; k++) c[k] = (0.0f + film_value(film.sum[p * 3 + k], flags, k)) * scale;
+  if (rgb) rgb[p * 3] = c[0], rgb[p * 3 + 1] = c[1], rgb[p * 3 + 2] = c[2];
+  if (packed) packed[p] = resolve_pixel(c[0], c[1], c[2]);
 }
 
 // ---- parity hooks: the same device functions / kernels, driven by caller-provided inputs ---------------------

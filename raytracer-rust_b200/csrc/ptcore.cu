@@ -26,6 +26,8 @@
 #include <string>
 #include <vector>
 
+#include <cub/device/device_select.cuh>
+
 #include "../../include/ptcore.h"
 #include "pt_build_dev.h"
 #include "pt_scene_host.h"
@@ -156,12 +158,21 @@ struct ptc_scene {
   float *h_film = nullptr;           // pinned staging for the film's way to the caller's (pageable) buffer, grow-only
   size_t h_film_n = 0;
   DevBuf<uint32_t> w_packed;
+  // ptc_render_adaptive, grow-only: the film snapshot of the last decision, the needs-more byte map, the keep flag of
+  // each list entry, the active list and the next one, every pixel's final count, the compaction's count and scratch
+  DevBuf<float> w_adapt_vp;
+  DevBuf<uint8_t> w_adapt_needs, w_adapt_keep;
+  DevBuf<uint32_t> w_adapt_list[2];
+  DevBuf<int32_t> w_adapt_spp;
+  DevBuf<uint32_t> w_adapt_n;
+  DevBuf<uint8_t> w_adapt_tmp;
   DevBuf<Ctl> d_ctl;
   Ctl *h_ctl = nullptr;  // pinned ring
   uint32_t *h_progress = nullptr;  // pinned + mapped: the word k_extend_pre reports the state of the render in
   static constexpr int kRing = 4;
   cudaEvent_t ring_ev[kRing] = {nullptr, nullptr, nullptr, nullptr};
   cudaEvent_t ev_begin = nullptr, ev_end = nullptr;  // render_ms brackets, created once (ensure_ctl)
+  cudaEvent_t ev_adapt_begin = nullptr, ev_adapt_end = nullptr;  // ... of ptc_render_adaptive, around all its passes
   cudaStream_t own_stream = nullptr;
   std::vector<cudaEvent_t> timing_events;
 
@@ -183,6 +194,8 @@ struct ptc_scene {
       if (e) cudaEventDestroy(e);
     if (ev_begin) cudaEventDestroy(ev_begin);
     if (ev_end) cudaEventDestroy(ev_end);
+    if (ev_adapt_begin) cudaEventDestroy(ev_adapt_begin);
+    if (ev_adapt_end) cudaEventDestroy(ev_adapt_end);
     for (auto &e : timing_events) cudaEventDestroy(e);
     if (own_stream) cudaStreamDestroy(own_stream);
   }
@@ -251,12 +264,22 @@ void ensure_ctl(ptc_scene *s) {
   for (auto &e : s->ring_ev) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
   CK(cudaEventCreate(&s->ev_begin));
   CK(cudaEventCreate(&s->ev_end));
+  CK(cudaEventCreate(&s->ev_adapt_begin));
+  CK(cudaEventCreate(&s->ev_adapt_end));
 }
+
+// What one call of render_accumulate renders besides its settings.  Default: the tiles of the settings into a cleared
+// film.  ptc_render_adaptive's passes add samples to the film as it stands, the later ones for a list of pixels only.
+struct Pass {
+  bool clear_film = true;
+  const uint32_t *pixels = nullptr;  // device, ascending; nullptr: the tiles of tile_mod / tile_rem
+  uint32_t n_pixels = 0;
+};
 
 // the wavefront loop; renders into the scene's fixed-point film and then adds its fp32 image into d_accum on `stream`
 // (d_accum == nullptr: the caller takes the fixed-point film itself, ptc_multi_*'s int64 reduce)
 void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_settings *st, float *d_accum,
-                       cudaStream_t stream, ptc_stats *stats) {
+                       cudaStream_t stream, ptc_stats *stats, const Pass &pass = Pass()) {
   require_committed(s);
   if (!cam || !st) throw std::invalid_argument("null argument");
   if (st->width <= 0 || st->height <= 0 || st->spp <= 0) throw std::invalid_argument("bad render settings");
@@ -272,9 +295,13 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
   const bool nee = (st->flags & PTC_FLAG_NEE) != 0;
   // the sky joins the sampled lights only where there is a sky distribution; elsewhere the flag changes nothing
   const bool nee_sky = nee && (st->flags & PTC_FLAG_NEE_SKY) != 0 && s->ds.sky_dist != nullptr;
-  // paths this call starts (its tiles x its samples; border tiles padded to 32 x 32 like the path index space)
+  // paths this call starts (its tiles x its samples; border tiles padded to 32 x 32 like the path index space; a pixel
+  // list padded to 32 entries)
+  const uint64_t list_padded = ((uint64_t)pass.n_pixels + 31u) & ~31ull;
   uint64_t want_paths;
-  {
+  if (pass.pixels) {
+    want_paths = list_padded * (uint64_t)(s_end - s_begin);
+  } else {
     const int tx = (st->width + 31) / 32, ty = (st->height + 31) / 32, nt = tx * ty;
     const int mine = tile_rem < nt ? (nt - tile_rem + tile_mod - 1) / tile_mod : 0;
     want_paths = (uint64_t)mine * 1024ull * (uint64_t)(s_end - s_begin);
@@ -327,7 +354,9 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
   rp.n_my_tiles = tile_rem < n_tiles ? (n_tiles - tile_rem + tile_mod - 1) / tile_mod : 0;
   rp.tile_mod = tile_mod, rp.tile_rem = tile_rem;
   rp.seed = st->seed;
-  {  // odd multiplier coprime with the number of 32-pixel rows (= n_my_tiles * 32): a bijection on row indices
+  rp.pixel_list = pass.pixels, rp.n_list = pass.n_pixels;
+  {  // odd multiplier coprime with the number of 32-pixel rows (= n_my_tiles * 32, or padded list entries / 32): a bijection
+     // on row indices
     auto gcd = [](uint64_t a, uint64_t b) {
       while (b) {
         const uint64_t t = a % b;
@@ -336,15 +365,15 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
       }
       return a;
     };
-    const uint64_t rows = (uint64_t)std::max(rp.n_my_tiles, 1) * 32ull;
+    const uint64_t rows = pass.pixels ? std::max<uint64_t>(list_padded / 32u, 1u) : (uint64_t)std::max(rp.n_my_tiles, 1) * 32ull;
     uint64_t m = (0x9E3779B1ull % rows) | 1ull;
     while (gcd(m, rows) != 1) m += 2;
     rp.row_mult = (uint32_t)m;
   }
 
   // valid pixels of this rank (for the paths statistic)
-  uint64_t my_pixels = 0;
-  for (int t = tile_rem; t < n_tiles; t += tile_mod) {
+  uint64_t my_pixels = pass.pixels ? pass.n_pixels : 0;
+  for (int t = tile_rem; !pass.pixels && t < n_tiles; t += tile_mod) {
     const int tx = t % rp.tiles_x, ty = t / rp.tiles_x;
     const int w = std::min(32, st->width - tx * 32), h = std::min(32, st->height - ty * 32);
     my_pixels += (uint64_t)w * h;
@@ -352,14 +381,16 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
 
   Ctl init;
   memset(&init, 0, sizeof(init));
-  init.total_paths = rp.max_depth > 0 ? (unsigned long long)rp.n_my_tiles * 1024ull * (unsigned long long)rp.n_samples : 0ull;
+  init.total_paths = rp.max_depth > 0 ? (pass.pixels ? list_padded : (unsigned long long)rp.n_my_tiles * 1024ull) * (unsigned long long)rp.n_samples : 0ull;
   init.n_active = init.total_paths != 0ull ? segments : 0u;  // every segment reports once when it is empty for good (stage_shade)
   const size_t n_px = (size_t)st->width * st->height;
   if (s->film_sum.n < n_px * 3) s->film_sum.alloc(n_px * 3);
   if (s->film_flags.n < n_px) s->film_flags.alloc(n_px);
   const Film film{s->film_sum.p, s->film_flags.p};
-  CK(cudaMemsetAsync(film.sum, 0, n_px * 3 * sizeof(long long), stream));
-  CK(cudaMemsetAsync(film.flags, 0, n_px * sizeof(unsigned long long), stream));
+  if (pass.clear_film) {
+    CK(cudaMemsetAsync(film.sum, 0, n_px * 3 * sizeof(long long), stream));
+    CK(cudaMemsetAsync(film.flags, 0, n_px * sizeof(unsigned long long), stream));
+  }
   CK(cudaMemcpyAsync(s->d_ctl.p, &init, sizeof(Ctl), cudaMemcpyHostToDevice, stream));
   CK(cudaMemsetAsync(bufs[0].cnt, 0, segments * sizeof(uint32_t), stream));
   CK(cudaMemsetAsync(s->ws.seg_flags.p, 0, 3 * (size_t)segments * sizeof(uint32_t), stream));
@@ -444,9 +475,10 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
     auto run_shade = [&]() {  // reads set `flip`, writes the other one, which the next extend then reads
       if (timing) mark(ST_SHADE);
       const SegRange ssr = seg_range(0u, 1u);
-      if (nee_sky) launch_stage(pdl, stream, segments, k_shade<2>, s->d_ctl.p, ssr, s->ds, rp, bufs[flip], film);
-      else if (nee) launch_stage(pdl, stream, segments, k_shade<1>, s->d_ctl.p, ssr, s->ds, rp, bufs[flip], film);
-      else launch_stage(pdl, stream, segments, k_shade<0>, s->d_ctl.p, ssr, s->ds, rp, bufs[flip], film);
+      const int mode = nee_sky ? 2 : (nee ? 1 : 0);
+      auto *kernel = pass.pixels ? (mode == 2 ? k_shade<2, true> : mode == 1 ? k_shade<1, true> : k_shade<0, true>)
+                                 : (mode == 2 ? k_shade<2> : mode == 1 ? k_shade<1> : k_shade<0>);
+      launch_stage(pdl, stream, segments, kernel, s->d_ctl.p, ssr, s->ds, rp, bufs[flip], film);
       launches += 1;
       flip ^= 1;
     };
@@ -954,6 +986,114 @@ int ptc_render_u32(ptc_scene *s, const ptc_camera *cam, const ptc_render_setting
   CK(cudaMemcpyAsync(out_u32, s->w_packed.p, px * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
   CK(cudaStreamSynchronize(stream));
   if (stats) stats->kernel_launches += 1;
+  return 0;
+  PTC_GUARD_END
+}
+
+int ptc_render_adaptive(ptc_scene *s, const ptc_camera *cam, const ptc_render_settings *st, const ptc_adaptive *ad, float *out_rgb,
+                        uint32_t *out_u32, int32_t *out_spp, ptc_stats *stats) {
+  PTC_GUARD_BEGIN
+  // the arguments first, the scene's state after them
+  if (!s || !cam || !st || !ad) throw std::invalid_argument("null argument");
+  if (st->width <= 0 || st->height <= 0 || st->spp <= 0) throw std::invalid_argument("bad render settings");
+  if (st->sample_begin != 0 || st->sample_end != 0 || st->tile_mod != 0)
+    throw std::invalid_argument("ptc_render_adaptive schedules the samples itself: sample_begin, sample_end and tile_mod must be 0");
+  if (ad->min_spp < 2 || ad->min_spp % 2 != 0 || ad->min_spp > st->spp) throw std::invalid_argument("min_spp must be even, >= 2 and <= spp");
+  if (!(ad->threshold >= 0.0f)) throw std::invalid_argument("threshold must be >= 0");
+  check_render_flags(st);
+  require_committed(s);
+  if ((int64_t)st->width * st->height > (int64_t)0x3fffffff) throw std::invalid_argument("image too large");
+  CK(cudaSetDevice(s->device));
+  ensure_ctl(s);
+  const uint32_t n_px = (uint32_t)st->width * (uint32_t)st->height;
+  if (s->w_adapt_vp.n < (size_t)n_px * 3) s->w_adapt_vp.alloc((size_t)n_px * 3);
+  if (s->w_adapt_needs.n < n_px) s->w_adapt_needs.alloc(n_px), s->w_adapt_keep.alloc(n_px), s->w_adapt_spp.alloc(n_px);
+  for (auto &l : s->w_adapt_list)
+    if (l.n < n_px) l.alloc(n_px);
+  if (!s->w_adapt_n.p) s->w_adapt_n.alloc(1);
+  size_t tmp_bytes = 0;
+  CK(cub::DeviceSelect::Flagged(nullptr, tmp_bytes, (const uint32_t *)nullptr, (const uint8_t *)nullptr, (uint32_t *)nullptr,
+                                (uint32_t *)nullptr, (int)n_px));
+  if (s->w_adapt_tmp.n < tmp_bytes) s->w_adapt_tmp.alloc(tmp_bytes);
+  cudaStream_t stream = s->own_stream;
+  const unsigned nb = (n_px + 255u) / 256u;
+
+  ptc_stats total;
+  memset(&total, 0, sizeof(total));
+  uint64_t launches = 0;
+  auto run_pass = [&](int first, int last, const Pass &pass) {
+    ptc_render_settings ps = *st;
+    ps.sample_begin = first, ps.sample_end = last;
+    ptc_stats p;
+    render_accumulate(s, cam, &ps, nullptr, stream, &p, pass);
+    total.paths += p.paths, total.rays += p.rays, total.iterations += p.iterations, launches += p.kernel_launches;
+    total.extend_ms += p.extend_ms, total.shade_ms += p.shade_ms, total.extend_launches += p.extend_launches;
+    total.pre_ms += p.pre_ms, total.traverse_ms += p.traverse_ms, total.post_ms += p.post_ms;
+    total.nodes_visited += p.nodes_visited, total.tris_tested += p.tris_tested, total.mesh_rays += p.mesh_rays;
+  };
+
+  // passes 0 and 1 over the tiles, the snapshot between them
+  const int half = ad->min_spp / 2;
+  CK(cudaEventRecord(s->ev_adapt_begin, stream));
+  run_pass(0, half, Pass());
+  const Film f{s->film_sum.p, s->film_flags.p};
+  float *vp = s->w_adapt_vp.p;
+  CK(cudaMemsetAsync(vp, 0, (size_t)n_px * 3 * sizeof(float), stream));
+  k_film_to_accum<<<(unsigned)(((size_t)n_px * 3 + 255) / 256), 256, 0, stream>>>(f, n_px, vp);
+  launches += 1;
+  Pass more;
+  more.clear_film = false;
+  run_pass(half, ad->min_spp, more);
+  k_adapt_init<<<nb, 256, 0, stream>>>(n_px, st->spp, s->w_adapt_list[0].p, s->w_adapt_needs.p, s->w_adapt_spp.p);
+  launches += 1;
+  CK(cudaGetLastError());
+
+  // decision, then a pass over the pixels that stay, until none stays or they have all reached spp
+  uint32_t n_list = n_px;
+  int cur = 0, n = ad->min_spp, m = half;
+  while (n < st->spp) {
+    const uint32_t *list = s->w_adapt_list[cur].p;
+    const unsigned lb = (n_list + 255u) / 256u;
+    k_adapt_decide<<<lb, 256, 0, stream>>>(f, list, n_list, n, m, ad->threshold, vp, s->w_adapt_needs.p);
+    k_adapt_keep<<<lb, 256, 0, stream>>>(list, n_list, s->w_adapt_needs.p, st->width, st->height, s->w_adapt_keep.p);
+    k_adapt_leave<<<lb, 256, 0, stream>>>(list, n_list, s->w_adapt_keep.p, n, s->w_adapt_needs.p, s->w_adapt_spp.p);
+    CK(cudaGetLastError());
+    size_t tb = s->w_adapt_tmp.n;
+    CK(cub::DeviceSelect::Flagged(s->w_adapt_tmp.p, tb, list, s->w_adapt_keep.p, s->w_adapt_list[cur ^ 1].p, s->w_adapt_n.p,
+                                  (int)n_list, stream));  // stable: the next list is ascending again
+    launches += 5;
+    uint32_t kept = 0;
+    CK(cudaMemcpyAsync(&kept, s->w_adapt_n.p, sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+    CK(cudaStreamSynchronize(stream));
+    n_list = kept, cur ^= 1;
+    if (n_list == 0) break;
+    more.pixels = s->w_adapt_list[cur].p, more.n_pixels = n_list;
+    const int next = adapt_next_end(n, st->spp);
+    run_pass(n, next, more);
+    m = n, n = next;
+  }
+
+  // one resolve of every pixel at its own count
+  if (out_rgb && s->w_film_out.n < (size_t)n_px * 3) s->w_film_out.alloc((size_t)n_px * 3);
+  if (out_u32 && s->w_packed.n < n_px) s->w_packed.alloc(n_px);
+  if (out_rgb || out_u32) {
+    k_resolve_adaptive<<<nb, 256, 0, stream>>>(f, n_px, s->w_adapt_spp.p, out_rgb ? s->w_film_out.p : nullptr,
+                                               out_u32 ? s->w_packed.p : nullptr);
+    launches += 1;
+    CK(cudaGetLastError());
+  }
+  CK(cudaEventRecord(s->ev_adapt_end, stream));
+  if (out_u32) CK(cudaMemcpyAsync(out_u32, s->w_packed.p, (size_t)n_px * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+  if (out_spp) CK(cudaMemcpyAsync(out_spp, s->w_adapt_spp.p, (size_t)n_px * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+  if (out_rgb) film_to_host(s, s->w_film_out.p, out_rgb, (size_t)n_px * 3, stream);
+  CK(cudaStreamSynchronize(stream));
+  if (stats) {
+    *stats = total;
+    stats->kernel_launches = launches;
+    float ms = 0.0f;
+    CK(cudaEventElapsedTime(&ms, s->ev_adapt_begin, s->ev_adapt_end));
+    stats->render_ms = ms;
+  }
   return 0;
   PTC_GUARD_END
 }

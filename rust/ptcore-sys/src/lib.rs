@@ -92,6 +92,14 @@ pub struct ptc_stats {
     pub regen_ms: f64,
 }
 
+/// ptc_render_adaptive's parameters: min_spp even, >= 2, <= spp; threshold >= 0 (0: never stop early, +inf: stop at min_spp)
+#[repr(C)]
+#[derive(Clone, Copy, Default)]
+pub struct ptc_adaptive {
+    pub min_spp: i32,
+    pub threshold: f32,
+}
+
 #[repr(C)]
 pub struct ptc_scene {
     _private: [u8; 0],
@@ -122,6 +130,9 @@ extern "C" {
                       stats: *mut ptc_stats) -> c_int;
     pub fn ptc_render_u32(s: *mut ptc_scene, cam: *const ptc_camera, st: *const ptc_render_settings, out_u32: *mut u32,
                           stats: *mut ptc_stats) -> c_int;
+    /// adaptive sampling, one device (include/ptcore.h); every output may be null
+    pub fn ptc_render_adaptive(s: *mut ptc_scene, cam: *const ptc_camera, st: *const ptc_render_settings, ad: *const ptc_adaptive,
+                               out_rgb: *mut f32, out_u32: *mut u32, out_spp: *mut i32, stats: *mut ptc_stats) -> c_int;
     pub fn ptc_render_accumulate(s: *mut ptc_scene, cam: *const ptc_camera, st: *const ptc_render_settings, d_accum: *mut f32,
                                  cuda_stream: *mut c_void, stats: *mut ptc_stats) -> c_int;
     pub fn ptc_resolve_u32(s: *mut ptc_scene, rgb: *const f32, n_pixels: i64, scale: f32, out: *mut u32) -> c_int;

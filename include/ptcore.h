@@ -220,8 +220,10 @@ int ptc_resolve_u32(ptc_scene *, const float *rgb, int64_t n_pixels, float scale
 /* In-process multi-GPU, for a single-process host like the reference's binary (SURVEY.md 8e): the scene is replicated
  * on every device of `devices` (devices[0] = the device `primary` was committed on; the host-side flattening is not
  * repeated), one host thread per device renders its shard — a balanced sample range or the interleaved 32x32 tiles
- * with index % n == i, Philox keyed on the global pixel / sample so the shards are invisible — and the fp32 radiance
- * films are summed onto devices[0] with ONE ncclReduce over NVLink before the 1/spp scale and the copy to the host.
+ * with index % n == i, Philox keyed on the global pixel / sample so the shards are invisible — and the fixed-point films
+ * (int64 radiance sums, then the NaN / inf flag words) are summed onto devices[0] by two ncclReduce calls over NVLink, so
+ * the image is the one-GPU image bit for bit.  devices[0] then resolves the film (1/spp, and the packing for
+ * ptc_multi_render_u32) and copies the image to the host.
  * The one-process-per-GPU route (ptc_render_accumulate + torch.distributed, bench.py) stays available.
  * NCCL is loaded at run time (libnccl.so.2) by ptc_multi_create for n > 1 only. */
 typedef struct ptc_multi ptc_multi;

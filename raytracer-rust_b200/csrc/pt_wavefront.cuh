@@ -974,25 +974,35 @@ __global__ void __launch_bounds__(kBlock, kSegPerSM) k_shade(Ctl *ctl, SegRange 
   stage_end(sr, sr.seg0 + blockIdx.x);
 }
 
-// accum[i] += fp32(film sum i): the end of every render (ptc_render_accumulate ADDS into the caller's fp32 film)
+// accum[i] += fp32(film sum i): the end of ptc_render_accumulate (which ADDS into the caller's fp32 film), and
+// ptc_render_adaptive's snapshot
 __global__ void k_film_to_accum(Film film, size_t n_pixels, float *accum) {
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n_pixels * 3) return;
   const size_t px = i / 3;
   accum[i] += film_value(film.sum[i], film.flags[px], (int)(i - px * 3));
 }
-// out = rgb * scale (renderer.rs:103)
-__global__ void k_scale(const float *in, float *out, size_t n, float scale) {
-  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) out[i] = in[i] * scale;
-}
-// renderer.rs:112-120 + color.rs:87-93
+// renderer.rs:112-120 + color.rs:87-93 on a caller's fp32 film (ptc_resolve_device / ptc_resolve_u32)
 __global__ void k_resolve(const float *rgb, size_t n_pixels, float scale, uint32_t *out) {
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n_pixels) out[i] = resolve_pixel(rgb[i * 3] * scale, rgb[i * 3 + 1] * scale, rgb[i * 3 + 2] * scale);
 }
+// The end of every render that returns an image: rgb = film sum x scale (renderer.rs:103; counts != nullptr: x 1 / the
+// pixel's own count, ptc_render_adaptive), packed = resolve_pixel of that (renderer.rs:112-120 + color.rs:87-93).
+// 0.0f + the sum is what k_film_to_accum leaves in a zeroed fp32 film, so the result is bit for bit that film x scale,
+// then k_resolve.  Either output may be nullptr.
+__global__ void k_resolve_film(Film film, size_t n_pixels, float scale, const int32_t *counts, float *rgb, uint32_t *packed) {
+  const size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= n_pixels) return;
+  if (counts) scale = 1.0f / (float)counts[p];
+  const unsigned long long flags = film.flags[p];
+  float c[3];
+  for (int k = 0; k < 3; k++) c[k] = (0.0f + film_value(film.sum[p * 3 + k], flags, k)) * scale;
+  if (rgb) rgb[p * 3] = c[0], rgb[p * 3 + 1] = c[1], rgb[p * 3 + 2] = c[2];
+  if (packed) packed[p] = resolve_pixel(c[0], c[1], c[2]);
+}
 
-// ---- ptc_render_adaptive (pt_adaptive.h): decision, dilation and the per-pixel resolve ------------------------
+// ---- ptc_render_adaptive (pt_adaptive.h): decision and dilation ------------------------------------------------
 // every pixel active, none needing more, every final count spp until the pixel leaves earlier
 __global__ void k_adapt_init(uint32_t n_pixels, int32_t spp, uint32_t *list, uint8_t *needs, int32_t *counts) {
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1022,18 +1032,6 @@ __global__ void k_adapt_leave(const uint32_t *list, uint32_t n_list, const uint8
   if (i >= n_list || keep[i]) return;
   const uint32_t p = list[i];
   needs[p] = 0u, counts[p] = n;
-}
-// rgb = film sum x (1 / its own count), packed = resolve_pixel of that: per pixel what k_film_to_accum into a zeroed
-// film, then k_scale / k_resolve with 1 / spp compute for a uniform render at that count.  Either output may be nullptr.
-__global__ void k_resolve_adaptive(Film film, size_t n_pixels, const int32_t *counts, float *rgb, uint32_t *packed) {
-  const size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (p >= n_pixels) return;
-  const float scale = 1.0f / (float)counts[p];
-  const unsigned long long flags = film.flags[p];
-  float c[3];
-  for (int k = 0; k < 3; k++) c[k] = (0.0f + film_value(film.sum[p * 3 + k], flags, k)) * scale;
-  if (rgb) rgb[p * 3] = c[0], rgb[p * 3 + 1] = c[1], rgb[p * 3 + 2] = c[2];
-  if (packed) packed[p] = resolve_pixel(c[0], c[1], c[2]);
 }
 
 // ---- parity hooks: the same device functions / kernels, driven by caller-provided inputs ---------------------

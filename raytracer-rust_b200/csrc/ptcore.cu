@@ -152,11 +152,11 @@ struct ptc_scene {
   uint64_t pool_budget_bytes = 0;  // what the default pool may occupy: a quarter of the memory free at the first render, at most 48 GiB
   Workspace ws;       // render
   Workspace ws_hook;  // ptc_intersect (kept apart so a parity call never disturbs a render's pool)
-  DevBuf<float> w_film, w_film_out;  // ptc_render / ptc_resolve_u32 staging, grow-only
   DevBuf<long long> film_sum;            // the fixed-point film of the render in flight (pt_wavefront.cuh: Film), grow-only
   DevBuf<unsigned long long> film_flags;
-  float *h_film = nullptr;           // pinned staging for the film's way to the caller's (pageable) buffer, grow-only
-  size_t h_film_n = 0;
+  char *h_film = nullptr;  // pinned staging for an image's way to the caller's (pageable) buffer, grow-only
+  size_t h_film_bytes = 0;
+  DevBuf<float> w_film_out;  // the resolved images (resolve_film_to_host) and ptc_resolve_u32's input, grow-only
   DevBuf<uint32_t> w_packed;
   // ptc_render_adaptive, grow-only: the film snapshot of the last decision, the needs-more byte map, the keep flag of
   // each list entry, the active list and the next one, every pixel's final count, the compaction's count and scratch
@@ -177,6 +177,7 @@ struct ptc_scene {
   std::vector<cudaEvent_t> timing_events;
 
   uint32_t segments() const { return (uint32_t)(sm_count * kSegPerSM); }
+  Film film() const { return Film{film_sum.p, film_flags.p}; }
 
   ~ptc_scene() {
     if (device >= 0) cudaSetDevice(device);
@@ -252,8 +253,30 @@ void require_committed(const ptc_scene *s) {
   if (!s->committed) throw std::logic_error("scene not committed (call ptc_scene_commit first)");
 }
 
-void check_render_flags(const ptc_render_settings *st) {
+// What every render entry point checks of its arguments; `has_output`: the caller passed the output(s) it needs.  The
+// scene's state is checked apart (ptc_render_adaptive checks it after its own arguments).
+void check_render_args(const ptc_camera *cam, const ptc_render_settings *st, bool has_output) {
+  if (!cam || !st || !has_output) throw std::invalid_argument("null argument");
+  if (st->width <= 0 || st->height <= 0 || st->spp <= 0) throw std::invalid_argument("bad render settings");
+  if ((int64_t)st->width * st->height > (int64_t)0x3fffffff) throw std::invalid_argument("image too large");
   if ((st->flags & PTC_FLAG_NEE_SKY) && !(st->flags & PTC_FLAG_NEE)) throw std::invalid_argument("PTC_FLAG_NEE_SKY needs PTC_FLAG_NEE");
+}
+
+// The samples [begin, end) a call renders: sample_begin = sample_end = 0 means [0, spp)
+void sample_range(const ptc_render_settings *st, int &begin, int &end) {
+  begin = st->sample_begin, end = st->sample_end;
+  if (begin == 0 && end == 0) end = st->spp;
+  if (begin < 0 || end < begin) throw std::invalid_argument("bad sample range");
+}
+
+// The scene's fixed-point film for n_px pixels: grow-only, and cleared on `stream` before every render that starts it
+void ensure_film(ptc_scene *s, size_t n_px) {
+  if (s->film_sum.n < n_px * 3) s->film_sum.alloc(n_px * 3);
+  if (s->film_flags.n < n_px) s->film_flags.alloc(n_px);
+}
+void clear_film(ptc_scene *s, size_t n_px, cudaStream_t stream) {
+  CK(cudaMemsetAsync(s->film_sum.p, 0, n_px * 3 * sizeof(long long), stream));
+  CK(cudaMemsetAsync(s->film_flags.p, 0, n_px * sizeof(unsigned long long), stream));
 }
 
 void ensure_ctl(ptc_scene *s) {
@@ -277,35 +300,25 @@ struct Pass {
 };
 
 // the wavefront loop; renders into the scene's fixed-point film and then adds its fp32 image into d_accum on `stream`
-// (d_accum == nullptr: the caller takes the fixed-point film itself, ptc_multi_*'s int64 reduce)
+// (d_accum == nullptr: the caller takes the fixed-point film itself).  The caller has checked the scene's state and
+// check_render_args.
 void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_settings *st, float *d_accum,
                        cudaStream_t stream, ptc_stats *stats, const Pass &pass = Pass()) {
-  require_committed(s);
-  if (!cam || !st) throw std::invalid_argument("null argument");
-  if (st->width <= 0 || st->height <= 0 || st->spp <= 0) throw std::invalid_argument("bad render settings");
-  if ((int64_t)st->width * st->height > (int64_t)0x3fffffff) throw std::invalid_argument("image too large");
-  check_render_flags(st);
   CK(cudaSetDevice(s->device));
-  int s_begin = st->sample_begin, s_end = st->sample_end;
-  if (s_begin == 0 && s_end == 0) s_end = st->spp;
-  if (s_begin < 0 || s_end < s_begin) throw std::invalid_argument("bad sample range");
+  int s_begin, s_end;
+  sample_range(st, s_begin, s_end);
   const int tile_mod = st->tile_mod > 0 ? st->tile_mod : 1;
   const int tile_rem = st->tile_mod > 0 ? st->tile_rem : 0;
   if (tile_rem < 0 || tile_rem >= tile_mod) throw std::invalid_argument("tile_rem out of range");
   const bool nee = (st->flags & PTC_FLAG_NEE) != 0;
   // the sky joins the sampled lights only where there is a sky distribution; elsewhere the flag changes nothing
   const bool nee_sky = nee && (st->flags & PTC_FLAG_NEE_SKY) != 0 && s->ds.sky_dist != nullptr;
+  const int tiles_x = (st->width + 31) / 32, n_tiles = tiles_x * ((st->height + 31) / 32);
+  const int n_my_tiles = tile_rem < n_tiles ? (n_tiles - tile_rem + tile_mod - 1) / tile_mod : 0;
   // paths this call starts (its tiles x its samples; border tiles padded to 32 x 32 like the path index space; a pixel
   // list padded to 32 entries)
   const uint64_t list_padded = ((uint64_t)pass.n_pixels + 31u) & ~31ull;
-  uint64_t want_paths;
-  if (pass.pixels) {
-    want_paths = list_padded * (uint64_t)(s_end - s_begin);
-  } else {
-    const int tx = (st->width + 31) / 32, ty = (st->height + 31) / 32, nt = tx * ty;
-    const int mine = tile_rem < nt ? (nt - tile_rem + tile_mod - 1) / tile_mod : 0;
-    want_paths = (uint64_t)mine * 1024ull * (uint64_t)(s_end - s_begin);
-  }
+  const uint64_t want_paths = (pass.pixels ? list_padded : (uint64_t)n_my_tiles * 1024ull) * (uint64_t)(s_end - s_begin);
   uint64_t pool;
   if (st->pool_paths > 0) {
     pool = (uint64_t)st->pool_paths;
@@ -348,10 +361,8 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
   rp.width = st->width, rp.height = st->height;
   rp.max_depth = st->max_depth;
   rp.sample_begin = s_begin, rp.n_samples = s_end - s_begin;
-  rp.tiles_x = (st->width + 31) / 32;
-  const int tiles_y = (st->height + 31) / 32;
-  const int n_tiles = rp.tiles_x * tiles_y;
-  rp.n_my_tiles = tile_rem < n_tiles ? (n_tiles - tile_rem + tile_mod - 1) / tile_mod : 0;
+  rp.tiles_x = tiles_x;
+  rp.n_my_tiles = n_my_tiles;
   rp.tile_mod = tile_mod, rp.tile_rem = tile_rem;
   rp.seed = st->seed;
   rp.pixel_list = pass.pixels, rp.n_list = pass.n_pixels;
@@ -381,16 +392,12 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
 
   Ctl init;
   memset(&init, 0, sizeof(init));
-  init.total_paths = rp.max_depth > 0 ? (pass.pixels ? list_padded : (unsigned long long)rp.n_my_tiles * 1024ull) * (unsigned long long)rp.n_samples : 0ull;
+  init.total_paths = rp.max_depth > 0 ? want_paths : 0ull;
   init.n_active = init.total_paths != 0ull ? segments : 0u;  // every segment reports once when it is empty for good (stage_shade)
   const size_t n_px = (size_t)st->width * st->height;
-  if (s->film_sum.n < n_px * 3) s->film_sum.alloc(n_px * 3);
-  if (s->film_flags.n < n_px) s->film_flags.alloc(n_px);
-  const Film film{s->film_sum.p, s->film_flags.p};
-  if (pass.clear_film) {
-    CK(cudaMemsetAsync(film.sum, 0, n_px * 3 * sizeof(long long), stream));
-    CK(cudaMemsetAsync(film.flags, 0, n_px * sizeof(unsigned long long), stream));
-  }
+  ensure_film(s, n_px);
+  const Film film = s->film();
+  if (pass.clear_film) clear_film(s, n_px, stream);
   CK(cudaMemcpyAsync(s->d_ctl.p, &init, sizeof(Ctl), cudaMemcpyHostToDevice, stream));
   CK(cudaMemsetAsync(bufs[0].cnt, 0, segments * sizeof(uint32_t), stream));
   CK(cudaMemsetAsync(s->ws.seg_flags.p, 0, 3 * (size_t)segments * sizeof(uint32_t), stream));
@@ -621,33 +628,54 @@ int fail(int code, const std::string &msg) {
 
 }  // namespace
 
-// Device film -> caller's host buffer.  A copy straight into pageable memory runs at ~5 GB/s (C5's 99.5 MB film: 20 ms,
+// Device image -> caller's host buffer.  A copy straight into pageable memory runs at ~5 GB/s (C5's 99.5 MB film: 20 ms,
 // as long as a quarter of the 8-GPU render); through a pinned staging buffer the PCIe leg runs at link speed and the
 // host-side copy is split over a few threads.
-void film_to_host(ptc_scene *s, const float *d_src, float *dst, size_t n, cudaStream_t stream) {
-  const size_t bytes = n * sizeof(float);
+void film_to_host(ptc_scene *s, const void *d_src, void *dst, size_t bytes, cudaStream_t stream) {
   if (bytes < ((size_t)8 << 20)) {
     CK(cudaMemcpyAsync(dst, d_src, bytes, cudaMemcpyDeviceToHost, stream));
     CK(cudaStreamSynchronize(stream));
     return;
   }
-  if (s->h_film_n < n) {
+  if (s->h_film_bytes < bytes) {
     if (s->h_film) cudaFreeHost(s->h_film);
-    s->h_film = nullptr, s->h_film_n = 0;
+    s->h_film = nullptr, s->h_film_bytes = 0;
     CK(cudaMallocHost(&s->h_film, bytes));
-    s->h_film_n = n;
+    s->h_film_bytes = bytes;
   }
   CK(cudaMemcpyAsync(s->h_film, d_src, bytes, cudaMemcpyDeviceToHost, stream));
   CK(cudaStreamSynchronize(stream));
   const int nt = (int)std::min<size_t>(8, std::max<size_t>(1, std::thread::hardware_concurrency()));
   std::vector<std::thread> th;
-  const size_t per = (n + (size_t)nt - 1) / (size_t)nt;
+  const size_t per = (bytes + (size_t)nt - 1) / (size_t)nt;
   for (int t = 0; t < nt; t++) {
-    const size_t a = (size_t)t * per, b = std::min(n, a + per);
+    const size_t a = (size_t)t * per, b = std::min(bytes, a + per);
     if (a >= b) break;
-    th.emplace_back([=] { memcpy(dst + a, s->h_film + a, (b - a) * sizeof(float)); });
+    th.emplace_back([=] { memcpy(static_cast<char *>(dst) + a, s->h_film + a, b - a); });
   }
   for (auto &t : th) t.join();
+}
+
+// The scene's film -> the caller's host images, the one way every render that returns an image ends: k_resolve_film
+// into the staging buffers, then whichever of out_rgb (W*H*3 linear mean radiance) and out_u32 (W*H 0x00RRGGBB) is not
+// nullptr to the host.  counts == nullptr: every pixel x scale, else x 1 / counts[p].  `resolved`, if given, is recorded
+// once the resolve is done, before the copies.  Returns, with all the work queued on `stream` done (the event included,
+// also when no image is asked for), the number of kernels launched.
+int resolve_film_to_host(ptc_scene *s, size_t n_px, float scale, const int32_t *counts, float *out_rgb, uint32_t *out_u32,
+                         cudaStream_t stream, cudaEvent_t resolved = nullptr) {
+  if (out_rgb && s->w_film_out.n < n_px * 3) s->w_film_out.alloc(n_px * 3);
+  if (out_u32 && s->w_packed.n < n_px) s->w_packed.alloc(n_px);
+  const int launches = (out_rgb || out_u32) ? 1 : 0;
+  if (launches) {
+    k_resolve_film<<<(unsigned)((n_px + 255) / 256), 256, 0, stream>>>(s->film(), n_px, scale, counts, out_rgb ? s->w_film_out.p : nullptr,
+                                                                       out_u32 ? s->w_packed.p : nullptr);
+    CK(cudaGetLastError());
+  }
+  if (resolved) CK(cudaEventRecord(resolved, stream));
+  if (out_u32) film_to_host(s, s->w_packed.p, out_u32, n_px * sizeof(uint32_t), stream);
+  if (out_rgb) film_to_host(s, s->w_film_out.p, out_rgb, n_px * 3 * sizeof(float), stream);
+  CK(cudaStreamSynchronize(stream));
+  return launches;
 }
 
 // Device half of commit: upload the flattened scene `hs` (built) to `device` and fill s->ds.  `s` may be the handle that
@@ -707,7 +735,7 @@ void upload_scene(ptc_scene *s, const HostScene &hs, int device) {
   s->committed = true;
 }
 
-// ---- in-process multi-GPU (ptc_multi_*): scene replicated per device, work sharded, ONE NCCL reduce of the film ----
+// ---- in-process multi-GPU (ptc_multi_*): scene replicated per device, work sharded, the films reduced by NCCL ----
 // NCCL is bound at run time: a process that also hosts PyTorch must end up with ONE libnccl (dlopen by soname returns
 // the copy that is already loaded), and processes that never call ptc_multi_create never load it.
 struct NcclApi {
@@ -938,71 +966,47 @@ int ptc_render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_
                           void *cuda_stream, ptc_stats *stats) {
   PTC_GUARD_BEGIN
   require_committed(s);
+  check_render_args(cam, st, d_accum != nullptr);
   // the caller's handle is honoured as given: NULL is the legacy default stream, which orders the film atomics after
   // whatever the caller queued there (a memset of d_accum, a wait on a collective)
-  if (!d_accum) throw std::invalid_argument("null argument");
   render_accumulate(s, cam, st, d_accum, (cudaStream_t)cuda_stream, stats);
   return 0;
   PTC_GUARD_END
 }
 
-int ptc_render(ptc_scene *s, const ptc_camera *cam, const ptc_render_settings *st, float *out_rgb, ptc_stats *stats) {
+// ptc_render (out_rgb) and ptc_render_u32 (out_u32): the render into the scene's film, then one resolve of it with the
+// 1/spp of renderer.rs:85 — only the asked-for image crosses PCIe
+static int render_to_host(ptc_scene *s, const ptc_camera *cam, const ptc_render_settings *st, float *out_rgb, uint32_t *out_u32,
+                          ptc_stats *stats) {
   PTC_GUARD_BEGIN
   require_committed(s);
-  if (!st || !out_rgb) throw std::invalid_argument("null argument");
-  if (st->width <= 0 || st->height <= 0 || st->spp <= 0) throw std::invalid_argument("bad render settings");
-  CK(cudaSetDevice(s->device));
-  const size_t n = (size_t)st->width * st->height * 3;
-  if (s->w_film.n < n) s->w_film.alloc(n);
-  if (s->w_film_out.n < n) s->w_film_out.alloc(n);
-  DevBuf<float> &accum = s->w_film, &out = s->w_film_out;
-  cudaStream_t stream = s->own_stream;
-  CK(cudaMemsetAsync(accum.p, 0, n * sizeof(float), stream));
-  render_accumulate(s, cam, st, accum.p, stream, stats);
-  const float inv_spp = 1.0f / (float)st->spp;  // renderer.rs:85
-  k_scale<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(accum.p, out.p, n, inv_spp);
-  CK(cudaGetLastError());
-  film_to_host(s, out.p, out_rgb, n, stream);
-  if (stats) stats->kernel_launches += 1;
+  check_render_args(cam, st, out_rgb || out_u32);
+  render_accumulate(s, cam, st, nullptr, s->own_stream, stats);
+  const int launches = resolve_film_to_host(s, (size_t)st->width * st->height, 1.0f / (float)st->spp, nullptr, out_rgb, out_u32, s->own_stream);
+  if (stats) stats->kernel_launches += launches;
   return 0;
   PTC_GUARD_END
 }
 
+int ptc_render(ptc_scene *s, const ptc_camera *cam, const ptc_render_settings *st, float *out_rgb, ptc_stats *stats) {
+  return render_to_host(s, cam, st, out_rgb, nullptr, stats);
+}
+
 int ptc_render_u32(ptc_scene *s, const ptc_camera *cam, const ptc_render_settings *st, uint32_t *out_u32, ptc_stats *stats) {
-  PTC_GUARD_BEGIN
-  require_committed(s);
-  if (!st || !out_u32) throw std::invalid_argument("null argument");
-  if (st->width <= 0 || st->height <= 0 || st->spp <= 0) throw std::invalid_argument("bad render settings");
-  CK(cudaSetDevice(s->device));
-  const size_t px = (size_t)st->width * st->height, n = px * 3;
-  if (s->w_film.n < n) s->w_film.alloc(n);
-  if (s->w_packed.n < px) s->w_packed.alloc(px);
-  cudaStream_t stream = s->own_stream;
-  CK(cudaMemsetAsync(s->w_film.p, 0, n * sizeof(float), stream));
-  render_accumulate(s, cam, st, s->w_film.p, stream, stats);
-  // renderer.rs:103 (x 1/spp) and :112-120 (sqrt, clamp, x255, truncate, pack) on the device: only the packed image crosses PCIe
-  k_resolve<<<(unsigned)((px + 255) / 256), 256, 0, stream>>>(s->w_film.p, px, 1.0f / (float)st->spp, s->w_packed.p);
-  CK(cudaGetLastError());
-  CK(cudaMemcpyAsync(out_u32, s->w_packed.p, px * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
-  CK(cudaStreamSynchronize(stream));
-  if (stats) stats->kernel_launches += 1;
-  return 0;
-  PTC_GUARD_END
+  return render_to_host(s, cam, st, nullptr, out_u32, stats);
 }
 
 int ptc_render_adaptive(ptc_scene *s, const ptc_camera *cam, const ptc_render_settings *st, const ptc_adaptive *ad, float *out_rgb,
                         uint32_t *out_u32, int32_t *out_spp, ptc_stats *stats) {
   PTC_GUARD_BEGIN
   // the arguments first, the scene's state after them
-  if (!s || !cam || !st || !ad) throw std::invalid_argument("null argument");
-  if (st->width <= 0 || st->height <= 0 || st->spp <= 0) throw std::invalid_argument("bad render settings");
+  if (!s || !ad) throw std::invalid_argument("null argument");
+  check_render_args(cam, st, true);  // every output may be NULL
   if (st->sample_begin != 0 || st->sample_end != 0 || st->tile_mod != 0)
     throw std::invalid_argument("ptc_render_adaptive schedules the samples itself: sample_begin, sample_end and tile_mod must be 0");
   if (ad->min_spp < 2 || ad->min_spp % 2 != 0 || ad->min_spp > st->spp) throw std::invalid_argument("min_spp must be even, >= 2 and <= spp");
   if (!(ad->threshold >= 0.0f)) throw std::invalid_argument("threshold must be >= 0");
-  check_render_flags(st);
   require_committed(s);
-  if ((int64_t)st->width * st->height > (int64_t)0x3fffffff) throw std::invalid_argument("image too large");
   CK(cudaSetDevice(s->device));
   ensure_ctl(s);
   const uint32_t n_px = (uint32_t)st->width * (uint32_t)st->height;
@@ -1036,7 +1040,7 @@ int ptc_render_adaptive(ptc_scene *s, const ptc_camera *cam, const ptc_render_se
   const int half = ad->min_spp / 2;
   CK(cudaEventRecord(s->ev_adapt_begin, stream));
   run_pass(0, half, Pass());
-  const Film f{s->film_sum.p, s->film_flags.p};
+  const Film f = s->film();
   float *vp = s->w_adapt_vp.p;
   CK(cudaMemsetAsync(vp, 0, (size_t)n_px * 3 * sizeof(float), stream));
   k_film_to_accum<<<(unsigned)(((size_t)n_px * 3 + 255) / 256), 256, 0, stream>>>(f, n_px, vp);
@@ -1073,20 +1077,9 @@ int ptc_render_adaptive(ptc_scene *s, const ptc_camera *cam, const ptc_render_se
     m = n, n = next;
   }
 
-  // one resolve of every pixel at its own count
-  if (out_rgb && s->w_film_out.n < (size_t)n_px * 3) s->w_film_out.alloc((size_t)n_px * 3);
-  if (out_u32 && s->w_packed.n < n_px) s->w_packed.alloc(n_px);
-  if (out_rgb || out_u32) {
-    k_resolve_adaptive<<<nb, 256, 0, stream>>>(f, n_px, s->w_adapt_spp.p, out_rgb ? s->w_film_out.p : nullptr,
-                                               out_u32 ? s->w_packed.p : nullptr);
-    launches += 1;
-    CK(cudaGetLastError());
-  }
-  CK(cudaEventRecord(s->ev_adapt_end, stream));
-  if (out_u32) CK(cudaMemcpyAsync(out_u32, s->w_packed.p, (size_t)n_px * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
-  if (out_spp) CK(cudaMemcpyAsync(out_spp, s->w_adapt_spp.p, (size_t)n_px * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
-  if (out_rgb) film_to_host(s, s->w_film_out.p, out_rgb, (size_t)n_px * 3, stream);
-  CK(cudaStreamSynchronize(stream));
+  // one resolve of every pixel at its own count (the scale is unused), the end of render_ms
+  launches += resolve_film_to_host(s, n_px, 1.0f, s->w_adapt_spp.p, out_rgb, out_u32, stream, s->ev_adapt_end);
+  if (out_spp) film_to_host(s, s->w_adapt_spp.p, out_spp, (size_t)n_px * sizeof(int32_t), stream);
   if (stats) {
     *stats = total;
     stats->kernel_launches = launches;
@@ -1336,28 +1329,24 @@ void ptc_multi_destroy(ptc_multi *m) { delete m; }
 static int multi_render(ptc_multi *m, const ptc_camera *cam, const ptc_render_settings *st, int shard_mode, float *out_rgb, uint32_t *out_u32,
                         ptc_stats *stats) {
   PTC_GUARD_BEGIN
-  if (!m || !cam || !st || (!out_rgb && !out_u32)) throw std::invalid_argument("null argument");
-  if (st->width <= 0 || st->height <= 0 || st->spp <= 0) throw std::invalid_argument("bad render settings");
+  if (!m) throw std::invalid_argument("null argument");
+  check_render_args(cam, st, out_rgb || out_u32);
   if (st->tile_mod > 0) throw std::invalid_argument("ptc_multi_render shards by itself: tile_mod must be 0");
   if (shard_mode != PTC_SHARD_SAMPLES && shard_mode != PTC_SHARD_TILES) throw std::invalid_argument("bad shard mode");
-  check_render_flags(st);
   const int n = (int)m->scenes.size();
-  int s_begin = st->sample_begin, s_end = st->sample_end;
-  if (s_begin == 0 && s_end == 0) s_end = st->spp;
-  if (s_begin < 0 || s_end < s_begin) throw std::invalid_argument("bad sample range");
-  const size_t count = (size_t)st->width * st->height * 3;
+  int s_begin, s_end;
+  sample_range(st, s_begin, s_end);
+  const size_t n_px = (size_t)st->width * st->height;
   std::vector<ptc_stats> per((size_t)n);
   std::vector<std::string> errors((size_t)n);
   const auto t0 = std::chrono::steady_clock::now();
   // Everything that can fail for lack of memory happens before the first thread starts: a worker that dropped out
   // ahead of the collective would leave the other devices waiting in ncclReduce for ever.
   if (n > 1 && m->comms_dead) m->init_comms();
-  const size_t n_px = count / 3;
   for (int i = 0; i < n; i++) {
     ptc_scene *s = m->scenes[(size_t)i];
     CK(cudaSetDevice(s->device));
-    if (s->film_sum.n < count) s->film_sum.alloc(count);
-    if (s->film_flags.n < n_px) s->film_flags.alloc(n_px);
+    ensure_film(s, n_px);
   }
   std::mutex abort_mutex;
   auto work = [&](int i) {
@@ -1378,12 +1367,8 @@ static int multi_render(ptc_multi *m, const ptc_camera *cam, const ptc_render_se
         mine.tile_mod = n, mine.tile_rem = i;
       }
       memset(&per[(size_t)i], 0, sizeof(ptc_stats));
-      if (idle) {
-        CK(cudaMemsetAsync(s->film_sum.p, 0, count * sizeof(long long), stream));
-        CK(cudaMemsetAsync(s->film_flags.p, 0, n_px * sizeof(unsigned long long), stream));
-      } else {
-        render_accumulate(s, cam, &mine, nullptr, stream, &per[(size_t)i]);  // leaves the shard in the device's fixed-point film
-      }
+      if (idle) clear_film(s, n_px, stream);
+      else render_accumulate(s, cam, &mine, nullptr, stream, &per[(size_t)i]);  // leaves the shard in the device's fixed-point film
       film_ok = true;
     } catch (std::exception &e) {
       errors[(size_t)i] = e.what();
@@ -1397,11 +1382,8 @@ static int multi_render(ptc_multi *m, const ptc_camera *cam, const ptc_render_se
     // the order NCCL adds in.  A device whose render failed still takes part, with a zeroed film, so that the others return;
     // if it cannot even do that the communicators are aborted (and re-created by the next call).
     try {
-      if (!film_ok) {
-        CK(cudaMemsetAsync(s->film_sum.p, 0, count * sizeof(long long), stream));
-        CK(cudaMemsetAsync(s->film_flags.p, 0, n_px * sizeof(unsigned long long), stream));
-      }
-      m->nccl.check(m->nccl.Reduce(s->film_sum.p, s->film_sum.p, count, ncclInt64, ncclSum, 0, m->comms[(size_t)i], stream), "ncclReduce(film)");
+      if (!film_ok) clear_film(s, n_px, stream);
+      m->nccl.check(m->nccl.Reduce(s->film_sum.p, s->film_sum.p, n_px * 3, ncclInt64, ncclSum, 0, m->comms[(size_t)i], stream), "ncclReduce(film)");
       m->nccl.check(m->nccl.Reduce(s->film_flags.p, s->film_flags.p, n_px, ncclUint64, ncclSum, 0, m->comms[(size_t)i], stream), "ncclReduce(flags)");
       CK(cudaStreamSynchronize(stream));
     } catch (std::exception &e) {
@@ -1418,23 +1400,7 @@ static int multi_render(ptc_multi *m, const ptc_camera *cam, const ptc_render_se
     if (!errors[(size_t)i].empty()) throw CudaError("device " + std::to_string(m->devices[(size_t)i]) + ": " + errors[(size_t)i]);
   ptc_scene *root = m->primary;
   CK(cudaSetDevice(root->device));
-  if (root->w_film.n < count) root->w_film.alloc(count);
-  CK(cudaMemsetAsync(root->w_film.p, 0, count * sizeof(float), root->own_stream));
-  k_film_to_accum<<<(unsigned)((count + 255) / 256), 256, 0, root->own_stream>>>(Film{root->film_sum.p, root->film_flags.p}, n_px, root->w_film.p);
-  CK(cudaGetLastError());
-  const float inv_spp = 1.0f / (float)st->spp;  // renderer.rs:85
-  if (out_rgb) {
-    if (root->w_film_out.n < count) root->w_film_out.alloc(count);
-    k_scale<<<(unsigned)((count + 255) / 256), 256, 0, root->own_stream>>>(root->w_film.p, root->w_film_out.p, count, inv_spp);
-    CK(cudaGetLastError());
-    film_to_host(root, root->w_film_out.p, out_rgb, count, root->own_stream);
-  } else {  // renderer.rs:103,112-120 on the device; the packed image is a third of the film
-    const size_t px = count / 3;
-    if (root->w_packed.n < px) root->w_packed.alloc(px);
-    k_resolve<<<(unsigned)((px + 255) / 256), 256, 0, root->own_stream>>>(root->w_film.p, px, inv_spp, root->w_packed.p);
-    CK(cudaGetLastError());
-    film_to_host(root, reinterpret_cast<const float *>(root->w_packed.p), reinterpret_cast<float *>(out_u32), px, root->own_stream);
-  }
+  const int launches = resolve_film_to_host(root, n_px, 1.0f / (float)st->spp, nullptr, out_rgb, out_u32, root->own_stream);  // renderer.rs:85
   if (stats) {
     memset(stats, 0, sizeof(*stats));
     for (const ptc_stats &p : per) {
@@ -1442,8 +1408,8 @@ static int multi_render(ptc_multi *m, const ptc_camera *cam, const ptc_render_se
       stats->iterations = std::max(stats->iterations, p.iterations);
       stats->nodes_visited += p.nodes_visited, stats->tris_tested += p.tris_tested, stats->mesh_rays += p.mesh_rays;
     }
-    stats->kernel_launches += 1;
-    // wall clock of the whole call on the host: renders on all devices, the reduce, the scale and the copy out
+    stats->kernel_launches += launches;
+    // wall clock of the whole call on the host: renders on all devices, the reduce, the resolve and the copy out
     stats->render_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
   }
   return 0;

@@ -192,3 +192,17 @@ def test_deterministic_and_pool_invariant(pt):
         for k in range(3):
             assert np.array_equal(a[k], x[k]), k
         assert x[3].paths == a[3].paths and x[3].rays == a[3].rays
+
+
+@pytest.mark.parametrize("min_spp", [64, 4])  # min_spp = spp: the last work queued is k_adapt_init, not a render pass
+def test_stats_only_call_without_outputs(pt, min_spp):
+    # every output may be NULL: the call still returns once its work (and the render_ms event) is done
+    import ctypes as C
+    s, cs, base, _ = _commit(pt, "cornell")
+    st = s.render_settings(**base)
+    *_, want = cs.render_adaptive(s.camera, st, min_spp, 0.05)
+    stats = pt.Stats()
+    ad = pt.Adaptive(min_spp, 0.05)
+    rc = pt.core().ptc_render_adaptive(cs._h, C.byref(s.camera), C.byref(st), C.byref(ad), None, None, None, C.byref(stats))
+    assert rc == 0, pt.core().ptc_last_error()
+    assert stats.paths == want.paths and stats.render_ms > 0

@@ -213,6 +213,31 @@ typedef struct ptc_adaptive {
 } ptc_adaptive;
 int ptc_render_adaptive(ptc_scene *, const ptc_camera *, const ptc_render_settings *, const ptc_adaptive *, float *out_rgb,
                         uint32_t *out_u32, int32_t *out_spp, ptc_stats *stats);
+/* Progressive rendering: the frame is rendered in passes, and after each pass on_preview is shown the image of all
+ * samples so far.  Schedule: n_0 = first_spp, n_{j+1} = min(n_j + step_j, spp) with step_j = n_j (max_pass_spp = 0: the
+ * samples double every pass) or min(n_j, max_pass_spp); pass j renders samples [n_{j-1}, n_j) of every pixel.  Philox is
+ * keyed on (pixel, sample) and the film sums are fixed-point, so preview j is, bit for bit, ptc_render_u32 at spp = n_j,
+ * and the final images are ptc_render / ptc_render_u32 at settings->spp.
+ * Threads: a worker thread inside the call drives the render; on_preview always runs on the calling thread, once per
+ * pass, in pass order.  The device renders pass j + 1 while on_preview shows preview j, and pass j starts only once
+ * on_preview of pass j - 2 has returned.  `image` (W*H 0x00RRGGBB) is valid during the callback only.
+ * Stop: a nonzero return from on_preview of pass k starts no later pass and makes no later callback; the pass in flight,
+ * if any, is finished and discarded; the outputs are preview k's images and *out_samples = n_k.  Otherwise the outputs
+ * are the last pass's images and *out_samples = spp.  on_preview may be NULL (the passes run back to back), and every
+ * output may be NULL: out_rgb W*H*3 linear mean radiance, out_u32 W*H 0x00RRGGBB, out_samples the samples they hold.
+ * settings: sample_begin = sample_end = 0 and tile_mod = 0, else PTC_E_INVALID; flags as in ptc_render.  Single device.
+ * stats: summed over every pass rendered (a discarded one included); render_ms from the first pass to the last preview
+ * image written (device events).  The arguments are checked before the scene's state: PTC_E_INVALID for bad ones even
+ * on an uncommitted scene. */
+typedef struct ptc_progressive {
+  int32_t first_spp;    /* samples of pass 0: 1 <= first_spp <= spp */
+  int32_t max_pass_spp; /* 0: every later pass doubles the samples so far; > 0: no later pass renders more than this */
+} ptc_progressive;
+/* return 0 to go on, anything else to stop; `image` = W*H 0x00RRGGBB, valid during the call only */
+typedef int32_t (*ptc_preview_fn)(void *user, int32_t pass, int32_t samples, const uint32_t *image);
+int ptc_render_progressive(ptc_scene *, const ptc_camera *, const ptc_render_settings *, const ptc_progressive *,
+                           ptc_preview_fn on_preview, void *user, float *out_rgb, uint32_t *out_u32,
+                           int32_t *out_samples, ptc_stats *stats);
 /* Film resolve, renderer.rs:112-120 + color.rs:87-93: out = pack(sqrt(rgb * scale)).  Device and host buffers. */
 int ptc_resolve_device(const float *d_rgb, int64_t n_pixels, float scale, uint32_t *d_out, void *cuda_stream);
 int ptc_resolve_u32(ptc_scene *, const float *rgb, int64_t n_pixels, float scale, uint32_t *out);

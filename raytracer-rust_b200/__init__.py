@@ -49,6 +49,14 @@ class Adaptive(C.Structure):  # ptc_adaptive
     _fields_ = [("min_spp", C.c_int32), ("threshold", C.c_float)]
 
 
+class ProgressiveSettings(C.Structure):  # ptc_progressive
+    _fields_ = [("first_spp", C.c_int32), ("max_pass_spp", C.c_int32)]
+
+
+# ptc_preview_fn: (user, pass, samples, image) -> 0 to go on, anything else to stop
+PREVIEW_FN = C.CFUNCTYPE(C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.POINTER(C.c_uint32))
+
+
 class Hit(C.Structure):  # ptc_hit
     _fields_ = [("object", C.c_int32), ("triangle", C.c_int32), ("t", C.c_float), ("position", C.c_float * 3),
                 ("normal", C.c_float * 3), ("front_face", C.c_int32), ("material", C.c_int32)]
@@ -151,6 +159,8 @@ def core():
     L.ptc_render_u32.argtypes = [_vp, C.POINTER(Camera), C.POINTER(RenderSettings), _vp, C.POINTER(Stats)]
     L.ptc_render_adaptive.argtypes = [_vp, C.POINTER(Camera), C.POINTER(RenderSettings), C.POINTER(Adaptive), _F, _vp, _vp,
                                       C.POINTER(Stats)]
+    L.ptc_render_progressive.argtypes = [_vp, C.POINTER(Camera), C.POINTER(RenderSettings), C.POINTER(ProgressiveSettings),
+                                         PREVIEW_FN, _vp, _F, _vp, C.POINTER(C.c_int32), C.POINTER(Stats)]
     L.ptc_render_accumulate.argtypes = [_vp, C.POINTER(Camera), C.POINTER(RenderSettings), _vp, _vp, C.POINTER(Stats)]
     L.ptc_resolve_device.argtypes = [_vp, C.c_int64, C.c_float, _vp, _vp]
     L.ptc_resolve_u32.argtypes = [_vp, _F, C.c_int64, C.c_float, _vp]
@@ -558,6 +568,36 @@ class CoreScene:
         _ck(core().ptc_render_adaptive(self._h, C.byref(camera), C.byref(settings), C.byref(ad), _fptr(rgb), u32.ctypes.data,
                                        spp.ctypes.data, C.byref(st)))
         return rgb, u32, spp, st
+
+    def render_progressive(self, camera, settings, first_spp=1, max_pass_spp=0, on_preview=None):
+        """Progressive rendering (ptc_render_progressive): the frame in passes of first_spp, then doubling (capped at
+        max_pass_spp samples per pass if > 0) up to settings.spp samples.  on_preview(pass, samples, u32) is called on
+        this thread after every pass with a copy of the packed image [H*W] so far, which is render_u32 at spp = samples;
+        a truthy return stops the render, and an exception raised in it stops the render and is re-raised here.
+        -> (rgb [H,W,3] float32, u32 [H*W] 0x00RRGGBB, samples, Stats): the last preview's images and sample count."""
+        rgb = np.empty((settings.height, settings.width, 3), np.float32)
+        u32 = np.empty(settings.height * settings.width, np.uint32)
+        samples = C.c_int32()
+        st = Stats()
+        raised = []
+        callback = PREVIEW_FN()  # NULL
+        if on_preview is not None:
+            n_px = settings.height * settings.width
+
+            def preview(_user, pass_, n, image):
+                try:
+                    return 1 if on_preview(pass_, n, np.ctypeslib.as_array(image, shape=(n_px,)).copy()) else 0
+                except BaseException as e:  # nothing may unwind through the C frames: stop, and raise it after the call
+                    raised.append(e)
+                    return 1
+            callback = PREVIEW_FN(preview)
+        pg = ProgressiveSettings(first_spp, max_pass_spp)
+        rc = core().ptc_render_progressive(self._h, C.byref(camera), C.byref(settings), C.byref(pg), callback, None, _fptr(rgb),
+                                           u32.ctypes.data, C.byref(samples), C.byref(st))
+        if raised:
+            raise raised[0]
+        _ck(rc)
+        return rgb, u32, samples.value, st
 
     def multi(self, devices):
         """In-process multi-GPU (ptc_multi_*): this committed scene replicated on `devices` (devices[0] = its own)."""

@@ -15,6 +15,8 @@
 
 #include <algorithm>
 #include <chrono>
+#include <condition_variable>
+#include <exception>
 #include <memory>
 #include <mutex>
 #include <thread>
@@ -166,6 +168,15 @@ struct ptc_scene {
   DevBuf<int32_t> w_adapt_spp;
   DevBuf<uint32_t> w_adapt_n;
   DevBuf<uint8_t> w_adapt_tmp;
+  // ptc_render_progressive: two preview slots (pass j resolves into slot j % 2; the rgb image only when the caller wants
+  // it), grow-only; the pinned buffer the calling thread shows previews from, and the stream it copies them on
+  DevBuf<uint32_t> w_prog_packed[2];
+  DevBuf<float> w_prog_rgb[2];
+  uint32_t *h_preview = nullptr;
+  size_t h_preview_px = 0;
+  cudaStream_t preview_stream = nullptr;
+  cudaEvent_t ev_prog_slot[2] = {nullptr, nullptr};  // recorded once slot j % 2 holds preview j
+  cudaEvent_t ev_prog_begin = nullptr;                // render_ms: from here to the last slot event
   DevBuf<Ctl> d_ctl;
   Ctl *h_ctl = nullptr;  // pinned ring
   uint32_t *h_progress = nullptr;  // pinned + mapped: the word k_extend_pre reports the state of the render in
@@ -197,6 +208,11 @@ struct ptc_scene {
     if (ev_end) cudaEventDestroy(ev_end);
     if (ev_adapt_begin) cudaEventDestroy(ev_adapt_begin);
     if (ev_adapt_end) cudaEventDestroy(ev_adapt_end);
+    if (h_preview) cudaFreeHost(h_preview);
+    for (auto &e : ev_prog_slot)
+      if (e) cudaEventDestroy(e);
+    if (ev_prog_begin) cudaEventDestroy(ev_prog_begin);
+    if (preview_stream) cudaStreamDestroy(preview_stream);
     for (auto &e : timing_events) cudaEventDestroy(e);
     if (own_stream) cudaStreamDestroy(own_stream);
   }
@@ -609,6 +625,20 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
     stats->tris_tested = fin.tris;
     stats->mesh_rays = fin.mesh_rays;
   }
+}
+
+// One pass of a render made of passes (ptc_render_adaptive, ptc_render_progressive): samples [first, last) of `pass`
+// into the scene's film, its stats added to `total`.  render_ms is left alone: the caller brackets all its passes.
+void render_pass(ptc_scene *s, const ptc_camera *cam, const ptc_render_settings *st, int first, int last, const Pass &pass,
+                 cudaStream_t stream, ptc_stats &total) {
+  ptc_render_settings ps = *st;
+  ps.sample_begin = first, ps.sample_end = last;
+  ptc_stats p;
+  render_accumulate(s, cam, &ps, nullptr, stream, &p, pass);
+  total.paths += p.paths, total.rays += p.rays, total.iterations += p.iterations, total.kernel_launches += p.kernel_launches;
+  total.extend_ms += p.extend_ms, total.shade_ms += p.shade_ms, total.extend_launches += p.extend_launches;
+  total.pre_ms += p.pre_ms, total.traverse_ms += p.traverse_ms, total.post_ms += p.post_ms;
+  total.nodes_visited += p.nodes_visited, total.tris_tested += p.tris_tested, total.mesh_rays += p.mesh_rays;
 }
 
 int fail(int code, const std::string &msg) {
@@ -1024,22 +1054,12 @@ int ptc_render_adaptive(ptc_scene *s, const ptc_camera *cam, const ptc_render_se
 
   ptc_stats total;
   memset(&total, 0, sizeof(total));
-  uint64_t launches = 0;
-  auto run_pass = [&](int first, int last, const Pass &pass) {
-    ptc_render_settings ps = *st;
-    ps.sample_begin = first, ps.sample_end = last;
-    ptc_stats p;
-    render_accumulate(s, cam, &ps, nullptr, stream, &p, pass);
-    total.paths += p.paths, total.rays += p.rays, total.iterations += p.iterations, launches += p.kernel_launches;
-    total.extend_ms += p.extend_ms, total.shade_ms += p.shade_ms, total.extend_launches += p.extend_launches;
-    total.pre_ms += p.pre_ms, total.traverse_ms += p.traverse_ms, total.post_ms += p.post_ms;
-    total.nodes_visited += p.nodes_visited, total.tris_tested += p.tris_tested, total.mesh_rays += p.mesh_rays;
-  };
+  uint64_t &launches = total.kernel_launches;
 
   // passes 0 and 1 over the tiles, the snapshot between them
   const int half = ad->min_spp / 2;
   CK(cudaEventRecord(s->ev_adapt_begin, stream));
-  run_pass(0, half, Pass());
+  render_pass(s, cam, st, 0, half, Pass(), stream, total);
   const Film f = s->film();
   float *vp = s->w_adapt_vp.p;
   CK(cudaMemsetAsync(vp, 0, (size_t)n_px * 3 * sizeof(float), stream));
@@ -1047,7 +1067,7 @@ int ptc_render_adaptive(ptc_scene *s, const ptc_camera *cam, const ptc_render_se
   launches += 1;
   Pass more;
   more.clear_film = false;
-  run_pass(half, ad->min_spp, more);
+  render_pass(s, cam, st, half, ad->min_spp, more, stream, total);
   k_adapt_init<<<nb, 256, 0, stream>>>(n_px, st->spp, s->w_adapt_list[0].p, s->w_adapt_needs.p, s->w_adapt_spp.p);
   launches += 1;
   CK(cudaGetLastError());
@@ -1073,7 +1093,7 @@ int ptc_render_adaptive(ptc_scene *s, const ptc_camera *cam, const ptc_render_se
     if (n_list == 0) break;
     more.pixels = s->w_adapt_list[cur].p, more.n_pixels = n_list;
     const int next = adapt_next_end(n, st->spp);
-    run_pass(n, next, more);
+    render_pass(s, cam, st, n, next, more, stream, total);
     m = n, n = next;
   }
 
@@ -1082,9 +1102,154 @@ int ptc_render_adaptive(ptc_scene *s, const ptc_camera *cam, const ptc_render_se
   if (out_spp) film_to_host(s, s->w_adapt_spp.p, out_spp, (size_t)n_px * sizeof(int32_t), stream);
   if (stats) {
     *stats = total;
-    stats->kernel_launches = launches;
     float ms = 0.0f;
     CK(cudaEventElapsedTime(&ms, s->ev_adapt_begin, s->ev_adapt_end));
+    stats->render_ms = ms;
+  }
+  return 0;
+  PTC_GUARD_END
+}
+
+// ptc_render_progressive's schedule: the samples after pass j + 1, given n after pass j
+static int progressive_next(int n, int spp, int max_pass_spp) {
+  const int64_t step = max_pass_spp > 0 ? std::min(n, max_pass_spp) : n;
+  return (int)std::min<int64_t>((int64_t)n + step, spp);
+}
+
+int ptc_render_progressive(ptc_scene *s, const ptc_camera *cam, const ptc_render_settings *st, const ptc_progressive *pg,
+                           ptc_preview_fn on_preview, void *user, float *out_rgb, uint32_t *out_u32, int32_t *out_samples,
+                           ptc_stats *stats) {
+  PTC_GUARD_BEGIN
+  // the arguments first, the scene's state after them
+  if (!s || !pg) throw std::invalid_argument("null argument");
+  check_render_args(cam, st, true);  // every output may be NULL
+  if (st->sample_begin != 0 || st->sample_end != 0 || st->tile_mod != 0)
+    throw std::invalid_argument("ptc_render_progressive schedules the samples itself: sample_begin, sample_end and tile_mod must be 0");
+  if (pg->first_spp < 1 || pg->first_spp > st->spp) throw std::invalid_argument("first_spp must be >= 1 and <= spp");
+  if (pg->max_pass_spp < 0) throw std::invalid_argument("max_pass_spp must be >= 0");
+  require_committed(s);
+  CK(cudaSetDevice(s->device));
+  ensure_ctl(s);
+  const size_t n_px = (size_t)st->width * st->height;
+  for (int k = 0; k < 2; k++) {
+    if (s->w_prog_packed[k].n < n_px) s->w_prog_packed[k].alloc(n_px);
+    if (out_rgb && s->w_prog_rgb[k].n < n_px * 3) s->w_prog_rgb[k].alloc(n_px * 3);
+    if (!s->ev_prog_slot[k]) CK(cudaEventCreate(&s->ev_prog_slot[k]));
+  }
+  if (!s->ev_prog_begin) CK(cudaEventCreate(&s->ev_prog_begin));
+  if (!s->preview_stream) CK(cudaStreamCreateWithFlags(&s->preview_stream, cudaStreamNonBlocking));
+  if (on_preview && s->h_preview_px < n_px) {
+    if (s->h_preview) cudaFreeHost(s->h_preview);
+    s->h_preview = nullptr, s->h_preview_px = 0;
+    CK(cudaMallocHost(&s->h_preview, n_px * sizeof(uint32_t)));
+    s->h_preview_px = n_px;
+  }
+  cudaStream_t stream = s->own_stream;
+
+  // What the two threads share, under `mu`.  The worker publishes pass j (ready = j + 1, samples[j % 2]) once its slot
+  // event is recorded; the calling thread publishes callback j's return (shown = j + 1) and a stop.
+  std::mutex mu;
+  std::condition_variable cv;
+  int ready = 0, shown = 0;
+  int32_t samples[2] = {0, 0};
+  bool stop = false, worker_done = false;
+  std::exception_ptr worker_error;
+  ptc_stats total;
+  memset(&total, 0, sizeof(total));
+  cudaEvent_t last_slot_event = nullptr;
+
+  auto worker = [&]() {
+    try {
+      CK(cudaSetDevice(s->device));
+      CK(cudaEventRecord(s->ev_prog_begin, stream));
+      int n = 0;
+      for (int j = 0; n < st->spp; j++) {
+        {  // pass j overwrites slot j % 2: preview j - 2 must have been shown
+          std::unique_lock<std::mutex> lk(mu);
+          cv.wait(lk, [&] { return stop || !on_preview || shown >= j - 1; });
+          if (stop) break;
+        }
+        const int next = j == 0 ? pg->first_spp : progressive_next(n, st->spp, pg->max_pass_spp);
+        Pass pass;
+        pass.clear_film = j == 0;
+        render_pass(s, cam, st, n, next, pass, stream, total);
+        k_resolve_film<<<(unsigned)((n_px + 255) / 256), 256, 0, stream>>>(s->film(), n_px, 1.0f / (float)next, nullptr,
+                                                                           out_rgb ? s->w_prog_rgb[j & 1].p : nullptr,
+                                                                           s->w_prog_packed[j & 1].p);
+        CK(cudaGetLastError());
+        total.kernel_launches += 1;
+        CK(cudaEventRecord(s->ev_prog_slot[j & 1], stream));
+        last_slot_event = s->ev_prog_slot[j & 1];
+        n = next;
+        {
+          std::lock_guard<std::mutex> lk(mu);
+          samples[j & 1] = n, ready = j + 1;
+        }
+        cv.notify_all();
+      }
+    } catch (...) {
+      std::lock_guard<std::mutex> lk(mu);
+      worker_error = std::current_exception();
+    }
+    {
+      std::lock_guard<std::mutex> lk(mu);
+      worker_done = true;
+    }
+    cv.notify_all();
+  };
+
+  // The worker is joined on every way out of this scope: told to stop, it finishes the pass in flight and starts no other.
+  struct Joiner {
+    std::thread th;
+    std::mutex &mu;
+    std::condition_variable &cv;
+    bool &stop;
+    void join() {
+      if (!th.joinable()) return;
+      {
+        std::lock_guard<std::mutex> lk(mu);
+        stop = true;
+      }
+      cv.notify_all();
+      th.join();
+    }
+    ~Joiner() { join(); }
+  } joiner{std::thread(worker), mu, cv, stop};
+
+  int last = -1;  // the preview the outputs are: the one the callback stopped at, else the last pass's
+  for (int j = 0;; j++) {
+    int32_t n_j;
+    {
+      std::unique_lock<std::mutex> lk(mu);
+      cv.wait(lk, [&] { return ready > j || worker_done; });
+      if (ready <= j) break;
+      n_j = samples[j & 1];
+    }
+    last = j;
+    if (!on_preview) continue;
+    CK(cudaStreamWaitEvent(s->preview_stream, s->ev_prog_slot[j & 1], 0));
+    CK(cudaMemcpyAsync(s->h_preview, s->w_prog_packed[j & 1].p, n_px * sizeof(uint32_t), cudaMemcpyDeviceToHost, s->preview_stream));
+    CK(cudaStreamSynchronize(s->preview_stream));
+    const bool stop_here = on_preview(user, j, n_j, s->h_preview) != 0;
+    {
+      std::lock_guard<std::mutex> lk(mu);
+      shown = j + 1;
+      stop = stop || stop_here;
+    }
+    cv.notify_all();
+    if (stop_here) break;
+  }
+  joiner.join();
+  if (worker_error) std::rethrow_exception(worker_error);  // (without an error the worker has published pass 0 at least)
+  // the worker is gone: the render stream and the staging buffer are this thread's again
+  CK(cudaStreamSynchronize(stream));
+  if (out_u32) film_to_host(s, s->w_prog_packed[last & 1].p, out_u32, n_px * sizeof(uint32_t), stream);
+  if (out_rgb) film_to_host(s, s->w_prog_rgb[last & 1].p, out_rgb, n_px * 3 * sizeof(float), stream);
+  if (out_samples) *out_samples = samples[last & 1];
+  if (stats) {
+    *stats = total;
+    float ms = 0.0f;
+    CK(cudaEventElapsedTime(&ms, s->ev_prog_begin, last_slot_event));
     stats->render_ms = ms;
   }
   return 0;

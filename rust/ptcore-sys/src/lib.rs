@@ -100,6 +100,18 @@ pub struct ptc_adaptive {
     pub threshold: f32,
 }
 
+/// ptc_render_progressive's schedule: pass 0 renders first_spp samples (1 <= first_spp <= spp), every later pass doubles
+/// the samples so far (max_pass_spp = 0) or adds at most max_pass_spp (> 0)
+#[repr(C)]
+#[derive(Clone, Copy, Default)]
+pub struct ptc_progressive {
+    pub first_spp: i32,
+    pub max_pass_spp: i32,
+}
+
+/// (user, pass, samples, image: W*H 0x00RRGGBB, valid during the call only) -> 0 to go on, anything else to stop
+pub type ptc_preview_fn = Option<unsafe extern "C" fn(*mut c_void, i32, i32, *const u32) -> i32>;
+
 #[repr(C)]
 pub struct ptc_scene {
     _private: [u8; 0],
@@ -133,6 +145,11 @@ extern "C" {
     /// adaptive sampling, one device (include/ptcore.h); every output may be null
     pub fn ptc_render_adaptive(s: *mut ptc_scene, cam: *const ptc_camera, st: *const ptc_render_settings, ad: *const ptc_adaptive,
                                out_rgb: *mut f32, out_u32: *mut u32, out_spp: *mut i32, stats: *mut ptc_stats) -> c_int;
+    /// progressive rendering, one device (include/ptcore.h): on_preview runs on the calling thread after every pass;
+    /// on_preview and every output may be null
+    pub fn ptc_render_progressive(s: *mut ptc_scene, cam: *const ptc_camera, st: *const ptc_render_settings, pg: *const ptc_progressive,
+                                  on_preview: ptc_preview_fn, user: *mut c_void, out_rgb: *mut f32, out_u32: *mut u32,
+                                  out_samples: *mut i32, stats: *mut ptc_stats) -> c_int;
     pub fn ptc_render_accumulate(s: *mut ptc_scene, cam: *const ptc_camera, st: *const ptc_render_settings, d_accum: *mut f32,
                                  cuda_stream: *mut c_void, stats: *mut ptc_stats) -> c_int;
     pub fn ptc_resolve_u32(s: *mut ptc_scene, rgb: *const f32, n_pixels: i64, scale: f32, out: *mut u32) -> c_int;

@@ -1,18 +1,18 @@
 #!/usr/bin/env python3
 """Progressive preview through the C ABI (SURVEY.md 8f-4, second half: what would replace the reference's minifb window,
-src/main.rs:60-75, which only shows the finished frame).  Nothing new in the library is needed: `ptc_render_accumulate`
-ADDS a sample range into a device-resident film, `ptc_resolve_device` packs it with the scale of the samples so far — so a
-host renders the frame in passes and shows (here: saves) the image after each.  Philox is keyed on the global sample index
-so the last pass is the one-shot render of the same spp up to the fp32 rounding of the per-pass film conversions (the
-script prints the difference).
+src/main.rs:60-75, which only shows the finished frame).  `ptc_render_progressive` renders the frame in passes of
+first_spp, then doubling samples, and calls back on this thread after each pass with the packed image of all samples so
+far, while the device renders the next pass.  Here the callback saves one PNG per preview.  Philox is keyed on the global
+(pixel, sample) and the film is a fixed-point sum, so each preview is the one-shot render at its sample count bit for
+bit; the script checks that for the last one.
 
-  python tools/progressive_preview.py [scene.json] [passes] [spp_per_pass] [out_dir]
+  python tools/progressive_preview.py [scene.json] [spp] [first_spp] [out_dir]
 """
 import os
 import sys
+import time
 
 import numpy as np
-import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -23,29 +23,29 @@ pt = ptload.load()
 
 def main():
     path = sys.argv[1] if len(sys.argv) > 1 else os.path.join(ROOT, "scenes", "cornell-box", "scene.json")
-    passes = int(sys.argv[2]) if len(sys.argv) > 2 else 4
-    per = int(sys.argv[3]) if len(sys.argv) > 3 else 4
+    spp = int(sys.argv[2]) if len(sys.argv) > 2 else 64
+    first = int(sys.argv[3]) if len(sys.argv) > 3 else 1
     out_dir = sys.argv[4] if len(sys.argv) > 4 else os.path.join(ROOT, "gpurun_out")
     os.makedirs(out_dir, exist_ok=True)
     scene = pt.load_scene_from_json(path)
-    w, h, _, depth = scene.settings
+    w, h, _, _ = scene.settings
     w, h = min(w, 512), min(h, 512)
     cs = scene.to_core().commit(0)
-    film = torch.zeros(w * h * 3, dtype=torch.float32, device="cuda:0")
-    packed = torch.zeros(w * h, dtype=torch.int32, device="cuda:0")
-    stream = torch.cuda.current_stream().cuda_stream
-    total = passes * per
-    for k in range(passes):
-        st = scene.render_settings(width=w, height=h, spp=total, sample_begin=k * per, sample_end=(k + 1) * per, seed=0)
-        stats = cs.render_accumulate(scene.camera, st, film.data_ptr(), stream)
-        pt._ck(pt.core().ptc_resolve_device(film.data_ptr(), w * h, 1.0 / ((k + 1) * per), packed.data_ptr(), stream))
-        img = packed.cpu().numpy().view(np.uint32)
+    st = scene.render_settings(width=w, height=h, spp=spp, seed=0)
+    t0 = time.perf_counter()
+    last = {}
+
+    def show(k, n, img):
         pt.save_image(os.path.join(out_dir, f"preview_{k:02d}.png"), img, w, h)
-        print(f"pass {k}: {(k + 1) * per} spp so far, {stats.render_ms:.2f} ms")
-    # the last frame is the one-shot render (up to fp32 rounding of the per-pass film conversions)
-    once, _ = cs.render_u32(scene.camera, scene.render_settings(width=w, height=h, spp=total, seed=0))
-    diff = np.abs(((img[:, None] >> np.array([16, 8, 0])) & 255).astype(int) - ((once[:, None] >> np.array([16, 8, 0])) & 255).astype(int))
-    print(f"last pass vs one-shot render of {total} spp: max channel difference {diff.max()} level(s), {float((diff > 0).mean()) * 100:.3f} % of channels")
+        print(f"pass {k}: {n} spp so far, preview at {(time.perf_counter() - t0) * 1e3:.2f} ms")
+        last["n"], last["img"] = n, img
+        return 0
+
+    _, u32, n, stats = cs.render_progressive(scene.camera, st, first_spp=first, on_preview=show)
+    print(f"{n} spp in {stats.render_ms:.2f} ms of device time, {(time.perf_counter() - t0) * 1e3:.2f} ms in all")
+    once, _ = cs.render_u32(scene.camera, st)
+    assert last["n"] == n == spp and np.array_equal(last["img"], once) and np.array_equal(u32, once)
+    print(f"the last preview is the one-shot render of {spp} spp, bit for bit")
 
 
 if __name__ == "__main__":

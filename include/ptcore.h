@@ -238,6 +238,35 @@ typedef int32_t (*ptc_preview_fn)(void *user, int32_t pass, int32_t samples, con
 int ptc_render_progressive(ptc_scene *, const ptc_camera *, const ptc_render_settings *, const ptc_progressive *,
                            ptc_preview_fn on_preview, void *user, float *out_rgb, uint32_t *out_u32,
                            int32_t *out_samples, ptc_stats *stats);
+/* Denoised rendering.  The frame is rendered exactly as ptc_render renders it (samples [0, spp/2), then [spp/2, spp) into
+ * the same film: out_noisy_rgb is ptc_render's image bit for bit), the per-pixel variance of the mean is estimated from the
+ * two halves, camera samples [0, feature_spp) are intersected once more for first-hit albedo and normal, and a
+ * variance-guided edge-avoiding à-trous filter runs on the device.  settings: spp >= 2, sample_begin = sample_end = 0,
+ * tile_mod = 0, else PTC_E_INVALID; flags as in ptc_render.  Single device.  Every output is a host buffer and may be NULL:
+ * out_rgb W*H*3 denoised linear radiance, out_u32 W*H 0x00RRGGBB of out_rgb (resolve at scale 1), out_noisy_rgb W*H*3,
+ * out_albedo / out_normal W*H*3 (feature means), out_variance W*H (what the filter starts from).  stats: the two render
+ * passes summed as in ptc_render; render_ms from the first pass to the end of the filter (device events).  The
+ * ptc_denoise arguments are checked before the scene's state: PTC_E_INVALID even on an uncommitted scene.
+ * Filter (DESIGN.md 5h): x = noisy / max(albedo, 1e-3) per channel; level i = 0 .. iterations-1 prefilters its variance
+ * with (1 2 1)x(1 2 1), then takes 5x5 taps at spacing 2^i with B3-spline weights times 1 / (1 + d^2 / sigma^2) for the
+ * luminance (sigma_luminance^2 x the prefiltered variance), normal and albedo differences; frame borders are not clamped
+ * but skipped.  A pixel with a non-finite channel is passed through unchanged and never used as a neighbour.  The
+ * result is remodulated by max(albedo, 1e-3). */
+typedef struct ptc_denoise {
+  int32_t feature_spp;    /* 1 <= feature_spp <= settings->spp */
+  int32_t iterations;     /* 1..10 à-trous levels, step 2^i */
+  float sigma_luminance;  /* > 0, finite */
+  float sigma_normal;     /* > 0, finite */
+  float sigma_albedo;     /* > 0, finite */
+} ptc_denoise;
+int ptc_render_denoised(ptc_scene *, const ptc_camera *, const ptc_render_settings *, const ptc_denoise *, float *out_rgb,
+                        uint32_t *out_u32, float *out_noisy_rgb, float *out_albedo, float *out_normal, float *out_variance,
+                        ptc_stats *stats);
+/* The filter alone on caller-provided host images (the inputs ptc_render_denoised returns): out_rgb W*H*3.  Needs a
+ * committed scene only for its device and stream.  feature_spp is not used; the other ptc_denoise fields are checked as
+ * above, before the scene's state. */
+int ptc_denoise_image(ptc_scene *, const ptc_denoise *, int32_t width, int32_t height, const float *rgb, const float *variance,
+                      const float *albedo, const float *normal, float *out_rgb);
 /* Film resolve, renderer.rs:112-120 + color.rs:87-93: out = pack(sqrt(rgb * scale)).  Device and host buffers. */
 int ptc_resolve_device(const float *d_rgb, int64_t n_pixels, float scale, uint32_t *d_out, void *cuda_stream);
 int ptc_resolve_u32(ptc_scene *, const float *rgb, int64_t n_pixels, float scale, uint32_t *out);

@@ -53,6 +53,11 @@ class ProgressiveSettings(C.Structure):  # ptc_progressive
     _fields_ = [("first_spp", C.c_int32), ("max_pass_spp", C.c_int32)]
 
 
+class Denoise(C.Structure):  # ptc_denoise
+    _fields_ = [("feature_spp", C.c_int32), ("iterations", C.c_int32), ("sigma_luminance", C.c_float),
+                ("sigma_normal", C.c_float), ("sigma_albedo", C.c_float)]
+
+
 # ptc_preview_fn: (user, pass, samples, image) -> 0 to go on, anything else to stop
 PREVIEW_FN = C.CFUNCTYPE(C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.POINTER(C.c_uint32))
 
@@ -161,6 +166,9 @@ def core():
                                       C.POINTER(Stats)]
     L.ptc_render_progressive.argtypes = [_vp, C.POINTER(Camera), C.POINTER(RenderSettings), C.POINTER(ProgressiveSettings),
                                          PREVIEW_FN, _vp, _F, _vp, C.POINTER(C.c_int32), C.POINTER(Stats)]
+    L.ptc_render_denoised.argtypes = [_vp, C.POINTER(Camera), C.POINTER(RenderSettings), C.POINTER(Denoise), _F, _vp, _F, _F, _F,
+                                      _F, C.POINTER(Stats)]
+    L.ptc_denoise_image.argtypes = [_vp, C.POINTER(Denoise), C.c_int32, C.c_int32, _F, _F, _F, _F, _F]
     L.ptc_render_accumulate.argtypes = [_vp, C.POINTER(Camera), C.POINTER(RenderSettings), _vp, _vp, C.POINTER(Stats)]
     L.ptc_resolve_device.argtypes = [_vp, C.c_int64, C.c_float, _vp, _vp]
     L.ptc_resolve_u32.argtypes = [_vp, _F, C.c_int64, C.c_float, _vp]
@@ -598,6 +606,38 @@ class CoreScene:
             raise raised[0]
         _ck(rc)
         return rgb, u32, samples.value, st
+
+    def render_denoised(self, camera, settings, feature_spp=None, iterations=5, sigma_luminance=4.0, sigma_normal=0.1,
+                        sigma_albedo=0.1):
+        """Denoised rendering (ptc_render_denoised): the frame rendered as render() renders it, the variance of each pixel's
+        mean from two halves of its samples, first-hit albedo and normal averaged over camera samples [0, feature_spp)
+        (None: min(settings.spp, 4)), then `iterations` levels of the à-trous filter.  -> (rgb [H,W,3] float32 denoised,
+        u32 [H*W] 0x00RRGGBB of rgb, noisy [H,W,3] = render()'s image, albedo [H,W,3], normal [H,W,3], variance [H,W],
+        Stats)."""
+        h, w = settings.height, settings.width
+        rgb, noisy, albedo, normal = (np.empty((h, w, 3), np.float32) for _ in range(4))
+        u32 = np.empty(h * w, np.uint32)
+        var = np.empty((h, w), np.float32)
+        st = Stats()
+        dn = Denoise(min(settings.spp, 4) if feature_spp is None else feature_spp, iterations, sigma_luminance, sigma_normal,
+                     sigma_albedo)
+        _ck(core().ptc_render_denoised(self._h, C.byref(camera), C.byref(settings), C.byref(dn), _fptr(rgb), u32.ctypes.data,
+                                       _fptr(noisy), _fptr(albedo), _fptr(normal), _fptr(var), C.byref(st)))
+        return rgb, u32, noisy, albedo, normal, var, st
+
+    def denoise_image(self, rgb, variance, albedo, normal, iterations=5, sigma_luminance=4.0, sigma_normal=0.1,
+                      sigma_albedo=0.1):
+        """The filter of render_denoised alone (ptc_denoise_image) on the device: rgb, albedo, normal [H,W,3], variance
+        [H,W] -> the denoised rgb [H,W,3] float32."""
+        c = _f32(rgb)
+        if c.ndim != 3 or c.shape[2] != 3:
+            raise ValueError("rgb must be [H, W, 3]")
+        h, w = c.shape[0], c.shape[1]
+        v, a, n = _f32(variance, (h, w)), _f32(albedo, (h, w, 3)), _f32(normal, (h, w, 3))
+        out = np.empty((h, w, 3), np.float32)
+        dn = Denoise(1, iterations, sigma_luminance, sigma_normal, sigma_albedo)
+        _ck(core().ptc_denoise_image(self._h, C.byref(dn), w, h, _fptr(c), _fptr(v), _fptr(a), _fptr(n), _fptr(out)))
+        return out
 
     def multi(self, devices):
         """In-process multi-GPU (ptc_multi_*): this committed scene replicated on `devices` (devices[0] = its own)."""

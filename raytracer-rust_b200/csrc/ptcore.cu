@@ -15,6 +15,7 @@
 
 #include <algorithm>
 #include <chrono>
+#include <cmath>
 #include <condition_variable>
 #include <exception>
 #include <memory>
@@ -34,6 +35,7 @@
 #include "pt_build_dev.h"
 #include "pt_scene_host.h"
 #include "pt_wavefront.cuh"
+#include "pt_denoise.cuh"
 
 using namespace pt;
 using namespace ptw;
@@ -177,6 +179,13 @@ struct ptc_scene {
   cudaStream_t preview_stream = nullptr;
   cudaEvent_t ev_prog_slot[2] = {nullptr, nullptr};  // recorded once slot j % 2 holds preview j
   cudaEvent_t ev_prog_begin = nullptr;                // render_ms: from here to the last slot event
+  // ptc_render_denoised / ptc_denoise_image, grow-only: the fp32 film sums after the first half of the samples, one
+  // sample's camera rays (origins, then directions), the feature sums (then means), the variance, the denoised image,
+  // the filter's ping-pong input and its guides; the feature pass's control block; render_ms brackets
+  DevBuf<float> w_dn_half, w_dn_rays, w_dn_albedo, w_dn_normal, w_dn_var, w_dn_out;
+  DevBuf<float4> w_dn_xv[2], w_dn_ga, w_dn_gn;
+  DevBuf<Ctl> w_dn_ctl;
+  cudaEvent_t ev_dn_begin = nullptr, ev_dn_end = nullptr;
   DevBuf<Ctl> d_ctl;
   Ctl *h_ctl = nullptr;  // pinned ring
   uint32_t *h_progress = nullptr;  // pinned + mapped: the word k_extend_pre reports the state of the render in
@@ -212,6 +221,8 @@ struct ptc_scene {
     for (auto &e : ev_prog_slot)
       if (e) cudaEventDestroy(e);
     if (ev_prog_begin) cudaEventDestroy(ev_prog_begin);
+    if (ev_dn_begin) cudaEventDestroy(ev_dn_begin);
+    if (ev_dn_end) cudaEventDestroy(ev_dn_end);
     if (preview_stream) cudaStreamDestroy(preview_stream);
     for (auto &e : timing_events) cudaEventDestroy(e);
     if (own_stream) cudaStreamDestroy(own_stream);
@@ -262,6 +273,28 @@ int launch_extend(cudaStream_t stream, uint32_t segments, int rounds, Ctl *ctl, 
     k_extend_post<<<segments, kBlock, 0, stream>>>(ctl, sr, ds, eo, tq, r, t_min, t_max);
   }
   return 1 + 2 * rounds;
+}
+
+// n rays (device arrays of n x 3 floats) laid out like a render's pool in the hook workspace (segment b = slots
+// [b * cap, ...), ray i in slot i) and run through the render's extend kernels: the hit records are left in ws_hook's
+// hit0 / hit1 / ids.  ptc_intersect's rays and ptc_render_denoised's feature rays.  `before` / `after`, if given, are
+// recorded around the extend launches.  Returns the number of extend launches.
+int extend_hook_rays(ptc_scene *s, const float *d_o, const float *d_d, uint32_t n, float t_min, float t_max, Ctl *ctl, bool counters,
+                     cudaStream_t st, cudaEvent_t before = nullptr, cudaEvent_t after = nullptr) {
+  const uint32_t segments = s->segments();
+  const uint32_t cap = (uint32_t)(((uint64_t)n + segments - 1) / segments + kBlock - 1) / kBlock * kBlock;
+  s->ws_hook.ensure(segments, cap, s->mesh_objects, true, false);
+  Buffers b = s->ws_hook.buffers();
+  b.cap = cap;
+  const TaskQ tq = s->ws_hook.taskq();
+  k_fill_counts<<<(segments + 255) / 256, 256, 0, st>>>(b.cnt, segments, cap, n);
+  k_pack_rays<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_o, d_d, (size_t)n, b.ray_o, b.ray_d);
+  const ExtendOut eo{b, s->ws_hook.ids.p};
+  if (before) CK(cudaEventRecord(before, st));
+  const int launches = launch_extend(st, segments, s->mesh_objects, ctl, s->ds, eo, tq, t_min, t_max, counters);
+  CK(cudaGetLastError());
+  if (after) CK(cudaEventRecord(after, st));
+  return launches;
 }
 
 void require_committed(const ptc_scene *s) {
@@ -1256,6 +1289,145 @@ int ptc_render_progressive(ptc_scene *s, const ptc_camera *cam, const ptc_render
   PTC_GUARD_END
 }
 
+// ptc_denoise's filter parameters (the arguments of both denoise entry points; feature_spp is ptc_render_denoised's)
+static void check_denoise_filter(const ptc_denoise *dn) {
+  if (dn->iterations < 1 || dn->iterations > kDenoiseMaxIterations) throw std::invalid_argument("iterations must be 1..10");
+  for (const float sg : {dn->sigma_luminance, dn->sigma_normal, dn->sigma_albedo})
+    if (!(sg > 0.0f) || !std::isfinite(sg)) throw std::invalid_argument("the sigmas must be > 0 and finite");
+}
+
+// The filter on the device, queued on `stream`: the noisy image (W*H*3, in s->w_film_out), var (W*H), albedo and normal
+// (W*H*3) -> s->w_dn_out (W*H*3 denoised) and s->w_packed (W*H, resolve_pixel of it at scale 1).  Returns the number of
+// kernels launched.
+static int denoise_filter(ptc_scene *s, const ptc_denoise *dn, int32_t width, int32_t height, const float *var, const float *albedo,
+                          const float *normal, cudaStream_t stream) {
+  const uint32_t n_px = (uint32_t)width * (uint32_t)height;
+  for (auto &b : s->w_dn_xv)
+    if (b.n < n_px) b.alloc(n_px);
+  if (s->w_dn_ga.n < n_px) s->w_dn_ga.alloc(n_px), s->w_dn_gn.alloc(n_px);
+  if (s->w_dn_out.n < (size_t)n_px * 3) s->w_dn_out.alloc((size_t)n_px * 3);
+  if (s->w_packed.n < n_px) s->w_packed.alloc(n_px);
+  const unsigned nb = (n_px + 255u) / 256u;
+  k_denoise_prepare<<<nb, 256, 0, stream>>>(s->w_film_out.p, var, albedo, normal, n_px, s->w_dn_xv[0].p, s->w_dn_ga.p, s->w_dn_gn.p);
+  const DenoiseParams dp = denoise_params(dn->sigma_luminance, dn->sigma_normal, dn->sigma_albedo);
+  const dim3 block(kAtrousBlockX, kAtrousBlockY);
+  const dim3 grid((unsigned)(width + kAtrousBlockX - 1) / kAtrousBlockX, (unsigned)(height + kAtrousBlockY - 1) / kAtrousBlockY);
+  for (int i = 0; i < dn->iterations; i++)
+    k_atrous<<<grid, block, 0, stream>>>(s->w_dn_xv[i & 1].p, s->w_dn_ga.p, s->w_dn_gn.p, width, height, 1 << i, dp, s->w_dn_xv[(i + 1) & 1].p);
+  k_denoise_finish<<<nb, 256, 0, stream>>>(s->w_dn_xv[dn->iterations & 1].p, s->w_film_out.p, albedo, n_px, s->w_dn_out.p, s->w_packed.p);
+  CK(cudaGetLastError());
+  return 2 + dn->iterations;
+}
+
+int ptc_render_denoised(ptc_scene *s, const ptc_camera *cam, const ptc_render_settings *st, const ptc_denoise *dn, float *out_rgb,
+                        uint32_t *out_u32, float *out_noisy_rgb, float *out_albedo, float *out_normal, float *out_variance,
+                        ptc_stats *stats) {
+  PTC_GUARD_BEGIN
+  // the arguments first, the scene's state after them
+  if (!s || !dn) throw std::invalid_argument("null argument");
+  check_render_args(cam, st, true);  // every output may be NULL
+  if (st->sample_begin != 0 || st->sample_end != 0 || st->tile_mod != 0)
+    throw std::invalid_argument("ptc_render_denoised schedules the samples itself: sample_begin, sample_end and tile_mod must be 0");
+  if (st->spp < 2) throw std::invalid_argument("ptc_render_denoised needs spp >= 2: the variance comes from two halves of the samples");
+  if (dn->feature_spp < 1 || dn->feature_spp > st->spp) throw std::invalid_argument("feature_spp must be >= 1 and <= spp");
+  check_denoise_filter(dn);
+  require_committed(s);
+  CK(cudaSetDevice(s->device));
+  ensure_ctl(s);
+  const uint32_t n_px = (uint32_t)st->width * (uint32_t)st->height;
+  const size_t n3 = (size_t)n_px * 3;
+  if (s->w_dn_half.n < n3) s->w_dn_half.alloc(n3);
+  if (s->w_dn_albedo.n < n3) s->w_dn_albedo.alloc(n3), s->w_dn_normal.alloc(n3);
+  if (s->w_dn_rays.n < 2 * n3) s->w_dn_rays.alloc(2 * n3);
+  if (s->w_dn_var.n < n_px) s->w_dn_var.alloc(n_px);
+  if (s->w_film_out.n < n3) s->w_film_out.alloc(n3);
+  if (!s->w_dn_ctl.p) s->w_dn_ctl.alloc(1);
+  if (!s->ev_dn_begin) CK(cudaEventCreate(&s->ev_dn_begin));
+  if (!s->ev_dn_end) CK(cudaEventCreate(&s->ev_dn_end));
+  cudaStream_t stream = s->own_stream;
+  const unsigned nb = (n_px + 255u) / 256u;
+  ptc_stats total;
+  memset(&total, 0, sizeof(total));
+  uint64_t &launches = total.kernel_launches;
+
+  // 1. the render in two halves, the fp32 film sums of the first one kept: the film is ptc_render's
+  const int half = st->spp / 2;
+  CK(cudaEventRecord(s->ev_dn_begin, stream));
+  render_pass(s, cam, st, 0, half, Pass(), stream, total);
+  CK(cudaMemsetAsync(s->w_dn_half.p, 0, n3 * sizeof(float), stream));
+  k_film_to_accum<<<(unsigned)((n3 + 255) / 256), 256, 0, stream>>>(s->film(), n_px, s->w_dn_half.p);
+  Pass more;
+  more.clear_film = false;
+  render_pass(s, cam, st, half, st->spp, more, stream, total);
+  launches += 1;
+
+  // 2. features: camera samples 0 .. feature_spp - 1 in order, each one's first hits added to the per-pixel sums
+  CK(cudaMemsetAsync(s->w_dn_albedo.p, 0, n3 * sizeof(float), stream));
+  CK(cudaMemsetAsync(s->w_dn_normal.p, 0, n3 * sizeof(float), stream));
+  CK(cudaMemsetAsync(s->w_dn_ctl.p, 0, sizeof(Ctl), stream));
+  RenderParams rp;
+  memset(&rp, 0, sizeof(rp));
+  memcpy(&rp.cam, cam, sizeof(DCamera));
+  rp.width = st->width, rp.height = st->height, rp.seed = st->seed;
+  float *ray_o = s->w_dn_rays.p, *ray_d = s->w_dn_rays.p + n3;
+  for (int k = 0; k < dn->feature_spp; k++) {
+    k_primary_rays<<<nb, 256, 0, stream>>>(rp, (uint32_t)k, ray_o, ray_d);
+    launches += 3 + extend_hook_rays(s, ray_o, ray_d, n_px, kEps, INFINITY, s->w_dn_ctl.p, false, stream);
+    const Buffers b = s->ws_hook.buffers();
+    k_feature_add<<<nb, 256, 0, stream>>>(b.hit0, b.hit1, s->ds.materials, n_px, s->w_dn_albedo.p, s->w_dn_normal.p);
+    launches += 1;
+  }
+  k_feature_mean<<<(unsigned)((n3 + 255) / 256), 256, 0, stream>>>(s->w_dn_albedo.p, s->w_dn_normal.p, n3, 1.0f / (float)dn->feature_spp);
+
+  // 3. the noisy image (ptc_render's), the variance from the halves, the filter
+  k_resolve_film<<<nb, 256, 0, stream>>>(s->film(), n_px, 1.0f / (float)st->spp, nullptr, s->w_film_out.p, nullptr);
+  k_denoise_variance<<<nb, 256, 0, stream>>>(s->w_dn_half.p, s->film(), n_px, half, st->spp, s->w_dn_albedo.p, s->w_dn_var.p);
+  CK(cudaGetLastError());
+  launches += 3 + denoise_filter(s, dn, st->width, st->height, s->w_dn_var.p, s->w_dn_albedo.p, s->w_dn_normal.p, stream);
+  CK(cudaEventRecord(s->ev_dn_end, stream));
+
+  if (out_rgb) film_to_host(s, s->w_dn_out.p, out_rgb, n3 * sizeof(float), stream);
+  if (out_u32) film_to_host(s, s->w_packed.p, out_u32, (size_t)n_px * sizeof(uint32_t), stream);
+  if (out_noisy_rgb) film_to_host(s, s->w_film_out.p, out_noisy_rgb, n3 * sizeof(float), stream);
+  if (out_albedo) film_to_host(s, s->w_dn_albedo.p, out_albedo, n3 * sizeof(float), stream);
+  if (out_normal) film_to_host(s, s->w_dn_normal.p, out_normal, n3 * sizeof(float), stream);
+  if (out_variance) film_to_host(s, s->w_dn_var.p, out_variance, (size_t)n_px * sizeof(float), stream);
+  CK(cudaStreamSynchronize(stream));
+  if (stats) {
+    *stats = total;
+    float ms = 0.0f;
+    CK(cudaEventElapsedTime(&ms, s->ev_dn_begin, s->ev_dn_end));
+    stats->render_ms = ms;
+  }
+  return 0;
+  PTC_GUARD_END
+}
+
+int ptc_denoise_image(ptc_scene *s, const ptc_denoise *dn, int32_t width, int32_t height, const float *rgb, const float *variance,
+                      const float *albedo, const float *normal, float *out_rgb) {
+  PTC_GUARD_BEGIN
+  if (!s || !dn || !rgb || !variance || !albedo || !normal || !out_rgb) throw std::invalid_argument("null argument");
+  if (width <= 0 || height <= 0) throw std::invalid_argument("bad image size");
+  if ((int64_t)width * height > (int64_t)0x3fffffff) throw std::invalid_argument("image too large");
+  check_denoise_filter(dn);
+  require_committed(s);
+  CK(cudaSetDevice(s->device));
+  const uint32_t n_px = (uint32_t)width * (uint32_t)height;
+  const size_t n3 = (size_t)n_px * 3;
+  if (s->w_film_out.n < n3) s->w_film_out.alloc(n3);
+  if (s->w_dn_albedo.n < n3) s->w_dn_albedo.alloc(n3), s->w_dn_normal.alloc(n3);
+  if (s->w_dn_var.n < n_px) s->w_dn_var.alloc(n_px);
+  cudaStream_t stream = s->own_stream;
+  CK(cudaMemcpyAsync(s->w_film_out.p, rgb, n3 * sizeof(float), cudaMemcpyHostToDevice, stream));
+  CK(cudaMemcpyAsync(s->w_dn_var.p, variance, (size_t)n_px * sizeof(float), cudaMemcpyHostToDevice, stream));
+  CK(cudaMemcpyAsync(s->w_dn_albedo.p, albedo, n3 * sizeof(float), cudaMemcpyHostToDevice, stream));
+  CK(cudaMemcpyAsync(s->w_dn_normal.p, normal, n3 * sizeof(float), cudaMemcpyHostToDevice, stream));
+  denoise_filter(s, dn, width, height, s->w_dn_var.p, s->w_dn_albedo.p, s->w_dn_normal.p, stream);
+  film_to_host(s, s->w_dn_out.p, out_rgb, n3 * sizeof(float), stream);
+  return 0;
+  PTC_GUARD_END
+}
+
 int ptc_resolve_device(const float *d_rgb, int64_t n_pixels, float scale, uint32_t *d_out, void *cuda_stream) {
   PTC_GUARD_BEGIN
   if (!d_rgb || !d_out || n_pixels < 0) throw std::invalid_argument("bad argument");
@@ -1295,13 +1467,6 @@ int ptc_intersect(ptc_scene *s, const float *origins, const float *dirs, int64_t
   if (n > (int64_t)0x3fffffff) throw std::invalid_argument("too many rays for one call");
   CK(cudaSetDevice(s->device));
   ensure_ctl(s);
-  // the rays are laid out like a render's pool (segment b = slots [b * cap, ...)) and go through the SAME kernels
-  const uint32_t segments = s->segments();
-  const uint32_t cap = (uint32_t)(((uint64_t)n + segments - 1) / segments + kBlock - 1) / kBlock * kBlock;
-  s->ws_hook.ensure(segments, cap, s->mesh_objects, true, false);
-  Buffers b = s->ws_hook.buffers();
-  b.cap = cap;
-  const TaskQ tq = s->ws_hook.taskq();
   DevBuf<float> d_o, d_d;
   DevBuf<ptc_hit> d_out;
   DevBuf<Ctl> ctl;
@@ -1312,18 +1477,12 @@ int ptc_intersect(ptc_scene *s, const float *origins, const float *dirs, int64_t
   memset(&init, 0, sizeof(init));
   ctl.upload(&init, 1);
   cudaStream_t st = s->own_stream;
-  const unsigned nb = (unsigned)((n + 255) / 256);
-  k_fill_counts<<<(segments + 255) / 256, 256, 0, st>>>(b.cnt, segments, cap, (uint32_t)n);
-  k_pack_rays<<<nb, 256, 0, st>>>(d_o.p, d_d.p, (size_t)n, b.ray_o, b.ray_d);
-  const ExtendOut eo{b, s->ws_hook.ids.p};
   cudaEvent_t ea, eb;
   CK(cudaEventCreate(&ea));
   CK(cudaEventCreate(&eb));
-  CK(cudaEventRecord(ea, st));
-  const int ext_launches = launch_extend(st, segments, s->mesh_objects, ctl.p, s->ds, eo, tq, t_min, t_max, true);
-  CK(cudaGetLastError());
-  CK(cudaEventRecord(eb, st));
-  k_unpack_hits<<<nb, 256, 0, st>>>(b.hit0, b.hit1, s->ws_hook.ids.p, (size_t)n, d_out.p);
+  const int ext_launches = extend_hook_rays(s, d_o.p, d_d.p, (uint32_t)n, t_min, t_max, ctl.p, true, st, ea, eb);
+  const Buffers b = s->ws_hook.buffers();
+  k_unpack_hits<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(b.hit0, b.hit1, s->ws_hook.ids.p, (size_t)n, d_out.p);
   CK(cudaGetLastError());
   CK(cudaMemcpyAsync(out, d_out.p, (size_t)n * sizeof(ptc_hit), cudaMemcpyDeviceToHost, st));
   Ctl fin;

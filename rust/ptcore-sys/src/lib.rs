@@ -112,6 +112,18 @@ pub struct ptc_progressive {
 /// (user, pass, samples, image: W*H 0x00RRGGBB, valid during the call only) -> 0 to go on, anything else to stop
 pub type ptc_preview_fn = Option<unsafe extern "C" fn(*mut c_void, i32, i32, *const u32) -> i32>;
 
+/// ptc_render_denoised's / ptc_denoise_image's parameters: 1 <= feature_spp <= spp (ptc_render_denoised only), 1..10
+/// à-trous levels, and the three edge-stopping sigmas, each > 0 and finite
+#[repr(C)]
+#[derive(Clone, Copy, Default)]
+pub struct ptc_denoise {
+    pub feature_spp: i32,
+    pub iterations: i32,
+    pub sigma_luminance: f32,
+    pub sigma_normal: f32,
+    pub sigma_albedo: f32,
+}
+
 #[repr(C)]
 pub struct ptc_scene {
     _private: [u8; 0],
@@ -150,6 +162,13 @@ extern "C" {
     pub fn ptc_render_progressive(s: *mut ptc_scene, cam: *const ptc_camera, st: *const ptc_render_settings, pg: *const ptc_progressive,
                                   on_preview: ptc_preview_fn, user: *mut c_void, out_rgb: *mut f32, out_u32: *mut u32,
                                   out_samples: *mut i32, stats: *mut ptc_stats) -> c_int;
+    /// denoised rendering, one device (include/ptcore.h): out_noisy_rgb is ptc_render's image; every output may be null
+    pub fn ptc_render_denoised(s: *mut ptc_scene, cam: *const ptc_camera, st: *const ptc_render_settings, dn: *const ptc_denoise,
+                               out_rgb: *mut f32, out_u32: *mut u32, out_noisy_rgb: *mut f32, out_albedo: *mut f32,
+                               out_normal: *mut f32, out_variance: *mut f32, stats: *mut ptc_stats) -> c_int;
+    /// the denoiser's filter alone on host images (W*H*3 rgb / albedo / normal, W*H variance) -> out_rgb W*H*3
+    pub fn ptc_denoise_image(s: *mut ptc_scene, dn: *const ptc_denoise, width: i32, height: i32, rgb: *const f32, variance: *const f32,
+                             albedo: *const f32, normal: *const f32, out_rgb: *mut f32) -> c_int;
     pub fn ptc_render_accumulate(s: *mut ptc_scene, cam: *const ptc_camera, st: *const ptc_render_settings, d_accum: *mut f32,
                                  cuda_stream: *mut c_void, stats: *mut ptc_stats) -> c_int;
     pub fn ptc_resolve_u32(s: *mut ptc_scene, rgb: *const f32, n_pixels: i64, scale: f32, out: *mut u32) -> c_int;

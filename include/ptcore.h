@@ -267,6 +267,24 @@ int ptc_render_denoised(ptc_scene *, const ptc_camera *, const ptc_render_settin
  * above, before the scene's state. */
 int ptc_denoise_image(ptc_scene *, const ptc_denoise *, int32_t width, int32_t height, const float *rgb, const float *variance,
                       const float *albedo, const float *normal, float *out_rgb);
+/* Batch rendering: n_views cameras of one committed scene rendered as ONE wavefront job (one pool, one launch chain, one
+ * drain), for turntables, camera paths and multi-view datasets.  View k is, bit for bit, ptc_render / ptc_render_u32 with
+ * camera cams[k], seed seeds[k] (seeds == NULL: every view uses settings->seed) and the other settings as given: Philox
+ * is keyed on (seed of the view, pixel within the view, sample) and the film is fixed-point.
+ * settings: width/height/spp/max_depth/sample_begin/sample_end/pool_paths/flags as in ptc_render (the default pool is
+ * sized for the whole job); tile_mod must be 0; n_views >= 1 and n_views * ceil32(width) * ceil32(height) <= 2^30, else
+ * PTC_E_INVALID.  Single device.  Outputs are host buffers, view-major, each may be NULL but not both: out_rgb
+ * n_views*W*H*3 linear mean radiance, out_u32 n_views*W*H 0x00RRGGBB.  stats: paths and rays of the whole job (= the sums
+ * over the single-view renders), launches and render_ms of the whole job.  The arguments are checked before the scene's
+ * state: PTC_E_INVALID for bad ones even on an uncommitted scene. */
+int ptc_render_batch(ptc_scene *, const ptc_camera *cams, int32_t n_views, const uint64_t *seeds,
+                     const ptc_render_settings *, float *out_rgb, uint32_t *out_u32, ptc_stats *stats);
+/* Same, device-resident, as ptc_render_accumulate: ADDS each view's radiance sum (not divided by spp) into d_accum
+ * (n_views*W*H*3 floats in device memory of the scene's device, view-major), ordered on `cuda_stream` (NULL = the legacy
+ * default stream).  View k's slice is what ptc_render_accumulate adds for cams[k] and seeds[k].  Returns after the work
+ * is enqueued AND finished. */
+int ptc_render_batch_accumulate(ptc_scene *, const ptc_camera *cams, int32_t n_views, const uint64_t *seeds,
+                                const ptc_render_settings *, float *d_accum, void *cuda_stream, ptc_stats *stats);
 /* Film resolve, renderer.rs:112-120 + color.rs:87-93: out = pack(sqrt(rgb * scale)).  Device and host buffers. */
 int ptc_resolve_device(const float *d_rgb, int64_t n_pixels, float scale, uint32_t *d_out, void *cuda_stream);
 int ptc_resolve_u32(ptc_scene *, const float *rgb, int64_t n_pixels, float scale, uint32_t *out);

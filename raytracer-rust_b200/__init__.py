@@ -170,6 +170,9 @@ def core():
                                       _F, C.POINTER(Stats)]
     L.ptc_denoise_image.argtypes = [_vp, C.POINTER(Denoise), C.c_int32, C.c_int32, _F, _F, _F, _F, _F]
     L.ptc_render_accumulate.argtypes = [_vp, C.POINTER(Camera), C.POINTER(RenderSettings), _vp, _vp, C.POINTER(Stats)]
+    L.ptc_render_batch.argtypes = [_vp, C.POINTER(Camera), C.c_int32, _vp, C.POINTER(RenderSettings), _F, _vp, C.POINTER(Stats)]
+    L.ptc_render_batch_accumulate.argtypes = [_vp, C.POINTER(Camera), C.c_int32, _vp, C.POINTER(RenderSettings), _vp, _vp,
+                                              C.POINTER(Stats)]
     L.ptc_resolve_device.argtypes = [_vp, C.c_int64, C.c_float, _vp, _vp]
     L.ptc_resolve_u32.argtypes = [_vp, _F, C.c_int64, C.c_float, _vp]
     L.ptc_intersect.argtypes = [_vp, _F, _F, C.c_int64, C.c_float, C.c_float, _vp, C.POINTER(Stats)]
@@ -646,6 +649,37 @@ class CoreScene:
     def render_accumulate(self, camera, settings, d_accum_ptr, stream_ptr=None):
         st = Stats()
         _ck(core().ptc_render_accumulate(self._h, C.byref(camera), C.byref(settings), d_accum_ptr, stream_ptr, C.byref(st)))
+        return st
+
+    @staticmethod
+    def _batch_args(cameras, seeds):
+        cams = (Camera * len(cameras))(*cameras)
+        if seeds is None:
+            return cams, None, None
+        s = np.ascontiguousarray(seeds, dtype=np.uint64)
+        if s.shape != (len(cameras),):
+            raise ValueError("seeds must hold one seed per camera")
+        return cams, s, s.ctypes.data
+
+    def render_batch(self, cameras, settings, seeds=None):
+        """Batch rendering (ptc_render_batch): every camera of `cameras` rendered in one wavefront job.  seeds: one per
+        camera (None: settings.seed for all).  -> (rgb [K,H,W,3] float32 linear mean radiance, u32 [K,H*W] 0x00RRGGBB,
+        Stats of the whole job); view k is render / render_u32 of cameras[k] with seed seeds[k], bit for bit."""
+        cams, _keep, sp = self._batch_args(cameras, seeds)
+        k, h, w = len(cameras), settings.height, settings.width
+        rgb = np.empty((k, h, w, 3), np.float32)
+        u32 = np.empty((k, h * w), np.uint32)
+        st = Stats()
+        _ck(core().ptc_render_batch(self._h, cams, k, sp, C.byref(settings), _fptr(rgb), u32.ctypes.data, C.byref(st)))
+        return rgb, u32, st
+
+    def render_batch_accumulate(self, cameras, settings, d_accum_ptr, stream_ptr=None, seeds=None):
+        """ptc_render_batch_accumulate: ADDS each view's radiance sum into the device buffer d_accum_ptr (K*H*W*3 float32,
+        view-major), ordered on stream_ptr; view k's slice is render_accumulate of cameras[k] with seed seeds[k]."""
+        cams, _keep, sp = self._batch_args(cameras, seeds)
+        st = Stats()
+        _ck(core().ptc_render_batch_accumulate(self._h, cams, len(cameras), sp, C.byref(settings), d_accum_ptr, stream_ptr,
+                                               C.byref(st)))
         return st
 
     def resolve_u32(self, rgb, scale=1.0):

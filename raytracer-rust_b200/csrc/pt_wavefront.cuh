@@ -84,6 +84,18 @@ struct RenderParams {
   uint32_t n_list;
 };
 
+// ptc_render_batch: n views of one scene as ONE job.  The path index space is n_views stacked tile grids (local tile t
+// -> view t / tiles_per_view, tile t % tiles_per_view); a pool entry's pixel word holds the global film index
+// view * view_px + pixel.  Philox is keyed on the view's seed and the pixel within the view, so view k is, bit for bit,
+// the single render of cams[k] with seeds[k].  Read by k_shade_batch only: a kernel argument of its own, so that the
+// parameters of every other kernel keep their layout.
+struct BatchTables {
+  const DCamera *cams;    // [n_views]
+  const uint64_t *seeds;  // [n_views]
+  uint32_t view_px;       // width * height
+  uint32_t tiles_per_view;
+};
+
 // Path state, SoA of float4.  Segment b = slots [b * cap, b * cap + cnt[b]).
 struct Buffers {
   float4 *ray_o;  // origin.xyz, pixel index
@@ -532,11 +544,14 @@ __device__ __forceinline__ uint32_t block_rank(bool flag, uint32_t *s_warp /* [k
 // `seg_done` (or nullptr): one word per segment, set when the segment is found empty with the path supply exhausted — it
 // will never hold a ray again — and counted off ctl->n_active, once.
 // (The path state is read with plain loads: launches overlap, see stage_begin, so it is not read-only while a k_shade runs.)
-// List: regeneration starts paths from rp.pixel_list instead of the tiles (ptc_render_adaptive's later passes); a
-// template argument, so that the shade kernels of every other render compile to the instructions they had.
-template <int Mode, bool List>
+// Src: where regeneration starts paths.  kSrcTiles: the tiles of tile_mod / tile_rem; kSrcList: rp.pixel_list
+// (ptc_render_adaptive's later passes); kSrcBatch: the stacked tile grids of `bt` (ptc_render_batch).  A template
+// argument, so that the shade kernels of every other render compile to the instructions they had.
+constexpr int kSrcTiles = 0, kSrcList = 1, kSrcBatch = 2;
+template <int Mode, int Src>
 __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, uint32_t *seg_done, Ctl *ctl, const DScene &sc, const RenderParams &rp,
-                                                const Buffers &b, const Film &film) {
+                                                const Buffers &b, const Film &film, const BatchTables &bt) {
+  constexpr bool List = Src == kSrcList, Batch = Src == kSrcBatch;
   __shared__ uint16_t s_perm[kShadeWindow];
   __shared__ uint32_t s_hist[2][16];
   __shared__ uint32_t s_warp[kBlock / 32 + 1];
@@ -605,7 +620,15 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
         const float4 o4 = b.ray_o[i], d4 = b.ray_d[i], b4 = b.beta[i];
         const float4 h1 = b.hit1[i];
         const uint32_t pixel_word = f2u(o4.w), sample = f2u(d4.w), bounce = f2u(b4.w);
-        const uint32_t pixel = NEE ? (pixel_word & ~kShadowBit) : pixel_word;
+        const uint32_t pixel = NEE ? (pixel_word & ~kShadowBit) : pixel_word;  // the film index (global in a batch)
+        // Philox key: the view's seed and the pixel within the view
+        uint64_t seed = rp.seed;
+        uint32_t key_pixel = pixel;
+        if (Batch) {
+          const uint32_t view = pixel / bt.view_px;
+          seed = bt.seeds[view];
+          key_pixel = pixel - view * bt.view_px;
+        }
         const uint32_t bits = f2u(h1.w);
         const V3 beta = v3(b4.x, b4.y, b4.z);
         const V3 ray_d = v3(d4.x, d4.y, d4.z);
@@ -645,7 +668,7 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
             radiance = beta * e * w_mis;
             add = true;
           }
-          const Uniforms4 u = philox_uniforms(rp.seed, pixel, sample, bounce, 0u);
+          const Uniforms4 u = philox_uniforms(seed, key_pixel, sample, bounce, 0u);
           Ray sc_ray;
           V3 att;
           if (mat_scatter(m, ray_d, pos, nrm, (bits & kFrontBit) != 0u, u.u, sc_ray, att)) {
@@ -662,14 +685,14 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
                 if (SKY) {
                   // one emitter: the sky with probability p_sky (own uniforms, Philox block 2; infinitely far, so any hit
                   // occludes), else a uniformly chosen analytic light with the rest of u[0]
-                  const Uniforms4 ul = philox_uniforms(rp.seed, pixel, sample, bounce, 1u);
+                  const Uniforms4 ul = philox_uniforms(seed, key_pixel, sample, bounce, 1u);
                   const float p_sky = sc.n_lights > 0 ? 0.5f : 1.0f;
                   const V3 so = pos + nrm * kEps;
                   V3 wi, fcos, le;
                   float dist, pl, pb;
                   bool ok;
                   if (ul.u[0] < p_sky) {
-                    const Uniforms4 us = philox_uniforms(rp.seed, pixel, sample, bounce, 2u);
+                    const Uniforms4 us = philox_uniforms(seed, key_pixel, sample, bounce, 2u);
                     wi = sky_sample(sc, us.u, pl);
                     pl *= p_sky;
                     dist = INFINITY;
@@ -691,7 +714,7 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
                     sb4 = make_float4(c.x, c.y, c.z, u2f(bounce + 1u));
                   }
                 } else if (sc.n_lights > 0) {
-                  const Uniforms4 ul = philox_uniforms(rp.seed, pixel, sample, bounce, 1u);
+                  const Uniforms4 ul = philox_uniforms(seed, key_pixel, sample, bounce, 1u);
                   const uint32_t li = min((uint32_t)(ul.u[0] * (float)sc.n_lights), (uint32_t)sc.n_lights - 1u);
                   const DLight L = sc.lights[li];
                   const V3 so = pos + nrm * kEps;
@@ -778,7 +801,7 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
     for (uint32_t j0 = 0; j0 < avail; j0 += (uint32_t)kBlock) {
       const uint32_t j = j0 + tid;
       bool valid = j < avail;
-      uint32_t pixel = 0, sample = 0;
+      uint32_t pixel = 0, sample = 0, view = 0;
       int x = 0, y = 0;
       if (valid) {
         const unsigned long long p = first_path + j;
@@ -793,7 +816,11 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
           y = (int)(pixel / (uint32_t)rp.width);
         } else {
           const uint32_t local_tile = r >> 10, in_tile = r & 1023u;
-          const uint32_t tile = local_tile * (uint32_t)rp.tile_mod + (uint32_t)rp.tile_rem;
+          uint32_t tile = local_tile * (uint32_t)rp.tile_mod + (uint32_t)rp.tile_rem;
+          if (Batch) {  // (tile_mod = 1, tile_rem = 0) the row scatter above runs over the rows of every view
+            view = local_tile / bt.tiles_per_view;
+            tile = local_tile - view * bt.tiles_per_view;
+          }
           x = (int)((tile % (uint32_t)rp.tiles_x) * 32u + (in_tile & 31u));
           y = (int)((tile / (uint32_t)rp.tiles_x) * 32u + (in_tile >> 5));
           valid = x < rp.width && y < rp.height;
@@ -805,11 +832,11 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
       const uint32_t off = block_rank(valid, s_warp, &total);
       if (valid) {
         const uint32_t slot = seg_base + w + off;
-        const Uniforms4 jit = philox_uniforms(rp.seed, pixel, sample, 0xffffffffu, 0u);
+        const Uniforms4 jit = philox_uniforms(Batch ? bt.seeds[view] : rp.seed, pixel, sample, 0xffffffffu, 0u);
         const float u = ((float)x + jit.u[0]) / (float)rp.width;   // renderer.rs:96
         const float v = ((float)y + jit.u[1]) / (float)rp.height;  // renderer.rs:97
-        const Ray ray = camera_get_ray(rp.cam, u, v);
-        b.nray_o[slot] = make_float4(ray.o.x, ray.o.y, ray.o.z, u2f(pixel));
+        const Ray ray = camera_get_ray(Batch ? bt.cams[view] : rp.cam, u, v);
+        b.nray_o[slot] = make_float4(ray.o.x, ray.o.y, ray.o.z, u2f(Batch ? view * bt.view_px + pixel : pixel));
         b.nray_d[slot] = make_float4(ray.d.x, ray.d.y, ray.d.z, u2f(sample));
         b.nbeta[slot] = make_float4(1.0f, 1.0f, 1.0f, u2f(0u));
         if (NEE) b.naux[slot] = -1.0f;
@@ -970,7 +997,16 @@ __global__ void __launch_bounds__(kBlock, kSegPerSM) k_extend_post(Ctl *ctl, Seg
 template <int Mode, bool List = false>
 __global__ void __launch_bounds__(kBlock, kSegPerSM) k_shade(Ctl *ctl, SegRange sr, DScene sc, RenderParams rp, Buffers b, Film film) {
   stage_begin(sr, sr.seg0 + blockIdx.x, ctl);
-  stage_shade<Mode, List>(sr.seg0 + blockIdx.x, sr.n_seg, sr.flags ? sr.flags + sr.n_seg : nullptr, ctl, sc, rp, b, film);
+  stage_shade<Mode, List ? kSrcList : kSrcTiles>(sr.seg0 + blockIdx.x, sr.n_seg, sr.flags ? sr.flags + sr.n_seg : nullptr, ctl, sc, rp, b,
+                                                 film, BatchTables{});
+  stage_end(sr, sr.seg0 + blockIdx.x);
+}
+// ptc_render_batch: paths of every view of `bt` (stage_shade, kSrcBatch); rp.tile_mod = 1, rp.n_my_tiles = views x tiles
+template <int Mode>
+__global__ void __launch_bounds__(kBlock, kSegPerSM) k_shade_batch(Ctl *ctl, SegRange sr, DScene sc, RenderParams rp, Buffers b, Film film,
+                                                                   BatchTables bt) {
+  stage_begin(sr, sr.seg0 + blockIdx.x, ctl);
+  stage_shade<Mode, kSrcBatch>(sr.seg0 + blockIdx.x, sr.n_seg, sr.flags ? sr.flags + sr.n_seg : nullptr, ctl, sc, rp, b, film, bt);
   stage_end(sr, sr.seg0 + blockIdx.x);
 }
 

@@ -186,6 +186,9 @@ struct ptc_scene {
   DevBuf<float4> w_dn_xv[2], w_dn_ga, w_dn_gn;
   DevBuf<Ctl> w_dn_ctl;
   cudaEvent_t ev_dn_begin = nullptr, ev_dn_end = nullptr;
+  // ptc_render_batch, grow-only: the cameras and seeds of the views (pt_wavefront.cuh: BatchTables)
+  DevBuf<DCamera> d_batch_cams;
+  DevBuf<uint64_t> d_batch_seeds;
   DevBuf<Ctl> d_ctl;
   Ctl *h_ctl = nullptr;  // pinned ring
   uint32_t *h_progress = nullptr;  // pinned + mapped: the word k_extend_pre reports the state of the render in
@@ -342,10 +345,14 @@ void ensure_ctl(ptc_scene *s) {
 
 // What one call of render_accumulate renders besides its settings.  Default: the tiles of the settings into a cleared
 // film.  ptc_render_adaptive's passes add samples to the film as it stands, the later ones for a list of pixels only.
+// ptc_render_batch renders the tiles of `views` cameras into one film of views x W x H pixels, view-major.
 struct Pass {
   bool clear_film = true;
   const uint32_t *pixels = nullptr;  // device, ascending; nullptr: the tiles of tile_mod / tile_rem
   uint32_t n_pixels = 0;
+  uint32_t views = 0;                // > 0: a batch (tile_mod = 0); its cameras and seeds, device tables of `views` entries
+  const DCamera *cams = nullptr;
+  const uint64_t *seeds = nullptr;
 };
 
 // the wavefront loop; renders into the scene's fixed-point film and then adds its fp32 image into d_accum on `stream`
@@ -363,7 +370,8 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
   // the sky joins the sampled lights only where there is a sky distribution; elsewhere the flag changes nothing
   const bool nee_sky = nee && (st->flags & PTC_FLAG_NEE_SKY) != 0 && s->ds.sky_dist != nullptr;
   const int tiles_x = (st->width + 31) / 32, n_tiles = tiles_x * ((st->height + 31) / 32);
-  const int n_my_tiles = tile_rem < n_tiles ? (n_tiles - tile_rem + tile_mod - 1) / tile_mod : 0;
+  const uint32_t views = std::max<uint32_t>(pass.views, 1u);  // a batch's tile grids are stacked (the caller checked the size)
+  const int n_my_tiles = (tile_rem < n_tiles ? (n_tiles - tile_rem + tile_mod - 1) / tile_mod : 0) * (int)views;
   // paths this call starts (its tiles x its samples; border tiles padded to 32 x 32 like the path index space; a pixel
   // list padded to 32 entries)
   const uint64_t list_padded = ((uint64_t)pass.n_pixels + 31u) & ~31ull;
@@ -438,12 +446,17 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
     const int w = std::min(32, st->width - tx * 32), h = std::min(32, st->height - ty * 32);
     my_pixels += (uint64_t)w * h;
   }
+  my_pixels *= views;
 
   Ctl init;
   memset(&init, 0, sizeof(init));
   init.total_paths = rp.max_depth > 0 ? want_paths : 0ull;
   init.n_active = init.total_paths != 0ull ? segments : 0u;  // every segment reports once when it is empty for good (stage_shade)
-  const size_t n_px = (size_t)st->width * st->height;
+  // Does the initial fill reserve every path?  Each segment's first reservation takes min(room, share) paths (stage_shade:
+  // room = cap, cap / 2 with NEE; share = its fair share of the job in whole rows) unless the supply is already out.
+  const uint64_t fill_share = ((init.total_paths + segments - 1) / segments + 31ull) & ~31ull;
+  const bool job_in_first_fill = (uint64_t)segments * std::min<uint64_t>(nee ? cap64 / 2 : cap64, fill_share) >= init.total_paths;
+  const size_t n_px = (size_t)st->width * st->height * views;
   ensure_film(s, n_px);
   const Film film = s->film();
   if (pass.clear_film) clear_film(s, n_px, stream);
@@ -532,9 +545,15 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
       if (timing) mark(ST_SHADE);
       const SegRange ssr = seg_range(0u, 1u);
       const int mode = nee_sky ? 2 : (nee ? 1 : 0);
-      auto *kernel = pass.pixels ? (mode == 2 ? k_shade<2, true> : mode == 1 ? k_shade<1, true> : k_shade<0, true>)
-                                 : (mode == 2 ? k_shade<2> : mode == 1 ? k_shade<1> : k_shade<0>);
-      launch_stage(pdl, stream, segments, kernel, s->d_ctl.p, ssr, s->ds, rp, bufs[flip], film);
+      if (pass.views > 0) {
+        const BatchTables bt{pass.cams, pass.seeds, (uint32_t)st->width * (uint32_t)st->height, (uint32_t)n_tiles};
+        auto *kernel = mode == 2 ? k_shade_batch<2> : mode == 1 ? k_shade_batch<1> : k_shade_batch<0>;
+        launch_stage(pdl, stream, segments, kernel, s->d_ctl.p, ssr, s->ds, rp, bufs[flip], film, bt);
+      } else {
+        auto *kernel = pass.pixels ? (mode == 2 ? k_shade<2, true> : mode == 1 ? k_shade<1, true> : k_shade<0, true>)
+                                   : (mode == 2 ? k_shade<2> : mode == 1 ? k_shade<1> : k_shade<0>);
+        launch_stage(pdl, stream, segments, kernel, s->d_ctl.p, ssr, s->ds, rp, bufs[flip], film);
+      }
       launches += 1;
       flip ^= 1;
     };
@@ -550,9 +569,12 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
         // the extend of iteration k reports what the shade of iteration k - 1 left: nothing alive and nothing to start
         // means every launch from k on is empty.  Ahead of the device by kAhead iterations at most (4 launches of ~2.5 us
         // each against >= 45 us per iteration: two would do), so that few empty launches trail the render.
-        // And once the supply is known to be exhausted the end is known too: a path started by the shade of iteration
-        // k - 1 at the latest has its last segment in iteration k - 1 + max_depth (the whole job in flight at once:
-        // exactly max_depth iterations, no trailing launch at all).
+        // And once the supply is known to be exhausted the end is known too.  When the initial fill reserved every path,
+        // a path started by the shade of iteration k - 1 at the latest has its last segment in iteration k - 1 +
+        // max_depth (the whole job in flight at once: exactly max_depth iterations, no trailing launch at all).
+        // Otherwise segment 0's report says nothing about the others: segments run ahead of each other, and another one
+        // may have reserved the last paths in a later shade.  Every shade it can have run has been enqueued, though, so
+        // the paths end by iteration it + max_depth.
         const uint64_t kAhead = getenv("PTC_AHEAD") ? (uint64_t)std::max(1, atoi(getenv("PTC_AHEAD"))) : 3u;
         for (uint32_t spins = 0;; spins++) {
           const uint32_t w = *prog;
@@ -562,7 +584,7 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
           }
           if ((w & 2u) && !draining) {
             draining = true;
-            last_iteration = (uint64_t)(w >> 2) - 1u + (uint64_t)rp.max_depth + (nee ? 1u : 0u);  // + the last hit's shadow ray
+            last_iteration = (job_in_first_fill ? (uint64_t)(w >> 2) - 1u : it) + (uint64_t)rp.max_depth + (nee ? 1u : 0u);  // + the last hit's shadow ray
           }
           if (it >= last_iteration) {
             finished = true;
@@ -1057,6 +1079,62 @@ int ptc_render(ptc_scene *s, const ptc_camera *cam, const ptc_render_settings *s
 
 int ptc_render_u32(ptc_scene *s, const ptc_camera *cam, const ptc_render_settings *st, uint32_t *out_u32, ptc_stats *stats) {
   return render_to_host(s, cam, st, nullptr, out_u32, stats);
+}
+
+// ptc_render_batch / ptc_render_batch_accumulate: the arguments, before the scene's state
+static void check_batch_args(const ptc_camera *cams, int32_t n_views, const ptc_render_settings *st, bool has_output) {
+  check_render_args(cams, st, has_output);
+  if (n_views < 1) throw std::invalid_argument("n_views must be >= 1");
+  if (st->tile_mod != 0) throw std::invalid_argument("ptc_render_batch renders whole views: tile_mod must be 0");
+  // the film index of every padded pixel of every view stays below 2^30 (a pool entry's pixel word keeps kShadowBit)
+  const uint64_t padded = (uint64_t)n_views * (((uint64_t)st->width + 31u) & ~31ull) * (((uint64_t)st->height + 31u) & ~31ull);
+  if (padded > (1ull << 30)) throw std::invalid_argument("batch too large: n_views * ceil32(width) * ceil32(height) > 2^30");
+}
+
+// The batch's cameras and seeds (seeds == NULL: settings->seed for every view) into the scene's device tables, one copy
+// each on the stream the render runs on; -> the Pass that renders them.
+static Pass batch_pass(ptc_scene *s, const ptc_camera *cams, int32_t n_views, const uint64_t *seeds, const ptc_render_settings *st,
+                       cudaStream_t stream) {
+  static_assert(sizeof(ptc_camera) == sizeof(DCamera), "ptc_camera and DCamera share one layout");
+  CK(cudaSetDevice(s->device));
+  const size_t n = (size_t)n_views;
+  if (s->d_batch_cams.n < n) s->d_batch_cams.alloc(n), s->d_batch_seeds.alloc(n);
+  std::vector<uint64_t> same;
+  if (!seeds) same.assign(n, st->seed), seeds = same.data();
+  // (from pageable memory: the call returns once the source has been read)
+  CK(cudaMemcpyAsync(s->d_batch_cams.p, cams, n * sizeof(DCamera), cudaMemcpyHostToDevice, stream));
+  CK(cudaMemcpyAsync(s->d_batch_seeds.p, seeds, n * sizeof(uint64_t), cudaMemcpyHostToDevice, stream));
+  Pass pass;
+  pass.views = (uint32_t)n_views, pass.cams = s->d_batch_cams.p, pass.seeds = s->d_batch_seeds.p;
+  return pass;
+}
+
+int ptc_render_batch(ptc_scene *s, const ptc_camera *cams, int32_t n_views, const uint64_t *seeds, const ptc_render_settings *st,
+                     float *out_rgb, uint32_t *out_u32, ptc_stats *stats) {
+  PTC_GUARD_BEGIN
+  // the arguments first, the scene's state after them
+  if (!s) throw std::invalid_argument("null argument");
+  check_batch_args(cams, n_views, st, out_rgb || out_u32);
+  require_committed(s);
+  const Pass pass = batch_pass(s, cams, n_views, seeds, st, s->own_stream);
+  render_accumulate(s, cams, st, nullptr, s->own_stream, stats, pass);
+  const size_t n_px = (size_t)n_views * st->width * st->height;
+  const int launches = resolve_film_to_host(s, n_px, 1.0f / (float)st->spp, nullptr, out_rgb, out_u32, s->own_stream);  // as ptc_render
+  if (stats) stats->kernel_launches += launches;
+  return 0;
+  PTC_GUARD_END
+}
+
+int ptc_render_batch_accumulate(ptc_scene *s, const ptc_camera *cams, int32_t n_views, const uint64_t *seeds, const ptc_render_settings *st,
+                                float *d_accum, void *cuda_stream, ptc_stats *stats) {
+  PTC_GUARD_BEGIN
+  if (!s) throw std::invalid_argument("null argument");
+  check_batch_args(cams, n_views, st, d_accum != nullptr);
+  require_committed(s);
+  const Pass pass = batch_pass(s, cams, n_views, seeds, st, (cudaStream_t)cuda_stream);
+  render_accumulate(s, cams, st, d_accum, (cudaStream_t)cuda_stream, stats, pass);
+  return 0;
+  PTC_GUARD_END
 }
 
 int ptc_render_adaptive(ptc_scene *s, const ptc_camera *cam, const ptc_render_settings *st, const ptc_adaptive *ad, float *out_rgb,

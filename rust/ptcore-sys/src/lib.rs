@@ -171,6 +171,14 @@ extern "C" {
                              albedo: *const f32, normal: *const f32, out_rgb: *mut f32) -> c_int;
     pub fn ptc_render_accumulate(s: *mut ptc_scene, cam: *const ptc_camera, st: *const ptc_render_settings, d_accum: *mut f32,
                                  cuda_stream: *mut c_void, stats: *mut ptc_stats) -> c_int;
+    /// n_views cameras as one wavefront job: view k is ptc_render / ptc_render_u32 of cams[k] with seeds[k] (seeds NULL:
+    /// settings' seed), bit for bit; out_rgb n_views*W*H*3, out_u32 n_views*W*H, view-major, either may be NULL
+    pub fn ptc_render_batch(s: *mut ptc_scene, cams: *const ptc_camera, n_views: i32, seeds: *const u64, st: *const ptc_render_settings,
+                            out_rgb: *mut f32, out_u32: *mut u32, stats: *mut ptc_stats) -> c_int;
+    /// same, device-resident: adds each view's radiance sum into d_accum (n_views*W*H*3 floats, view-major) on cuda_stream
+    pub fn ptc_render_batch_accumulate(s: *mut ptc_scene, cams: *const ptc_camera, n_views: i32, seeds: *const u64,
+                                       st: *const ptc_render_settings, d_accum: *mut f32, cuda_stream: *mut c_void,
+                                       stats: *mut ptc_stats) -> c_int;
     pub fn ptc_resolve_u32(s: *mut ptc_scene, rgb: *const f32, n_pixels: i64, scale: f32, out: *mut u32) -> c_int;
     /// the HDR sky as a light (PTC_FLAG_NEE_SKY): sample / pdf hooks; PTC_E_STATE without a sky distribution
     pub fn ptc_sky_sample(s: *mut ptc_scene, u4: *const f32, n: i64, out_dir: *mut f32, out_pdf: *mut f32, out_rgb: *mut f32) -> c_int;

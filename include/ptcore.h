@@ -91,11 +91,18 @@ enum {
                             non-specular hit also samples one emissive sphere / quad through a shadow ray, and emitters found
                             by BSDF sampling are weighted with the power heuristic.  Same expected image, far less noise where
                             emitters are small (veach-mis).  stats.rays then counts the shadow rays too. */
-  PTC_FLAG_NEE_SKY = 8   /* with PTC_FLAG_NEE only (alone: PTC_E_INVALID): NEE also samples the HDR sky as an environment light,
+  PTC_FLAG_NEE_SKY = 8,  /* with PTC_FLAG_NEE only (alone: PTC_E_INVALID): NEE also samples the HDR sky as an environment light,
                             importance-sampled by its radiance over the cells of the reference's equirectangular lookup, with
                             the power heuristic against BSDF sampling (the Tungsten scenes' "enable_light_sampling").  Same
                             expected image, less noise under a sky with bright spots (the teapot's envmap).  On a scene
                             without an HDR sky, or with an all-zero one, it changes nothing: the image is PTC_FLAG_NEE's. */
+  PTC_FLAG_NEE_EMITTERS = 16 /* with PTC_FLAG_NEE only (alone: PTC_E_INVALID), may be combined with PTC_FLAG_NEE_SKY: NEE also
+                            samples emissive meshes (uniform by world area over the triangles a ray can hit) and cubes (their
+                            six faces by area), and chooses among all sampled emitters by power, max(r, g, b) x area, instead of
+                            uniformly.  The first 63 emissive spheres, quads, cubes and meshes of finite positive power, in
+                            object order, are sampled; planes and the rest are found by BSDF sampling alone.  With the sky,
+                            p_sky stays 0.5 when an emitter is sampled.  Same expected image; a scene whose only sampled
+                            emitters are one sphere or quad renders exactly as with PTC_FLAG_NEE. */
 };
 
 /* HitRecord (src/hittable.rs:10-16) plus the ids the parity bar is stated on. */
@@ -327,6 +334,16 @@ int ptc_scatter(ptc_scene *, int material, const float *ray_dirs, const float *p
  * PTC_E_STATE when the committed scene has no sky distribution (no HDR sky, or an all-zero one). */
 int ptc_sky_sample(ptc_scene *, const float *u4, int64_t n, float *out_dir, float *out_pdf, float *out_rgb);
 int ptc_sky_pdf(ptc_scene *, const float *dirs, int64_t n, float *out_pdf);
+/* PTC_FLAG_NEE_EMITTERS parity hooks.  ptc_light_sample: what the shade stage draws from n points x (n x 3) with the n x 4
+ * uniforms u4 of its light sample (u[0] the emitter, u[1], u[2] the point, u[3] the triangle or cube face), without the
+ * sky's share: the point (n x 3), the estimator's divisor (solid-angle density the sampler realises), the object and the
+ * triangle (original index; -1 for other emitters).  A rejected sample has object and triangle -1 and pdf 0.
+ * ptc_light_pdf: the n rays (origins, unit dirs; n x 3) go through the render's extend kernels; out_pdf is the MIS
+ * density the shade stage gives a BSDF-sampled ray whose closest hit is a sampled emitter (0 otherwise), without the
+ * sky's share.  Both PTC_E_STATE when the committed scene has no emitter this mode samples. */
+int ptc_light_sample(ptc_scene *, const float *x, const float *u4, int64_t n, float *out_point, float *out_pdf,
+                     int32_t *out_object, int32_t *out_triangle);
+int ptc_light_pdf(ptc_scene *, const float *origins, const float *dirs, int64_t n, float *out_pdf);
 /* Philox4x32-10 known-answer hook (runs on the device). */
 int ptc_philox(ptc_scene *, const uint32_t ctr[4], const uint32_t key[2], uint32_t out[4]);
 

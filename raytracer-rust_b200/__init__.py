@@ -21,7 +21,7 @@ REPO_ROOT = os.path.dirname(_HERE)
 PTC_OK, PTC_E_INVALID, PTC_E_CUDA, PTC_E_NOMEM, PTC_E_STATE = 0, -1, -2, -3, -4
 MAT_LAMBERT, MAT_LAMBERT_CHECKER, MAT_METAL, MAT_DIELECTRIC, MAT_EMISSIVE, MAT_PLASTIC, MAT_ROUGH_CONDUCTOR, MAT_NULL = range(8)
 DIST_GGX, DIST_BECKMANN = 0, 1
-FLAG_COUNTERS, FLAG_TIMING, FLAG_NEE, FLAG_NEE_SKY = 1, 2, 4, 8
+FLAG_COUNTERS, FLAG_TIMING, FLAG_NEE, FLAG_NEE_SKY, FLAG_NEE_EMITTERS = 1, 2, 4, 8, 16
 COMMIT_FAST_BUILD = 1
 COMMIT_DEVICE_SAH = 2
 LOAD_INFINITE_SPHERE_SKY, LOAD_WO3_STRIDE16, LOAD_SKIP_UNKNOWN = 1, 2, 4
@@ -181,6 +181,8 @@ def core():
     L.ptc_philox.argtypes = [_vp, _vp, _vp, _vp]
     L.ptc_sky_sample.argtypes = [_vp, _F, C.c_int64, _F, _F, _F]
     L.ptc_sky_pdf.argtypes = [_vp, _F, C.c_int64, _F]
+    L.ptc_light_sample.argtypes = [_vp, _F, _F, C.c_int64, _F, _F, _vp, _vp]
+    L.ptc_light_pdf.argtypes = [_vp, _F, _F, C.c_int64, _F]
     L.ptc_multi_create.argtypes = [_vp, C.POINTER(C.c_int), C.c_int, C.POINTER(_vp)]
     L.ptc_multi_destroy.argtypes = [_vp]
     L.ptc_multi_destroy.restype = None
@@ -725,6 +727,29 @@ class CoreScene:
         d = _f32(dirs, (-1, 3))
         pdf = np.empty(len(d), np.float32)
         _ck(core().ptc_sky_pdf(self._h, _fptr(d), len(d), _fptr(pdf)))
+        return pdf
+
+    def light_sample(self, x, u4):
+        """FLAG_NEE_EMITTERS' light sample from points x (n x 3) with Philox block 1's uniforms u4 (n x 4), without the
+        sky's share -> (points n x 3, the estimator's solid-angle divisor n, object n, triangle n; -1 where rejected or,
+        for the triangle, where the emitter is not a mesh), by the shade stage's own device function."""
+        xx, u = _f32(x, (-1, 3)), _f32(u4, (-1, 4))
+        if len(xx) != len(u):
+            raise ValueError("x and u4 must have the same number of rows")
+        n = len(u)
+        pts, pdf = np.empty((n, 3), np.float32), np.empty(n, np.float32)
+        obj, tri = np.empty(n, np.int32), np.empty(n, np.int32)
+        _ck(core().ptc_light_sample(self._h, _fptr(xx), _fptr(u), n, _fptr(pts), _fptr(pdf), obj.ctypes.data, tri.ctypes.data))
+        return pts, pdf, obj, tri
+
+    def light_pdf(self, origins, dirs):
+        """The MIS density FLAG_NEE_EMITTERS gives a BSDF-sampled ray (origins, unit dirs: n x 3) whose closest hit, traced
+        by the render's extend kernels, is a sampled emitter; 0 otherwise.  Without the sky's share."""
+        o, d = _f32(origins, (-1, 3)), _f32(dirs, (-1, 3))
+        if len(o) != len(d):
+            raise ValueError("origins and dirs must have the same number of rows")
+        pdf = np.empty(len(d), np.float32)
+        _ck(core().ptc_light_pdf(self._h, _fptr(o), _fptr(d), len(d), _fptr(pdf)))
         return pdf
 
     def philox(self, ctr, key):

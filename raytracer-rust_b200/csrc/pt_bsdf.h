@@ -398,6 +398,68 @@ PT_HD uint32_t cdf_search(const float *cdf, uint32_t n, float u) {
   }
   return lo;
 }
+// ---- PTC_FLAG_NEE_EMITTERS: lights chosen by power; meshes and cubes sampled by area (tables: pt_types.h, EmitterTables).
+// Two densities.  The estimator divides by what the sampler realises: p_sel x (the entry's CDF bin / its world area),
+// converted to solid angle with the entry's GEOMETRIC cosine.  The power heuristic weighs both strategies with one
+// formula, emitter_mis_pdf = p_sel d^2 / (|cos| A_light), cos against the normal the hit record reports and d the true
+// distance, evaluated alike where a light sample is drawn and where a BSDF-sampled ray hits the emitter: so the two
+// weights sum to 1 even where a caller's stored normals are not the geometric ones.  (Spheres and quads: light_sample /
+// light_pdf as under PTC_FLAG_NEE, times p_sel.)
+PT_HD float emitter_select_prob(const EmitterTables &et, uint32_t light) { return et.sel_cdf[light + 1] - et.sel_cdf[light]; }
+PT_HD bool emitter_area_sampled(const DLight &L) { return L.type == OBJ_MESH || L.type == OBJ_CUBE; }
+PT_HD float emitter_mis_pdf(const DLight &L, float p_sel, float dist, float cos_rec) { return light_pdf(L, dist, cos_rec) * p_sel; }
+struct EmitterSample {
+  V3 wi;
+  float dist;
+  float pdf;   // the estimator's divisor
+  float pmis;  // the power heuristic's density of this light strategy
+  uint32_t light;
+  int32_t entry;  // triangle (original index) or cube face; -1 for spheres and quads
+};
+// One light sample from x: u0 chooses the light, u1 u2 the point, u3 the triangle or face.  false: rejected (x on the
+// light, or the light seen edge-on).
+PT_HD bool emitter_sample(const DScene &sc, const EmitterTables &et, V3 x, float u0, float u1, float u2, float u3, EmitterSample &s) {
+  s.light = cdf_search(et.sel_cdf, (uint32_t)sc.n_lights, u0);
+  s.entry = -1;
+  const DLight &L = sc.lights[s.light];
+  const float p_sel = emitter_select_prob(et, s.light);
+  if (!emitter_area_sampled(L)) {
+    if (!light_sample(L, x, u1, u2, s.wi, s.dist, s.pdf)) return false;
+    s.pdf *= p_sel;
+    s.pmis = s.pdf;
+    return true;
+  }
+  uint32_t first, count, coff;
+  memcpy(&first, &L.f[0], 4), memcpy(&count, &L.f[1], 4), memcpy(&coff, &L.f[2], 4);
+  const float *cdf = et.ent_cdf + coff;
+  const uint32_t e = cdf_search(cdf, count, u3);
+  const float p_bin = cdf[e + 1] - cdf[e];
+  const float4 *q = et.ent + (size_t)(first + e) * 3u;
+  const float4 q0 = q[0], q1 = q[1], q2 = q[2];
+  const V3 v0 = v3(q0.x, q0.y, q0.z), e1 = v3(q1.x, q1.y, q1.z), e2 = v3(q2.x, q2.y, q2.z), nrec = v3(q0.w, q1.w, q2.w);
+  const bool tri = L.type == OBJ_MESH;
+  float a = u1, b = u2;
+  if (tri) {  // uniform on the triangle: (1 - sqrt u1, sqrt u1 (1 - u2), sqrt u1 u2)
+    const float r = sqrtf(u1);
+    a = r * (1.0f - u2), b = r * u2;
+  }
+  const V3 y = v0 + e1 * a + e2 * b;
+  const V3 ng = cross(e1, e2);
+  const float len = length(ng);
+  const float area = tri ? 0.5f * len : len;
+  const V3 d = y - x;
+  const float d2 = length_squared(d);
+  if (!(d2 > 1e-12f) || !(area > 0.0f)) return false;
+  s.dist = sqrtf(d2);
+  s.wi = d * (1.0f / s.dist);
+  const float cos_g = fabsf(dot(ng, s.wi)) / len;
+  if (!(cos_g > 1e-6f)) return false;
+  s.entry = (int32_t)e;
+  s.pdf = p_sel * p_bin * d2 / (cos_g * area);
+  s.pmis = emitter_mis_pdf(L, p_sel, s.dist, fabsf(dot(nrec, s.wi)));
+  return true;
+}
+
 // a direction with density sky_pdf from four uniforms: row, column, then uniform in phi and cos(theta) inside the cell
 // (uniform in solid angle), mapped back through the lookup's angles: atan2(z, x) = phi - pi, y = cos(theta)
 PT_HD V3 sky_sample(const DScene &sc, const float *u4, float &pdf) {

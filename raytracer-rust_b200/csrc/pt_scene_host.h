@@ -10,6 +10,7 @@
 
 #include "../../include/ptcore.h"
 #include "pt_build.h"
+#include "pt_math.h"
 #include "pt_types.h"
 
 namespace pt {
@@ -149,6 +150,112 @@ struct HostScene {
       o.hit_bits = (m.type << 26) | (light_id << 20) | o.material;
     }
     build_sky_dist();
+    build_emitters();
+  }
+  // PTC_FLAG_NEE_EMITTERS (layout in pt_types.h: EmitterTables): the first kMaxLights emissive spheres, quads, cubes and
+  // meshes of finite positive power max(r, g, b) x area, in object order, and a copy of the object table whose hit_bits
+  // carry these light ids.  Areas and weights are summed in double in a fixed order, then stored as float CDFs.
+  std::vector<DObject> objects_em;
+  std::vector<DLight> lights_em;
+  std::vector<float> em_sel_cdf;  // [lights_em.size() + 1], or empty
+  std::vector<float4> em_ent;
+  std::vector<float> em_ent_cdf;
+  void build_emitters() {
+    objects_em = objects;
+    lights_em.clear(), em_sel_cdf.clear(), em_ent.clear(), em_ent_cdf.clear();
+    std::vector<double> power, area;
+    std::vector<double> ent_area;
+    for (size_t k = 0; k < objects.size(); k++) {
+      DObject &o = objects_em[k];
+      const DMaterial &m = materials[(size_t)o.material];
+      o.hit_bits &= ~(63 << 20);
+      if (m.type != PTC_MAT_EMISSIVE || o.type == OBJ_PLANE || (int)lights_em.size() >= kMaxLights) continue;
+      // every channel finite (std::max would drop a NaN in the second argument), the largest positive
+      if (!std::isfinite(m.albedo[0]) || !std::isfinite(m.albedo[1]) || !std::isfinite(m.albedo[2])) continue;
+      const double radiance = std::max((double)m.albedo[0], std::max((double)m.albedo[1], (double)m.albedo[2]));
+      if (!(radiance > 0.0)) continue;
+      DLight l;
+      memset(&l, 0, sizeof(l));
+      l.type = o.type, l.object = (int32_t)k;
+      for (int i = 0; i < 3; i++) l.emission[i] = m.albedo[i];
+      double a = 0.0;
+      const size_t first = em_ent.size() / 3;
+      ent_area.clear();
+      if (o.type == OBJ_SPHERE || o.type == OBJ_QUAD) {  // as in the PTC_FLAG_NEE list
+        if (o.type == OBJ_SPHERE) {
+          for (int i = 0; i < 4; i++) l.f[i] = o.f[i];
+          l.area = 4.0f * 3.14159265358979323846f * o.f[3] * o.f[3];
+        } else {
+          for (int i = 0; i < 12; i++) l.f[i] = o.f[i];
+          const float *ea = o.f + 3, *eb = o.f + 6;
+          const float cx = ea[1] * eb[2] - ea[2] * eb[1], cy = ea[2] * eb[0] - ea[0] * eb[2], cz = ea[0] * eb[1] - ea[1] * eb[0];
+          l.area = std::sqrt(cx * cx + cy * cy + cz * cz);
+        }
+        a = l.area;
+      } else {
+        const float *w2o = o.f, *o2w = o.f + 16;
+        auto push = [&](V3 v0, V3 e1, V3 e2, V3 n_obj, double scale, bool live) {
+          const V3 nrec = normalized(mat_t_vector(w2o, n_obj));
+          em_ent.push_back(make_float4(v0.x, v0.y, v0.z, nrec.x));
+          em_ent.push_back(make_float4(e1.x, e1.y, e1.z, nrec.y));
+          em_ent.push_back(make_float4(e2.x, e2.y, e2.z, nrec.z));
+          const double cx = (double)e1.y * e2.z - (double)e1.z * e2.y, cy = (double)e1.z * e2.x - (double)e1.x * e2.z,
+                       cz = (double)e1.x * e2.y - (double)e1.y * e2.x;
+          const double ar = live ? scale * std::sqrt(cx * cx + cy * cy + cz * cz) : 0.0;
+          ent_area.push_back(std::isfinite(ar) ? ar : 0.0);
+        };
+        if (o.type == OBJ_CUBE) {  // faces of [-0.5, 0.5]^3: +-x, +-y, +-z, each base + two unit edges
+          for (int ax = 0; ax < 3; ax++)
+            for (int sgn = 0; sgn < 2; sgn++) {
+              float b[3] = {-0.5f, -0.5f, -0.5f}, u[3] = {0, 0, 0}, v[3] = {0, 0, 0}, n[3] = {0, 0, 0};
+              b[ax] = sgn ? 0.5f : -0.5f;
+              u[(ax + 1) % 3] = 1.0f, v[(ax + 2) % 3] = 1.0f, n[ax] = sgn ? 1.0f : -1.0f;
+              push(mat_point(o2w, v3(b[0], b[1], b[2])), mat_vector(o2w, v3(u[0], u[1], u[2])), mat_vector(o2w, v3(v[0], v[1], v[2])),
+                   v3(n[0], n[1], n[2]), 1.0, true);
+            }
+        } else {  // every triangle in original order; a dead one (never hit) with weight 0
+          const MeshBuild &mb = *meshes[(size_t)o.mesh];
+          for (int64_t t = 0; t < mb.n; t++) {
+            const float *q = mb.tris.data() + (size_t)t * 12;
+            const V3 v0 = mat_point(o2w, v3(q[0], q[1], q[2]));
+            const V3 e1 = mat_point(o2w, v3(q[3], q[4], q[5])) - v0, e2 = mat_point(o2w, v3(q[6], q[7], q[8])) - v0;
+            push(v0, e1, e2, v3(q[9], q[10], q[11]), 0.5, !mb.dead[(size_t)t]);
+          }
+        }
+        for (double x : ent_area) a += x;
+        l.area = (float)a;
+      }
+      const double pw = radiance * a;
+      if (!(a > 0.0) || !(l.area > 0.0f) || !std::isfinite(pw) || !std::isfinite(l.area)) {
+        em_ent.resize(first * 3);
+        continue;
+      }
+      if (o.type == OBJ_CUBE || o.type == OBJ_MESH) {
+        // (DLight holds 32-bit offsets: entry and CDF tables of at most 2^32 - 1 floats each)
+        if (em_ent.size() / 3 > 0xffffffffull || em_ent_cdf.size() + ent_area.size() + 1 > 0xffffffffull)
+          throw std::runtime_error("emissive meshes too large for the PTC_FLAG_NEE_EMITTERS tables");
+        const uint32_t first32 = (uint32_t)first, count = (uint32_t)ent_area.size(), coff = (uint32_t)em_ent_cdf.size();
+        memcpy(&l.f[0], &first32, 4), memcpy(&l.f[1], &count, 4), memcpy(&l.f[2], &coff, 4);
+        double c = 0.0;
+        for (uint32_t i = 0; i < count; i++) {
+          em_ent_cdf.push_back((float)(c / a));
+          c += ent_area[i];
+        }
+        em_ent_cdf.push_back(1.0f);
+      }
+      lights_em.push_back(l);
+      power.push_back(pw);
+      o.hit_bits |= (int32_t)lights_em.size() << 20;
+    }
+    if (lights_em.empty()) return;
+    double total = 0.0;
+    for (double p : power) total += p;
+    double c = 0.0;
+    for (size_t i = 0; i < power.size(); i++) {
+      em_sel_cdf.push_back((float)(c / total));
+      c += power[i];
+    }
+    em_sel_cdf.push_back(1.0f);
   }
   // the sky as a light (PTC_FLAG_NEE_SKY, layout in pt_types.h: SkyDist): cell weight = max(r, g, b) x solid angle, summed
   // in double in a fixed order; left empty without a sky or when every weight is 0

@@ -72,9 +72,10 @@ struct DMesh {
 };
 
 // An emitter that next-event estimation can sample (PTC_FLAG_NEE; the reference has no light sampling): emissive spheres
-// and quads.  Other emissive objects are found by BSDF sampling alone, like every emitter in the reference.
+// and quads.  Other emissive objects are found by BSDF sampling alone, like every emitter in the reference, unless
+// PTC_FLAG_NEE_EMITTERS samples them too (EmitterTables below).
 struct alignas(16) DLight {
-  int32_t type;    // OBJ_SPHERE or OBJ_QUAD
+  int32_t type;    // OBJ_SPHERE or OBJ_QUAD (PTC_FLAG_NEE_EMITTERS: also OBJ_MESH, OBJ_CUBE)
   int32_t object;  // index in the object table
   float area;      // 4 pi r^2 / |edge0 x edge1|
   float pad;
@@ -83,6 +84,21 @@ struct alignas(16) DLight {
   float pad2;
 };
 constexpr int kMaxLights = 63;  // light id 1..63 in the hit record's 6 bits; further emitters are simply not sampled
+
+// PTC_FLAG_NEE_EMITTERS: a second light list (HostScene::lights_em) that also holds emissive meshes and cubes, chosen by
+// power.  Such a DLight has type OBJ_MESH or OBJ_CUBE, `area` = its total world area (a mesh: live triangles only), and
+//   f[0] first entry in EmitterTables::ent, f[1] entry count, f[2] offset of its entry CDF in EmitterTables::ent_cdf
+// (bit-cast uint32).  The entries of a mesh are its triangles in ORIGINAL order (entry i = triangle i; a dead triangle has
+// a CDF bin of width 0), those of a cube its six faces; each entry is three float4, in world space:
+//   (v0.xyz, nrec.x), (e1.xyz, nrec.y), (e2.xyz, nrec.z)
+// a triangle v0 + s e1 + t e2 (s, t >= 0, s + t <= 1) or, for a cube face, a parallelogram (s, t in [0, 1]); nrec is the
+// normal the hit record reports there (mesh_finish / cube_finish_normal: normalized((w2o)^T n_obj)) up to its sign.
+// Read by the shade kernels of this mode only, as a kernel argument of their own.
+struct EmitterTables {
+  const float *sel_cdf;  // [n_lights + 1]: selection CDF over the lights, by max(r, g, b) x area, 0 ... 1
+  const float4 *ent;     // [3 x entries]
+  const float *ent_cdf;  // per mesh / cube light: [count + 1] by area, 0 ... 1
+};
 
 // The HDR sky as a light (PTC_FLAG_NEE_SKY).  The reference's lookup (pt_bsdf.h: sky_texel) makes a w x h sky piecewise
 // constant over Wc x Hc cells, Wc = max(w - 1, 1), Hc = max(h - 1, 1): cell (x, y) has the radiance of texel (x, y) and

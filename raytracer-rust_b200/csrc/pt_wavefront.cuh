@@ -172,6 +172,13 @@ __device__ __forceinline__ float film_value(long long sum, unsigned long long fl
 constexpr uint32_t kHitBit = 0x80000000u, kFrontBit = 0x40000000u, kMatMask = 0x000fffffu;
 constexpr int kTypeShift = 26, kLightShift = 20;  // DObject::hit_bits: type << 26 | NEE light id << 20 | material index
 constexpr uint32_t kShadowBit = 0x80000000u;       // in a pool entry's pixel word: the entry is an NEE shadow ray (see stage_shade)
+// PTC_FLAG_NEE_EMITTERS: in a shadow ray's bounce word (beta.w), the ray goes to a mesh or cube light, whose id is in the
+// low 6 bits: it is unoccluded iff its closest hit is that light at the sampled point (see stage_shade)
+constexpr uint32_t kPosTestBit = 0x80000000u;
+// The hit point must lie within kPosTestTol x distance + kPosTestAbs x max|coordinate| of the sampled point: the two
+// points differ by the rounding of the transforms (a few ulps of the coordinates) only, and two sheets of one emitter
+// that are farther apart than this are told apart (10^-4 x distance: 0.2 mm at 2 m)
+constexpr float kPosTestTol = 1e-4f, kPosTestAbs = 1e-5f;
 
 __device__ __forceinline__ void write_hit(const ExtendOut &out, uint32_t i, const Hit &h) {
   out.b.hit0[i] = make_float4(h.px, h.py, h.pz, h.t);
@@ -540,6 +547,13 @@ __device__ __forceinline__ uint32_t block_rank(bool flag, uint32_t *s_warp /* [k
 // n_lights), its direction is drawn from the sky's own distribution (pt_bsdf.h: sky_sample, Philox block 2) and the
 // shadow ray has an infinite distance: any hit occludes.  A BSDF-sampled ray that misses is weighted with the power
 // heuristic against p_sky * sky_pdf.  Mode 0 = plain, 1 = NEE.
+// Modes 3 and 4 (PTC_FLAG_NEE_EMITTERS, without and with the sky): the lights are `sc.lights` = HostScene::lights_em,
+// emissive meshes and cubes included, chosen by power from `et`'s selection CDF (u[0] of Philox block 1; with the sky,
+// what is left of it after the sky's share), a triangle or cube face by area with u[3] (pt_bsdf.h: emitter_sample).  The
+// extend stages ran on the object table whose hit_bits carry these light ids.  A mesh's t is not a distance
+// (mesh_finish), so the shadow ray of a mesh or cube light is unoccluded iff its closest hit carries that light's id
+// at the sampled point, to within rounding (kPosTestTol; a concave emitter occludes itself), and the hit-side MIS density
+// uses |hit point - ray origin|.  Spheres and quads keep Mode 1 / 2's rules bit for bit.
 // Returns the new ray count of the segment.
 // `seg_done` (or nullptr): one word per segment, set when the segment is found empty with the path supply exhausted — it
 // will never hold a ray again — and counted off ctl->n_active, once.
@@ -550,14 +564,14 @@ __device__ __forceinline__ uint32_t block_rank(bool flag, uint32_t *s_warp /* [k
 constexpr int kSrcTiles = 0, kSrcList = 1, kSrcBatch = 2;
 template <int Mode, int Src>
 __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, uint32_t *seg_done, Ctl *ctl, const DScene &sc, const RenderParams &rp,
-                                                const Buffers &b, const Film &film, const BatchTables &bt) {
+                                                const Buffers &b, const Film &film, const BatchTables &bt, const EmitterTables &et) {
   constexpr bool List = Src == kSrcList, Batch = Src == kSrcBatch;
   __shared__ uint16_t s_perm[kShadeWindow];
   __shared__ uint32_t s_hist[2][16];
   __shared__ uint32_t s_warp[kBlock / 32 + 1];
   __shared__ unsigned long long s_first;
   __shared__ uint32_t s_avail, s_more, s_w, s_wp;
-  constexpr bool NEE = Mode != 0, SKY = Mode == 2;
+  constexpr bool NEE = Mode != 0, SKY = Mode == 2 || Mode == 4, EM = Mode >= 3;
   const uint32_t n = b.cnt[seg], seg_base = seg * b.cap;
   const uint32_t tid = threadIdx.x, lane = tid & 31u;
   const uint32_t lt_mask = (1u << lane) - 1u;
@@ -638,7 +652,15 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
           // a shadow ray: beta is the MIS-weighted contribution, the sample field the distance to the light point.  The light
           // itself is hit at that distance; anything nearer (by more than the tolerance) occludes.
           const float t_light = d4.w;
-          if (!(bits & kHitBit) || !(b.hit0[i].w < t_light * (1.0f - 2e-4f))) radiance = beta, add = true;
+          if (EM && (bounce & kPosTestBit)) {
+            const float4 h0 = b.hit0[i];
+            const V3 y = v3(o4.x, o4.y, o4.z) + ray_d * t_light;
+            const float tol = kPosTestTol * t_light + kPosTestAbs * fmaxf(fabsf(y.x), fmaxf(fabsf(y.y), fabsf(y.z)));
+            if ((bits & kHitBit) && ((bits >> kLightShift) & 63u) == (bounce & 63u) && length_squared(v3(h0.x, h0.y, h0.z) - y) <= tol * tol)
+              radiance = beta, add = true;
+          } else if (!(bits & kHitBit) || !(b.hit0[i].w < t_light * (1.0f - 2e-4f))) {
+            radiance = beta, add = true;
+          }
         } else if (!(bits & kHitBit)) {
           radiance = beta * sky_color(sc, ray_d);
           if (SKY) {  // power heuristic against the sky's light-sampling pdf (camera rays and delta lobes: weight 1)
@@ -659,7 +681,13 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
             if (NEE) {  // power heuristic against the light-sampling pdf of this very point, if the emitter is a sampled light
               const float pb = b.aux[i];
               const uint32_t light = (bits >> kLightShift) & 63u;
-              if (pb >= 0.0f && light != 0u) {
+              if (EM && pb >= 0.0f && light != 0u) {
+                // selection probability by power, times 1 - p_sky when the sky is sampled too
+                const DLight &L = sc.lights[light - 1u];
+                const float dl = emitter_area_sampled(L) ? length(pos - v3(o4.x, o4.y, o4.z)) : h0.w;
+                const float pl = emitter_mis_pdf(L, emitter_select_prob(et, light - 1u) * (SKY ? 0.5f : 1.0f), dl, fabsf(dot(nrm, ray_d)));
+                w_mis = pb * pb / (pb * pb + pl * pl);
+              } else if (!EM && pb >= 0.0f && light != 0u) {
                 // selection probability 1 / n_lights, or (1 - p_sky) / n_lights when the sky is sampled too
                 const float pl = light_pdf(sc.lights[light - 1u], h0.w, fabsf(dot(nrm, ray_d))) * ((SKY ? 0.5f : 1.0f) / (float)sc.n_lights);
                 w_mis = pb * pb / (pb * pb + pl * pl);
@@ -689,7 +717,8 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
                   const float p_sky = sc.n_lights > 0 ? 0.5f : 1.0f;
                   const V3 so = pos + nrm * kEps;
                   V3 wi, fcos, le;
-                  float dist, pl, pb;
+                  float dist, pl, pb, pm;
+                  uint32_t tag = bounce + 1u;
                   bool ok;
                   if (ul.u[0] < p_sky) {
                     const Uniforms4 us = philox_uniforms(seed, key_pixel, sample, bounce, 2u);
@@ -698,22 +727,47 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
                     dist = INFINITY;
                     le = sky_color(sc, wi);
                     ok = pl > 0.0f;
+                    pm = pl;
+                  } else if (EM) {
+                    EmitterSample es;
+                    ok = emitter_sample(sc, et, so, (ul.u[0] - p_sky) * 2.0f, ul.u[1], ul.u[2], ul.u[3], es);
+                    const DLight &L = sc.lights[es.light];
+                    wi = es.wi, dist = es.dist, pl = es.pdf * 0.5f, pm = es.pmis * 0.5f;  // (1 - p_sky) x the light's own
+                    le = v3(L.emission[0], L.emission[1], L.emission[2]);
+                    if (emitter_area_sampled(L)) tag = kPosTestBit | (es.light + 1u);
                   } else {
                     const uint32_t li = min((uint32_t)((ul.u[0] - p_sky) * 2.0f * (float)sc.n_lights), (uint32_t)sc.n_lights - 1u);
                     const DLight L = sc.lights[li];
                     ok = light_sample(L, so, ul.u[1], ul.u[2], wi, dist, pl);
                     pl *= 0.5f / (float)sc.n_lights;  // (1 - p_sky) / n_lights, as where a BSDF-sampled ray hits the light
                     le = v3(L.emission[0], L.emission[1], L.emission[2]);
+                    pm = pl;
                   }
                   if (ok && mat_eval_pdf(m, ray_d, pos, nrm, wi, fcos, pb) && (fcos.x > 0.0f || fcos.y > 0.0f || fcos.z > 0.0f)) {
-                    const float w_mis = pl * pl / (pl * pl + pb * pb);
+                    const float w_mis = pm * pm / (pm * pm + pb * pb);
                     const V3 c = beta * fcos * le * (w_mis / pl);
                     shadow = true;
                     so4 = make_float4(so.x, so.y, so.z, u2f(pixel | kShadowBit));
                     sd4 = make_float4(wi.x, wi.y, wi.z, dist);
-                    sb4 = make_float4(c.x, c.y, c.z, u2f(bounce + 1u));
+                    sb4 = make_float4(c.x, c.y, c.z, u2f(tag));
                   }
-                } else if (sc.n_lights > 0) {
+                } else if (EM && sc.n_lights > 0) {
+                  const Uniforms4 ul = philox_uniforms(seed, key_pixel, sample, bounce, 1u);
+                  const V3 so = pos + nrm * kEps;
+                  EmitterSample es;
+                  V3 fcos;
+                  float pb;
+                  if (emitter_sample(sc, et, so, ul.u[0], ul.u[1], ul.u[2], ul.u[3], es) && mat_eval_pdf(m, ray_d, pos, nrm, es.wi, fcos, pb) &&
+                      (fcos.x > 0.0f || fcos.y > 0.0f || fcos.z > 0.0f)) {
+                    const DLight &L = sc.lights[es.light];
+                    const float w_mis = es.pmis * es.pmis / (es.pmis * es.pmis + pb * pb);
+                    const V3 c = beta * fcos * v3(L.emission[0], L.emission[1], L.emission[2]) * (w_mis / es.pdf);
+                    shadow = true;
+                    so4 = make_float4(so.x, so.y, so.z, u2f(pixel | kShadowBit));
+                    sd4 = make_float4(es.wi.x, es.wi.y, es.wi.z, es.dist);
+                    sb4 = make_float4(c.x, c.y, c.z, u2f(emitter_area_sampled(L) ? kPosTestBit | (es.light + 1u) : bounce + 1u));
+                  }
+                } else if (!EM && sc.n_lights > 0) {
                   const Uniforms4 ul = philox_uniforms(seed, key_pixel, sample, bounce, 1u);
                   const uint32_t li = min((uint32_t)(ul.u[0] * (float)sc.n_lights), (uint32_t)sc.n_lights - 1u);
                   const DLight L = sc.lights[li];
@@ -998,7 +1052,7 @@ template <int Mode, bool List = false>
 __global__ void __launch_bounds__(kBlock, kSegPerSM) k_shade(Ctl *ctl, SegRange sr, DScene sc, RenderParams rp, Buffers b, Film film) {
   stage_begin(sr, sr.seg0 + blockIdx.x, ctl);
   stage_shade<Mode, List ? kSrcList : kSrcTiles>(sr.seg0 + blockIdx.x, sr.n_seg, sr.flags ? sr.flags + sr.n_seg : nullptr, ctl, sc, rp, b,
-                                                 film, BatchTables{});
+                                                 film, BatchTables{}, EmitterTables{});
   stage_end(sr, sr.seg0 + blockIdx.x);
 }
 // ptc_render_batch: paths of every view of `bt` (stage_shade, kSrcBatch); rp.tile_mod = 1, rp.n_my_tiles = views x tiles
@@ -1006,7 +1060,17 @@ template <int Mode>
 __global__ void __launch_bounds__(kBlock, kSegPerSM) k_shade_batch(Ctl *ctl, SegRange sr, DScene sc, RenderParams rp, Buffers b, Film film,
                                                                    BatchTables bt) {
   stage_begin(sr, sr.seg0 + blockIdx.x, ctl);
-  stage_shade<Mode, kSrcBatch>(sr.seg0 + blockIdx.x, sr.n_seg, sr.flags ? sr.flags + sr.n_seg : nullptr, ctl, sc, rp, b, film, bt);
+  stage_shade<Mode, kSrcBatch>(sr.seg0 + blockIdx.x, sr.n_seg, sr.flags ? sr.flags + sr.n_seg : nullptr, ctl, sc, rp, b, film, bt,
+                               EmitterTables{});
+  stage_end(sr, sr.seg0 + blockIdx.x);
+}
+// PTC_FLAG_NEE_EMITTERS: Mode 3 (NEE + emitters) or 4 (NEE + sky + emitters), paths from any Src; the emitter tables are a
+// kernel argument of these instantiations only, so that the parameters of every other kernel keep their layout
+template <int Mode, int Src>
+__global__ void __launch_bounds__(kBlock, kSegPerSM) k_shade_em(Ctl *ctl, SegRange sr, DScene sc, RenderParams rp, Buffers b, Film film,
+                                                                BatchTables bt, EmitterTables et) {
+  stage_begin(sr, sr.seg0 + blockIdx.x, ctl);
+  stage_shade<Mode, Src>(sr.seg0 + blockIdx.x, sr.n_seg, sr.flags ? sr.flags + sr.n_seg : nullptr, ctl, sc, rp, b, film, bt, et);
   stage_end(sr, sr.seg0 + blockIdx.x);
 }
 
@@ -1145,6 +1209,37 @@ __global__ void k_sky_sample(DScene sc, const float *u4, size_t n, float *dirs, 
 __global__ void k_sky_pdf(DScene sc, const float *dirs, size_t n, float *pdf) {
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) pdf[i] = sky_pdf(sc, v3(dirs[i * 3], dirs[i * 3 + 1], dirs[i * 3 + 2]));
+}
+
+// PTC_FLAG_NEE_EMITTERS parity hooks: emitter_sample as the shade stage runs it (u4 = Philox block 1's uniforms), and the
+// MIS density the shade stage gives a BSDF ray whose closest hit (extend kernels, hit0 / hit1) is a sampled emitter
+__global__ void k_light_sample(DScene sc, EmitterTables et, const float *x, const float *u4, size_t n, float *point, float *pdf,
+                               int32_t *object, int32_t *triangle) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const V3 xi = v3(x[i * 3], x[i * 3 + 1], x[i * 3 + 2]);
+  EmitterSample es;
+  const bool ok = emitter_sample(sc, et, xi, u4[i * 4], u4[i * 4 + 1], u4[i * 4 + 2], u4[i * 4 + 3], es);
+  const V3 y = ok ? xi + es.wi * es.dist : v3(0, 0, 0);
+  point[i * 3] = y.x, point[i * 3 + 1] = y.y, point[i * 3 + 2] = y.z;
+  pdf[i] = ok ? es.pdf : 0.0f;
+  object[i] = ok ? sc.lights[es.light].object : -1;
+  triangle[i] = ok && sc.lights[es.light].type == OBJ_MESH ? es.entry : -1;
+}
+__global__ void k_light_pdf(DScene sc, EmitterTables et, const float *o, const float *d, const float4 *hit0, const float4 *hit1, size_t n,
+                            float *pdf) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const float4 h0 = hit0[i], h1 = hit1[i];
+  const uint32_t bits = f2u(h1.w), light = (bits >> kLightShift) & 63u;
+  float p = 0.0f;
+  if ((bits & kHitBit) && light != 0u) {
+    const DLight &L = sc.lights[light - 1u];
+    const V3 pos = v3(h0.x, h0.y, h0.z), ray_d = normalized(v3(d[i * 3], d[i * 3 + 1], d[i * 3 + 2]));
+    const float dl = emitter_area_sampled(L) ? length(pos - v3(o[i * 3], o[i * 3 + 1], o[i * 3 + 2])) : h0.w;
+    p = emitter_mis_pdf(L, emitter_select_prob(et, light - 1u), dl, fabsf(dot(v3(h1.x, h1.y, h1.z), ray_d)));
+  }
+  pdf[i] = p;
 }
 
 __global__ void k_philox(U4 c, uint32_t k0, uint32_t k1, uint32_t *out) {

@@ -147,9 +147,16 @@ struct ptc_scene {
   DevBuf<float> d_sky;
   DevBuf<DLight> d_lights;
   DevBuf<float> d_sky_dist;
+  // PTC_FLAG_NEE_EMITTERS (HostScene::build_emitters): the object table with these light ids, the light list, its tables
+  DevBuf<DObject> d_objects_em;
+  DevBuf<DLight> d_lights_em;
+  DevBuf<float> d_em_sel_cdf, d_em_ent_cdf;
+  DevBuf<float4> d_em_ent;
   std::vector<std::unique_ptr<DevBuf<float4>>> mesh_bufs;
   std::vector<DevMeshBuffers> dev_built;  // per mesh: device arrays left behind by the device-side builder (adopted by upload_scene)
   DScene ds;
+  DScene ds_em;      // ds with d_objects_em and d_lights_em: what every launch of a PTC_FLAG_NEE_EMITTERS render sees
+  EmitterTables et;  // the tables of ds_em's lights
   int mesh_objects = 0;  // mesh entries in object_list = extend rounds needed
 
   int64_t last_pool_slots = 0;  // path-pool slots of the last render (ptc_scene_last_pool_slots)
@@ -283,7 +290,7 @@ int launch_extend(cudaStream_t stream, uint32_t segments, int rounds, Ctl *ctl, 
 // hit0 / hit1 / ids.  ptc_intersect's rays and ptc_render_denoised's feature rays.  `before` / `after`, if given, are
 // recorded around the extend launches.  Returns the number of extend launches.
 int extend_hook_rays(ptc_scene *s, const float *d_o, const float *d_d, uint32_t n, float t_min, float t_max, Ctl *ctl, bool counters,
-                     cudaStream_t st, cudaEvent_t before = nullptr, cudaEvent_t after = nullptr) {
+                     cudaStream_t st, cudaEvent_t before = nullptr, cudaEvent_t after = nullptr, const DScene *ds = nullptr) {
   const uint32_t segments = s->segments();
   const uint32_t cap = (uint32_t)(((uint64_t)n + segments - 1) / segments + kBlock - 1) / kBlock * kBlock;
   s->ws_hook.ensure(segments, cap, s->mesh_objects, true, false);
@@ -294,7 +301,7 @@ int extend_hook_rays(ptc_scene *s, const float *d_o, const float *d_d, uint32_t 
   k_pack_rays<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_o, d_d, (size_t)n, b.ray_o, b.ray_d);
   const ExtendOut eo{b, s->ws_hook.ids.p};
   if (before) CK(cudaEventRecord(before, st));
-  const int launches = launch_extend(st, segments, s->mesh_objects, ctl, s->ds, eo, tq, t_min, t_max, counters);
+  const int launches = launch_extend(st, segments, s->mesh_objects, ctl, ds ? *ds : s->ds, eo, tq, t_min, t_max, counters);
   CK(cudaGetLastError());
   if (after) CK(cudaEventRecord(after, st));
   return launches;
@@ -312,6 +319,7 @@ void check_render_args(const ptc_camera *cam, const ptc_render_settings *st, boo
   if (st->width <= 0 || st->height <= 0 || st->spp <= 0) throw std::invalid_argument("bad render settings");
   if ((int64_t)st->width * st->height > (int64_t)0x3fffffff) throw std::invalid_argument("image too large");
   if ((st->flags & PTC_FLAG_NEE_SKY) && !(st->flags & PTC_FLAG_NEE)) throw std::invalid_argument("PTC_FLAG_NEE_SKY needs PTC_FLAG_NEE");
+  if ((st->flags & PTC_FLAG_NEE_EMITTERS) && !(st->flags & PTC_FLAG_NEE)) throw std::invalid_argument("PTC_FLAG_NEE_EMITTERS needs PTC_FLAG_NEE");
 }
 
 // The samples [begin, end) a call renders: sample_begin = sample_end = 0 means [0, spp)
@@ -369,6 +377,9 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
   const bool nee = (st->flags & PTC_FLAG_NEE) != 0;
   // the sky joins the sampled lights only where there is a sky distribution; elsewhere the flag changes nothing
   const bool nee_sky = nee && (st->flags & PTC_FLAG_NEE_SKY) != 0 && s->ds.sky_dist != nullptr;
+  // emissive meshes and cubes join the sampled lights: every launch sees the object table that carries their light ids
+  const bool nee_em = nee && (st->flags & PTC_FLAG_NEE_EMITTERS) != 0;
+  const DScene &ds = nee_em ? s->ds_em : s->ds;
   const int tiles_x = (st->width + 31) / 32, n_tiles = tiles_x * ((st->height + 31) / 32);
   const uint32_t views = std::max<uint32_t>(pass.views, 1u);  // a batch's tile grids are stacked (the caller checked the size)
   const int n_my_tiles = (tile_rem < n_tiles ? (n_tiles - tile_rem + tile_mod - 1) / tile_mod : 0) * (int)views;
@@ -527,17 +538,17 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
     auto run_extend = [&]() {
       const ExtendOut eo{bufs[flip], nullptr};
       if (timing) mark(ST_PRE);
-      launch_stage(pdl, stream, segments, k_extend_pre, s->d_ctl.p, seg_range(0u, 1u), s->ds, eo, tq, kEps, INFINITY,
+      launch_stage(pdl, stream, segments, k_extend_pre, s->d_ctl.p, seg_range(0u, 1u), ds, eo, tq, kEps, INFINITY,
                    (volatile uint32_t *)d_progress, (uint32_t)(it + 1));  // renderer.rs:24
       for (int r = 0; r < rounds; r++) {
         if (timing) mark(ST_TRAVERSE);
         // (a split launch needs a hand-out counter of its own; a render with more launches than counters goes on unsplit)
         const SegRange tsr = seg_range(trav_seq, (draining || trav_seq >= kTravCounters) ? 1u : trav_parts_bulk);
         trav_seq++;
-        if (counters) launch_stage(pdl, stream, segments, k_traverse<true>, s->d_ctl.p, tsr, s->ds, tq, r, kEps, eo.b.cap, refill);
-        else launch_stage(pdl, stream, segments, k_traverse<false>, s->d_ctl.p, tsr, s->ds, tq, r, kEps, eo.b.cap, refill);
+        if (counters) launch_stage(pdl, stream, segments, k_traverse<true>, s->d_ctl.p, tsr, ds, tq, r, kEps, eo.b.cap, refill);
+        else launch_stage(pdl, stream, segments, k_traverse<false>, s->d_ctl.p, tsr, ds, tq, r, kEps, eo.b.cap, refill);
         if (timing) mark(ST_POST);
-        launch_stage(pdl, stream, segments, k_extend_post, s->d_ctl.p, seg_range(0u, 1u), s->ds, eo, tq, r, kEps, INFINITY);
+        launch_stage(pdl, stream, segments, k_extend_post, s->d_ctl.p, seg_range(0u, 1u), ds, eo, tq, r, kEps, INFINITY);
       }
       launches += 1 + 2 * (uint64_t)rounds;
     };
@@ -545,7 +556,14 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
       if (timing) mark(ST_SHADE);
       const SegRange ssr = seg_range(0u, 1u);
       const int mode = nee_sky ? 2 : (nee ? 1 : 0);
-      if (pass.views > 0) {
+      if (nee_em) {
+        const BatchTables bt = pass.views > 0 ? BatchTables{pass.cams, pass.seeds, (uint32_t)st->width * (uint32_t)st->height, (uint32_t)n_tiles}
+                                              : BatchTables{};
+        auto *kernel = pass.views > 0 ? (nee_sky ? k_shade_em<4, kSrcBatch> : k_shade_em<3, kSrcBatch>)
+                       : pass.pixels  ? (nee_sky ? k_shade_em<4, kSrcList> : k_shade_em<3, kSrcList>)
+                                      : (nee_sky ? k_shade_em<4, kSrcTiles> : k_shade_em<3, kSrcTiles>);
+        launch_stage(pdl, stream, segments, kernel, s->d_ctl.p, ssr, ds, rp, bufs[flip], film, bt, s->et);
+      } else if (pass.views > 0) {
         const BatchTables bt{pass.cams, pass.seeds, (uint32_t)st->width * (uint32_t)st->height, (uint32_t)n_tiles};
         auto *kernel = mode == 2 ? k_shade_batch<2> : mode == 1 ? k_shade_batch<1> : k_shade_batch<0>;
         launch_stage(pdl, stream, segments, kernel, s->d_ctl.p, ssr, s->ds, rp, bufs[flip], film, bt);
@@ -813,6 +831,16 @@ void upload_scene(ptc_scene *s, const HostScene &hs, int device) {
   s->ds.n_meshes = (int32_t)dm.size();
   s->ds.sky_w = hs.sky_w;
   s->ds.sky_h = hs.sky_h;
+  s->d_objects_em.upload(hs.objects_em.data(), hs.objects_em.size());
+  s->d_lights_em.upload(hs.lights_em.data(), hs.lights_em.size());
+  s->d_em_sel_cdf.upload(hs.em_sel_cdf.data(), hs.em_sel_cdf.size());
+  s->d_em_ent.upload(hs.em_ent.data(), hs.em_ent.size());
+  s->d_em_ent_cdf.upload(hs.em_ent_cdf.data(), hs.em_ent_cdf.size());
+  s->ds_em = s->ds;
+  s->ds_em.objects = s->d_objects_em.p;
+  s->ds_em.lights = s->d_lights_em.p;
+  s->ds_em.n_lights = (int32_t)hs.lights_em.size();
+  s->et = EmitterTables{s->d_em_sel_cdf.p, s->d_em_ent.p, s->d_em_ent_cdf.p};
   s->mesh_objects = 0;
   for (const DObject &o : hs.objects)
     if (o.type == OBJ_MESH) s->mesh_objects++;
@@ -1674,6 +1702,61 @@ int ptc_sky_pdf(ptc_scene *s, const float *dirs, int64_t n, float *out_pdf) {
   CK(cudaGetLastError());
   CK(cudaMemcpyAsync(out_pdf, d_pdf.p, N * 4, cudaMemcpyDeviceToHost, s->own_stream));
   CK(cudaStreamSynchronize(s->own_stream));
+  return 0;
+  PTC_GUARD_END
+}
+
+int ptc_light_sample(ptc_scene *s, const float *x, const float *u4, int64_t n, float *out_point, float *out_pdf, int32_t *out_object,
+                     int32_t *out_triangle) {
+  PTC_GUARD_BEGIN
+  require_committed(s);
+  if (n < 0 || (n > 0 && (!x || !u4 || !out_point || !out_pdf || !out_object || !out_triangle))) throw std::invalid_argument("bad argument");
+  if (s->ds_em.n_lights == 0) throw std::logic_error("the committed scene has no emitter PTC_FLAG_NEE_EMITTERS samples");
+  if (n == 0) return 0;
+  CK(cudaSetDevice(s->device));
+  const size_t N = (size_t)n;
+  DevBuf<float> d_x, d_u, d_pt, d_pdf;
+  DevBuf<int32_t> d_obj, d_tri;
+  d_x.upload(x, N * 3);
+  d_u.upload(u4, N * 4);
+  d_pt.alloc(N * 3), d_pdf.alloc(N), d_obj.alloc(N), d_tri.alloc(N);
+  k_light_sample<<<(unsigned)((N + 127) / 128), 128, 0, s->own_stream>>>(s->ds_em, s->et, d_x.p, d_u.p, N, d_pt.p, d_pdf.p, d_obj.p, d_tri.p);
+  CK(cudaGetLastError());
+  CK(cudaMemcpyAsync(out_point, d_pt.p, N * 12, cudaMemcpyDeviceToHost, s->own_stream));
+  CK(cudaMemcpyAsync(out_pdf, d_pdf.p, N * 4, cudaMemcpyDeviceToHost, s->own_stream));
+  CK(cudaMemcpyAsync(out_object, d_obj.p, N * 4, cudaMemcpyDeviceToHost, s->own_stream));
+  CK(cudaMemcpyAsync(out_triangle, d_tri.p, N * 4, cudaMemcpyDeviceToHost, s->own_stream));
+  CK(cudaStreamSynchronize(s->own_stream));
+  return 0;
+  PTC_GUARD_END
+}
+
+int ptc_light_pdf(ptc_scene *s, const float *origins, const float *dirs, int64_t n, float *out_pdf) {
+  PTC_GUARD_BEGIN
+  require_committed(s);
+  if (n < 0 || (n > 0 && (!origins || !dirs || !out_pdf))) throw std::invalid_argument("bad argument");
+  if (s->ds_em.n_lights == 0) throw std::logic_error("the committed scene has no emitter PTC_FLAG_NEE_EMITTERS samples");
+  if (n == 0) return 0;
+  if (n > (int64_t)0x3fffffff) throw std::invalid_argument("too many rays for one call");
+  CK(cudaSetDevice(s->device));
+  ensure_ctl(s);
+  const size_t N = (size_t)n;
+  DevBuf<float> d_o, d_d, d_pdf;
+  DevBuf<Ctl> ctl;
+  d_o.upload(origins, N * 3);
+  d_d.upload(dirs, N * 3);
+  d_pdf.alloc(N);
+  Ctl init;
+  memset(&init, 0, sizeof(init));
+  ctl.upload(&init, 1);
+  cudaStream_t st = s->own_stream;
+  // the render's extend kernels, on the object table whose hit records carry the PTC_FLAG_NEE_EMITTERS light ids
+  extend_hook_rays(s, d_o.p, d_d.p, (uint32_t)n, kEps, INFINITY, ctl.p, false, st, nullptr, nullptr, &s->ds_em);
+  const Buffers b = s->ws_hook.buffers();
+  k_light_pdf<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(s->ds_em, s->et, d_o.p, d_d.p, b.hit0, b.hit1, N, d_pdf.p);
+  CK(cudaGetLastError());
+  CK(cudaMemcpyAsync(out_pdf, d_pdf.p, N * 4, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
   return 0;
   PTC_GUARD_END
 }

@@ -18,6 +18,8 @@ pub const PTC_FLAG_TIMING: i32 = 2;
 pub const PTC_FLAG_NEE: i32 = 4;
 /// with PTC_FLAG_NEE only: NEE also samples the HDR sky as an environment light
 pub const PTC_FLAG_NEE_SKY: i32 = 8;
+/// with PTC_FLAG_NEE only: NEE also samples emissive meshes and cubes, and chooses among emitters by power
+pub const PTC_FLAG_NEE_EMITTERS: i32 = 16;
 
 pub const PTC_MAT_LAMBERT: i32 = 0;
 pub const PTC_MAT_LAMBERT_CHECKER: i32 = 1;
@@ -183,6 +185,10 @@ extern "C" {
     /// the HDR sky as a light (PTC_FLAG_NEE_SKY): sample / pdf hooks; PTC_E_STATE without a sky distribution
     pub fn ptc_sky_sample(s: *mut ptc_scene, u4: *const f32, n: i64, out_dir: *mut f32, out_pdf: *mut f32, out_rgb: *mut f32) -> c_int;
     pub fn ptc_sky_pdf(s: *mut ptc_scene, dirs: *const f32, n: i64, out_pdf: *mut f32) -> c_int;
+    /// PTC_FLAG_NEE_EMITTERS: light sample / MIS density hooks; PTC_E_STATE without a sampled emitter
+    pub fn ptc_light_sample(s: *mut ptc_scene, x: *const f32, u4: *const f32, n: i64, out_point: *mut f32, out_pdf: *mut f32,
+                            out_object: *mut i32, out_triangle: *mut i32) -> c_int;
+    pub fn ptc_light_pdf(s: *mut ptc_scene, origins: *const f32, dirs: *const f32, n: i64, out_pdf: *mut f32) -> c_int;
     pub fn ptc_resolve_device(d_rgb: *const f32, n_pixels: i64, scale: f32, d_out: *mut u32, cuda_stream: *mut c_void) -> c_int;
 
     // in-process multi-GPU: one host thread per device inside the library, one ncclReduce of the film (include/ptcore.h)

@@ -168,6 +168,29 @@ int ptc_scene_add_mesh(ptc_scene *, const float *tris, int64_t n, const float ob
 /* Scene.skybox_hdr_image (src/scene.rs:9): w*h*3 linear floats, row-major, top row first */
 int ptc_scene_set_sky_hdr(ptc_scene *, const float *rgb, int32_t w, int32_t h);
 
+/* Thin-lens depth of field (DESIGN.md 5k).  Let (o, d) be the pinhole ray Camera::get_ray(u, v) of the jittered (u, v) and
+ * f^, r^, u^ the normalised forward, right and true_up.  With R = aperture_radius > 0 and F = focus_distance:
+ *   (dx, dy) = the Shirley-Chiu concentric map of (u[2], u[3]) of the camera jitter's Philox draw onto the unit disk (u[0],
+ *              u[1] stay the pixel jitter, so no random stream moves);
+ *   P = o + d F / dot(d, f^), the focus point: focus is planar, a plane at distance F along the view axis;
+ *   the ray starts at o' = o + R (dx r^ + dy u^) and points along P - o' (normalised).
+ * If dot(d, f^) <= 0, or anything above is not finite (a malformed camera), the ray is the pinhole ray.  R == 0 gives the
+ * pinhole ray itself.  A point at depth z along f^ is smeared over a disk of radius R |1/z - 1/F| in the units of
+ * half_width / half_height. */
+typedef struct ptc_lens {
+  float aperture_radius; /* R >= 0, finite; 0 = pinhole */
+  float focus_distance;  /* F > 0, finite */
+} ptc_lens;
+/* Sets the lenses every render of this handle uses from now on (handle state, as a render in flight is; allowed before
+ * commit, needs no device).  n == 0: pinhole (lenses may be NULL), the state of a new handle.  Every entry needs
+ * aperture_radius >= 0 and finite and focus_distance > 0 and finite; otherwise PTC_E_INVALID and the state is unchanged.
+ * Single-camera calls (ptc_render, _u32, _accumulate, _adaptive, _progressive, _denoised and its feature pass,
+ * ptc_multi_render* through the primary handle's lens at the time of the call, ptc_primary_rays) use lenses[0], and return
+ * PTC_E_INVALID with n > 1.  ptc_render_batch / _batch_accumulate take n == 1 (every view uses it) or n == n_views (view k
+ * uses lenses[k]); any other n is PTC_E_INVALID.  These lens checks come before the scene's state.  A call whose lenses
+ * all have aperture_radius == 0 runs exactly the kernels and launches it runs without a lens. */
+int ptc_scene_set_lens(ptc_scene *, const ptc_lens *lenses, int32_t n);
+
 /* Host half of commit only (reference-BVH dead mask -> SAH -> 8-wide quantised BVH); needs no device.  Optional:
  * ptc_scene_commit runs it if it has not been run. */
 int ptc_scene_build(ptc_scene *);

@@ -49,8 +49,12 @@ pth_scene *pth_load_scene_from_json(const char *json_path);
  *                        reference rejects the whole file, e.g. its own tungsten/teapot/scene.json) becomes the sky
  *   WO3_STRIDE16         read .wo3 triangles with Tungsten's 16-byte records; without it the reader restates the
  *                        reference's 12-byte mis-read (mesh_object.rs:188-190) index for index
- *   SKIP_UNKNOWN         other unknown primitive types are skipped with a warning instead of failing the file */
-enum { PTH_LOAD_INFINITE_SPHERE_SKY = 1, PTH_LOAD_WO3_STRIDE16 = 2, PTH_LOAD_SKIP_UNKNOWN = 4 };
+ *   SKIP_UNKNOWN         other unknown primitive types are skipped with a warning instead of failing the file
+ *   THIN_LENS            a camera of `"type": "thinlens"` gets a lens (pth_scene_lens): aperture_size is the lens radius,
+ *                        focus_distance the focus distance, or |look_at - position| when the key is missing (our rule);
+ *                        aperture textures, cat-eye and focus_pivot are ignored with a warning.  Without the flag the
+ *                        camera is a pinhole, as in the reference */
+enum { PTH_LOAD_INFINITE_SPHERE_SKY = 1, PTH_LOAD_WO3_STRIDE16 = 2, PTH_LOAD_SKIP_UNKNOWN = 4, PTH_LOAD_THIN_LENS = 8 };
 pth_scene *pth_load_scene_from_json_ex(const char *json_path, int flags);
 /* An empty scene to be filled programmatically (tests, synthetic scenes). */
 pth_scene *pth_scene_new(void);
@@ -65,6 +69,8 @@ const pth_object *pth_scene_objects(const pth_scene *);
 int64_t pth_scene_mesh(const pth_scene *, int32_t mesh, const float **tris);
 int pth_scene_sky(const pth_scene *, const float **rgb, int32_t *w, int32_t *h);
 void pth_scene_camera(const pth_scene *, ptc_camera *);
+/* 1 and *out = the camera's lens when the scene has one (PTH_LOAD_THIN_LENS), 0 for a pinhole (out untouched) */
+int pth_scene_lens(const pth_scene *, ptc_lens *out);
 /* RenderSettings: width, height, samples_per_pixel, max_depth (parser.rs:255-292) */
 void pth_scene_settings(const pth_scene *, int32_t *width, int32_t *height, int32_t *spp, int32_t *max_depth);
 
@@ -97,7 +103,8 @@ void pth_transform(const float scale[3], const float rot_deg[3], const float pos
 void pth_camera_new(const float position[3], const float look_at[3], const float up[3], float vfov_deg, float aspect,
                     ptc_camera *out);
 
-/* Feed the description to the product core in object_list order (what the Rust `describe()` walk does). */
+/* Feed the description to the product core in object_list order (what the Rust `describe()` walk does), and the lens if
+ * the scene has one (ptc_scene_set_lens). */
 ptc_scene *pth_build_ptc_scene(const pth_scene *);
 /* render_scene (renderer.rs:67-123): Vec<u32> 0x00RRGGBB, row-major, top row first, on device `device`. */
 int pth_render_scene(const pth_scene *, int device, uint32_t *out_u32, ptc_stats *stats);

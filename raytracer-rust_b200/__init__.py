@@ -24,7 +24,7 @@ DIST_GGX, DIST_BECKMANN = 0, 1
 FLAG_COUNTERS, FLAG_TIMING, FLAG_NEE, FLAG_NEE_SKY, FLAG_NEE_EMITTERS = 1, 2, 4, 8, 16
 COMMIT_FAST_BUILD = 1
 COMMIT_DEVICE_SAH = 2
-LOAD_INFINITE_SPHERE_SKY, LOAD_WO3_STRIDE16, LOAD_SKIP_UNKNOWN = 1, 2, 4
+LOAD_INFINITE_SPHERE_SKY, LOAD_WO3_STRIDE16, LOAD_SKIP_UNKNOWN, LOAD_THIN_LENS = 1, 2, 4, 8
 OBJ_SPHERE, OBJ_PLANE, OBJ_QUAD, OBJ_CUBE, OBJ_MESH = range(5)
 
 
@@ -37,6 +37,10 @@ class Material(C.Structure):  # ptc_material
 class Camera(C.Structure):  # ptc_camera == src/camera.rs:4-11
     _fields_ = [("position", C.c_float * 3), ("forward", C.c_float * 3), ("right", C.c_float * 3),
                 ("true_up", C.c_float * 3), ("half_width", C.c_float), ("half_height", C.c_float)]
+
+
+class Lens(C.Structure):  # ptc_lens
+    _fields_ = [("aperture_radius", C.c_float), ("focus_distance", C.c_float)]
 
 
 class RenderSettings(C.Structure):  # ptc_render_settings
@@ -160,6 +164,7 @@ def core():
     L.ptc_scene_mesh_info.argtypes = [_vp, C.c_int, C.POINTER(MeshInfo), _vp, _vp]
     L.ptc_scene_last_pool_slots.argtypes = [_vp]
     L.ptc_scene_last_pool_slots.restype = C.c_int64
+    L.ptc_scene_set_lens.argtypes = [_vp, C.POINTER(Lens), C.c_int32]
     L.ptc_render.argtypes = [_vp, C.POINTER(Camera), C.POINTER(RenderSettings), _F, C.POINTER(Stats)]
     L.ptc_render_u32.argtypes = [_vp, C.POINTER(Camera), C.POINTER(RenderSettings), _vp, C.POINTER(Stats)]
     L.ptc_render_adaptive.argtypes = [_vp, C.POINTER(Camera), C.POINTER(RenderSettings), C.POINTER(Adaptive), _F, _vp, _vp,
@@ -220,6 +225,7 @@ def host():
     L.pth_scene_sky.argtypes = [_vp, C.POINTER(_F), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
     L.pth_scene_camera.argtypes = [_vp, C.POINTER(Camera)]
     L.pth_scene_camera.restype = None
+    L.pth_scene_lens.argtypes = [_vp, C.POINTER(Lens)]
     L.pth_scene_settings.argtypes = [_vp] + [C.POINTER(C.c_int32)] * 4
     L.pth_scene_settings.restype = None
     L.pth_scene_push_material.argtypes = [_vp, C.POINTER(Material)]
@@ -380,6 +386,14 @@ class Scene:
         c = Camera()
         host().pth_scene_camera(self._h, C.byref(c))
         return c
+
+    @property
+    def lens(self):
+        """(aperture_radius, focus_distance) of a thin-lens camera (LOAD_THIN_LENS), None for a pinhole."""
+        ln = Lens()
+        if not host().pth_scene_lens(self._h, C.byref(ln)):
+            return None
+        return ln.aperture_radius, ln.focus_distance
 
     @property
     def settings(self):
@@ -545,6 +559,20 @@ class CoreScene:
 
     def last_pool_slots(self):
         return int(core().ptc_scene_last_pool_slots(self._h))
+
+    def set_lens(self, aperture_radius=None, focus_distance=None):
+        """Thin-lens depth of field (ptc_scene_set_lens) for every later render of this handle:
+        set_lens(aperture_radius, focus_distance) for one lens, set_lens([(r, f), ...]) for one per batch view, set_lens()
+        or set_lens([]) for a pinhole again."""
+        if aperture_radius is None:
+            pairs = []
+        elif focus_distance is None:
+            pairs = [tuple(p) for p in aperture_radius]
+        else:
+            pairs = [(aperture_radius, focus_distance)]
+        arr = (Lens * max(len(pairs), 1))(*[Lens(float(r), float(f)) for r, f in pairs])
+        _ck(core().ptc_scene_set_lens(self._h, arr if pairs else None, len(pairs)))
+        return self
 
     def mesh_info(self, obj):
         info = MeshInfo()

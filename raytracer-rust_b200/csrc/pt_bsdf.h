@@ -495,6 +495,42 @@ PT_HD Ray camera_get_ray(const DCamera &c, float u, float v) {
   return ray_new(v3(c.position[0], c.position[1], c.position[2]), dir);
 }
 
+// Thin lens (ptc_scene_set_lens): aperture radius R, focus distance F.  (o, d) = the pinhole ray of (u, v); (dx, dy) =
+// the Shirley-Chiu concentric map of (u2, u3) onto the unit disk; the lens origin o' = o + R (dx r^ + dy u^); the ray
+// goes from o' through the focus point P = o + d F / dot(d, f^) (a focus PLANE at distance F along the view axis).
+// P - o' = (F / dot(d, f^)) (d - R (dx r^ + dy u^) dot(d, f^) / F) is normalised in the second form: the same direction,
+// without cancelling against the position or overflowing for a large F.
+// R == 0 returns the pinhole ray itself; so does a degenerate case (dot(d, f^) <= 0, anything not finite).
+PT_HD Ray camera_get_ray_lens(const DCamera &c, float R, float F, float u, float v, float u2, float u3) {
+  const Ray p = camera_get_ray(c, u, v);
+  if (!(R > 0.0f)) return p;
+  const float a = 2.0f * u2 - 1.0f, b = 2.0f * u3 - 1.0f;
+  float r = 0.0f, phi = 0.0f;
+  if (a != 0.0f || b != 0.0f) {
+    if (fabsf(a) > fabsf(b)) r = a, phi = (kPi / 4.0f) * (b / a);
+    else r = b, phi = kPi / 2.0f - (kPi / 4.0f) * (a / b);
+  }
+  float sp, cp;
+#if defined(__CUDA_ARCH__)
+  sincosf(phi, &sp, &cp);
+#else
+  sp = sinf(phi);
+  cp = cosf(phi);
+#endif
+  const float dx = r * cp, dy = r * sp;
+  const V3 fwd = normalized(v3(c.forward[0], c.forward[1], c.forward[2]));
+  const V3 rgt = normalized(v3(c.right[0], c.right[1], c.right[2]));
+  const V3 up = normalized(v3(c.true_up[0], c.true_up[1], c.true_up[2]));
+  const float cd = dot(p.d, fwd);
+  if (!(cd > 0.0f)) return p;
+  const V3 lens = (rgt * dx + up * dy) * R;
+  const V3 o = p.o + lens;
+  const V3 dir = p.d - lens * (cd / F);
+  const Ray q = ray_new(o, dir);
+  if (!(isfinite(q.o.x) && isfinite(q.o.y) && isfinite(q.o.z) && isfinite(q.d.x) && isfinite(q.d.y) && isfinite(q.d.z))) return p;
+  return q;
+}
+
 // renderer.rs:112-120 + color.rs:87-93: sqrt "gamma", clamp, *255, truncate, 0x00RRGGBB
 PT_HD uint32_t resolve_channel(float c) {
   float r = sqrtf(c);

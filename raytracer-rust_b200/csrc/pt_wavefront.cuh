@@ -96,6 +96,12 @@ struct BatchTables {
   uint32_t tiles_per_view;
 };
 
+// ptc_scene_set_lens: (aperture radius, focus distance) per view (a single render is view 0).  Read by k_shade_lens and
+// k_primary_rays_lens only: a trailing kernel argument of their own, like BatchTables.
+struct LensTables {
+  const float2 *lens;
+};
+
 // Path state, SoA of float4.  Segment b = slots [b * cap, b * cap + cnt[b]).
 struct Buffers {
   float4 *ray_o;  // origin.xyz, pixel index
@@ -561,10 +567,13 @@ __device__ __forceinline__ uint32_t block_rank(bool flag, uint32_t *s_warp /* [k
 // Src: where regeneration starts paths.  kSrcTiles: the tiles of tile_mod / tile_rem; kSrcList: rp.pixel_list
 // (ptc_render_adaptive's later passes); kSrcBatch: the stacked tile grids of `bt` (ptc_render_batch).  A template
 // argument, so that the shade kernels of every other render compile to the instructions they had.
+// Lens: camera paths start through the thin lens of `lt` (camera_get_ray_lens, with u[2], u[3] of the jitter draw);
+// only regeneration changes.
 constexpr int kSrcTiles = 0, kSrcList = 1, kSrcBatch = 2;
-template <int Mode, int Src>
+template <int Mode, int Src, bool Lens = false>
 __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, uint32_t *seg_done, Ctl *ctl, const DScene &sc, const RenderParams &rp,
-                                                const Buffers &b, const Film &film, const BatchTables &bt, const EmitterTables &et) {
+                                                const Buffers &b, const Film &film, const BatchTables &bt, const EmitterTables &et,
+                                                const LensTables &lt = LensTables{}) {
   constexpr bool List = Src == kSrcList, Batch = Src == kSrcBatch;
   __shared__ uint16_t s_perm[kShadeWindow];
   __shared__ uint32_t s_hist[2][16];
@@ -889,7 +898,13 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
         const Uniforms4 jit = philox_uniforms(Batch ? bt.seeds[view] : rp.seed, pixel, sample, 0xffffffffu, 0u);
         const float u = ((float)x + jit.u[0]) / (float)rp.width;   // renderer.rs:96
         const float v = ((float)y + jit.u[1]) / (float)rp.height;  // renderer.rs:97
-        const Ray ray = camera_get_ray(Batch ? bt.cams[view] : rp.cam, u, v);
+        Ray ray;
+        if (Lens) {
+          const float2 ln = lt.lens[Batch ? view : 0u];
+          ray = camera_get_ray_lens(Batch ? bt.cams[view] : rp.cam, ln.x, ln.y, u, v, jit.u[2], jit.u[3]);
+        } else {
+          ray = camera_get_ray(Batch ? bt.cams[view] : rp.cam, u, v);
+        }
         b.nray_o[slot] = make_float4(ray.o.x, ray.o.y, ray.o.z, u2f(Batch ? view * bt.view_px + pixel : pixel));
         b.nray_d[slot] = make_float4(ray.d.x, ray.d.y, ray.d.z, u2f(sample));
         b.nbeta[slot] = make_float4(1.0f, 1.0f, 1.0f, u2f(0u));
@@ -1073,6 +1088,15 @@ __global__ void __launch_bounds__(kBlock, kSegPerSM) k_shade_em(Ctl *ctl, SegRan
   stage_shade<Mode, Src>(sr.seg0 + blockIdx.x, sr.n_seg, sr.flags ? sr.flags + sr.n_seg : nullptr, ctl, sc, rp, b, film, bt, et);
   stage_end(sr, sr.seg0 + blockIdx.x);
 }
+// ptc_scene_set_lens with a nonzero aperture: Mode 0-4, paths from any Src, through the thin lens of `lt`.  The lens table
+// is a trailing argument of these instantiations only (see k_shade_em).
+template <int Mode, int Src>
+__global__ void __launch_bounds__(kBlock, kSegPerSM) k_shade_lens(Ctl *ctl, SegRange sr, DScene sc, RenderParams rp, Buffers b, Film film,
+                                                                  BatchTables bt, EmitterTables et, LensTables lt) {
+  stage_begin(sr, sr.seg0 + blockIdx.x, ctl);
+  stage_shade<Mode, Src, true>(sr.seg0 + blockIdx.x, sr.n_seg, sr.flags ? sr.flags + sr.n_seg : nullptr, ctl, sc, rp, b, film, bt, et, lt);
+  stage_end(sr, sr.seg0 + blockIdx.x);
+}
 
 // accum[i] += fp32(film sum i): the end of ptc_render_accumulate (which ADDS into the caller's fp32 film), and
 // ptc_render_adaptive's snapshot
@@ -1172,6 +1196,20 @@ __global__ void k_primary_rays(RenderParams rp, uint32_t sample, float *out_o, f
   const float u = ((float)x + jit.u[0]) / (float)rp.width;
   const float v = ((float)y + jit.u[1]) / (float)rp.height;
   const Ray ray = camera_get_ray(rp.cam, u, v);
+  out_o[pixel * 3 + 0] = ray.o.x, out_o[pixel * 3 + 1] = ray.o.y, out_o[pixel * 3 + 2] = ray.o.z;
+  out_d[pixel * 3 + 0] = ray.d.x, out_d[pixel * 3 + 1] = ray.d.y, out_d[pixel * 3 + 2] = ray.d.z;
+}
+// the same through the thin lens lt.lens[0]: ptc_primary_rays and ptc_render_denoised's feature pass under a lens see
+// exactly the camera rays k_shade_lens starts
+__global__ void k_primary_rays_lens(RenderParams rp, uint32_t sample, float *out_o, float *out_d, LensTables lt) {
+  const uint32_t pixel = blockIdx.x * blockDim.x + threadIdx.x;
+  if (pixel >= (uint32_t)(rp.width * rp.height)) return;
+  const int x = (int)(pixel % (uint32_t)rp.width), y = (int)(pixel / (uint32_t)rp.width);
+  const Uniforms4 jit = philox_uniforms(rp.seed, pixel, sample, 0xffffffffu, 0u);
+  const float u = ((float)x + jit.u[0]) / (float)rp.width;
+  const float v = ((float)y + jit.u[1]) / (float)rp.height;
+  const float2 ln = lt.lens[0];
+  const Ray ray = camera_get_ray_lens(rp.cam, ln.x, ln.y, u, v, jit.u[2], jit.u[3]);
   out_o[pixel * 3 + 0] = ray.o.x, out_o[pixel * 3 + 1] = ray.o.y, out_o[pixel * 3 + 2] = ray.o.z;
   out_d[pixel * 3 + 0] = ray.d.x, out_d[pixel * 3 + 1] = ray.d.y, out_d[pixel * 3 + 2] = ray.d.z;
 }

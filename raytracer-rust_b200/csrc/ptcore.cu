@@ -196,6 +196,10 @@ struct ptc_scene {
   // ptc_render_batch, grow-only: the cameras and seeds of the views (pt_wavefront.cuh: BatchTables)
   DevBuf<DCamera> d_batch_cams;
   DevBuf<uint64_t> d_batch_seeds;
+  // ptc_scene_set_lens: the lenses as set (empty = pinhole), and the (R, F) table of the render in flight, grow-only
+  // (pt_wavefront.cuh: LensTables)
+  std::vector<ptc_lens> lens;
+  DevBuf<float2> d_lens;
   DevBuf<Ctl> d_ctl;
   Ctl *h_ctl = nullptr;  // pinned ring
   uint32_t *h_progress = nullptr;  // pinned + mapped: the word k_extend_pre reports the state of the render in
@@ -361,7 +365,41 @@ struct Pass {
   uint32_t views = 0;                // > 0: a batch (tile_mod = 0); its cameras and seeds, device tables of `views` entries
   const DCamera *cams = nullptr;
   const uint64_t *seeds = nullptr;
+  const float2 *lens = nullptr;      // device, (R, F) per view (one for a single camera); nullptr: pinhole, today's kernels
 };
+
+// The lens a single-camera call uses: lenses[0] of ptc_scene_set_lens, nullptr for a pinhole or a zero aperture (the call
+// then runs exactly the kernels it runs without a lens).  Checked before the scene's state.
+const ptc_lens *single_lens(const ptc_scene *s) {
+  if (s->lens.size() > 1) throw std::invalid_argument("a single-camera call uses one lens: ptc_scene_set_lens was given n > 1");
+  return !s->lens.empty() && s->lens[0].aperture_radius > 0.0f ? &s->lens[0] : nullptr;
+}
+
+// n lenses into the device table of `d` (the scene a render runs on), one copy on `stream`; nullptr when none has an
+// aperture.  The table grows only, and is allocated before the copy (ptc_multi allocates it before its threads start).
+const float2 *upload_lens(ptc_scene *d, const ptc_lens *l, size_t n, cudaStream_t stream) {
+  static_assert(sizeof(ptc_lens) == sizeof(float2), "ptc_lens and float2 share one layout");
+  bool any = false;
+  for (size_t k = 0; k < n; k++) any = any || l[k].aperture_radius > 0.0f;
+  if (!any) return nullptr;
+  if (d->d_lens.n < n) d->d_lens.alloc(n);
+  // (from pageable memory: the call returns once the source has been read)
+  CK(cudaMemcpyAsync(d->d_lens.p, l, n * sizeof(float2), cudaMemcpyHostToDevice, stream));
+  return d->d_lens.p;
+}
+
+// k_shade_lens<mode, Src>: 0 plain, 1 NEE, 2 NEE + sky, 3 NEE + emitters, 4 NEE + sky + emitters
+using ShadeLensKernel = void (*)(Ctl *, SegRange, DScene, RenderParams, Buffers, Film, BatchTables, EmitterTables, LensTables);
+template <int Src>
+ShadeLensKernel shade_lens_kernel(int mode) {
+  switch (mode) {
+    case 0: return k_shade_lens<0, Src>;
+    case 1: return k_shade_lens<1, Src>;
+    case 2: return k_shade_lens<2, Src>;
+    case 3: return k_shade_lens<3, Src>;
+    default: return k_shade_lens<4, Src>;
+  }
+}
 
 // the wavefront loop; renders into the scene's fixed-point film and then adds its fp32 image into d_accum on `stream`
 // (d_accum == nullptr: the caller takes the fixed-point film itself).  The caller has checked the scene's state and
@@ -556,7 +594,16 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
       if (timing) mark(ST_SHADE);
       const SegRange ssr = seg_range(0u, 1u);
       const int mode = nee_sky ? 2 : (nee ? 1 : 0);
-      if (nee_em) {
+      if (pass.lens) {
+        const BatchTables bt = pass.views > 0 ? BatchTables{pass.cams, pass.seeds, (uint32_t)st->width * (uint32_t)st->height, (uint32_t)n_tiles}
+                                              : BatchTables{};
+        const int lmode = nee_em ? (nee_sky ? 4 : 3) : mode;
+        auto *kernel = pass.views > 0 ? shade_lens_kernel<kSrcBatch>(lmode)
+                       : pass.pixels  ? shade_lens_kernel<kSrcList>(lmode)
+                                      : shade_lens_kernel<kSrcTiles>(lmode);
+        launch_stage(pdl, stream, segments, kernel, s->d_ctl.p, ssr, ds, rp, bufs[flip], film, bt, nee_em ? s->et : EmitterTables{},
+                     LensTables{pass.lens});
+      } else if (nee_em) {
         const BatchTables bt = pass.views > 0 ? BatchTables{pass.cams, pass.seeds, (uint32_t)st->width * (uint32_t)st->height, (uint32_t)n_tiles}
                                               : BatchTables{};
         auto *kernel = pass.views > 0 ? (nee_sky ? k_shade_em<4, kSrcBatch> : k_shade_em<3, kSrcBatch>)
@@ -985,6 +1032,19 @@ int ptc_scene_set_sky_hdr(ptc_scene *s, const float *rgb, int32_t w, int32_t h) 
   PTC_GUARD_END
 }
 
+int ptc_scene_set_lens(ptc_scene *s, const ptc_lens *lenses, int32_t n) {
+  PTC_GUARD_BEGIN
+  if (!s || n < 0 || (n > 0 && !lenses)) throw std::invalid_argument("bad argument");
+  for (int32_t k = 0; k < n; k++) {
+    const float r = lenses[k].aperture_radius, f = lenses[k].focus_distance;
+    if (!(r >= 0.0f) || !std::isfinite(r)) throw std::invalid_argument("aperture_radius must be >= 0 and finite");
+    if (!(f > 0.0f) || !std::isfinite(f)) throw std::invalid_argument("focus_distance must be > 0 and finite");
+  }
+  s->lens.assign(lenses, lenses + n);
+  return 0;
+  PTC_GUARD_END
+}
+
 int ptc_scene_build(ptc_scene *s) {
   PTC_GUARD_BEGIN
   if (!s) throw std::invalid_argument("null argument");
@@ -1078,11 +1138,18 @@ int ptc_scene_mesh_info(const ptc_scene *s, int object, ptc_mesh_info *info, uin
 int ptc_render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_settings *st, float *d_accum,
                           void *cuda_stream, ptc_stats *stats) {
   PTC_GUARD_BEGIN
+  if (!s) throw std::invalid_argument("null argument");
+  const ptc_lens *lens = single_lens(s);
   require_committed(s);
   check_render_args(cam, st, d_accum != nullptr);
   // the caller's handle is honoured as given: NULL is the legacy default stream, which orders the film atomics after
   // whatever the caller queued there (a memset of d_accum, a wait on a collective)
-  render_accumulate(s, cam, st, d_accum, (cudaStream_t)cuda_stream, stats);
+  Pass pass;
+  if (lens) {
+    CK(cudaSetDevice(s->device));
+    pass.lens = upload_lens(s, lens, 1, (cudaStream_t)cuda_stream);
+  }
+  render_accumulate(s, cam, st, d_accum, (cudaStream_t)cuda_stream, stats, pass);
   return 0;
   PTC_GUARD_END
 }
@@ -1092,9 +1159,16 @@ int ptc_render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_
 static int render_to_host(ptc_scene *s, const ptc_camera *cam, const ptc_render_settings *st, float *out_rgb, uint32_t *out_u32,
                           ptc_stats *stats) {
   PTC_GUARD_BEGIN
+  if (!s) throw std::invalid_argument("null argument");
+  const ptc_lens *lens = single_lens(s);
   require_committed(s);
   check_render_args(cam, st, out_rgb || out_u32);
-  render_accumulate(s, cam, st, nullptr, s->own_stream, stats);
+  Pass pass;
+  if (lens) {
+    CK(cudaSetDevice(s->device));
+    pass.lens = upload_lens(s, lens, 1, s->own_stream);
+  }
+  render_accumulate(s, cam, st, nullptr, s->own_stream, stats, pass);
   const int launches = resolve_film_to_host(s, (size_t)st->width * st->height, 1.0f / (float)st->spp, nullptr, out_rgb, out_u32, s->own_stream);
   if (stats) stats->kernel_launches += launches;
   return 0;
@@ -1110,9 +1184,11 @@ int ptc_render_u32(ptc_scene *s, const ptc_camera *cam, const ptc_render_setting
 }
 
 // ptc_render_batch / ptc_render_batch_accumulate: the arguments, before the scene's state
-static void check_batch_args(const ptc_camera *cams, int32_t n_views, const ptc_render_settings *st, bool has_output) {
+static void check_batch_args(const ptc_scene *s, const ptc_camera *cams, int32_t n_views, const ptc_render_settings *st, bool has_output) {
   check_render_args(cams, st, has_output);
   if (n_views < 1) throw std::invalid_argument("n_views must be >= 1");
+  if (s->lens.size() > 1 && s->lens.size() != (size_t)n_views)
+    throw std::invalid_argument("ptc_scene_set_lens gave n lenses: a batch needs n == 1 or n == n_views");
   if (st->tile_mod != 0) throw std::invalid_argument("ptc_render_batch renders whole views: tile_mod must be 0");
   // the film index of every padded pixel of every view stays below 2^30 (a pool entry's pixel word keeps kShadowBit)
   const uint64_t padded = (uint64_t)n_views * (((uint64_t)st->width + 31u) & ~31ull) * (((uint64_t)st->height + 31u) & ~31ull);
@@ -1134,6 +1210,11 @@ static Pass batch_pass(ptc_scene *s, const ptc_camera *cams, int32_t n_views, co
   CK(cudaMemcpyAsync(s->d_batch_seeds.p, seeds, n * sizeof(uint64_t), cudaMemcpyHostToDevice, stream));
   Pass pass;
   pass.views = (uint32_t)n_views, pass.cams = s->d_batch_cams.p, pass.seeds = s->d_batch_seeds.p;
+  if (!s->lens.empty()) {  // one lens for every view, or one per view
+    std::vector<ptc_lens> per(n, s->lens[0]);
+    if (s->lens.size() == n) per = s->lens;
+    pass.lens = upload_lens(s, per.data(), n, stream);
+  }
   return pass;
 }
 
@@ -1142,7 +1223,7 @@ int ptc_render_batch(ptc_scene *s, const ptc_camera *cams, int32_t n_views, cons
   PTC_GUARD_BEGIN
   // the arguments first, the scene's state after them
   if (!s) throw std::invalid_argument("null argument");
-  check_batch_args(cams, n_views, st, out_rgb || out_u32);
+  check_batch_args(s, cams, n_views, st, out_rgb || out_u32);
   require_committed(s);
   const Pass pass = batch_pass(s, cams, n_views, seeds, st, s->own_stream);
   render_accumulate(s, cams, st, nullptr, s->own_stream, stats, pass);
@@ -1157,7 +1238,7 @@ int ptc_render_batch_accumulate(ptc_scene *s, const ptc_camera *cams, int32_t n_
                                 float *d_accum, void *cuda_stream, ptc_stats *stats) {
   PTC_GUARD_BEGIN
   if (!s) throw std::invalid_argument("null argument");
-  check_batch_args(cams, n_views, st, d_accum != nullptr);
+  check_batch_args(s, cams, n_views, st, d_accum != nullptr);
   require_committed(s);
   const Pass pass = batch_pass(s, cams, n_views, seeds, st, (cudaStream_t)cuda_stream);
   render_accumulate(s, cams, st, d_accum, (cudaStream_t)cuda_stream, stats, pass);
@@ -1175,6 +1256,7 @@ int ptc_render_adaptive(ptc_scene *s, const ptc_camera *cam, const ptc_render_se
     throw std::invalid_argument("ptc_render_adaptive schedules the samples itself: sample_begin, sample_end and tile_mod must be 0");
   if (ad->min_spp < 2 || ad->min_spp % 2 != 0 || ad->min_spp > st->spp) throw std::invalid_argument("min_spp must be even, >= 2 and <= spp");
   if (!(ad->threshold >= 0.0f)) throw std::invalid_argument("threshold must be >= 0");
+  const ptc_lens *lens = single_lens(s);
   require_committed(s);
   CK(cudaSetDevice(s->device));
   ensure_ctl(s);
@@ -1197,14 +1279,16 @@ int ptc_render_adaptive(ptc_scene *s, const ptc_camera *cam, const ptc_render_se
 
   // passes 0 and 1 over the tiles, the snapshot between them
   const int half = ad->min_spp / 2;
+  Pass first;
+  first.lens = lens ? upload_lens(s, lens, 1, stream) : nullptr;
   CK(cudaEventRecord(s->ev_adapt_begin, stream));
-  render_pass(s, cam, st, 0, half, Pass(), stream, total);
+  render_pass(s, cam, st, 0, half, first, stream, total);
   const Film f = s->film();
   float *vp = s->w_adapt_vp.p;
   CK(cudaMemsetAsync(vp, 0, (size_t)n_px * 3 * sizeof(float), stream));
   k_film_to_accum<<<(unsigned)(((size_t)n_px * 3 + 255) / 256), 256, 0, stream>>>(f, n_px, vp);
   launches += 1;
-  Pass more;
+  Pass more = first;
   more.clear_film = false;
   render_pass(s, cam, st, half, ad->min_spp, more, stream, total);
   k_adapt_init<<<nb, 256, 0, stream>>>(n_px, st->spp, s->w_adapt_list[0].p, s->w_adapt_needs.p, s->w_adapt_spp.p);
@@ -1266,6 +1350,7 @@ int ptc_render_progressive(ptc_scene *s, const ptc_camera *cam, const ptc_render
     throw std::invalid_argument("ptc_render_progressive schedules the samples itself: sample_begin, sample_end and tile_mod must be 0");
   if (pg->first_spp < 1 || pg->first_spp > st->spp) throw std::invalid_argument("first_spp must be >= 1 and <= spp");
   if (pg->max_pass_spp < 0) throw std::invalid_argument("max_pass_spp must be >= 0");
+  const ptc_lens *lens = single_lens(s);
   require_committed(s);
   CK(cudaSetDevice(s->device));
   ensure_ctl(s);
@@ -1284,6 +1369,7 @@ int ptc_render_progressive(ptc_scene *s, const ptc_camera *cam, const ptc_render
     s->h_preview_px = n_px;
   }
   cudaStream_t stream = s->own_stream;
+  const float2 *d_lens = lens ? upload_lens(s, lens, 1, stream) : nullptr;
 
   // What the two threads share, under `mu`.  The worker publishes pass j (ready = j + 1, samples[j % 2]) once its slot
   // event is recorded; the calling thread publishes callback j's return (shown = j + 1) and a stop.
@@ -1311,6 +1397,7 @@ int ptc_render_progressive(ptc_scene *s, const ptc_camera *cam, const ptc_render
         const int next = j == 0 ? pg->first_spp : progressive_next(n, st->spp, pg->max_pass_spp);
         Pass pass;
         pass.clear_film = j == 0;
+        pass.lens = d_lens;
         render_pass(s, cam, st, n, next, pass, stream, total);
         k_resolve_film<<<(unsigned)((n_px + 255) / 256), 256, 0, stream>>>(s->film(), n_px, 1.0f / (float)next, nullptr,
                                                                            out_rgb ? s->w_prog_rgb[j & 1].p : nullptr,
@@ -1437,6 +1524,7 @@ int ptc_render_denoised(ptc_scene *s, const ptc_camera *cam, const ptc_render_se
   if (st->spp < 2) throw std::invalid_argument("ptc_render_denoised needs spp >= 2: the variance comes from two halves of the samples");
   if (dn->feature_spp < 1 || dn->feature_spp > st->spp) throw std::invalid_argument("feature_spp must be >= 1 and <= spp");
   check_denoise_filter(dn);
+  const ptc_lens *lens = single_lens(s);
   require_committed(s);
   CK(cudaSetDevice(s->device));
   ensure_ctl(s);
@@ -1458,11 +1546,13 @@ int ptc_render_denoised(ptc_scene *s, const ptc_camera *cam, const ptc_render_se
 
   // 1. the render in two halves, the fp32 film sums of the first one kept: the film is ptc_render's
   const int half = st->spp / 2;
+  Pass first;
+  first.lens = lens ? upload_lens(s, lens, 1, stream) : nullptr;
   CK(cudaEventRecord(s->ev_dn_begin, stream));
-  render_pass(s, cam, st, 0, half, Pass(), stream, total);
+  render_pass(s, cam, st, 0, half, first, stream, total);
   CK(cudaMemsetAsync(s->w_dn_half.p, 0, n3 * sizeof(float), stream));
   k_film_to_accum<<<(unsigned)((n3 + 255) / 256), 256, 0, stream>>>(s->film(), n_px, s->w_dn_half.p);
-  Pass more;
+  Pass more = first;
   more.clear_film = false;
   render_pass(s, cam, st, half, st->spp, more, stream, total);
   launches += 1;
@@ -1477,7 +1567,8 @@ int ptc_render_denoised(ptc_scene *s, const ptc_camera *cam, const ptc_render_se
   rp.width = st->width, rp.height = st->height, rp.seed = st->seed;
   float *ray_o = s->w_dn_rays.p, *ray_d = s->w_dn_rays.p + n3;
   for (int k = 0; k < dn->feature_spp; k++) {
-    k_primary_rays<<<nb, 256, 0, stream>>>(rp, (uint32_t)k, ray_o, ray_d);
+    if (first.lens) k_primary_rays_lens<<<nb, 256, 0, stream>>>(rp, (uint32_t)k, ray_o, ray_d, LensTables{first.lens});
+    else k_primary_rays<<<nb, 256, 0, stream>>>(rp, (uint32_t)k, ray_o, ray_d);
     launches += 3 + extend_hook_rays(s, ray_o, ray_d, n_px, kEps, INFINITY, s->w_dn_ctl.p, false, stream);
     const Buffers b = s->ws_hook.buffers();
     k_feature_add<<<nb, 256, 0, stream>>>(b.hit0, b.hit1, s->ds.materials, n_px, s->w_dn_albedo.p, s->w_dn_normal.p);
@@ -1615,6 +1706,8 @@ int ptc_intersect(ptc_scene *s, const float *origins, const float *dirs, int64_t
 int ptc_primary_rays(ptc_scene *s, const ptc_camera *cam, const ptc_render_settings *st, int32_t sample, float *out_o,
                      float *out_d) {
   PTC_GUARD_BEGIN
+  if (!s) throw std::invalid_argument("null argument");
+  const ptc_lens *lens = single_lens(s);
   require_committed(s);
   if (!cam || !st || !out_o || !out_d || st->width <= 0 || st->height <= 0) throw std::invalid_argument("bad argument");
   CK(cudaSetDevice(s->device));
@@ -1626,7 +1719,12 @@ int ptc_primary_rays(ptc_scene *s, const ptc_camera *cam, const ptc_render_setti
   DevBuf<float> d_o, d_d;
   d_o.alloc(n * 3);
   d_d.alloc(n * 3);
-  k_primary_rays<<<(unsigned)((n + 255) / 256), 256, 0, s->own_stream>>>(rp, (uint32_t)sample, d_o.p, d_d.p);
+  if (lens) {
+    k_primary_rays_lens<<<(unsigned)((n + 255) / 256), 256, 0, s->own_stream>>>(rp, (uint32_t)sample, d_o.p, d_d.p,
+                                                                                LensTables{upload_lens(s, lens, 1, s->own_stream)});
+  } else {
+    k_primary_rays<<<(unsigned)((n + 255) / 256), 256, 0, s->own_stream>>>(rp, (uint32_t)sample, d_o.p, d_d.p);
+  }
   CK(cudaGetLastError());
   CK(cudaMemcpyAsync(out_o, d_o.p, n * 12, cudaMemcpyDeviceToHost, s->own_stream));
   CK(cudaMemcpyAsync(out_d, d_d.p, n * 12, cudaMemcpyDeviceToHost, s->own_stream));
@@ -1818,6 +1916,8 @@ static int multi_render(ptc_multi *m, const ptc_camera *cam, const ptc_render_se
   check_render_args(cam, st, out_rgb || out_u32);
   if (st->tile_mod > 0) throw std::invalid_argument("ptc_multi_render shards by itself: tile_mod must be 0");
   if (shard_mode != PTC_SHARD_SAMPLES && shard_mode != PTC_SHARD_TILES) throw std::invalid_argument("bad shard mode");
+  // every device renders through the primary handle's lens
+  const ptc_lens *lens = single_lens(m->primary);
   const int n = (int)m->scenes.size();
   int s_begin, s_end;
   sample_range(st, s_begin, s_end);
@@ -1832,6 +1932,7 @@ static int multi_render(ptc_multi *m, const ptc_camera *cam, const ptc_render_se
     ptc_scene *s = m->scenes[(size_t)i];
     CK(cudaSetDevice(s->device));
     ensure_film(s, n_px);
+    if (lens && s->d_lens.n < 1) s->d_lens.alloc(1);
   }
   std::mutex abort_mutex;
   auto work = [&](int i) {
@@ -1852,8 +1953,10 @@ static int multi_render(ptc_multi *m, const ptc_camera *cam, const ptc_render_se
         mine.tile_mod = n, mine.tile_rem = i;
       }
       memset(&per[(size_t)i], 0, sizeof(ptc_stats));
+      Pass pass;
+      pass.lens = lens && !idle ? upload_lens(s, lens, 1, stream) : nullptr;
       if (idle) clear_film(s, n_px, stream);
-      else render_accumulate(s, cam, &mine, nullptr, stream, &per[(size_t)i]);  // leaves the shard in the device's fixed-point film
+      else render_accumulate(s, cam, &mine, nullptr, stream, &per[(size_t)i], pass);  // leaves the shard in the device's fixed-point film
       film_ok = true;
     } catch (std::exception &e) {
       errors[(size_t)i] = e.what();

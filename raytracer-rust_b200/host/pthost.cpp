@@ -125,6 +125,8 @@ struct pth_scene {
   std::vector<float> sky;
   int32_t sky_w = 0, sky_h = 0;
   ptc_camera camera;
+  bool has_lens = false;  // PTH_LOAD_THIN_LENS: a "thinlens" camera's lens
+  ptc_lens lens = {0.0f, 0.0f};
   int32_t width = 800, height = 600, spp = 16, max_depth = 10;  // parser.rs:255-258
   pth_scene() { memset(&camera, 0, sizeof(camera)); }
 };
@@ -649,6 +651,19 @@ pth_scene *load_scene(const std::string &json_path, int flags) {
   float aspect = (float)s->width / (float)s->height;
   if (const pth::Json *a = cam->find("aspect"); a && a->is_number()) aspect = (float)a->num;
   camera_new(cpos, clook, cup, (float)fov->num, aspect, &s->camera);
+  if (const pth::Json *ty = cam->find("type"); (flags & PTH_LOAD_THIN_LENS) && ty && ty->is_string() && ty->str == "thinlens") {
+    // Tungsten's aperture_size is the lens radius.  Without focus_distance we focus on look_at (our rule, not Tungsten's).
+    const pth::Json *ap = cam->find("aperture_size"), *fd = cam->find("focus_distance");
+    s->lens.aperture_radius = ap && ap->is_number() ? (float)ap->num : 0.0f;
+    const float dx = clook.x - cpos.x, dy = clook.y - cpos.y, dz = clook.z - cpos.z;
+    s->lens.focus_distance = fd && fd->is_number() ? (float)fd->num : std::sqrt(dx * dx + dy * dy + dz * dz);
+    s->has_lens = true;
+    for (const char *k : {"aperture", "cateye", "catEye", "focus_pivot"})
+      if (cam->find(k)) {
+        fprintf(stderr, "Warning: thinlens camera: aperture textures, cat-eye and focus_pivot are not supported and are ignored.\n");
+        break;
+      }
+  }
 
   // ---- bsdfs, parser.rs:308-495
   std::map<std::string, int> bsdfs;
@@ -971,6 +986,11 @@ int pth_scene_sky(const pth_scene *s, const float **rgb, int32_t *w, int32_t *h)
   return 1;
 }
 void pth_scene_camera(const pth_scene *s, ptc_camera *c) { *c = s->camera; }
+int pth_scene_lens(const pth_scene *s, ptc_lens *out) {
+  if (!s->has_lens) return 0;
+  if (out) *out = s->lens;
+  return 1;
+}
 void pth_scene_settings(const pth_scene *s, int32_t *w, int32_t *h, int32_t *spp, int32_t *md) {
   if (w) *w = s->width;
   if (h) *h = s->height;
@@ -1151,6 +1171,7 @@ struct CoreApi {
   decltype(&::ptc_scene_set_sky_hdr) set_sky_hdr = nullptr;
   decltype(&::ptc_scene_commit) commit = nullptr;
   decltype(&::ptc_render_u32) render_u32 = nullptr;
+  decltype(&::ptc_scene_set_lens) set_lens = nullptr;
   bool ok = false;
   std::string err;
   CoreApi() {
@@ -1176,6 +1197,7 @@ struct CoreApi {
     bind(add_material, "ptc_scene_add_material"), bind(add_sphere, "ptc_scene_add_sphere"), bind(add_plane, "ptc_scene_add_plane");
     bind(add_quad, "ptc_scene_add_quad"), bind(add_cube, "ptc_scene_add_cube"), bind(add_mesh, "ptc_scene_add_mesh");
     bind(set_sky_hdr, "ptc_scene_set_sky_hdr"), bind(commit, "ptc_scene_commit"), bind(render_u32, "ptc_render_u32");
+    bind(set_lens, "ptc_scene_set_lens");
     ok = all;
   }
 };
@@ -1223,6 +1245,7 @@ ptc_scene *pth_build_ptc_scene(const pth_scene *s) {
     if (r < 0) return fail();
   }
   if (!s->sky.empty() && api->set_sky_hdr(c, s->sky.data(), s->sky_w, s->sky_h) < 0) return fail();
+  if (s->has_lens && api->set_lens(c, &s->lens, 1) < 0) return fail();
   return c;
 }
 

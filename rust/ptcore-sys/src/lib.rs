@@ -126,6 +126,14 @@ pub struct ptc_denoise {
     pub sigma_albedo: f32,
 }
 
+/// Thin lens (ptc_scene_set_lens): aperture radius >= 0 (0 = pinhole) and focus distance > 0, both finite
+#[repr(C)]
+#[derive(Clone, Copy, Default)]
+pub struct ptc_lens {
+    pub aperture_radius: f32,
+    pub focus_distance: f32,
+}
+
 #[repr(C)]
 pub struct ptc_scene {
     _private: [u8; 0],
@@ -146,6 +154,8 @@ extern "C" {
     pub fn ptc_scene_add_mesh(s: *mut ptc_scene, tris: *const f32, n: i64, object_to_world: *const f32,
                               world_to_object: *const f32, material: c_int) -> c_int;
     pub fn ptc_scene_set_sky_hdr(s: *mut ptc_scene, rgb: *const f32, w: i32, h: i32) -> c_int;
+    /// n == 0: pinhole; single-camera renders use lenses[0] (n > 1: PTC_E_INVALID), batches n == 1 or n == n_views
+    pub fn ptc_scene_set_lens(s: *mut ptc_scene, lenses: *const ptc_lens, n: i32) -> c_int;
     pub fn ptc_scene_build(s: *mut ptc_scene) -> c_int;
     pub fn ptc_scene_last_pool_slots(s: *const ptc_scene) -> i64;
     pub fn ptc_scene_commit(s: *mut ptc_scene, device: c_int) -> c_int;

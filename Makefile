@@ -26,9 +26,9 @@ $(PKG)/libpthost.so: $(PKG)/host/pthost.cpp $(PKG)/host/json.hpp include/pthost.
 oracle/liboracle.so: oracle/oracle.cpp oracle/oracle.h
 	$(MAKE) -C oracle
 
-tests/hostsim/libhostsim.so: tests/hostsim/hostsim.cpp tests/hostsim/wfsim.cpp tests/hostsim/skysim.cpp tests/hostsim/adaptsim.cpp tests/hostsim/denoisesim.cpp tests/hostsim/emsim.cpp tests/hostsim/lenssim.cpp $(CSRC)/pt_build.cpp $(HDRS)
+tests/hostsim/libhostsim.so: tests/hostsim/hostsim.cpp tests/hostsim/wfsim.cpp tests/hostsim/skysim.cpp tests/hostsim/adaptsim.cpp tests/hostsim/denoisesim.cpp tests/hostsim/emsim.cpp tests/hostsim/lenssim.cpp tests/hostsim/motionsim.cpp $(CSRC)/pt_build.cpp $(HDRS)
 	$(CXX) $(CXXFLAGS) -shared -o $@ tests/hostsim/hostsim.cpp tests/hostsim/wfsim.cpp tests/hostsim/skysim.cpp tests/hostsim/adaptsim.cpp \
-		tests/hostsim/denoisesim.cpp tests/hostsim/emsim.cpp tests/hostsim/lenssim.cpp \
+		tests/hostsim/denoisesim.cpp tests/hostsim/emsim.cpp tests/hostsim/lenssim.cpp tests/hostsim/motionsim.cpp \
 		$(CSRC)/pt_build.cpp
 
 clean:

@@ -191,6 +191,34 @@ typedef struct ptc_lens {
  * all have aperture_radius == 0 runs exactly the kernels and launches it runs without a lens. */
 int ptc_scene_set_lens(ptc_scene *, const ptc_lens *lenses, int32_t n);
 
+/* Motion blur (DESIGN.md 5l).  Every camera sample has a shutter time tau = u[0] of
+ * philox_uniforms(seed of the view, pixel in the view, sample, 0xffffffff, 1), in [0, 1) (block 1 of the camera-jitter
+ * counter, which no other draw uses: every random stream stays as it is).  The path and every ray it spawns (bounces,
+ * NEE shadow rays) carry that tau.
+ *   Object motion: D_k is the world-space displacement of object k over the shutter; at tau the object is its committed
+ *   self translated by tau D_k (translation only: no rotation, scale or keyframes).  Object k is intersected with the ray
+ *   (o.x - tau D.x, o.y - tau D.y, o.z - tau D.z), the same d, t_min and shrinking closest, for every type (the cube's
+ *   normal and the mesh's object-space ray included); it reports t as found in that frame, the position p + tau D (per
+ *   component) and the normal unchanged.  An object whose D is exactly (0, 0, 0) is intersected as without motion.
+ *   Camera motion: each camera has an end camera; at tau every float field of ptc_camera is c0 + tau (c1 - c0) (a large
+ *   rotation is lerped component-wise, not slerped; the ray direction is normalised anyway).  An end camera equal to the
+ *   start camera bit for bit leaves the start camera unchanged.  A lens applies to the camera at tau.
+ *   Next-event estimation: a light of a moving object is sampled from x - tau D_L, so the sampled point moves by +tau D_L;
+ *   wi, the distance, every pdf and MIS weight come out as for the static light seen from the shifted point.  The sky does
+ *   not move.
+ * A call in which no object moves and every end camera equals its start camera runs exactly the kernels and launches it
+ * runs without motion. */
+/* D of `object` for every later render of this handle (handle state, like the lens: allowed before and after commit).
+ * (0, 0, 0) makes the object static again.  An object index out of range or a non-finite component: PTC_E_INVALID, and
+ * the previous state stays. */
+int ptc_scene_set_object_motion(ptc_scene *, int32_t object, const float displacement[3]);
+/* The end cameras every later render of this handle uses.  n == 0: a static camera (end_cameras may be NULL), the state
+ * of a new handle.  Any non-finite field: PTC_E_INVALID, and the previous state stays.  The counts follow
+ * ptc_scene_set_lens: single-camera calls use end_cameras[0] and return PTC_E_INVALID with n > 1; ptc_render_batch /
+ * _batch_accumulate take n == 1 (every view) or n == n_views (view k uses end_cameras[k]).  These checks come before the
+ * scene's state. */
+int ptc_scene_set_camera_motion(ptc_scene *, const ptc_camera *end_cameras, int32_t n);
+
 /* Host half of commit only (reference-BVH dead mask -> SAH -> 8-wide quantised BVH); needs no device.  Optional:
  * ptc_scene_commit runs it if it has not been run. */
 int ptc_scene_build(ptc_scene *);
@@ -344,7 +372,14 @@ int ptc_multi_render_u32(ptc_multi *, const ptc_camera *, const ptc_render_setti
 /* HittableList::hit for n caller-provided rays (directions used as given). */
 int ptc_intersect(ptc_scene *, const float *origins, const float *dirs, int64_t n, float t_min, float t_max,
                   ptc_hit *out, ptc_stats *stats);
-/* Camera::get_ray + the Philox jitter for sample `sample` of every pixel: out_o/out_d = W*H*3 floats. */
+/* ptc_intersect for rays at the shutter times `times` (n floats, each in [0, 1]; otherwise PTC_E_INVALID) under the
+ * handle's object motion. */
+int ptc_intersect_at(ptc_scene *, const float *origins, const float *dirs, const float *times, int64_t n, float t_min,
+                     float t_max, ptc_hit *out, ptc_stats *stats);
+/* The shutter time tau of camera sample `sample` of every pixel (settings' seed, width and height): W*H floats. */
+int ptc_ray_times(ptc_scene *, const ptc_render_settings *, int32_t sample, float *out_time);
+/* Camera::get_ray + the Philox jitter for sample `sample` of every pixel: out_o/out_d = W*H*3 floats.  Through the
+ * handle's lens and at each ray's shutter time under its camera motion, as the renders start their paths. */
 int ptc_primary_rays(ptc_scene *, const ptc_camera *, const ptc_render_settings *, int32_t sample, float *out_o,
                      float *out_d);
 /* Material::emitted + Material::scatter for n (ray_dir, position, normal, front_face, u[4]) tuples.

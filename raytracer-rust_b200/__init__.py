@@ -165,6 +165,8 @@ def core():
     L.ptc_scene_last_pool_slots.argtypes = [_vp]
     L.ptc_scene_last_pool_slots.restype = C.c_int64
     L.ptc_scene_set_lens.argtypes = [_vp, C.POINTER(Lens), C.c_int32]
+    L.ptc_scene_set_object_motion.argtypes = [_vp, C.c_int32, _F]
+    L.ptc_scene_set_camera_motion.argtypes = [_vp, C.POINTER(Camera), C.c_int32]
     L.ptc_render.argtypes = [_vp, C.POINTER(Camera), C.POINTER(RenderSettings), _F, C.POINTER(Stats)]
     L.ptc_render_u32.argtypes = [_vp, C.POINTER(Camera), C.POINTER(RenderSettings), _vp, C.POINTER(Stats)]
     L.ptc_render_adaptive.argtypes = [_vp, C.POINTER(Camera), C.POINTER(RenderSettings), C.POINTER(Adaptive), _F, _vp, _vp,
@@ -182,6 +184,8 @@ def core():
     L.ptc_resolve_u32.argtypes = [_vp, _F, C.c_int64, C.c_float, _vp]
     L.ptc_intersect.argtypes = [_vp, _F, _F, C.c_int64, C.c_float, C.c_float, _vp, C.POINTER(Stats)]
     L.ptc_primary_rays.argtypes = [_vp, C.POINTER(Camera), C.POINTER(RenderSettings), C.c_int32, _F, _F]
+    L.ptc_intersect_at.argtypes = [_vp, _F, _F, _F, C.c_int64, C.c_float, C.c_float, _vp, C.POINTER(Stats)]
+    L.ptc_ray_times.argtypes = [_vp, C.POINTER(RenderSettings), C.c_int32, _F]
     L.ptc_scatter.argtypes = [_vp, C.c_int, _F, _F, _F, _vp, _F, C.c_int64, _vp, _F, _F, _F, _F]
     L.ptc_philox.argtypes = [_vp, _vp, _vp, _vp]
     L.ptc_sky_sample.argtypes = [_vp, _F, C.c_int64, _F, _F, _F]
@@ -574,6 +578,33 @@ class CoreScene:
         _ck(core().ptc_scene_set_lens(self._h, arr if pairs else None, len(pairs)))
         return self
 
+    def set_object_motion(self, obj, displacement):
+        """Motion blur (ptc_scene_set_object_motion): object `obj` is translated by tau * displacement at shutter time tau
+        in every later render of this handle; (0, 0, 0) makes it static again."""
+        d = np.ascontiguousarray(displacement, dtype=np.float32).reshape(3)
+        _ck(core().ptc_scene_set_object_motion(self._h, int(obj), _fptr(d)))
+        return self
+
+    def set_camera_motion(self, end_cameras=None):
+        """Motion blur (ptc_scene_set_camera_motion): the camera at shutter time tau is start + tau (end - start), field by
+        field.  set_camera_motion(end) for one end camera, set_camera_motion([end, ...]) for one per batch view,
+        set_camera_motion() or set_camera_motion([]) for a static camera again."""
+        if end_cameras is None:
+            cams = []
+        elif isinstance(end_cameras, Camera):
+            cams = [end_cameras]
+        else:
+            cams = list(end_cameras)
+        arr = (Camera * max(len(cams), 1))(*cams)
+        _ck(core().ptc_scene_set_camera_motion(self._h, arr if cams else None, len(cams)))
+        return self
+
+    def ray_times(self, settings, sample):
+        """The shutter time of camera sample `sample` of every pixel (ptc_ray_times) -> [H*W] float32."""
+        out = np.empty(settings.width * settings.height, np.float32)
+        _ck(core().ptc_ray_times(self._h, C.byref(settings), sample, _fptr(out)))
+        return out
+
     def mesh_info(self, obj):
         info = MeshInfo()
         _ck(core().ptc_scene_mesh_info(self._h, obj, C.byref(info), None, None))
@@ -718,11 +749,18 @@ class CoreScene:
         _ck(core().ptc_resolve_u32(self._h, _fptr(a), len(a), scale, out.ctypes.data))
         return out
 
-    def intersect(self, origins, dirs, t_min=1e-4, t_max=float("inf")):
+    def intersect(self, origins, dirs, t_min=1e-4, t_max=float("inf"), times=None):
+        """Closest hits (ptc_intersect); with `times` (one shutter time in [0, 1] per ray) under the handle's object
+        motion (ptc_intersect_at)."""
         o, d = _f32(origins, (-1, 3)), _f32(dirs, (-1, 3))
         out = np.zeros(len(o), HIT_DTYPE)
         st = Stats()
-        _ck(core().ptc_intersect(self._h, _fptr(o), _fptr(d), len(o), t_min, t_max, out.ctypes.data, C.byref(st)))
+        if times is None:
+            _ck(core().ptc_intersect(self._h, _fptr(o), _fptr(d), len(o), t_min, t_max, out.ctypes.data, C.byref(st)))
+        else:
+            t = _f32(times, (len(o),))
+            _ck(core().ptc_intersect_at(self._h, _fptr(o), _fptr(d), _fptr(t), len(o), t_min, t_max, out.ctypes.data,
+                                        C.byref(st)))
         return out, st
 
     def primary_rays(self, camera, settings, sample):

@@ -416,10 +416,11 @@ struct EmitterSample {
   uint32_t light;
   int32_t entry;  // triangle (original index) or cube face; -1 for spheres and quads
 };
-// One light sample from x: u0 chooses the light, u1 u2 the point, u3 the triangle or face.  false: rejected (x on the
-// light, or the light seen edge-on).
-PT_HD bool emitter_sample(const DScene &sc, const EmitterTables &et, V3 x, float u0, float u1, float u2, float u3, EmitterSample &s) {
-  s.light = cdf_search(et.sel_cdf, (uint32_t)sc.n_lights, u0);
+// One light sample from x of the light `light` (chosen by cdf_search(et.sel_cdf, n_lights, u0)): u1 u2 the point, u3 the
+// triangle or face.  false: rejected (x on the light, or the light seen edge-on).
+PT_HD bool emitter_sample_light(const DScene &sc, const EmitterTables &et, uint32_t light, V3 x, float u1, float u2, float u3,
+                                EmitterSample &s) {
+  s.light = light;
   s.entry = -1;
   const DLight &L = sc.lights[s.light];
   const float p_sel = emitter_select_prob(et, s.light);
@@ -458,6 +459,10 @@ PT_HD bool emitter_sample(const DScene &sc, const EmitterTables &et, V3 x, float
   s.pdf = p_sel * p_bin * d2 / (cos_g * area);
   s.pmis = emitter_mis_pdf(L, p_sel, s.dist, fabsf(dot(nrec, s.wi)));
   return true;
+}
+// One light sample from x: u0 chooses the light, then emitter_sample_light.
+PT_HD bool emitter_sample(const DScene &sc, const EmitterTables &et, V3 x, float u0, float u1, float u2, float u3, EmitterSample &s) {
+  return emitter_sample_light(sc, et, cdf_search(et.sel_cdf, (uint32_t)sc.n_lights, u0), x, u1, u2, u3, s);
 }
 
 // a direction with density sky_pdf from four uniforms: row, column, then uniform in phi and cos(theta) inside the cell
@@ -529,6 +534,42 @@ PT_HD Ray camera_get_ray_lens(const DCamera &c, float R, float F, float u, float
   const Ray q = ray_new(o, dir);
   if (!(isfinite(q.o.x) && isfinite(q.o.y) && isfinite(q.o.z) && isfinite(q.d.x) && isfinite(q.d.y) && isfinite(q.d.z))) return p;
   return q;
+}
+
+// Motion blur (ptc_scene_set_object_motion / ptc_scene_set_camera_motion, DESIGN.md 5l).  A camera sample's shutter time
+// tau is u[0] of Philox block 1 of the camera-jitter counter (block 0 is the jitter and the lens); the path and every ray
+// it spawns carry it.
+// The camera at tau: every float field c0 + tau (c1 - c0), component-wise (a rotation is lerped, not slerped;
+// camera_get_ray normalises the direction).  An end camera equal to the start camera bit for bit gives c0 itself.
+PT_HD DCamera camera_at(const DCamera &c0, const DCamera &c1, float tau) {
+  constexpr int kN = (int)(sizeof(DCamera) / sizeof(float));
+  static_assert(sizeof(DCamera) == kN * sizeof(float), "DCamera is floats only");
+  float a[kN], b[kN];
+  memcpy(a, &c0, sizeof(a));
+  memcpy(b, &c1, sizeof(b));
+  bool same = true;
+  for (int k = 0; k < kN; k++) same = same && f2u(a[k]) == f2u(b[k]);
+  if (same) return c0;
+  for (int k = 0; k < kN; k++) a[k] = a[k] + tau * (b[k] - a[k]);
+  DCamera c;
+  memcpy(&c, a, sizeof(c));
+  return c;
+}
+// Object k translated by tau D over the shutter: it sees the ray (o - tau D, d).  D == (0, 0, 0) (either sign of zero)
+// is a static object: callers test motion_moves first and then use today's code on the unshifted ray.
+PT_HD bool motion_moves(float4 D) { return D.x != 0.0f || D.y != 0.0f || D.z != 0.0f; }
+PT_HD V3 motion_point(V3 p, float tau, float4 D) { return v3(p.x - tau * D.x, p.y - tau * D.y, p.z - tau * D.z); }
+PT_HD Ray motion_object_ray(const Ray &r, float tau, float4 D) {
+  Ray q;
+  q.o = motion_point(r.o, tau, D);
+  q.d = r.d;
+  return q;
+}
+// the record of a hit found in the shifted frame, back in the world at tau: position + tau D (t and normal unchanged)
+PT_HD void motion_hit_position(Hit &h, float tau, float4 D) {
+  h.px = h.px + tau * D.x;
+  h.py = h.py + tau * D.y;
+  h.pz = h.pz + tau * D.z;
 }
 
 // renderer.rs:112-120 + color.rs:87-93: sqrt "gamma", clamp, *255, truncate, 0x00RRGGBB

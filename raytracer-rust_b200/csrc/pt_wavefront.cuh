@@ -27,6 +27,8 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <type_traits>
+
 #include "../../include/ptcore.h"
 #include "pt_adaptive.h"
 #include "pt_bsdf.h"
@@ -100,6 +102,18 @@ struct BatchTables {
 // k_primary_rays_lens only: a trailing kernel argument of their own, like BatchTables.
 struct LensTables {
   const float2 *lens;
+};
+
+// Motion blur (DESIGN.md 5l): the displacement D_k of every object over the shutter, the end camera of every view (a
+// single render is view 0; nullptr: a static camera), and the shutter time of every ray of the two ray sets (`tau` is
+// read, `ntau` written by k_shade; the host swaps them with the nray_* arrays).  Read by the *_motion kernels only: a
+// trailing kernel argument of their own, like LensTables, so that Buffers, RenderParams, DObject and DScene keep their
+// layout and every other kernel its instructions.
+struct MotionTables {
+  const float4 *disp;        // [n_objects]: D_k in .xyz
+  const DCamera *end_cams;   // [views] or nullptr
+  const float *tau;
+  float *ntau;
 };
 
 // Path state, SoA of float4.  Segment b = slots [b * cap, b * cap + cnt[b]).
@@ -227,8 +241,44 @@ __device__ __forceinline__ int scan_objects(const DScene &sc, const DObject *obj
   }
   return -1;
 }
+// The same scan at shutter time tau (motion blur): object k is tested on the ray shifted by -tau D_k (disp, the table in
+// shared or global memory), and a hit it reports moves by +tau D_k; an object with D_k == 0 sees `ray` itself.  A mesh
+// is parked with the object-space ray of its shifted ray, so k_traverse needs nothing of the motion.
+__device__ __forceinline__ int scan_objects_motion(const DScene &sc, const DObject *objs, const Ray &ray, float t_min, float &closest,
+                                                   Hit &best, bool &improved, int k_begin, MeshRay &park_ray, const float4 *disp,
+                                                   float tau) {
+  for (int k = k_begin; k < sc.n_objects; k++) {
+    const DObject *ob = objs + k;
+    const int type = ob->type;
+    const float4 D = disp[k];
+    const bool moves = motion_moves(D);
+    const Ray r = moves ? motion_object_ray(ray, tau, D) : ray;
+    bool hit;
+    if (type == OBJ_MESH) {
+      const MeshRay mr = mesh_object_ray(ob->f, r);
+      if (!mesh_root_may_hit(sc.meshes[ob->mesh], mr, t_min, closest)) continue;
+      park_ray = mr;
+      return k;
+    }
+    if (type == OBJ_SPHERE) hit = hit_sphere(ob->f, r, t_min, closest, best);
+    else if (type == OBJ_QUAD) hit = hit_quad(ob->f, r, t_min, closest, best);
+    else if (type == OBJ_CUBE) hit = hit_cube_t(ob->f, r, t_min, closest, best);
+    else hit = hit_plane(ob->f, r, t_min, closest, best);
+    if (hit) {
+      if (moves) motion_hit_position(best, tau, D);
+      improved = true;
+      closest = best.t;
+      best.object = k;
+      best.triangle = -1;
+      best.material = ob->hit_bits;
+    }
+  }
+  return -1;
+}
 
 // Completes the record that won the scan (pt_prims.h: a cube hit carries its normal as "pending" through the scan).
+// cube_finish_normal reads the ray's direction only, which the motion shift leaves as it is: a moving cube's record is
+// completed with the same bits from the world ray as from its shifted one.
 __device__ __forceinline__ void finish_hit(const DObject *objs, const Ray &ray, Hit &best) {
   if (best.front_face == kCubeNormalPending) cube_finish_normal(objs[best.object].f, ray, best);
 }
@@ -246,6 +296,16 @@ __device__ __forceinline__ const DObject *stage_objects(const DScene &sc, DObjec
   const int n16 = sc.n_objects * (int)(sizeof(DObject) / 16);
   for (int i = threadIdx.x; i < n16; i += blockDim.x) dst[i] = src[i];
   return s_objs;  // visible after the caller's __syncthreads()
+}
+// ... and the motion kernels stage the displacement table next to it
+template <bool kSharedObjs>
+__device__ __forceinline__ const float4 *stage_disp(const DScene &sc, const float4 *disp, float4 *s_disp) {
+  if constexpr (!kSharedObjs) {
+    return disp;
+  } else {
+    for (int i = threadIdx.x; i < sc.n_objects; i += blockDim.x) s_disp[i] = disp[i];
+    return s_disp;  // visible after the caller's __syncthreads()
+  }
 }
 
 // Append the parked lanes of this warp to the block's task segment: ballot + one SHARED-memory atomic per warp.
@@ -289,6 +349,42 @@ __device__ __forceinline__ void stage_pre(uint32_t seg, uint32_t n_seg, const DS
       Hit best;
       bool improved = false;
       park = scan_objects(sc, objs, ray, t_min, closest, best, improved, 0, mr);  // renderer.rs:24
+      if (improved) finish_hit(objs, ray, best);
+      if (improved) write_hit(out, i, best);
+      else write_miss(out, i);
+    }
+    park_tasks(&s_ntask, tq, 0, seg_base, park, i, mr, closest);
+  }
+  __syncthreads();
+  if (tid == 0 && tq.cnt) tq.cnt[seg] = s_ntask;
+  (void)n_seg;
+}
+
+// Motion blur: stage_pre with every ray at its own shutter time mt.tau[i] (scan_objects_motion)
+template <bool kSharedObjs>
+__device__ __forceinline__ void stage_pre_motion(uint32_t seg, uint32_t n_seg, const DScene &sc, const ExtendOut &out, const TaskQ &tq,
+                                                 float t_min, float t_max, const MotionTables &mt) {
+  __shared__ uint32_t s_ntask;
+  __shared__ __align__(16) DObject s_objs[kSmemObjects];
+  const uint32_t tid = threadIdx.x;
+  const uint32_t n = out.b.cnt[seg], seg_base = seg * out.b.cap;
+  if (tid == 0) s_ntask = 0;
+  const DObject *objs = kSharedObjs ? s_objs : sc.objects;
+  stage_objects<kSharedObjs>(sc, s_objs);
+  __shared__ float4 s_disp[kSmemObjects];
+  const float4 *disp = stage_disp<kSharedObjs>(sc, mt.disp, s_disp);
+  __syncthreads();
+  for (uint32_t c0 = 0; c0 < n; c0 += (uint32_t)kBlock) {
+    const uint32_t i = seg_base + c0 + tid;
+    int park = -1;
+    MeshRay mr;
+    float closest = t_max;
+    if (c0 + tid < n) {
+      const float4 o4 = out.b.ray_o[i], d4 = out.b.ray_d[i];
+      const Ray ray{v3(o4.x, o4.y, o4.z), v3(d4.x, d4.y, d4.z)};
+      Hit best;
+      bool improved = false;
+      park = scan_objects_motion(sc, objs, ray, t_min, closest, best, improved, 0, mr, disp, mt.tau[i]);  // renderer.rs:24
       if (improved) finish_hit(objs, ray, best);
       if (improved) write_hit(out, i, best);
       else write_miss(out, i);
@@ -494,6 +590,77 @@ __device__ __forceinline__ void stage_post(uint32_t seg, uint32_t n_seg, const D
   if (tid == 0) tq.cnt[(uint32_t)(round + 1) * n_seg + seg] = s_ntask;
 }
 
+// Motion blur: stage_post with the ray at its shutter time mt.tau[i]; the mesh that parked it finishes on the shifted ray,
+// as k_extend_pre_motion parked it
+template <bool kSharedObjs>
+__device__ __forceinline__ void stage_post_motion(uint32_t seg, uint32_t n_seg, const DScene &sc, const ExtendOut &out, const TaskQ &tq,
+                                                  int round, float t_min, float t_max, const MotionTables &mt) {
+  __shared__ uint32_t s_ntask;
+  __shared__ __align__(16) DObject s_objs[kSmemObjects];
+  const uint32_t tid = threadIdx.x;
+  const uint32_t n = tq.cnt[(uint32_t)round * n_seg + seg], seg_base = seg * out.b.cap;
+  const int par = round & 1;
+  if (tid == 0) s_ntask = 0;
+  const DObject *objs = kSharedObjs ? s_objs : sc.objects;
+  stage_objects<kSharedObjs>(sc, s_objs);
+  __shared__ float4 s_disp[kSmemObjects];
+  const float4 *disp = stage_disp<kSharedObjs>(sc, mt.disp, s_disp);
+  __syncthreads();
+  for (uint32_t c0 = 0; c0 < n; c0 += (uint32_t)kBlock) {
+    const uint32_t j = seg_base + c0 + tid;
+    int park = -1;
+    MeshRay mr;
+    float closest = t_max;
+    uint32_t i = 0;
+    if (c0 + tid < n) {
+      const uint2 rk = tq.ray[par][j];
+      const unsigned long long res = tq.res[par][j];
+      i = rk.x;
+      const int k = (int)rk.y;
+      const DObject *ob = objs + k;
+      const bool tri_hit = res != kNoTriHit;
+      const uint32_t order = (uint32_t)res;
+      // the stage is bound by the latency of these gathers: issue all of them before the first use
+      const float4 o4 = out.b.ray_o[i], d4 = out.b.ray_d[i];
+      // closest_so_far travels with the task (the t_max the traversal ran with; == t_max when nothing was hit before the
+      // mesh): a sequential 4-byte read instead of two gathered sectors of the hit record (hit0.w, hit1.w) per task
+      closest = tq.o[par][j].w;
+      float4 nq = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+      if (tri_hit) nq = ldg4(sc.meshes[ob->mesh].normals + order);  // normal + original index, by DFS position
+      const Ray ray{v3(o4.x, o4.y, o4.z), v3(d4.x, d4.y, d4.z)};
+      const float tau = mt.tau[i];
+      Hit best;
+      best.triangle = -1;
+      bool improved = false;
+      if (tri_hit) {
+        MeshHit mh;
+        mh.t = u2f((uint32_t)(res >> 32)), mh.tri = f2u(nq.w), mh.order = order;
+        Hit tmp;
+        // the shifted ray the mesh was parked with, and its hit back at tau
+        const float4 D = disp[k];
+        const bool moves = motion_moves(D);
+        const Ray r = moves ? motion_object_ray(ray, tau, D) : ray;
+        const MeshRay omr = mesh_object_ray<false>(ob->f, r);  // same inputs, same bits as in k_extend_pre_motion
+        const bool found = mesh_finish(ob->f, nq, r, omr, mh, t_min, closest, tmp);
+        if (found && moves) motion_hit_position(tmp, tau, D);
+        if (found) {
+          improved = true;
+          closest = tmp.t;
+          best = tmp;
+          best.object = k;
+          best.material = ob->hit_bits;  // type << 26 | light << 20 | index, see write_hit
+        }
+      }
+      park = scan_objects_motion(sc, objs, ray, t_min, closest, best, improved, k + 1, mr, disp, tau);
+      if (improved) finish_hit(objs, ray, best);
+      if (improved) write_hit(out, i, best);  // otherwise the record parked by the previous stage stands
+    }
+    park_tasks(&s_ntask, tq, par ^ 1, seg_base, park, i, mr, closest);
+  }
+  __syncthreads();
+  if (tid == 0) tq.cnt[(uint32_t)(round + 1) * n_seg + seg] = s_ntask;
+}
+
 constexpr int kShadeClasses = 11;  // 0 = miss, 1 + material type (8 types), 9 = NEE shadow ray, 10 = no ray (tail of the last window)
 constexpr int kShadeWindow = 2048;                   // rays one block sorts together
 constexpr int kShadeGroups = kShadeWindow / kBlock;  // 32-ray groups each warp shades per window
@@ -569,11 +736,21 @@ __device__ __forceinline__ uint32_t block_rank(bool flag, uint32_t *s_warp /* [k
 // argument, so that the shade kernels of every other render compile to the instructions they had.
 // Lens: camera paths start through the thin lens of `lt` (camera_get_ray_lens, with u[2], u[3] of the jitter draw);
 // only regeneration changes.
+// Motion: every ray carries its shutter time (mt.tau -> mt.ntau for survivors and shadow rays); regeneration draws it
+// (Philox block 1 of the jitter counter), takes the camera at that time and then the lens of `lt` if lt.lens is set; a
+// light of a moving object is sampled from x - tau D_L (nee_origin).
 constexpr int kSrcTiles = 0, kSrcList = 1, kSrcBatch = 2;
-template <int Mode, int Src, bool Lens = false>
+struct MotionNone {};  // what stands for a value of the motion twins in every other instantiation
+// The point a light is sampled from: x, or x - tau D of the light's object when it moves.  wi, dist and the pdfs come out
+// as for the static light seen from the shifted point, which is the moving light seen from x at tau.
+__device__ __forceinline__ V3 nee_origin(V3 x, const MotionTables &mt, int32_t object, float tau) {
+  const float4 D = mt.disp[object];
+  return motion_moves(D) ? motion_point(x, tau, D) : x;
+}
+template <int Mode, int Src, bool Lens = false, bool Motion = false>
 __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, uint32_t *seg_done, Ctl *ctl, const DScene &sc, const RenderParams &rp,
                                                 const Buffers &b, const Film &film, const BatchTables &bt, const EmitterTables &et,
-                                                const LensTables &lt = LensTables{}) {
+                                                const LensTables &lt = LensTables{}, const MotionTables *mt = nullptr) {
   constexpr bool List = Src == kSrcList, Batch = Src == kSrcBatch;
   __shared__ uint16_t s_perm[kShadeWindow];
   __shared__ uint32_t s_hist[2][16];
@@ -638,10 +815,12 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
       bool alive = false, shadow = false;
       float4 no, nd, nb, so4, sd4, sb4;
       float npdf = -1.0f;
+      std::conditional_t<Motion, float, MotionNone> tau{};  // the ray's shutter time: a float in the motion twins only
       if (p < wn) {
         const uint32_t i = win_base + (uint32_t)s_perm[p];
         const float4 o4 = b.ray_o[i], d4 = b.ray_d[i], b4 = b.beta[i];
         const float4 h1 = b.hit1[i];
+        if constexpr (Motion) tau = mt->tau[i];
         const uint32_t pixel_word = f2u(o4.w), sample = f2u(d4.w), bounce = f2u(b4.w);
         const uint32_t pixel = NEE ? (pixel_word & ~kShadowBit) : pixel_word;  // the film index (global in a batch)
         // Philox key: the view's seed and the pixel within the view
@@ -739,7 +918,12 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
                     pm = pl;
                   } else if (EM) {
                     EmitterSample es;
-                    ok = emitter_sample(sc, et, so, (ul.u[0] - p_sky) * 2.0f, ul.u[1], ul.u[2], ul.u[3], es);
+                    if constexpr (Motion) {  // the light is chosen once, and sampled from x - tau D of its object
+                      const uint32_t pick = cdf_search(et.sel_cdf, (uint32_t)sc.n_lights, (ul.u[0] - p_sky) * 2.0f);
+                      ok = emitter_sample_light(sc, et, pick, nee_origin(so, *mt, sc.lights[pick].object, tau), ul.u[1], ul.u[2], ul.u[3], es);
+                    } else {
+                      ok = emitter_sample(sc, et, so, (ul.u[0] - p_sky) * 2.0f, ul.u[1], ul.u[2], ul.u[3], es);
+                    }
                     const DLight &L = sc.lights[es.light];
                     wi = es.wi, dist = es.dist, pl = es.pdf * 0.5f, pm = es.pmis * 0.5f;  // (1 - p_sky) x the light's own
                     le = v3(L.emission[0], L.emission[1], L.emission[2]);
@@ -747,7 +931,8 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
                   } else {
                     const uint32_t li = min((uint32_t)((ul.u[0] - p_sky) * 2.0f * (float)sc.n_lights), (uint32_t)sc.n_lights - 1u);
                     const DLight L = sc.lights[li];
-                    ok = light_sample(L, so, ul.u[1], ul.u[2], wi, dist, pl);
+                    if constexpr (Motion) ok = light_sample(L, nee_origin(so, *mt, L.object, tau), ul.u[1], ul.u[2], wi, dist, pl);
+                    else ok = light_sample(L, so, ul.u[1], ul.u[2], wi, dist, pl);
                     pl *= 0.5f / (float)sc.n_lights;  // (1 - p_sky) / n_lights, as where a BSDF-sampled ray hits the light
                     le = v3(L.emission[0], L.emission[1], L.emission[2]);
                     pm = pl;
@@ -766,7 +951,14 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
                   EmitterSample es;
                   V3 fcos;
                   float pb;
-                  if (emitter_sample(sc, et, so, ul.u[0], ul.u[1], ul.u[2], ul.u[3], es) && mat_eval_pdf(m, ray_d, pos, nrm, es.wi, fcos, pb) &&
+                  bool ok;
+                  if constexpr (Motion) {  // the light is chosen once, and sampled from x - tau D of its object
+                    const uint32_t pick = cdf_search(et.sel_cdf, (uint32_t)sc.n_lights, ul.u[0]);
+                    ok = emitter_sample_light(sc, et, pick, nee_origin(so, *mt, sc.lights[pick].object, tau), ul.u[1], ul.u[2], ul.u[3], es);
+                  } else {
+                    ok = emitter_sample(sc, et, so, ul.u[0], ul.u[1], ul.u[2], ul.u[3], es);
+                  }
+                  if (ok && mat_eval_pdf(m, ray_d, pos, nrm, es.wi, fcos, pb) &&
                       (fcos.x > 0.0f || fcos.y > 0.0f || fcos.z > 0.0f)) {
                     const DLight &L = sc.lights[es.light];
                     const float w_mis = es.pmis * es.pmis / (es.pmis * es.pmis + pb * pb);
@@ -783,7 +975,10 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
                   const V3 so = pos + nrm * kEps;
                   V3 wi, fcos;
                   float dist, pl, pb;
-                  if (light_sample(L, so, ul.u[1], ul.u[2], wi, dist, pl) && mat_eval_pdf(m, ray_d, pos, nrm, wi, fcos, pb) &&
+                  bool ok;
+                  if constexpr (Motion) ok = light_sample(L, nee_origin(so, *mt, L.object, tau), ul.u[1], ul.u[2], wi, dist, pl);
+                  else ok = light_sample(L, so, ul.u[1], ul.u[2], wi, dist, pl);
+                  if (ok && mat_eval_pdf(m, ray_d, pos, nrm, wi, fcos, pb) &&
                       (fcos.x > 0.0f || fcos.y > 0.0f || fcos.z > 0.0f)) {
                     pl *= 1.0f / (float)sc.n_lights;
                     const float w_mis = pl * pl / (pl * pl + pb * pb);
@@ -818,6 +1013,7 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
           b.nray_d[slot] = nd;
           b.nbeta[slot] = nb;
           if (NEE) b.naux[slot] = npdf;
+          if constexpr (Motion) mt->ntau[slot] = tau;
         }
         if (NEE && shadow) {
           const uint32_t slot = seg_base + base + (uint32_t)__popc(amask) + (uint32_t)__popc(smask & lt_mask);
@@ -825,6 +1021,7 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
           b.nray_d[slot] = sd4;
           b.nbeta[slot] = sb4;
           b.naux[slot] = -1.0f;
+          if constexpr (Motion) mt->ntau[slot] = tau;
         }
       }
     }
@@ -899,7 +1096,19 @@ __device__ __forceinline__ uint32_t stage_shade(uint32_t seg, uint32_t n_seg, ui
         const float u = ((float)x + jit.u[0]) / (float)rp.width;   // renderer.rs:96
         const float v = ((float)y + jit.u[1]) / (float)rp.height;  // renderer.rs:97
         Ray ray;
-        if (Lens) {
+        if constexpr (Motion) {
+          // the shutter time: Philox block 1 of the jitter counter, never drawn otherwise
+          const float tau = philox_uniforms(Batch ? bt.seeds[view] : rp.seed, pixel, sample, 0xffffffffu, 1u).u[0];
+          DCamera cam = Batch ? bt.cams[view] : rp.cam;
+          if (mt->end_cams) cam = camera_at(cam, mt->end_cams[Batch ? view : 0u], tau);
+          if (lt.lens) {
+            const float2 ln = lt.lens[Batch ? view : 0u];
+            ray = camera_get_ray_lens(cam, ln.x, ln.y, u, v, jit.u[2], jit.u[3]);
+          } else {
+            ray = camera_get_ray(cam, u, v);
+          }
+          mt->ntau[slot] = tau;
+        } else if (Lens) {
           const float2 ln = lt.lens[Batch ? view : 0u];
           ray = camera_get_ray_lens(Batch ? bt.cams[view] : rp.cam, ln.x, ln.y, u, v, jit.u[2], jit.u[3]);
         } else {
@@ -1013,6 +1222,27 @@ __global__ void __launch_bounds__(kBlock, kSegPerSM) k_extend_pre(Ctl *ctl, SegR
   else stage_pre<false>(seg, sr.n_seg, sc, out, tq, t_min, t_max);
   stage_end(sr, seg);
 }
+// Motion blur: k_extend_pre with every ray at its shutter time mt.tau (stage_pre_motion); the same bookkeeping
+__global__ void __launch_bounds__(kBlock, kSegPerSM) k_extend_pre_motion(Ctl *ctl, SegRange sr, DScene sc, ExtendOut out, TaskQ tq, float t_min,
+                                                                         float t_max, volatile uint32_t *progress, uint32_t seq,
+                                                                         MotionTables mt) {
+  const uint32_t seg = sr.seg0 + blockIdx.x;
+  stage_begin(sr, seg, ctl);
+  if (threadIdx.x == 0) {
+    const uint32_t n = out.b.cnt[seg];
+    if (n) {
+      atomicAdd(&ctl->rays, (unsigned long long)n);
+      atomicMax(&ctl->iterations[0], seq);
+    }
+    if (progress && blockIdx.x == 0) {
+      *progress = seq << 2 | (ctl->next_path >= ctl->total_paths ? 2u : 0u) | (ctl->n_active == 0u ? 1u : 0u);
+      __threadfence_system();
+    }
+  }
+  if (sc.n_objects <= kSmemObjects) stage_pre_motion<true>(seg, sr.n_seg, sc, out, tq, t_min, t_max, mt);
+  else stage_pre_motion<false>(seg, sr.n_seg, sc, out, tq, t_min, t_max, mt);
+  stage_end(sr, seg);
+}
 template <bool COUNT>
 __global__ void __launch_bounds__(kBlock, kSegPerSM) k_traverse(Ctl *ctl, SegRange sr, DScene sc, TaskQ tq, int round, float t_min,
                                                                 uint32_t cap, uint32_t refill_lanes) {
@@ -1061,6 +1291,14 @@ __global__ void __launch_bounds__(kBlock, kSegPerSM) k_extend_post(Ctl *ctl, Seg
   else stage_post<false>(sr.seg0 + blockIdx.x, sr.n_seg, sc, out, tq, round, t_min, t_max);
   stage_end(sr, sr.seg0 + blockIdx.x);
 }
+// Motion blur: k_extend_post with every ray at its shutter time mt.tau (stage_post_motion)
+__global__ void __launch_bounds__(kBlock, kSegPerSM) k_extend_post_motion(Ctl *ctl, SegRange sr, DScene sc, ExtendOut out, TaskQ tq, int round,
+                                                                          float t_min, float t_max, MotionTables mt) {
+  stage_begin(sr, sr.seg0 + blockIdx.x, ctl);
+  if (sc.n_objects <= kSmemObjects) stage_post_motion<true>(sr.seg0 + blockIdx.x, sr.n_seg, sc, out, tq, round, t_min, t_max, mt);
+  else stage_post_motion<false>(sr.seg0 + blockIdx.x, sr.n_seg, sc, out, tq, round, t_min, t_max, mt);
+  stage_end(sr, sr.seg0 + blockIdx.x);
+}
 // Mode: 0 = plain, 1 = PTC_FLAG_NEE, 2 = PTC_FLAG_NEE | PTC_FLAG_NEE_SKY on a scene with a sky distribution.  List: paths
 // start from rp.pixel_list (stage_shade).
 template <int Mode, bool List = false>
@@ -1095,6 +1333,17 @@ __global__ void __launch_bounds__(kBlock, kSegPerSM) k_shade_lens(Ctl *ctl, SegR
                                                                   BatchTables bt, EmitterTables et, LensTables lt) {
   stage_begin(sr, sr.seg0 + blockIdx.x, ctl);
   stage_shade<Mode, Src, true>(sr.seg0 + blockIdx.x, sr.n_seg, sr.flags ? sr.flags + sr.n_seg : nullptr, ctl, sc, rp, b, film, bt, et, lt);
+  stage_end(sr, sr.seg0 + blockIdx.x);
+}
+// Motion blur (an object moves, or a camera differs from its end camera): Mode 0-4, paths from any Src, every ray at its
+// shutter time; the lens of `lt` if lt.lens is set (nullptr: a pinhole).  The tables are trailing arguments of these
+// instantiations only (see k_shade_em).
+template <int Mode, int Src>
+__global__ void __launch_bounds__(kBlock, kSegPerSM) k_shade_motion(Ctl *ctl, SegRange sr, DScene sc, RenderParams rp, Buffers b, Film film,
+                                                                    BatchTables bt, EmitterTables et, LensTables lt, MotionTables mt) {
+  stage_begin(sr, sr.seg0 + blockIdx.x, ctl);
+  stage_shade<Mode, Src, false, true>(sr.seg0 + blockIdx.x, sr.n_seg, sr.flags ? sr.flags + sr.n_seg : nullptr, ctl, sc, rp, b, film, bt, et,
+                                      lt, &mt);
   stage_end(sr, sr.seg0 + blockIdx.x);
 }
 
@@ -1212,6 +1461,35 @@ __global__ void k_primary_rays_lens(RenderParams rp, uint32_t sample, float *out
   const Ray ray = camera_get_ray_lens(rp.cam, ln.x, ln.y, u, v, jit.u[2], jit.u[3]);
   out_o[pixel * 3 + 0] = ray.o.x, out_o[pixel * 3 + 1] = ray.o.y, out_o[pixel * 3 + 2] = ray.o.z;
   out_d[pixel * 3 + 0] = ray.d.x, out_d[pixel * 3 + 1] = ray.d.y, out_d[pixel * 3 + 2] = ray.d.z;
+}
+// ... and at the shutter time: the camera at tau (mt.end_cams[0], if any), then the lens lt.lens[0] (if any), exactly as
+// k_shade_motion starts its paths; out_tau (or nullptr) receives tau.  ptc_primary_rays and the denoiser's feature pass
+// of a motion render.
+__global__ void k_primary_rays_motion(RenderParams rp, uint32_t sample, float *out_o, float *out_d, float *out_tau, LensTables lt,
+                                      MotionTables mt) {
+  const uint32_t pixel = blockIdx.x * blockDim.x + threadIdx.x;
+  if (pixel >= (uint32_t)(rp.width * rp.height)) return;
+  const int x = (int)(pixel % (uint32_t)rp.width), y = (int)(pixel / (uint32_t)rp.width);
+  const Uniforms4 jit = philox_uniforms(rp.seed, pixel, sample, 0xffffffffu, 0u);
+  const float u = ((float)x + jit.u[0]) / (float)rp.width;
+  const float v = ((float)y + jit.u[1]) / (float)rp.height;
+  const float tau = philox_uniforms(rp.seed, pixel, sample, 0xffffffffu, 1u).u[0];
+  const DCamera cam = mt.end_cams ? camera_at(rp.cam, mt.end_cams[0], tau) : rp.cam;
+  Ray ray;
+  if (lt.lens) {
+    const float2 ln = lt.lens[0];
+    ray = camera_get_ray_lens(cam, ln.x, ln.y, u, v, jit.u[2], jit.u[3]);
+  } else {
+    ray = camera_get_ray(cam, u, v);
+  }
+  out_o[pixel * 3 + 0] = ray.o.x, out_o[pixel * 3 + 1] = ray.o.y, out_o[pixel * 3 + 2] = ray.o.z;
+  out_d[pixel * 3 + 0] = ray.d.x, out_d[pixel * 3 + 1] = ray.d.y, out_d[pixel * 3 + 2] = ray.d.z;
+  if (out_tau) out_tau[pixel] = tau;
+}
+// ptc_ray_times: the shutter time of camera sample `sample` of every pixel
+__global__ void k_ray_times(uint64_t seed, uint32_t n_pixels, uint32_t sample, float *out_tau) {
+  const uint32_t pixel = blockIdx.x * blockDim.x + threadIdx.x;
+  if (pixel < n_pixels) out_tau[pixel] = philox_uniforms(seed, pixel, sample, 0xffffffffu, 1u).u[0];
 }
 
 __global__ void k_scatter(DMaterial m, const float *dirs, const float *pos, const float *nrm, const int32_t *front,

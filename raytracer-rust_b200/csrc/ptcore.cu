@@ -87,6 +87,7 @@ struct Workspace {
   DevBuf<float4> ray_o, ray_d, beta, hit0, hit1;
   DevBuf<float4> ray_o2, ray_d2, beta2;  // second set of ray arrays (renders only): k_shade reads one set, writes the other
   DevBuf<float> aux, aux2;               // PTC_FLAG_NEE only (allocated at the first such render)
+  DevBuf<float> tau, tau2;               // motion renders only: the shutter time of every ray of the two sets (MotionTables)
   DevBuf<uint32_t> cnt;
   DevBuf<uint32_t> seg_flags;      // [3 * segments]: SegRange::flags
   DevBuf<uint32_t> trav_counters;  // [kTravCounters]: SegRange::trav_counter of the render's split traversal launches
@@ -120,6 +121,14 @@ struct Workspace {
   // flip = 0: the stages read set 1 and k_shade writes set 2; flip = 1: the other way round
   void ensure_aux() {
     if (aux.n < slots()) aux.alloc(slots()), aux2.alloc(slots());
+  }
+  void ensure_tau() {
+    if (tau.n < slots()) tau.alloc(slots()), tau2.alloc(slots());
+  }
+  // the shutter times that go with buffers(flip): the stages read `tau`, k_shade writes `ntau`
+  MotionTables motion(int flip, const float4 *disp, const DCamera *end_cams) const {
+    if (flip == 0) return MotionTables{disp, end_cams, tau.p, tau2.p};
+    return MotionTables{disp, end_cams, tau2.p, tau.p};
   }
   Buffers buffers(int flip = 0) const {
     if (flip == 0) return Buffers{ray_o.p, ray_d.p, beta.p, hit0.p, hit1.p, cnt.p, cap, ray_o2.p, ray_d2.p, beta2.p, aux.p, aux2.p};
@@ -190,6 +199,7 @@ struct ptc_scene {
   // sample's camera rays (origins, then directions), the feature sums (then means), the variance, the denoised image,
   // the filter's ping-pong input and its guides; the feature pass's control block; render_ms brackets
   DevBuf<float> w_dn_half, w_dn_rays, w_dn_albedo, w_dn_normal, w_dn_var, w_dn_out;
+  DevBuf<float> w_dn_tau;  // a motion render's feature pass: the shutter time of every camera ray
   DevBuf<float4> w_dn_xv[2], w_dn_ga, w_dn_gn;
   DevBuf<Ctl> w_dn_ctl;
   cudaEvent_t ev_dn_begin = nullptr, ev_dn_end = nullptr;
@@ -200,6 +210,12 @@ struct ptc_scene {
   // (pt_wavefront.cuh: LensTables)
   std::vector<ptc_lens> lens;
   DevBuf<float2> d_lens;
+  // ptc_scene_set_object_motion / ptc_scene_set_camera_motion: D per object as set (missing entries are 0) and the end
+  // cameras (empty = static); the tables of the render in flight, grow-only (pt_wavefront.cuh: MotionTables)
+  std::vector<float4> motion;
+  std::vector<ptc_camera> end_cams;
+  DevBuf<float4> d_motion_disp;
+  DevBuf<DCamera> d_motion_cams;
   DevBuf<Ctl> d_ctl;
   Ctl *h_ctl = nullptr;  // pinned ring
   uint32_t *h_progress = nullptr;  // pinned + mapped: the word k_extend_pre reports the state of the render in
@@ -276,15 +292,18 @@ uint32_t traverse_refill_arg() {
 
 // One extend pass over ALL segments on one stream (ptc_intersect) = pre, then (traverse, post) once per mesh object a ray
 // can meet.  Returns the number of launches.
+// mt.tau != nullptr: the rays at their shutter times, through the motion twins of pre and post.
 int launch_extend(cudaStream_t stream, uint32_t segments, int rounds, Ctl *ctl, const DScene &ds, const ExtendOut &eo, const TaskQ &tq,
-                  float t_min, float t_max, bool counters) {
+                  float t_min, float t_max, bool counters, const MotionTables &mt = MotionTables{}) {
   const SegRange sr{0u, segments, 0u, 0u, 1u};
-  k_extend_pre<<<segments, kBlock, 0, stream>>>(ctl, sr, ds, eo, tq, t_min, t_max, nullptr, 0u);
+  if (mt.tau) k_extend_pre_motion<<<segments, kBlock, 0, stream>>>(ctl, sr, ds, eo, tq, t_min, t_max, nullptr, 0u, mt);
+  else k_extend_pre<<<segments, kBlock, 0, stream>>>(ctl, sr, ds, eo, tq, t_min, t_max, nullptr, 0u);
   for (int r = 0; r < rounds; r++) {
     const SegRange tsr{0u, segments, 0u, (uint32_t)r, 1u};
     if (counters) k_traverse<true><<<segments, kBlock, 0, stream>>>(ctl, tsr, ds, tq, r, t_min, eo.b.cap, traverse_refill_arg());
     else k_traverse<false><<<segments, kBlock, 0, stream>>>(ctl, tsr, ds, tq, r, t_min, eo.b.cap, traverse_refill_arg());
-    k_extend_post<<<segments, kBlock, 0, stream>>>(ctl, sr, ds, eo, tq, r, t_min, t_max);
+    if (mt.tau) k_extend_post_motion<<<segments, kBlock, 0, stream>>>(ctl, sr, ds, eo, tq, r, t_min, t_max, mt);
+    else k_extend_post<<<segments, kBlock, 0, stream>>>(ctl, sr, ds, eo, tq, r, t_min, t_max);
   }
   return 1 + 2 * rounds;
 }
@@ -292,9 +311,12 @@ int launch_extend(cudaStream_t stream, uint32_t segments, int rounds, Ctl *ctl, 
 // n rays (device arrays of n x 3 floats) laid out like a render's pool in the hook workspace (segment b = slots
 // [b * cap, ...), ray i in slot i) and run through the render's extend kernels: the hit records are left in ws_hook's
 // hit0 / hit1 / ids.  ptc_intersect's rays and ptc_render_denoised's feature rays.  `before` / `after`, if given, are
-// recorded around the extend launches.  Returns the number of extend launches.
+// recorded around the extend launches.  `d_tau` (n floats) and `disp` (the object displacements, device), if given: the
+// rays at their shutter times (ray i is in slot i, so d_tau is the time table as it stands).  Returns the number of
+// extend launches.
 int extend_hook_rays(ptc_scene *s, const float *d_o, const float *d_d, uint32_t n, float t_min, float t_max, Ctl *ctl, bool counters,
-                     cudaStream_t st, cudaEvent_t before = nullptr, cudaEvent_t after = nullptr, const DScene *ds = nullptr) {
+                     cudaStream_t st, cudaEvent_t before = nullptr, cudaEvent_t after = nullptr, const DScene *ds = nullptr,
+                     const float *d_tau = nullptr, const float4 *disp = nullptr) {
   const uint32_t segments = s->segments();
   const uint32_t cap = (uint32_t)(((uint64_t)n + segments - 1) / segments + kBlock - 1) / kBlock * kBlock;
   s->ws_hook.ensure(segments, cap, s->mesh_objects, true, false);
@@ -305,7 +327,8 @@ int extend_hook_rays(ptc_scene *s, const float *d_o, const float *d_d, uint32_t 
   k_pack_rays<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_o, d_d, (size_t)n, b.ray_o, b.ray_d);
   const ExtendOut eo{b, s->ws_hook.ids.p};
   if (before) CK(cudaEventRecord(before, st));
-  const int launches = launch_extend(st, segments, s->mesh_objects, ctl, ds ? *ds : s->ds, eo, tq, t_min, t_max, counters);
+  const MotionTables mt = d_tau ? MotionTables{disp, nullptr, d_tau, nullptr} : MotionTables{};
+  const int launches = launch_extend(st, segments, s->mesh_objects, ctl, ds ? *ds : s->ds, eo, tq, t_min, t_max, counters, mt);
   CK(cudaGetLastError());
   if (after) CK(cudaEventRecord(after, st));
   return launches;
@@ -366,7 +389,69 @@ struct Pass {
   const DCamera *cams = nullptr;
   const uint64_t *seeds = nullptr;
   const float2 *lens = nullptr;      // device, (R, F) per view (one for a single camera); nullptr: pinhole, today's kernels
+  // motion blur: the motion twins run, with the displacement table (device, one per object) and the end cameras (device,
+  // one per view; nullptr: a static camera).  false: no object moves and every end camera is its start camera, today's kernels
+  bool motion = false;
+  const float4 *disp = nullptr;
+  const DCamera *end_cams = nullptr;
 };
+
+// The end camera a single-camera call uses: end_cams[0] of ptc_scene_set_camera_motion, nullptr for a static camera.
+// Checked before the scene's state.
+const ptc_camera *single_end_cam(const ptc_scene *s) {
+  if (s->end_cams.size() > 1)
+    throw std::invalid_argument("a single-camera call uses one end camera: ptc_scene_set_camera_motion was given n > 1");
+  return s->end_cams.empty() ? nullptr : &s->end_cams[0];
+}
+
+// What one call moves, from the motion state of handle `s` (the primary handle of a ptc_multi): D per object, and an end
+// camera per view where the views' end cameras are not all equal to their start cameras bit for bit (ends[k % ends.size()]
+// goes with view k: one end camera for all views, or one each).
+struct MotionCall {
+  std::vector<float4> disp;
+  std::vector<DCamera> end_cams;  // empty: no camera moves
+  bool objects = false;
+  bool any() const { return objects || !end_cams.empty(); }
+};
+MotionCall motion_call(const ptc_scene *s, const ptc_camera *cams, size_t views, const ptc_camera *ends, size_t n_ends) {
+  MotionCall mc;
+  const size_t n_obj = s->hs.objects.size();
+  mc.disp.assign(std::max<size_t>(n_obj, 1), make_float4(0.0f, 0.0f, 0.0f, 0.0f));
+  for (size_t k = 0; k < n_obj && k < s->motion.size(); k++) {
+    mc.disp[k] = s->motion[k];
+    mc.objects = mc.objects || motion_moves(s->motion[k]);
+  }
+  bool camera = false;
+  for (size_t v = 0; v < views && n_ends > 0; v++) camera = camera || memcmp(&ends[v % n_ends], &cams[v], sizeof(ptc_camera)) != 0;
+  if (camera) {
+    mc.end_cams.resize(views);
+    for (size_t v = 0; v < views; v++) memcpy(&mc.end_cams[v], &ends[v % n_ends], sizeof(DCamera));
+  }
+  return mc;
+}
+// Grow `d`'s motion tables to hold `mc` (ptc_multi allocates them before its threads start)
+void ensure_motion(ptc_scene *d, const MotionCall &mc) {
+  if (d->d_motion_disp.n < mc.disp.size()) d->d_motion_disp.alloc(mc.disp.size());
+  if (d->d_motion_cams.n < mc.end_cams.size()) d->d_motion_cams.alloc(mc.end_cams.size());
+}
+// mc into the device tables of `d` (the scene a render runs on), one copy per table on `stream`, and into `pass`.  Nothing
+// when nothing moves: the call runs today's kernels.
+void upload_motion(ptc_scene *d, const MotionCall &mc, cudaStream_t stream, Pass &pass) {
+  static_assert(sizeof(ptc_camera) == sizeof(DCamera), "ptc_camera and DCamera share one layout");
+  if (!mc.any()) return;
+  ensure_motion(d, mc);
+  // (from pageable memory: the call returns once the source has been read)
+  CK(cudaMemcpyAsync(d->d_motion_disp.p, mc.disp.data(), mc.disp.size() * sizeof(float4), cudaMemcpyHostToDevice, stream));
+  if (!mc.end_cams.empty())
+    CK(cudaMemcpyAsync(d->d_motion_cams.p, mc.end_cams.data(), mc.end_cams.size() * sizeof(DCamera), cudaMemcpyHostToDevice, stream));
+  pass.motion = true;
+  pass.disp = d->d_motion_disp.p;
+  pass.end_cams = mc.end_cams.empty() ? nullptr : d->d_motion_cams.p;
+}
+// the motion of a single-camera call of `s` (end camera from single_end_cam)
+MotionCall single_motion(const ptc_scene *s, const ptc_camera *cam, const ptc_camera *end) {
+  return motion_call(s, cam, 1, end, end ? 1 : 0);
+}
 
 // The lens a single-camera call uses: lenses[0] of ptc_scene_set_lens, nullptr for a pinhole or a zero aperture (the call
 // then runs exactly the kernels it runs without a lens).  Checked before the scene's state.
@@ -398,6 +483,19 @@ ShadeLensKernel shade_lens_kernel(int mode) {
     case 2: return k_shade_lens<2, Src>;
     case 3: return k_shade_lens<3, Src>;
     default: return k_shade_lens<4, Src>;
+  }
+}
+
+// k_shade_motion<mode, Src>, the same modes
+using ShadeMotionKernel = void (*)(Ctl *, SegRange, DScene, RenderParams, Buffers, Film, BatchTables, EmitterTables, LensTables, MotionTables);
+template <int Src>
+ShadeMotionKernel shade_motion_kernel(int mode) {
+  switch (mode) {
+    case 0: return k_shade_motion<0, Src>;
+    case 1: return k_shade_motion<1, Src>;
+    case 2: return k_shade_motion<2, Src>;
+    case 3: return k_shade_motion<3, Src>;
+    default: return k_shade_motion<4, Src>;
   }
 }
 
@@ -434,7 +532,7 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
     // 43.2 ms at 48 Mi slots), next best with many fills of a large pool, worst when a second, ragged fill trails the
     // first (46.6 ms at 0.8 x the job).  So: the job itself if that fits a quarter of the free memory (and 48 GiB),
     // else 48 Mi slots, and never between one and 2.5 fills.
-    const uint64_t per_slot = 128ull + (s->mesh_objects > 0 ? 96ull : 0ull) + (nee ? 8ull : 0ull);
+    const uint64_t per_slot = 128ull + (s->mesh_objects > 0 ? 96ull : 0ull) + (nee ? 8ull : 0ull) + (pass.motion ? 8ull : 0ull);
     if (s->pool_budget_bytes == 0) {
       // asked once per scene: cudaMemGetInfo contends with NVML pollers (nvidia-smi -lms) for tens of milliseconds
       size_t free_b = 0, total_b = 0;
@@ -457,6 +555,7 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
   ensure_ctl(s);
   s->ws.ensure(segments, (uint32_t)cap64, s->mesh_objects, false, true);
   if (nee) s->ws.ensure_aux();
+  if (pass.motion) s->ws.ensure_tau();
   s->last_pool_slots = (int64_t)cap64 * segments;
   Buffers bufs[2] = {s->ws.buffers(0), s->ws.buffers(1)};
   bufs[0].cap = bufs[1].cap = (uint32_t)cap64;  // a pool smaller than the allocation simply uses a smaller segment stride
@@ -576,8 +675,12 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
     auto run_extend = [&]() {
       const ExtendOut eo{bufs[flip], nullptr};
       if (timing) mark(ST_PRE);
-      launch_stage(pdl, stream, segments, k_extend_pre, s->d_ctl.p, seg_range(0u, 1u), ds, eo, tq, kEps, INFINITY,
-                   (volatile uint32_t *)d_progress, (uint32_t)(it + 1));  // renderer.rs:24
+      if (pass.motion)
+        launch_stage(pdl, stream, segments, k_extend_pre_motion, s->d_ctl.p, seg_range(0u, 1u), ds, eo, tq, kEps, INFINITY,
+                     (volatile uint32_t *)d_progress, (uint32_t)(it + 1), s->ws.motion(flip, pass.disp, pass.end_cams));
+      else
+        launch_stage(pdl, stream, segments, k_extend_pre, s->d_ctl.p, seg_range(0u, 1u), ds, eo, tq, kEps, INFINITY,
+                     (volatile uint32_t *)d_progress, (uint32_t)(it + 1));  // renderer.rs:24
       for (int r = 0; r < rounds; r++) {
         if (timing) mark(ST_TRAVERSE);
         // (a split launch needs a hand-out counter of its own; a render with more launches than counters goes on unsplit)
@@ -586,7 +689,11 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
         if (counters) launch_stage(pdl, stream, segments, k_traverse<true>, s->d_ctl.p, tsr, ds, tq, r, kEps, eo.b.cap, refill);
         else launch_stage(pdl, stream, segments, k_traverse<false>, s->d_ctl.p, tsr, ds, tq, r, kEps, eo.b.cap, refill);
         if (timing) mark(ST_POST);
-        launch_stage(pdl, stream, segments, k_extend_post, s->d_ctl.p, seg_range(0u, 1u), ds, eo, tq, r, kEps, INFINITY);
+        if (pass.motion)
+          launch_stage(pdl, stream, segments, k_extend_post_motion, s->d_ctl.p, seg_range(0u, 1u), ds, eo, tq, r, kEps, INFINITY,
+                       s->ws.motion(flip, pass.disp, pass.end_cams));
+        else
+          launch_stage(pdl, stream, segments, k_extend_post, s->d_ctl.p, seg_range(0u, 1u), ds, eo, tq, r, kEps, INFINITY);
       }
       launches += 1 + 2 * (uint64_t)rounds;
     };
@@ -594,7 +701,16 @@ void render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_set
       if (timing) mark(ST_SHADE);
       const SegRange ssr = seg_range(0u, 1u);
       const int mode = nee_sky ? 2 : (nee ? 1 : 0);
-      if (pass.lens) {
+      if (pass.motion) {
+        const BatchTables bt = pass.views > 0 ? BatchTables{pass.cams, pass.seeds, (uint32_t)st->width * (uint32_t)st->height, (uint32_t)n_tiles}
+                                              : BatchTables{};
+        const int mmode = nee_em ? (nee_sky ? 4 : 3) : mode;
+        auto *kernel = pass.views > 0 ? shade_motion_kernel<kSrcBatch>(mmode)
+                       : pass.pixels  ? shade_motion_kernel<kSrcList>(mmode)
+                                      : shade_motion_kernel<kSrcTiles>(mmode);
+        launch_stage(pdl, stream, segments, kernel, s->d_ctl.p, ssr, ds, rp, bufs[flip], film, bt, nee_em ? s->et : EmitterTables{},
+                     LensTables{pass.lens}, s->ws.motion(flip, pass.disp, pass.end_cams));
+      } else if (pass.lens) {
         const BatchTables bt = pass.views > 0 ? BatchTables{pass.cams, pass.seeds, (uint32_t)st->width * (uint32_t)st->height, (uint32_t)n_tiles}
                                               : BatchTables{};
         const int lmode = nee_em ? (nee_sky ? 4 : 3) : mode;
@@ -1045,6 +1161,33 @@ int ptc_scene_set_lens(ptc_scene *s, const ptc_lens *lenses, int32_t n) {
   PTC_GUARD_END
 }
 
+int ptc_scene_set_object_motion(ptc_scene *s, int32_t object, const float displacement[3]) {
+  PTC_GUARD_BEGIN
+  if (!s || !displacement) throw std::invalid_argument("null argument");
+  if (object < 0 || (size_t)object >= s->hs.objects.size()) throw std::invalid_argument("object index out of range");
+  for (int c = 0; c < 3; c++)
+    if (!std::isfinite(displacement[c])) throw std::invalid_argument("displacement must be finite");
+  if (s->motion.size() <= (size_t)object) s->motion.resize((size_t)object + 1, make_float4(0.0f, 0.0f, 0.0f, 0.0f));
+  s->motion[(size_t)object] = make_float4(displacement[0], displacement[1], displacement[2], 0.0f);
+  return 0;
+  PTC_GUARD_END
+}
+
+int ptc_scene_set_camera_motion(ptc_scene *s, const ptc_camera *end_cameras, int32_t n) {
+  PTC_GUARD_BEGIN
+  if (!s || n < 0 || (n > 0 && !end_cameras)) throw std::invalid_argument("bad argument");
+  for (int32_t k = 0; k < n; k++) {
+    float f[sizeof(ptc_camera) / sizeof(float)];  // ptc_camera is floats only
+    static_assert(sizeof(f) == sizeof(ptc_camera), "ptc_camera is floats only");
+    memcpy(f, &end_cameras[k], sizeof(f));
+    for (float v : f)
+      if (!std::isfinite(v)) throw std::invalid_argument("every field of an end camera must be finite");
+  }
+  s->end_cams.assign(end_cameras, end_cameras + n);
+  return 0;
+  PTC_GUARD_END
+}
+
 int ptc_scene_build(ptc_scene *s) {
   PTC_GUARD_BEGIN
   if (!s) throw std::invalid_argument("null argument");
@@ -1140,6 +1283,7 @@ int ptc_render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_
   PTC_GUARD_BEGIN
   if (!s) throw std::invalid_argument("null argument");
   const ptc_lens *lens = single_lens(s);
+  const ptc_camera *end = single_end_cam(s);
   require_committed(s);
   check_render_args(cam, st, d_accum != nullptr);
   // the caller's handle is honoured as given: NULL is the legacy default stream, which orders the film atomics after
@@ -1148,6 +1292,11 @@ int ptc_render_accumulate(ptc_scene *s, const ptc_camera *cam, const ptc_render_
   if (lens) {
     CK(cudaSetDevice(s->device));
     pass.lens = upload_lens(s, lens, 1, (cudaStream_t)cuda_stream);
+  }
+  const MotionCall mc = single_motion(s, cam, end);
+  if (mc.any()) {
+    CK(cudaSetDevice(s->device));
+    upload_motion(s, mc, (cudaStream_t)cuda_stream, pass);
   }
   render_accumulate(s, cam, st, d_accum, (cudaStream_t)cuda_stream, stats, pass);
   return 0;
@@ -1161,12 +1310,18 @@ static int render_to_host(ptc_scene *s, const ptc_camera *cam, const ptc_render_
   PTC_GUARD_BEGIN
   if (!s) throw std::invalid_argument("null argument");
   const ptc_lens *lens = single_lens(s);
+  const ptc_camera *end = single_end_cam(s);
   require_committed(s);
   check_render_args(cam, st, out_rgb || out_u32);
   Pass pass;
   if (lens) {
     CK(cudaSetDevice(s->device));
     pass.lens = upload_lens(s, lens, 1, s->own_stream);
+  }
+  const MotionCall mc = single_motion(s, cam, end);
+  if (mc.any()) {
+    CK(cudaSetDevice(s->device));
+    upload_motion(s, mc, s->own_stream, pass);
   }
   render_accumulate(s, cam, st, nullptr, s->own_stream, stats, pass);
   const int launches = resolve_film_to_host(s, (size_t)st->width * st->height, 1.0f / (float)st->spp, nullptr, out_rgb, out_u32, s->own_stream);
@@ -1189,6 +1344,8 @@ static void check_batch_args(const ptc_scene *s, const ptc_camera *cams, int32_t
   if (n_views < 1) throw std::invalid_argument("n_views must be >= 1");
   if (s->lens.size() > 1 && s->lens.size() != (size_t)n_views)
     throw std::invalid_argument("ptc_scene_set_lens gave n lenses: a batch needs n == 1 or n == n_views");
+  if (s->end_cams.size() > 1 && s->end_cams.size() != (size_t)n_views)
+    throw std::invalid_argument("ptc_scene_set_camera_motion gave n end cameras: a batch needs n == 1 or n == n_views");
   if (st->tile_mod != 0) throw std::invalid_argument("ptc_render_batch renders whole views: tile_mod must be 0");
   // the film index of every padded pixel of every view stays below 2^30 (a pool entry's pixel word keeps kShadowBit)
   const uint64_t padded = (uint64_t)n_views * (((uint64_t)st->width + 31u) & ~31ull) * (((uint64_t)st->height + 31u) & ~31ull);
@@ -1215,6 +1372,8 @@ static Pass batch_pass(ptc_scene *s, const ptc_camera *cams, int32_t n_views, co
     if (s->lens.size() == n) per = s->lens;
     pass.lens = upload_lens(s, per.data(), n, stream);
   }
+  // one end camera for every view, or one per view
+  upload_motion(s, motion_call(s, cams, n, s->end_cams.data(), s->end_cams.size()), stream, pass);
   return pass;
 }
 
@@ -1257,6 +1416,7 @@ int ptc_render_adaptive(ptc_scene *s, const ptc_camera *cam, const ptc_render_se
   if (ad->min_spp < 2 || ad->min_spp % 2 != 0 || ad->min_spp > st->spp) throw std::invalid_argument("min_spp must be even, >= 2 and <= spp");
   if (!(ad->threshold >= 0.0f)) throw std::invalid_argument("threshold must be >= 0");
   const ptc_lens *lens = single_lens(s);
+  const ptc_camera *end = single_end_cam(s);
   require_committed(s);
   CK(cudaSetDevice(s->device));
   ensure_ctl(s);
@@ -1281,6 +1441,7 @@ int ptc_render_adaptive(ptc_scene *s, const ptc_camera *cam, const ptc_render_se
   const int half = ad->min_spp / 2;
   Pass first;
   first.lens = lens ? upload_lens(s, lens, 1, stream) : nullptr;
+  upload_motion(s, single_motion(s, cam, end), stream, first);
   CK(cudaEventRecord(s->ev_adapt_begin, stream));
   render_pass(s, cam, st, 0, half, first, stream, total);
   const Film f = s->film();
@@ -1351,6 +1512,7 @@ int ptc_render_progressive(ptc_scene *s, const ptc_camera *cam, const ptc_render
   if (pg->first_spp < 1 || pg->first_spp > st->spp) throw std::invalid_argument("first_spp must be >= 1 and <= spp");
   if (pg->max_pass_spp < 0) throw std::invalid_argument("max_pass_spp must be >= 0");
   const ptc_lens *lens = single_lens(s);
+  const ptc_camera *end = single_end_cam(s);
   require_committed(s);
   CK(cudaSetDevice(s->device));
   ensure_ctl(s);
@@ -1370,6 +1532,8 @@ int ptc_render_progressive(ptc_scene *s, const ptc_camera *cam, const ptc_render
   }
   cudaStream_t stream = s->own_stream;
   const float2 *d_lens = lens ? upload_lens(s, lens, 1, stream) : nullptr;
+  Pass moving;  // the motion tables of every pass
+  upload_motion(s, single_motion(s, cam, end), stream, moving);
 
   // What the two threads share, under `mu`.  The worker publishes pass j (ready = j + 1, samples[j % 2]) once its slot
   // event is recorded; the calling thread publishes callback j's return (shown = j + 1) and a stop.
@@ -1398,6 +1562,7 @@ int ptc_render_progressive(ptc_scene *s, const ptc_camera *cam, const ptc_render
         Pass pass;
         pass.clear_film = j == 0;
         pass.lens = d_lens;
+        pass.motion = moving.motion, pass.disp = moving.disp, pass.end_cams = moving.end_cams;
         render_pass(s, cam, st, n, next, pass, stream, total);
         k_resolve_film<<<(unsigned)((n_px + 255) / 256), 256, 0, stream>>>(s->film(), n_px, 1.0f / (float)next, nullptr,
                                                                            out_rgb ? s->w_prog_rgb[j & 1].p : nullptr,
@@ -1525,6 +1690,7 @@ int ptc_render_denoised(ptc_scene *s, const ptc_camera *cam, const ptc_render_se
   if (dn->feature_spp < 1 || dn->feature_spp > st->spp) throw std::invalid_argument("feature_spp must be >= 1 and <= spp");
   check_denoise_filter(dn);
   const ptc_lens *lens = single_lens(s);
+  const ptc_camera *end = single_end_cam(s);
   require_committed(s);
   CK(cudaSetDevice(s->device));
   ensure_ctl(s);
@@ -1548,6 +1714,8 @@ int ptc_render_denoised(ptc_scene *s, const ptc_camera *cam, const ptc_render_se
   const int half = st->spp / 2;
   Pass first;
   first.lens = lens ? upload_lens(s, lens, 1, stream) : nullptr;
+  upload_motion(s, single_motion(s, cam, end), stream, first);
+  if (first.motion && s->w_dn_tau.n < n_px) s->w_dn_tau.alloc(n_px);
   CK(cudaEventRecord(s->ev_dn_begin, stream));
   render_pass(s, cam, st, 0, half, first, stream, total);
   CK(cudaMemsetAsync(s->w_dn_half.p, 0, n3 * sizeof(float), stream));
@@ -1567,9 +1735,17 @@ int ptc_render_denoised(ptc_scene *s, const ptc_camera *cam, const ptc_render_se
   rp.width = st->width, rp.height = st->height, rp.seed = st->seed;
   float *ray_o = s->w_dn_rays.p, *ray_d = s->w_dn_rays.p + n3;
   for (int k = 0; k < dn->feature_spp; k++) {
-    if (first.lens) k_primary_rays_lens<<<nb, 256, 0, stream>>>(rp, (uint32_t)k, ray_o, ray_d, LensTables{first.lens});
-    else k_primary_rays<<<nb, 256, 0, stream>>>(rp, (uint32_t)k, ray_o, ray_d);
-    launches += 3 + extend_hook_rays(s, ray_o, ray_d, n_px, kEps, INFINITY, s->w_dn_ctl.p, false, stream);
+    if (first.motion) {
+      // the primary rays at their shutter times, intersected at those times
+      k_primary_rays_motion<<<nb, 256, 0, stream>>>(rp, (uint32_t)k, ray_o, ray_d, s->w_dn_tau.p, LensTables{first.lens},
+                                                    MotionTables{first.disp, first.end_cams, nullptr, nullptr});
+      launches += 3 + extend_hook_rays(s, ray_o, ray_d, n_px, kEps, INFINITY, s->w_dn_ctl.p, false, stream, nullptr, nullptr, nullptr,
+                                       s->w_dn_tau.p, first.disp);
+    } else {
+      if (first.lens) k_primary_rays_lens<<<nb, 256, 0, stream>>>(rp, (uint32_t)k, ray_o, ray_d, LensTables{first.lens});
+      else k_primary_rays<<<nb, 256, 0, stream>>>(rp, (uint32_t)k, ray_o, ray_d);
+      launches += 3 + extend_hook_rays(s, ray_o, ray_d, n_px, kEps, INFINITY, s->w_dn_ctl.p, false, stream);
+    }
     const Buffers b = s->ws_hook.buffers();
     k_feature_add<<<nb, 256, 0, stream>>>(b.hit0, b.hit1, s->ds.materials, n_px, s->w_dn_albedo.p, s->w_dn_normal.p);
     launches += 1;
@@ -1703,11 +1879,85 @@ int ptc_intersect(ptc_scene *s, const float *origins, const float *dirs, int64_t
   PTC_GUARD_END
 }
 
+int ptc_intersect_at(ptc_scene *s, const float *origins, const float *dirs, const float *times, int64_t n, float t_min, float t_max,
+                     ptc_hit *out, ptc_stats *stats) {
+  PTC_GUARD_BEGIN
+  require_committed(s);
+  if (n < 0 || (n > 0 && (!origins || !dirs || !times || !out))) throw std::invalid_argument("bad argument");
+  for (int64_t i = 0; i < n; i++)
+    if (!(times[i] >= 0.0f && times[i] <= 1.0f)) throw std::invalid_argument("a ray's time must be in [0, 1]");
+  if (stats) memset(stats, 0, sizeof(*stats));
+  if (n == 0) return 0;
+  if (n > (int64_t)0x3fffffff) throw std::invalid_argument("too many rays for one call");
+  CK(cudaSetDevice(s->device));
+  const MotionCall mc = motion_call(s, nullptr, 0, nullptr, 0);
+  if (!mc.objects) return ptc_intersect(s, origins, dirs, n, t_min, t_max, out, stats);  // nothing moves: today's kernels
+  ensure_ctl(s);
+  DevBuf<float> d_o, d_d, d_t;
+  DevBuf<ptc_hit> d_out;
+  DevBuf<Ctl> ctl;
+  d_o.upload(origins, (size_t)n * 3);
+  d_d.upload(dirs, (size_t)n * 3);
+  d_t.upload(times, (size_t)n);
+  d_out.alloc((size_t)n);
+  Ctl init;
+  memset(&init, 0, sizeof(init));
+  ctl.upload(&init, 1);
+  cudaStream_t st = s->own_stream;
+  Pass pass;
+  upload_motion(s, mc, st, pass);
+  cudaEvent_t ea, eb;
+  CK(cudaEventCreate(&ea));
+  CK(cudaEventCreate(&eb));
+  const int ext_launches = extend_hook_rays(s, d_o.p, d_d.p, (uint32_t)n, t_min, t_max, ctl.p, true, st, ea, eb, nullptr, d_t.p, pass.disp);
+  const Buffers b = s->ws_hook.buffers();
+  k_unpack_hits<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(b.hit0, b.hit1, s->ws_hook.ids.p, (size_t)n, d_out.p);
+  CK(cudaGetLastError());
+  CK(cudaMemcpyAsync(out, d_out.p, (size_t)n * sizeof(ptc_hit), cudaMemcpyDeviceToHost, st));
+  Ctl fin;
+  CK(cudaMemcpyAsync(&fin, ctl.p, sizeof(Ctl), cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  if (stats) {
+    float ms = 0.0f;
+    CK(cudaEventElapsedTime(&ms, ea, eb));
+    stats->rays = (uint64_t)n;
+    stats->kernel_launches = 3 + (uint64_t)ext_launches;
+    stats->render_ms = ms;
+    stats->extend_ms = ms;
+    stats->extend_launches = 1;
+    stats->nodes_visited = fin.nodes;
+    stats->tris_tested = fin.tris;
+    stats->mesh_rays = fin.mesh_rays;
+  }
+  cudaEventDestroy(ea);
+  cudaEventDestroy(eb);
+  return 0;
+  PTC_GUARD_END
+}
+
+int ptc_ray_times(ptc_scene *s, const ptc_render_settings *st, int32_t sample, float *out_time) {
+  PTC_GUARD_BEGIN
+  require_committed(s);
+  if (!st || !out_time || st->width <= 0 || st->height <= 0 || sample < 0) throw std::invalid_argument("bad argument");
+  if ((int64_t)st->width * st->height > (int64_t)0x3fffffff) throw std::invalid_argument("image too large");
+  CK(cudaSetDevice(s->device));
+  const uint32_t n = (uint32_t)st->width * (uint32_t)st->height;
+  DevBuf<float> d_t;
+  d_t.alloc(n);
+  k_ray_times<<<(n + 255) / 256, 256, 0, s->own_stream>>>(st->seed, n, (uint32_t)sample, d_t.p);
+  CK(cudaGetLastError());
+  CK(cudaMemcpyAsync(out_time, d_t.p, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, s->own_stream));
+  CK(cudaStreamSynchronize(s->own_stream));
+  return 0;
+  PTC_GUARD_END
+}
+
 int ptc_primary_rays(ptc_scene *s, const ptc_camera *cam, const ptc_render_settings *st, int32_t sample, float *out_o,
                      float *out_d) {
   PTC_GUARD_BEGIN
   if (!s) throw std::invalid_argument("null argument");
   const ptc_lens *lens = single_lens(s);
+  const ptc_camera *end = single_end_cam(s);
   require_committed(s);
   if (!cam || !st || !out_o || !out_d || st->width <= 0 || st->height <= 0) throw std::invalid_argument("bad argument");
   CK(cudaSetDevice(s->device));
@@ -1719,7 +1969,14 @@ int ptc_primary_rays(ptc_scene *s, const ptc_camera *cam, const ptc_render_setti
   DevBuf<float> d_o, d_d;
   d_o.alloc(n * 3);
   d_d.alloc(n * 3);
-  if (lens) {
+  const MotionCall mc = single_motion(s, cam, end);
+  if (!mc.end_cams.empty()) {  // the camera at each ray's shutter time (object motion does not change a camera ray)
+    Pass pass;
+    upload_motion(s, mc, s->own_stream, pass);
+    const LensTables lt{lens ? upload_lens(s, lens, 1, s->own_stream) : nullptr};
+    k_primary_rays_motion<<<(unsigned)((n + 255) / 256), 256, 0, s->own_stream>>>(rp, (uint32_t)sample, d_o.p, d_d.p, nullptr, lt,
+                                                                                  MotionTables{pass.disp, pass.end_cams, nullptr, nullptr});
+  } else if (lens) {
     k_primary_rays_lens<<<(unsigned)((n + 255) / 256), 256, 0, s->own_stream>>>(rp, (uint32_t)sample, d_o.p, d_d.p,
                                                                                 LensTables{upload_lens(s, lens, 1, s->own_stream)});
   } else {
@@ -1918,6 +2175,8 @@ static int multi_render(ptc_multi *m, const ptc_camera *cam, const ptc_render_se
   if (shard_mode != PTC_SHARD_SAMPLES && shard_mode != PTC_SHARD_TILES) throw std::invalid_argument("bad shard mode");
   // every device renders through the primary handle's lens
   const ptc_lens *lens = single_lens(m->primary);
+  // ... and with the primary handle's motion at the time of the call
+  const MotionCall mc = single_motion(m->primary, cam, single_end_cam(m->primary));
   const int n = (int)m->scenes.size();
   int s_begin, s_end;
   sample_range(st, s_begin, s_end);
@@ -1933,6 +2192,7 @@ static int multi_render(ptc_multi *m, const ptc_camera *cam, const ptc_render_se
     CK(cudaSetDevice(s->device));
     ensure_film(s, n_px);
     if (lens && s->d_lens.n < 1) s->d_lens.alloc(1);
+    if (mc.any()) ensure_motion(s, mc);
   }
   std::mutex abort_mutex;
   auto work = [&](int i) {
@@ -1955,6 +2215,7 @@ static int multi_render(ptc_multi *m, const ptc_camera *cam, const ptc_render_se
       memset(&per[(size_t)i], 0, sizeof(ptc_stats));
       Pass pass;
       pass.lens = lens && !idle ? upload_lens(s, lens, 1, stream) : nullptr;
+      if (!idle) upload_motion(s, mc, stream, pass);
       if (idle) clear_film(s, n_px, stream);
       else render_accumulate(s, cam, &mine, nullptr, stream, &per[(size_t)i], pass);  // leaves the shard in the device's fixed-point film
       film_ok = true;

@@ -156,6 +156,10 @@ extern "C" {
     pub fn ptc_scene_set_sky_hdr(s: *mut ptc_scene, rgb: *const f32, w: i32, h: i32) -> c_int;
     /// n == 0: pinhole; single-camera renders use lenses[0] (n > 1: PTC_E_INVALID), batches n == 1 or n == n_views
     pub fn ptc_scene_set_lens(s: *mut ptc_scene, lenses: *const ptc_lens, n: i32) -> c_int;
+    /// Motion blur: object `object` is translated by tau * displacement at shutter time tau; (0, 0, 0) = static
+    pub fn ptc_scene_set_object_motion(s: *mut ptc_scene, object: i32, displacement: *const f32) -> c_int;
+    /// n == 0: static camera; single-camera renders use end_cameras[0] (n > 1: PTC_E_INVALID), batches n == 1 or n == n_views
+    pub fn ptc_scene_set_camera_motion(s: *mut ptc_scene, end_cameras: *const ptc_camera, n: i32) -> c_int;
     pub fn ptc_scene_build(s: *mut ptc_scene) -> c_int;
     pub fn ptc_scene_last_pool_slots(s: *const ptc_scene) -> i64;
     pub fn ptc_scene_commit(s: *mut ptc_scene, device: c_int) -> c_int;
